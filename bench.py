@@ -5,7 +5,7 @@ A "step" is one Gibbs sweep (reference src/PHT_MCMC_Aslett.c:268-405) over all o
 latent-path draw per observation + the conjugate parameter update.  Metric: path draws per second
 (= observations x sweeps / time); Gibbs iterations/s is reported beside it.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--method MHRS|ECS|DCS] [--config 3] [--obs L]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--method MHRS|ECS|DCS] [--config 3] [--obs L] [--dump-outputs DIR]
   python bench.py --impl reference ...      # the reference's own C on the host cores
 
 Headline: BASELINE.json configs[2] = 8-phase general PHT, 10^7 observations, 20 % right-censored, method MHRS (the
@@ -176,6 +176,41 @@ def _peak_hbm():
         return 6650.0, "fallback (B200_PROFILING.md)"
 
 
+# ----------------------------------------------------------------------------- --dump-outputs
+DUMP_WINDOW = 256                # observations per sampled window of per-observation paths
+DUMP_PATH_BYTES = 32 << 20       # cap on the sampled paths' N array (float64, n*n per observation)
+
+
+def dump_outputs(path, wl, method, mhit, sum_y, sweeps, theta, device):
+    """Save what the last of `sweeps` chain sweeps computed, all float64, so that two builds can be compared output for
+    output: theta.npy (m, the parameter draw = the last row Engine.run returns), sweep_N/sweep_B/sweep_z.npy (the sweep's
+    totals: N column-major n*n, B n, z n in time units) and, for a fixed seeded sample of observation windows,
+    paths_obs.npy (observation index) with paths_B/paths_N/paths_z.npy (each observation's path statistics).
+    The totals and paths are recomputed by an untimed one-GPU engine on the whole data set that has run sweeps - 1
+    sweeps (the chain does not depend on the number of GPUs); its next sweep must reproduce `theta`."""
+    import phasetype_b200 as pb
+    e = pb.Engine(wl.n, wl.T, wl.C, wl.nu, wl.zeta, wl.y, wl.censored, method=METHOD_CODE[method], mhit=mhit, seed=SEED,
+                  device=device, sum_y_global=sum_y)
+    e.set_theta(wl.theta, next_iter=1)
+    e.run(sweeps - 1)
+    N, B, zfix = e.sweep_stats()
+    w = min(DUMP_WINDOW, wl.l)
+    k = max(1, min(64, wl.l // w, DUMP_PATH_BYTES // (8 * wl.n * wl.n * w)))
+    starts = np.sort(np.random.default_rng(SEED).choice(wl.l // w, k, replace=False)) * w
+    paths = [e.paths(int(a), w) for a in starts]
+    last = e.run(1)[0]
+    e.close()
+    if not np.array_equal(last, theta):
+        raise RuntimeError("the recomputed last sweep does not reproduce the timed chain's parameter draw")
+    os.makedirs(path, exist_ok=True)
+    out = {"theta": theta, "sweep_N": N, "sweep_B": B, "sweep_z": zfix * 2.0 ** -e.zbits,
+           "paths_obs": np.concatenate([np.arange(a, a + w) for a in starts]),
+           "paths_B": np.concatenate([p[0] for p in paths]), "paths_N": np.concatenate([p[1] for p in paths]),
+           "paths_z": np.concatenate([p[2] for p in paths])}
+    for name, a in out.items():
+        np.save(os.path.join(path, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 # ----------------------------------------------------------------------------- one measured configuration
 class Runner:
     def __init__(self, args, rank, world, local_rank):
@@ -259,9 +294,9 @@ class Runner:
         e.set_theta(wl.theta, next_iter=1)
         return e
 
-    def timed(self, wl, method, y_loc, c_loc, sum_y, steps, warmup, clocks=False):
+    def timed(self, wl, method, y_loc, c_loc, sum_y, steps, warmup, clocks=False, keep_theta=False):
         """W warm-up sweeps, then exactly `steps` sweeps between barriers; device time from CUDA events on the sweep
-        stream, max over ranks.  Returns a dict."""
+        stream, max over ranks.  keep_theta: also return the parameter draw of the last timed sweep.  Returns a dict."""
         eng = self.make_engine(wl, method, y_loc, c_loc, sum_y, True, True)
         eng.run(warmup)
         c0 = eng.counters()
@@ -277,6 +312,7 @@ class Runner:
         total_ms, _ = eng.last_ms()
         total_ms = self.reduce(total_ms)
         c1 = eng.counters()
+        theta = eng.get_theta() if keep_theta else None
         eng.close()
         # instrumented pass: duration of the path kernel alone (CUDA events around each launch, no graph)
         eng2 = self.make_engine(wl, method, y_loc, c_loc, sum_y, False, True)
@@ -293,7 +329,7 @@ class Runner:
         kern_ms = self.reduce(kern_ms)
         eng2.close()
         nloc = max(1, y_loc.shape[0])
-        return {"total_ms": total_ms, "wall": wall, "clocks": clk, "launches": int(c1["launches"] - c0["launches"]),
+        return {"total_ms": total_ms, "wall": wall, "clocks": clk, "launches": int(c1["launches"] - c0["launches"]), "theta": theta,
                 "kern_ms": kern_ms, "share": kern_ms * k / max(tot2, 1e-9),
                 "events": {q: (c1[q] - c0[q]) / float(steps * nloc) for q in ("attempts", "jumps", "deferred", "dens_evals", "env_updates", "brent_evals")},
                 "tail_rounds": (c1["tail_rounds"] - c0["tail_rounds"]) / float(steps)}
@@ -346,7 +382,12 @@ def main():
     ap.add_argument("--no-others", action="store_true", help="skip the ECS / DCS side measurements at N = 1")
     ap.add_argument("--no-weak", action="store_true", help="skip the weak-scaling side measurement at N > 1")
     ap.add_argument("--no-parity", action="store_true", help="skip the chain-parity check at N > 1")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="save what the last timed sweep computed as DIR/<name>.npy (parameter draw, sweep totals, a fixed "
+                         "sample of per-observation paths) so that two builds can be compared on the same seeded inputs")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to the b200 arm (the reference arm keeps no outputs)")
     args.warmup = max(args.warmup, 3)
 
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -389,7 +430,9 @@ def main():
     l_local = int(y_loc.shape[0]); l_global = wl.l
     sum_y = float(wl.y.sum())
 
-    res = R.timed(wl, method, y_loc, c_loc, sum_y, args.steps, args.warmup, clocks=True)
+    res = R.timed(wl, method, y_loc, c_loc, sum_y, args.steps, args.warmup, clocks=True, keep_theta=bool(args.dump_outputs))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, wl, method, args.mhit, sum_y, args.warmup + args.steps, res["theta"], local_rank)
     R.sm_mhz = (res.get("clocks") or {}).get("sm_mhz")
     value = l_global * args.steps / (res["total_ms"] * 1e-3)
 

@@ -6,7 +6,9 @@ legs may import this module; nothing under phasetype_b200/ does.
 Two libraries:
   * oracle/_build/libphtoracle.so -- the CPU restatement (pht_oracle.c), built by `make oracle`;
   * oracle/_ref/libphtref.so      -- the unmodified reference C + R stand-in, built by `make ref`
-                                     where /root/reference exists (prebuilt file travels to the GPU box).
+                                     where PHT_REFERENCE_SRC names an upstream PhaseType source tree
+                                     (https://github.com/louisaslett/PhaseType); without it the tests that
+                                     compare against the reference skip.
 """
 import ctypes as C
 import os
@@ -19,7 +21,7 @@ ORACLE_SO = os.path.join(HERE, "_build", "libphtoracle.so")
 REF_SO = os.path.join(HERE, "_ref", "libphtref.so")
 REF_LIBM_SO = os.path.join(HERE, "_ref", "libphtref_libm.so")
 REG_SO = os.path.join(HERE, "_ref", "PhaseType_reg.so")
-REFERENCE_ROOT = "/root/reference"
+REFERENCE_ROOT = os.environ.get("PHT_REFERENCE_SRC", "")
 
 N_COUNTERS = 16
 COUNTER_NAMES = ["paths", "attempts", "jumps", "dens_evals", "env_updates", "brent_evals",
@@ -32,14 +34,15 @@ _up = np.ctypeslib.ndpointer(dtype=np.uint64, flags="C_CONTIGUOUS")
 
 
 def build(target="all"):
-    """Compile the checkers (gcc).  `ref` is skipped when the reference tree is absent."""
+    """Compile the checkers (gcc).  `ref` is skipped when no reference tree is given (PHT_REFERENCE_SRC)."""
     targets = ["oracle"]
-    if target in ("all", "ref") and os.path.isdir(os.path.join(REFERENCE_ROOT, "src")):
+    if target in ("all", "ref") and REFERENCE_ROOT and os.path.isdir(os.path.join(REFERENCE_ROOT, "src")):
         targets.append("ref")
         targets.append("ref-libm")
         if os.path.exists(os.path.join(HERE, "..", "phasetype_b200", "libpht_b200.so")):
             targets.append("reg")
-    subprocess.run(["make", "-s", "-C", HERE] + targets, check=True)
+    ref = ["REF=" + os.path.abspath(REFERENCE_ROOT)] if REFERENCE_ROOT else []
+    subprocess.run(["make", "-s", "-C", HERE] + ref + targets, check=True)
 
 
 def _f64(a):

@@ -1,7 +1,7 @@
 """Generate the golden vectors in this directory from the UNMODIFIED reference C (oracle/_ref, i.e.
-/root/reference/src compiled against the R stand-in).  Run once in the build container:
+$PHT_REFERENCE_SRC/src compiled against the R stand-in).  Run once with an upstream PhaseType source tree:
 
-    python tests/golden/make_golden.py
+    PHT_REFERENCE_SRC=<PhaseType checkout> python tests/golden/make_golden.py
 
 Each .npz holds the inputs (S, s, y, censored, seed, iteration, mhit, and for ECS/DCS the LAPACK spectral data
 the reference itself computed) and the reference's per-observation outputs (B, N, z).  The reference's own
@@ -35,7 +35,7 @@ def model(kind, n, rng):
 
 def main():
     po.build()
-    assert po.have_ref(), "needs /root/reference to build oracle/_ref"
+    assert po.have_ref(), "set PHT_REFERENCE_SRC to an upstream PhaseType source tree to build oracle/_ref"
     cases = [("mhrs_package_y20", "MHRS", "package", 3, 0.0, 2), ("mhrs_dense8_cens", "MHRS", "dense", 8, 0.2, 1),
              ("mhrs_coxian4", "MHRS", "coxian", 4, 0.0, 1), ("dcs_package_y20", "DCS", "package", 3, 0.0, 1),
              ("dcs_sym8", "DCS", "sym", 8, 0.0, 1), ("dcs_coxian4", "DCS", "coxian", 4, 0.0, 1),

@@ -1,6 +1,6 @@
-"""Tier-3 fixture: the chain of the UNMODIFIED reference LJMA_Gibbs (oracle/_ref, built from /root/reference/src) on the
+"""Tier-3 fixture: the chain of the UNMODIFIED reference LJMA_Gibbs (oracle/_ref, built from $PHT_REFERENCE_SRC/src) on the
 structured repairable-system model of the reference's tests/phtMCMC2.R with 400 simulated observations, for each of the
-three methods.  Run in the build container (needs /root/reference):  python tests/golden/make_tier3.py"""
+three methods.  Run with an upstream PhaseType source tree:  PHT_REFERENCE_SRC=<checkout> python tests/golden/make_tier3.py"""
 import os
 import sys
 

@@ -172,7 +172,7 @@ def test_reference_registration_table_binds_the_drop_in():
     import ctypes as C
     from oracle import pyoracle as po
     if not os.path.exists(po.REG_SO):
-        pytest.skip("oracle/_ref/PhaseType_reg.so not built (needs /root/reference)")
+        pytest.skip("oracle/_ref/PhaseType_reg.so not built (needs PHT_REFERENCE_SRC)")
     reg = C.CDLL(po.REG_SO)
     fun = C.c_void_p(); nargs = C.c_int(); types = (C.c_uint * 32)(); dyn = C.c_int(); force = C.c_int()
     assert reg.phtreg_lookup(b"LJMA_Gibbs", C.byref(fun), C.byref(nargs), types, 32, C.byref(dyn), C.byref(force)) == 0
