@@ -24,7 +24,9 @@ extern "C" {
 /* ------------------------------------------------------------------ layer 1 */
 
 /* Replaces reference src/PHT_MCMC_Aslett.c:104 (same name, same 15 arguments,
- * same meaning: documented at src/PHT_MCMC_Aslett.c:72-103).  `res` (it x m,
+ * same meaning: documented at src/PHT_MCMC_Aslett.c:72-103).  R's `censored` has
+ * no slot for an upper bound, so interval-censored data go through layer 2
+ * (pht_engine_set_upper), not through this routine.  `res` (it x m,
  * column-major) is fully overwritten; row 0 is the start value.  Diagnostics go
  * through Rprintf; nothing is signalled (void), as in the reference.
  * Engine knobs that have no slot in the 15 arguments come from the environment:
@@ -134,6 +136,16 @@ int pht_engine_get_theta(pht_engine *e, double *theta);
 int pht_engine_set_pi(pht_engine *e, const double *pi, const double *beta);
 int pht_engine_get_pi(pht_engine *e, double *pi);
 int pht_engine_pi_rows(pht_engine *e, int rows, double *out);
+
+/* Interval-censored observations (method MHRS): the absorption time of local observation k is known to lie in
+ * [y_k, u_k].  upper_local holds one u per local observation, in the order of y_local; +INFINITY means no bound
+ * (exact or right-censored as before, with the same results bit for bit).  A finite u needs the censoring flag and
+ * u > y.  Paths are drawn from their law given y <= T <= u by the same rejection sampler (an attempt survives when it
+ * is absorbed in [y, u]); their statistics are those of a right-censored path.  Interval paths end by u, so the
+ * configured zbits may be at most pht_choose_zbits(sum over the observations of max(y, u)).  NULL clears the bounds.
+ * Every rank of a multi-rank run sets bounds (or none) before the exchange windows are attached.  Refused for ECS,
+ * DCS and the two MH variants. */
+int pht_engine_set_upper(pht_engine *e, const double *upper_local);
 
 /* run `nsweeps` Gibbs sweeps; row r of out (nsweeps x m, row-major) is the draw of sweep r.
  * out may be NULL (results stay on the device; fetch later with pht_engine_get_theta). */

@@ -19,6 +19,7 @@ SYMBOLS = [
     "pht_engine_get_theta", "pht_engine_run", "pht_engine_enqueue", "pht_engine_sync", "pht_engine_last_ms",
     "pht_engine_sweep_stats", "pht_engine_paths", "pht_engine_set_spectral", "pht_engine_get_model",
     "pht_engine_counters", "pht_fp64_fma_rate", "pht_engine_set_l2_flush", "pht_engine_peer_handle", "pht_engine_peer_attach", "pht_engine_round_trace", "pht_engine_set_pi", "pht_engine_get_pi", "pht_engine_pi_rows",
+    "pht_engine_set_upper",
 ]
 PEER_HANDLE_BYTES = 128
 CNT_NAMES = ["paths", "attempts", "jumps", "dens_evals", "env_updates", "brent_evals", "arms_calls",
@@ -76,6 +77,7 @@ def lib():
     L.pht_engine_set_pi.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
     L.pht_engine_get_pi.argtypes = [C.c_void_p, _dp]
     L.pht_engine_pi_rows.argtypes = [C.c_void_p, C.c_int, _dp]
+    L.pht_engine_set_upper.argtypes = [C.c_void_p, C.c_void_p]
     L.pht_engine_peer_handle.argtypes = [C.c_void_p, C.c_void_p]
     L.pht_engine_peer_attach.argtypes = [C.c_void_p, C.c_void_p]
     _lib = L
@@ -214,6 +216,21 @@ class Engine:
         out = np.zeros((int(rows), self.n))
         _check(lib().pht_engine_pi_rows(self._h, int(rows), out))
         return out
+
+    def set_upper(self, u):
+        """Interval-censored observations (method MHRS): u[k] is the upper bound of local observation k's absorption time
+        (+inf: none; a finite bound needs the censoring flag and u > y); None clears the bounds.  Interval paths end by u,
+        so construct the engine with sum_y_global = the sum of max(y, u) over all observations (or a zbits at most
+        pht_choose_zbits of it)."""
+        if u is None:
+            _check(lib().pht_engine_set_upper(self._h, None))
+            return
+        a = np.ascontiguousarray(u, dtype=np.float64)
+        if a.shape != (self.l_local,):
+            raise EngineError("set_upper: %d bounds for %d local observations" % (a.size, self.l_local))
+        if not self.l_local:
+            a = np.full(1, np.inf)           # an empty shard still takes part (never NULL, which clears)
+        _check(lib().pht_engine_set_upper(self._h, a.ctypes.data))
 
     def round_trace(self):
         """(48, 8) array: per tail round number, ns search / ns barrier / ns advance / sum of pending / sum of K / attempts run /

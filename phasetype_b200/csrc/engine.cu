@@ -84,6 +84,10 @@ struct pht_engine {
     ModelLayout L;
     int grid_blocks = 0, tail_blocks = 0, replay_blocks = 0;
     uint4 *d_recs = nullptr;           /* MHRS search -> replay records, one per observation position */
+    /* MHRS interval bounds (pht_engine_set_upper): u in upload order, u in the sorted layout, u of each tail item; the
+     * grids of the kernel instances that read them */
+    double *d_u = nullptr, *d_us = nullptr, *d_item_u = nullptr;
+    int iv_blocks[3] = { 0, 0, 0 };
     /* graph */
     cudaGraphExec_t graph_exec = nullptr; int graph_res_rows = -1; double *graph_res = nullptr;
     unsigned long long graph_launches = 0;      /* kernels one replay of the captured sweep launches */
@@ -122,6 +126,7 @@ static SweepParams sweep_params(pht_engine *e) {
     if (e->d_ys) { p.y = e->d_ys; p.cens = e->d_cs; p.perm = e->d_perm; }      /* production layout: decreasing y */
     p.glist = e->d_glist; p.k_switch = e->k_switch; p.recs = e->d_recs;
     if (e->peers_attached) { p.xw = e->d_xw; for (int r = 0; r < e->cfg.world && r < PHT_MAX_WORLD; r++) p.xpeer[r] = e->xpeer[r]; }
+    if (e->d_u) { p.u = e->d_ys ? e->d_us : e->d_u; p.item_u = e->d_item_u; }
     return p;
 }
 static UpdateParams update_params(pht_engine *e, double *res, int res_rows) {
@@ -189,7 +194,10 @@ static int enqueue_paths(pht_engine *e, const SweepParams &p, const uint32_t *id
         else CU(pht_launch_ecs(p, e->grid_blocks, e->d_idx_exact, e->n_exact, e->d_idx_cens, e->n_cens, e->stream));
         e->launches += (lists_given ? (n_exact != 0) + (n_cens != 0) : (e->n_exact != 0) + (e->n_cens != 0)) - 1;
         break;
-    case PHT_METHOD_MHRS: CU(pht_launch_mhrs(p, e->grid_blocks, e->tail_blocks, e->replay_blocks, e->stream)); e->launches += 2; break;
+    case PHT_METHOD_MHRS:
+        if (p.u) CU(pht_launch_mhrs(p, e->iv_blocks[0], e->iv_blocks[1], e->iv_blocks[2], e->stream));
+        else CU(pht_launch_mhrs(p, e->grid_blocks, e->tail_blocks, e->replay_blocks, e->stream));
+        e->launches += 2; break;
     case PHT_METHOD_DCS: CU(pht_launch_dcs(p, e->grid_blocks, e->stream)); e->launches++; break;           /* unit machine + complex-spectrum kernel */
     case PHT_METHOD_MHS_HOBOLTH: CU(pht_launch_dcs(p, e->grid_blocks, e->stream, true)); e->launches++; break;
     case PHT_METHOD_MHS_ASLETT:
@@ -255,7 +263,7 @@ extern "C" void pht_engine_destroy(pht_engine *e) {
     if (e->ev1) cudaEventDestroy(e->ev1);
     for (void *q : e->ipc_opened) cudaIpcCloseMemHandle(q);
     stage("events, ipc");
-    void *big[] = { e->d_recs, e->d_ys, e->d_cs, e->d_perm, e->d_y, e->d_cens, e->d_items /* arena: found, pend0, pend1, done live inside */, e->d_idx_exact, e->d_idx_cens,
+    void *big[] = { e->d_u, e->d_us, e->d_item_u, e->d_recs, e->d_ys, e->d_cs, e->d_perm, e->d_y, e->d_cens, e->d_items /* arena: found, pend0, pend1, done live inside */, e->d_idx_exact, e->d_idx_cens,
                     e->d_glist, e->d_model, e->d_stats, e->d_state, e->d_T, e->d_C, e->d_nu, e->d_zeta, e->d_var_ptr, e->d_cell_i, e->d_cell_j, e->d_pires, e->d_res };
     for (void *b : big) pht_dev_free(b, e->stream);
     if (e->stream) cudaStreamSynchronize(e->stream);
@@ -403,7 +411,7 @@ extern "C" int pht_engine_create(pht_engine **out, const pht_config *cfg, const 
         if (cfg->world > 1) CUE(pht_dev_alloc((void **)&e->d_glist, sizeof(uint32_t) * 2 * PHT_MAX_WORLD * PHT_GCAP, e->stream));      /* double buffered */
         CUE(pht_dev_alloc((void **)&e->d_recs, ln * sizeof(uint4), e->stream));
         stage("record list");
-        if (pht_mhrs_grid_blocks(cfg->device, n, &e->grid_blocks, &e->tail_blocks, &e->replay_blocks) != 0) e->grid_blocks = 0;
+        if (pht_mhrs_grid_blocks(cfg->device, n, false, &e->grid_blocks, &e->tail_blocks, &e->replay_blocks) != 0) e->grid_blocks = 0;
         if (e->grid_blocks <= 0) { fail("MHRS kernel does not fit on the device: %s", cudaGetErrorString(cudaGetLastError())); pht_engine_destroy(e); return -1; }
         if (auto_cap) {
             /* Attempts a lane spends on one observation before it hands it to the tail.  A lane is a slow worker (one
@@ -476,11 +484,13 @@ extern "C" int pht_engine_comm_init(pht_engine *e, const void *id128) {
 
 /* ---------------------------------------------------------------- peer exchange windows (MHRS global tail) */
 struct PeerHandle { unsigned long long pid; unsigned long long ptr; int device; int valid; cudaIpcMemHandle_t ipc; unsigned long long cfg_hash; };
-/* what every rank of a run must agree on (the chain is one chain): key, shape, sampler, fixed-point scale, world size */
-static unsigned long long cfg_hash(const pht_config &c) {
+/* what every rank of a run must agree on (the chain is one chain): key, shape, sampler, fixed-point scale, world size, and
+ * whether interval bounds are set (a global tail round searches every rank's items with one kernel instance) */
+static unsigned long long cfg_hash(const pht_engine *e) {
+    const pht_config &c = e->cfg;
     unsigned long long h = 0xcbf29ce484222325ULL;
     const unsigned long long v[] = { c.seed, (unsigned long long)c.n, (unsigned long long)c.m, (unsigned long long)c.method, (unsigned long long)c.mhit,
-                                     (unsigned long long)c.zbits, (unsigned long long)c.world };
+                                     (unsigned long long)c.zbits, (unsigned long long)c.world, e->d_u ? 1ull : 0ull };
     for (unsigned long long x : v) for (int b = 0; b < 8; b++) { h ^= (x >> (8 * b)) & 0xffull; h *= 0x100000001b3ULL; }
     return h;
 }
@@ -493,7 +503,7 @@ extern "C" int pht_engine_peer_handle(pht_engine *e, void *handle) {
     if (e->d_xw) {
         CU(cudaSetDevice(e->cfg.device));
         h.pid = (unsigned long long)getpid(); h.ptr = (unsigned long long)(uintptr_t)e->d_xw; h.device = e->cfg.device; h.valid = 1;
-        h.cfg_hash = cfg_hash(e->cfg);
+        h.cfg_hash = cfg_hash(e);
         CU(cudaIpcGetMemHandle(&h.ipc, e->d_xw));
     }
     memcpy(handle, &h, sizeof(h));
@@ -507,7 +517,7 @@ extern "C" int pht_engine_peer_attach(pht_engine *e, const void *handles) {
     for (int r = 0; r < e->cfg.world; r++) {
         PeerHandle h; memcpy(&h, (const char *)handles + (size_t)r * PHT_PEER_HANDLE_BYTES, sizeof(h));
         if (!h.valid) return fail("rank %d offers no exchange window", r);
-        if (h.cfg_hash != cfg_hash(e->cfg)) return fail("rank %d runs a different configuration (seed, n, m, method, mhit, zbits or world differ from rank %d's): the ranks of a run share one chain", r, e->cfg.rank);
+        if (h.cfg_hash != cfg_hash(e)) return fail("rank %d runs a different configuration (seed, n, m, method, mhit, zbits, world or the presence of interval bounds differ from rank %d's): the ranks of a run share one chain", r, e->cfg.rank);
         if (r == e->cfg.rank) { e->xpeer[r] = e->d_xw; continue; }
         if (h.pid == (unsigned long long)getpid()) {
             /* same process (one host thread per GPU): the peer's pointer is valid here once peer access is on */
@@ -589,6 +599,58 @@ extern "C" int pht_engine_pi_rows(pht_engine *e, int rows, double *out) {
     CU(cudaSetDevice(e->cfg.device));
     CU(cudaStreamSynchronize(e->stream));
     if (rows) CU(cudaMemcpy(out, e->d_pires, sizeof(double) * (size_t)rows * e->cfg.n, cudaMemcpyDeviceToHost));
+    return 0;
+}
+
+extern "C" int pht_engine_set_upper(pht_engine *e, const double *upper_local) {
+    if (!e) return fail("null engine");
+    CU(cudaSetDevice(e->cfg.device));
+    CU(cudaStreamSynchronize(e->stream));
+    if (e->peers_attached) return fail("the interval bounds of a multi-rank run are set on every rank before the exchange windows are attached");
+    if (e->graph_exec) { cudaGraphExecDestroy(e->graph_exec); e->graph_exec = nullptr; }     /* kernel parameters change */
+    if (!upper_local) {
+        double *bufs[] = { e->d_u, e->d_us, e->d_item_u };
+        for (double *b : bufs) CU(pht_dev_free(b, e->stream));
+        e->d_u = e->d_us = e->d_item_u = nullptr;
+        CU(cudaStreamSynchronize(e->stream));
+        return 0;
+    }
+    if (method_of(e->cfg) != PHT_METHOD_MHRS)
+        return fail("interval-censored observations need method MHRS (ECS, DCS and the MH variants have no conditional law for a bounded absorption time)");
+    const long l = e->l_local;
+    std::vector<double> y((size_t)(l > 0 ? l : 1)); std::vector<uint8_t> c((size_t)(l > 0 ? l : 1));
+    if (l > 0) {
+        CU(cudaMemcpy(y.data(), e->d_y, sizeof(double) * (size_t)l, cudaMemcpyDeviceToHost));
+        CU(cudaMemcpy(c.data(), e->d_cens, (size_t)l, cudaMemcpyDeviceToHost));
+    }
+    /* an interval path ends by u, not by y: the fixed-point scale must leave room for sum max(y, u) */
+    double sum = 0.0;
+    for (long i = 0; i < l; i++) {
+        const double u = upper_local[i];
+        if (std::isnan(u)) return fail("upper[%ld] is NaN", i);
+        if (u == INFINITY) { sum += y[(size_t)i]; continue; }
+        if (!(u > y[(size_t)i])) return fail("upper[%ld] = %g is not above y = %g", i, u, y[(size_t)i]);
+        if (!c[(size_t)i]) return fail("upper[%ld] = %g on an exact observation: a finite bound needs the censoring flag", i, u);
+        /* (the rejection loop `while (t < y || t > u)` runs no attempt at all when y = 0) */
+        if (!(y[(size_t)i] > 0.0)) return fail("upper[%ld] = %g with y = %g: an interval needs y > 0 (a tiny y for a failure before the first inspection)", i, u, y[(size_t)i]);
+        sum += u;
+    }
+    if (sum > 0.0 && e->cfg.zbits > pht_choose_zbits(sum))
+        return fail("zbits = %d is too fine for these bounds: interval paths end by u, and sum of max(y, u) = %g allows at most %d",
+                    e->cfg.zbits, sum, pht_choose_zbits(sum));
+    const size_t ln = (size_t)(l > 0 ? l : 1);
+    if (!e->iv_blocks[0] && pht_mhrs_grid_blocks(e->cfg.device, e->cfg.n, true, &e->iv_blocks[0], &e->iv_blocks[1], &e->iv_blocks[2]) != 0) {
+        e->iv_blocks[0] = 0;
+        return fail("MHRS interval kernels do not fit on the device: %s", cudaGetErrorString(cudaGetLastError()));
+    }
+    if (!e->d_u) CU(pht_dev_alloc((void **)&e->d_u, ln * sizeof(double), e->stream));
+    if (e->d_ys && !e->d_us) CU(pht_dev_alloc((void **)&e->d_us, ln * sizeof(double), e->stream));
+    if (!e->d_item_u) CU(pht_dev_alloc((void **)&e->d_item_u, (size_t)e->item_cap * sizeof(double), e->stream));
+    if (l > 0) {
+        CU(cudaMemcpyAsync(e->d_u, upper_local, sizeof(double) * (size_t)l, cudaMemcpyHostToDevice, e->stream));
+        if (e->d_ys) CU(pht_gather_f64(e->d_u, e->d_perm, e->d_us, l, e->stream));
+    }
+    CU(cudaStreamSynchronize(e->stream));
     return 0;
 }
 
@@ -731,6 +793,7 @@ extern "C" int pht_engine_paths(pht_engine *e, long first, long count, int *B, i
         if (enqueue_model(e, u)) goto out;
         SweepParams p = sweep_params(e);
         p.y = e->d_y; p.cens = e->d_cens; p.perm = nullptr;         /* the window [first, first + count) is in upload order */
+        if (p.u) p.u = e->d_u;
         p.outB = dB; p.outN = dN; p.outz = dz; p.first = first; p.count = count;
         if (method_of(e->cfg) == PHT_METHOD_ECS) {
             std::vector<uint32_t> ie, ic;

@@ -4,6 +4,8 @@
  * HBM layout (all per engine = per GPU):
  *   y[l_local]      fp64   observations of this rank's shard (global index rank + k*world)
  *   cens[l_local]   uint8  right-censoring flags (the ABI's int32 is repacked at upload)
+ *   u[l_local]      fp64   MHRS only, when interval bounds are set (pht_engine_set_upper): upper bound of each
+ *                          censored observation's absorption time, +inf = none; a copy in the decreasing-y layout
  *   model[]         fp64   the per-sweep model block, offsets from ModelLayout (< 70 KB at n = 32);
  *                          rebuilt on the device every sweep, copied to shared memory by the path kernels
  *   stats[]         int64  N (n*n) | B (n) | z fixed point in two limbs (2n) | error count: the only data that crosses NVLink
@@ -93,6 +95,9 @@ struct XchgWindow {
     unsigned long long gfound[2][PHT_MAX_WORLD * PHT_GCAP];        /* lowest surviving attempt per item, by round parity */
     uint32_t gcount[2][PHT_MAX_WORLD];                             /* items contributed by rank r, by sweep parity */
     TailItem gitems[2][PHT_MAX_WORLD * PHT_GCAP];                  /* the gathered items, by sweep parity */
+    /* upper bounds u of the gathered items (interval-censored observations, k_mhrs.cu IV instance): kept apart so that
+     * TailItem stays 32 bytes and no offset above moves; 512 KiB */
+    double gitem_u[2][PHT_MAX_WORLD * PHT_GCAP];
 };
 
 struct DevState {
@@ -138,6 +143,9 @@ struct SweepParams {
     uint32_t k_switch;         /* attempts per observation and round from which the tail goes global */
     /* per-observation recording (parity mode); all NULL in production */
     int *outB, *outN; double *outz; long first, count;
+    /* interval-censored observations (read by the IV instance of the MHRS kernels only; nullptr = no bounds set):
+     * u per position, same layout as y, +inf where there is no bound; and the bound of each tail item, indexed like items */
+    const double *u; double *item_u;
 };
 
 struct UpdateParams {
@@ -174,11 +182,14 @@ cudaError_t pht_launch_mhs_aslett(const SweepParams &p, int grid_blocks, const u
 int pht_mhs_aslett_grid_blocks(int device, int n);
 /* spectral data of the sweep: inject != nullptr copies host-supplied (evals | Q | Qinv) instead of solving on the device */
 cudaError_t pht_launch_spectral(const UpdateParams &p, const double *inject, cudaStream_t st);
-int pht_mhrs_grid_blocks(int device, int n, int *lane_blocks, int *tail_blocks, int *replay_blocks);
+/* iv: the instance that reads interval bounds (SweepParams::u != nullptr) */
+int pht_mhrs_grid_blocks(int device, int n, bool iv, int *lane_blocks, int *tail_blocks, int *replay_blocks);
 size_t pht_mhrs_smem_bytes(int n);
 /* large per-call buffers: stream-ordered pool allocations, cached across calls (engine.cu) */
 cudaError_t pht_dev_alloc(void **p, size_t bytes, cudaStream_t st);
 cudaError_t pht_dev_free(void *p, cudaStream_t st);
 cudaError_t pht_sort_by_y_desc(const double *y, const uint8_t *cens, long l, double *ys, uint8_t *cs, uint32_t *perm, cudaStream_t st);
+/* dst[i] = src[perm[i]] (device arrays of length l) */
+cudaError_t pht_gather_f64(const double *src, const uint32_t *perm, double *dst, long l, cudaStream_t st);
 
 #endif

@@ -252,16 +252,18 @@ __device__ __forceinline__ bool walk_step(Walk &w, double y, bool cens, uint32_t
 }
 
 /* Run attempt a of observation (y, cens, og) to its end with the exact walker.  Returns true when it survives
- * (alive at y in a state that can exit, eq_Bladt_MHRS.c:66,74); *jend = the state it is in at the end. */
+ * (alive at y in a state that can exit, eq_Bladt_MHRS.c:66,74); *jend = the state it is in at the end.
+ * IV: an interval-censored observation (cens with u < inf) survives only when it is absorbed at t <= u as well. */
 /* result word: bit 0 survived, bits 8..15 end state, bits 16..31 jump-steps taken */
-template <int NC>
+template <int NC, bool IV = false>
 MHRS_COLD uint32_t exact_attempt(uint32_t a, bool off, double y, bool cens, uint32_t og, const SweepParams &p,
-                                                      MhrsSmem<NC> &sm, uint32_t iter, int n, uint32_t smask) {
+                                                      MhrsSmem<NC> &sm, uint32_t iter, int n, uint32_t smask, double u = 0.0) {
     Walk w; Rec norec; norec.lastt = 0.0; norec.B = 0; norec.out_idx = 0; norec.z2 = nullptr;
     walk_begin(w, a, off, og, p, iter);
     unsigned st = 1;
     while (!walk_step<false>(w, y, cens, og, p, sm, iter, n, norec)) st++;
-    const bool ok = (w.t >= y) && ((smask >> w.j) & 1u);
+    bool ok = (w.t >= y) && ((smask >> w.j) & 1u);
+    if constexpr (IV) ok = ok && w.t <= u;
     return (ok ? 1u : 0u) | ((uint32_t)w.j << 8) | ((st > 0xffffu ? 0xffffu : st) << 16);
 }
 
@@ -370,6 +372,19 @@ __device__ __forceinline__ void replay_phase(const SweepParams &p, MhrsSmem<NC> 
  * per-step error bound that depends on y, the Philox word, and the censoring flag. */
 struct ObsF { float yn; uint32_t og; bool cens; };
 __device__ __forceinline__ void obs_set(ObsF &o, float yn, uint32_t og, bool cens) { o.yn = yn; o.og = og; o.cens = cens; }
+/* IV instance: also the upper bound u in the same units (+inf: none), and bn = the largest clock value a decision is
+ * made at (u when finite, else y), at which the part of the error bound that grows with the clock is taken */
+struct ObsFU : ObsF { float un, bn; };
+template <bool IV> struct ObsOf { typedef ObsF T; };
+template <> struct ObsOf<true> { typedef ObsFU T; };
+__device__ __forceinline__ void obs_set_u(ObsF &, float) {}
+__device__ __forceinline__ void obs_set_u(ObsFU &o, float un) { o.un = un; o.bn = (un < __int_as_float(0x7f800000)) ? un : o.yn; }
+__device__ __forceinline__ float obs_bound(const ObsF &o) { return o.yn; }
+__device__ __forceinline__ float obs_bound(const ObsFU &o) { return o.bn; }
+/* the bound of the observation at layout position pos (IV), or nothing */
+template <bool IV> __device__ __forceinline__ double upper_at(const double *u, uint32_t pos) {
+    if constexpr (IV) return u[pos]; else return 0.0;
+}
 /* the filter walk of one attempt: FP32 clock t with error bound dacc, sub-stream a, next block b, scan row */
 struct Fast { float t, dacc; uint32_t a, b; int row; };
 
@@ -391,9 +406,12 @@ __device__ __forceinline__ void fast_begin(Fast &f, uint32_t a, int n) { f.t = 0
  * The bound accumulated per step is TWICE that sum: 2 * 2^-e + (4.5e-7 + 1.2e-7 y) + 2.5e-7 |L|.  Uniforms with
  * w < 4096 and walks of 4096 steps make the bound infinite, i.e. leave the decision to the exact walker.
  * Outcome of the step: fail (the attempt is dead for certain), surv (alive at y for certain, in state kout), amb (the
- * clock is inside the error band at the moment of the test: ask the exact walker), none of them (the walk goes on). */
-template <int NC>
-__device__ __forceinline__ void fast_step(Fast &f, const ObsF &o, const SweepParams &p, const MhrsSmem<NC> &sm, uint32_t iter, int n,
+ * clock is inside the error band at the moment of the test: ask the exact walker), none of them (the walk goes on).
+ * IV (interval-censored observations, absorbed in [y, u]): the same bound, with its clock-proportional part taken at u
+ * instead of y, gives a second band around u.  The attempt fails as soon as the clock is past u for certain (the clock
+ * only grows), survives when absorbed above y and below u for certain, and goes to the exact walker inside either band. */
+template <int NC, bool IV = false>
+__device__ __forceinline__ void fast_step(Fast &f, const typename ObsOf<IV>::T &o, const SweepParams &p, const MhrsSmem<NC> &sm, uint32_t iter, int n,
                                           bool &fail, bool &surv, bool &amb, int &kout) {
     constexpr int R = NC + 1;
     const pht_u32x4 r = philox_block(f.b, f.a, o.og, iter, p);
@@ -410,7 +428,7 @@ __device__ __forceinline__ void fast_step(Fast &f, const ObsF &o, const SweepPar
     const float L = (__uint_as_float(0x4b400000u + eb) - 12583071.0f) + lg2m;        /* (eb - 159) + lg2m: log2 of u */
     f.t = __fmaf_rn(L, sm.A[k], f.t);
     const float trunc = __uint_as_float((254u - eb) << 23);                           /* 2^-(exponent of w) >= 1 / w */
-    const float c0y = __fmaf_rn(1.2e-7f, o.yn, 4.5e-7f);                              /* the part of the bound that depends on y */
+    const float c0y = __fmaf_rn(1.2e-7f, obs_bound(o), 4.5e-7f);                      /* the part of the bound that depends on y */
     const float step_err = __fmaf_rn(trunc, 2.0f, __fmaf_rn(fabsf(L), 2.5e-7f, c0y));
     const bool flagged = (w < 4096u) || (f.b >> 12) != 0u;
     f.dacc = flagged ? __int_as_float(0x7f800000) : f.dacc + step_err;
@@ -421,6 +439,13 @@ __device__ __forceinline__ void fast_step(Fast &f, const ObsF &o, const SweepPar
     surv = test && over;
     amb = test && !over && !under;
     fail = absd && (!o.cens || under);
+    if constexpr (IV) {
+        const float du = f.t - o.un;
+        const bool past = du > f.dacc, below = -du > f.dacc;        /* above u for certain / below u for certain */
+        fail = fail || past;
+        amb = test && !under && !past && !(over && below);
+        surv = surv && below;
+    }
     kout = absd ? f.row : k;             /* the state occupied at the end: absorption happens FROM the previous state */
     f.row = k;
 }
@@ -513,9 +538,10 @@ __device__ __forceinline__ void peer_barrier(cg::grid_group &grid, const SweepPa
 struct TailView {
     TailItem *items; const uint32_t *pend; unsigned long long *found; uint32_t P, K;
     bool global; uint32_t parity;
+    const double *u;           /* IV: the items' upper bounds, indexed like items */
 };
 
-template <int NC>
+template <int NC, bool IV = false>
 __device__ __forceinline__ void tail_search(const TailView &tv, const SweepParams &p, MhrsSmem<NC> &sm, uint32_t iter, int n,
                                             uint32_t smask, uint32_t nwarps,
                                             unsigned &c_jumps, unsigned &c_attempts) {
@@ -528,7 +554,7 @@ __device__ __forceinline__ void tail_search(const TailView &tv, const SweepParam
      * its own branch (one ATOMS), so the warp-wide hand-out code -- which with whole-warp ballots ran on almost every
      * iteration, some lane fails in most of them -- is left for the moment a pool runs out. */
     Fast f; fast_begin(f, 0u, n);
-    ObsF mo; obs_set(mo, 0.0f, 0u, false);
+    typename ObsOf<IV>::T mo; obs_set(mo, 0.0f, 0u, false); obs_set_u(mo, 0.0f);
     uint32_t my_item = 0xFFFFFFFFu; bool active = false;
     unsigned steps = 0;
     uint32_t *ctr = &sm.pctr[threadIdx.x >> 5];
@@ -537,7 +563,7 @@ __device__ __forceinline__ void tail_search(const TailView &tv, const SweepParam
     /* warp-uniform: the units this warp holds, and the pool being handed out ([*ctr, pool_end) of observation `item`) */
     unsigned long long u_next = 0, u_end = 0, last_base = 0, remaining = total_units;
     bool out_of_units = false, finished = false;
-    uint32_t item = 0, og = 0, a_first = 0, pool_end = 0; float yf = 0.0f; bool cens = false, first_off = false;
+    uint32_t item = 0, og = 0, a_first = 0, pool_end = 0; float yf = 0.0f, uf = 0.0f; bool cens = false, first_off = false;
     while (!finished) {
         /* ---- the search loop proper: no calls in here (the exact walker is asked from outside, see below) */
         bool want_exact = false, exact_off = false, survived = false; int kend = 0;
@@ -545,7 +571,7 @@ __device__ __forceinline__ void tail_search(const TailView &tv, const SweepParam
 #define TAIL_GRAB() do { \
             const uint32_t na_ = atomicAdd(ctr, 1u); \
             if (na_ < pool_end) { \
-                my_item = item; obs_set(mo, yf, og, cens); fast_begin(f, na_, n); \
+                my_item = item; obs_set(mo, yf, og, cens); obs_set_u(mo, uf); fast_begin(f, na_, n); \
                 /* the attempt that starts one draw into its sub-stream (after an MH accept test) is the exact walker's */ \
                 if (first_off && na_ == a_first) { want_exact = true; exact_off = true; active = false; } else active = true; \
             } else active = false; \
@@ -586,6 +612,7 @@ __device__ __forceinline__ void tail_search(const TailView &tv, const SweepParam
                             item = it_idx; a_first = it.a; first_off = (it.flags & TI_OFF) != 0u;
                             pool_end = pstart + len;
                             yf = (float)(it.y * sm.inv_smax); cens = (it.flags & TI_CENS) != 0u; og = it.og;
+                            if constexpr (IV) uf = (float)(tv.u[it_idx] * sm.inv_smax);
                         }
                     }
                     if (have) {
@@ -613,7 +640,7 @@ __device__ __forceinline__ void tail_search(const TailView &tv, const SweepParam
             __syncwarp();           /* lanes that have just taken an attempt step together with the rest */
             if (active) {
                 bool fail, surv, amb; int k;
-                fast_step(f, mo, p, sm, iter, n, fail, surv, amb, k);
+                fast_step<NC, IV>(f, mo, p, sm, iter, n, fail, surv, amb, k);
                 if (surv && !((smask >> k) & 1u)) { surv = false; fail = true; }     /* alive at y in a state that cannot exit: failed */
                 /* (jump-steps are counted when an attempt ends: f.b of them) */
                 if (fail) { c_attempts++; c_jumps += f.b; TAIL_GRAB(); }
@@ -626,7 +653,8 @@ __device__ __forceinline__ void tail_search(const TailView &tv, const SweepParam
         if (finished) break;
         /* ---- attempts the filter could not decide (or that start off the block boundary): the exact walker */
         if (want_exact) {
-            const uint32_t res = exact_attempt(f.a, exact_off, tv.items[my_item].y, mo.cens, mo.og, p, sm, iter, n, smask);
+            const uint32_t res = exact_attempt<NC, IV>(f.a, exact_off, tv.items[my_item].y, mo.cens, mo.og, p, sm, iter, n, smask,
+                                                       upper_at<IV>(tv.u, my_item));
             c_jumps += res >> 16; c_attempts++;
             survived = res & 1u; kend = (int)((res >> 8) & 0xffu);
         }
@@ -690,14 +718,14 @@ MHRS_COLD int tail_advance(TailItem &it, unsigned long long fword, uint32_t K, c
 #define LF_CENS 4u
 #define LF_NVALID 8u     /* the prefetch slot holds an observation */
 #define LF_NCENS 16u
-template <int NC>
+template <int NC, bool IV = false>
 __device__ __forceinline__ void lane_phase(const SweepParams &p, MhrsSmem<NC> &sm, uint32_t iter, int n, uint32_t smask,
                                            uint32_t obs_begin, uint32_t obs_end, uint32_t cap,
                                            unsigned &c_jumps, unsigned &c_attempts) {
     const unsigned FULL = 0xffffffffu;
     const int tid = threadIdx.x, lane = tid & 31;
     Fast f; fast_begin(f, 0u, n);
-    ObsF o; obs_set(o, 0.0f, 0u, false);
+    typename ObsOf<IV>::T o; obs_set(o, 0.0f, 0u, false); obs_set_u(o, 0.0f);
     const double inv_smax = sm.inv_smax;
     uint32_t pos = 0, a_lim = cap, fl = 0u;
     bool dry = false;                     /* warp-uniform: the observation stream has run out */
@@ -722,6 +750,7 @@ __device__ __forceinline__ void lane_phase(const SweepParams &p, MhrsSmem<NC> &s
         }
         if (!(fl & LF_RUN) && (fl & LF_NVALID)) {
             obs_set(o, sm.pf_yf[tid], sm.pf_og[tid], (fl & LF_NCENS) != 0u); pos = sm.pf_pos[tid];
+            if constexpr (IV) obs_set_u(o, (float)(p.u[pos] * inv_smax));
             fl = LF_RUN | (o.cens ? LF_CENS : 0u);
             sm.mh_cur_a[tid] = 0u; sm.mh_misc[tid] = 0u; a_lim = cap;
             fast_begin(f, 0u, n);
@@ -743,7 +772,7 @@ __device__ __forceinline__ void lane_phase(const SweepParams &p, MhrsSmem<NC> &s
         do {
             if (go) {
                 bool fail;
-                fast_step(f, o, p, sm, iter, n, fail, surv, amb, k);
+                fast_step<NC, IV>(f, o, p, sm, iter, n, fail, surv, amb, k);
                 if (fail) { c_jumps += f.b; fast_begin(f, f.a + 1u, n); c_attempts++; hand = f.a >= a_lim; }
                 go = !(surv || amb || hand);
             }
@@ -753,7 +782,7 @@ __device__ __forceinline__ void lane_phase(const SweepParams &p, MhrsSmem<NC> &s
         /* ---- events, a few lanes at a time */
         if (surv || amb) c_jumps += f.b;            /* the filter steps of the attempt that just ended (failed ones: above) */
         if (amb) {
-            const uint32_t res = exact_attempt(f.a, false, p.y[pos], o.cens, o.og, p, sm, iter, n, ~0u);
+            const uint32_t res = exact_attempt<NC, IV>(f.a, false, p.y[pos], o.cens, o.og, p, sm, iter, n, ~0u, upper_at<IV>(p.u, pos));
             surv = res & 1u; k = (int)((res >> 8) & 0xffu); c_jumps += res >> 16;
             if (!surv) { fast_begin(f, f.a + 1u, n); c_attempts++; hand = f.a >= a_lim; }
         }
@@ -790,7 +819,7 @@ __device__ __forceinline__ void lane_phase(const SweepParams &p, MhrsSmem<NC> &s
             } else {
                 /* next proposal: sub-stream a+1 from draw 1 (draw 0 was the accept uniform) */
                 const uint32_t a = f.a + 1u;
-                const uint32_t res = exact_attempt(a, true, p.y[pos], o.cens, o.og, p, sm, iter, n, smask);
+                const uint32_t res = exact_attempt<NC, IV>(a, true, p.y[pos], o.cens, o.og, p, sm, iter, n, smask, upper_at<IV>(p.u, pos));
                 surv = res & 1u; k = (int)((res >> 8) & 0xffu); c_jumps += res >> 16;
                 this_off = true;
                 if (!surv) c_attempts++;
@@ -805,6 +834,7 @@ __device__ __forceinline__ void lane_phase(const SweepParams &p, MhrsSmem<NC> &s
                 it.flags = pack_flags((fl & LF_HAVE) != 0u, (misc >> 8) & 1u, false, o.cens, (int)(misc & 0xffu), misc >> 16);
                 it.owner = p.obs_rank;
                 p.items[idx] = it; p.found[idx] = FOUND_NONE;
+                if constexpr (IV) p.item_u[idx] = p.u[pos];
                 atomicAdd(&p.state->counters[PHT_CNT_DEFERRED], 1ull);
                 fl &= ~LF_RUN;
             } else a_lim = 0xFFFFFFFFu;          /* no room: the lane keeps the observation */
@@ -840,8 +870,10 @@ __device__ __forceinline__ void model_scalars(const MhrsSmem<NC> &sm, int n, uin
     for (int i = 0; i < n; i++) smask |= (sm.s[i] != 0.0) ? (1u << i) : 0u;
 }
 
-/* Kernel 1 of the MHRS sweep: the lane phase (an ordinary launch; its own register budget). */
-template <int NC>
+/* Kernel 1 of the MHRS sweep: the lane phase (an ordinary launch; its own register budget).
+ * IV = true: the instance for sweeps with interval bounds set (SweepParams::u); kernels 1 and 2 have one each, the replay
+ * none (it replays an accepted attempt, whose path statistics are those of a right-censored observation). */
+template <int NC, bool IV>
 __global__ void __launch_bounds__(MHRS_THREADS, MHRS_MIN_BLOCKS) k_mhrs_lanes(const __grid_constant__ SweepParams p) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     MhrsSmem<NC> &sm = *reinterpret_cast<MhrsSmem<NC> *>(smem_raw);
@@ -856,13 +888,13 @@ __global__ void __launch_bounds__(MHRS_THREADS, MHRS_MIN_BLOCKS) k_mhrs_lanes(co
     const uint32_t obs_end = per_obs ? (uint32_t)(p.first + p.count) : (uint32_t)p.l_local;
     const uint32_t cap = p.mhrs_cap > 0 ? (uint32_t)p.mhrs_cap : 256u;
     unsigned c_attempts = 0, c_jumps = 0;      /* per thread and sweep: far below 2^32 */
-    lane_phase(p, sm, iter, n, smask, obs_begin, obs_end, cap, c_jumps, c_attempts);
+    lane_phase<NC, IV>(p, sm, iter, n, smask, obs_begin, obs_end, cap, c_jumps, c_attempts);
     flush_block(p, sm, n, false, c_attempts, c_jumps);
     if (blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(&p.state->counters[PHT_CNT_NS_LANE], gtimer() - t0);
 }
 
 /* Kernel 2: the tail (cooperative launch: grid barriers between rounds; peer barriers in global rounds). */
-template <int NC>
+template <int NC, bool IV>
 __global__ void __launch_bounds__(MHRS_THREADS, MHRS_TAIL_MIN_BLOCKS) k_mhrs_tail(const __grid_constant__ SweepParams p) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     cg::grid_group grid = cg::this_grid();
@@ -909,7 +941,10 @@ __global__ void __launch_bounds__(MHRS_THREADS, MHRS_TAIL_MIN_BLOCKS) k_mhrs_tai
                 if (timekeeper) { const unsigned long long t = gtimer(); atomicAdd(&p.state->counters[PHT_CNT_NS_TAIL], t - t_mark); t_mark = t; }
                 for (uint32_t r = 0; r < W; r++) {
                     XchgWindow *dst = p.xpeer[r];
-                    for (uint32_t i = gtid; i < P; i += gsize) dst->gitems[sp][me * PHT_GCAP + i] = p.items[pend[i]];
+                    for (uint32_t i = gtid; i < P; i += gsize) {
+                        dst->gitems[sp][me * PHT_GCAP + i] = p.items[pend[i]];
+                        if constexpr (IV) dst->gitem_u[sp][me * PHT_GCAP + i] = p.item_u[pend[i]];
+                    }
                     if (gtid == 0) dst->gcount[sp][me] = P;
                 }
                 peer_barrier(grid, p, ++epoch);
@@ -930,12 +965,12 @@ __global__ void __launch_bounds__(MHRS_THREADS, MHRS_TAIL_MIN_BLOCKS) k_mhrs_tai
         } else if (Pg == 0u || p.state->xdead != 0u) break;
         const uint32_t par = (rounds - g0) & 1u;
         TailView tv;
-        if (!global) { tv.items = p.items; tv.pend = pend; tv.found = p.found; tv.P = p.state->n_pend[cur]; }
-        else { tv.items = p.xw->gitems[sp]; tv.pend = gl_cur ? p.glist + PHT_MAX_WORLD * PHT_GCAP : p.glist; tv.found = p.xw->gfound[par]; tv.P = Pg; }
+        if (!global) { tv.items = p.items; tv.pend = pend; tv.found = p.found; tv.P = p.state->n_pend[cur]; tv.u = p.item_u; }
+        else { tv.items = p.xw->gitems[sp]; tv.pend = gl_cur ? p.glist + PHT_MAX_WORLD * PHT_GCAP : p.glist; tv.found = p.xw->gfound[par]; tv.P = Pg; tv.u = p.xw->gitem_u[sp]; }
         tv.K = K; tv.global = global; tv.parity = par;
         const unsigned long long tr0 = timekeeper ? gtimer() : 0ull;
         const unsigned att0 = c_attempts, jmp0 = c_jumps;
-        tail_search(tv, p, sm, iter, n, smask, nwarps, c_jumps, c_attempts);
+        tail_search<NC, IV>(tv, p, sm, iter, n, smask, nwarps, c_jumps, c_attempts);
         const unsigned long long tr1 = timekeeper ? gtimer() : 0ull;
         if (rounds < PHT_ROUND_TRACE) {          /* attempts this round ran, over the whole grid (measurement aid) */
             unsigned d = c_attempts - att0;
@@ -1039,44 +1074,57 @@ __global__ void __launch_bounds__(MHRS_THREADS, MHRS_REPLAY_MIN_BLOCKS) k_mhrs_r
 }
 
 /* ------------------------------------------------------------------------------------------ host side */
-template <int NC>
+template <int NC, bool IV>
 static int grid_blocks_of(int device, int *lane_blocks, int *tail_blocks, int *replay_blocks) {
     int a = 0, b = 0, c = 0, sms = 0;
     const size_t smem = sizeof(MhrsSmem<NC>);
-    if (cudaFuncSetAttribute(k_mhrs_lanes<NC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return -1;
-    if (cudaFuncSetAttribute(k_mhrs_tail<NC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return -1;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&a, k_mhrs_lanes<NC>, MHRS_THREADS, smem) != cudaSuccess) return -1;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, k_mhrs_tail<NC>, MHRS_THREADS, smem) != cudaSuccess) return -1;
+    if (cudaFuncSetAttribute(k_mhrs_lanes<NC, IV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return -1;
+    if (cudaFuncSetAttribute(k_mhrs_tail<NC, IV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return -1;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&a, k_mhrs_lanes<NC, IV>, MHRS_THREADS, smem) != cudaSuccess) return -1;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, k_mhrs_tail<NC, IV>, MHRS_THREADS, smem) != cudaSuccess) return -1;
     if (cudaFuncSetAttribute(k_mhrs_replay<NC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return -1;
     if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&c, k_mhrs_replay<NC>, MHRS_THREADS, smem) != cudaSuccess) return -1;
     if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device) != cudaSuccess) return -1;
     *lane_blocks = a * sms; *tail_blocks = b * sms; *replay_blocks = c * sms;
     return (a > 0 && b > 0 && c > 0) ? 0 : -1;
 }
-/* grid sizes: every SM full of resident blocks of each kernel (persistent warps; the tail launch is cooperative) */
-int pht_mhrs_grid_blocks(int device, int n, int *lane_blocks, int *tail_blocks, int *replay_blocks) {
-    if (n <= 8) return grid_blocks_of<8>(device, lane_blocks, tail_blocks, replay_blocks);
-    if (n <= 16) return grid_blocks_of<16>(device, lane_blocks, tail_blocks, replay_blocks);
-    return grid_blocks_of<32>(device, lane_blocks, tail_blocks, replay_blocks);
+/* grid sizes: every SM full of resident blocks of each kernel (persistent warps; the tail launch is cooperative).  The IV
+ * instances get grids of their own: their register counts need not be those of the plain ones. */
+int pht_mhrs_grid_blocks(int device, int n, bool iv, int *lane_blocks, int *tail_blocks, int *replay_blocks) {
+    if (iv) {
+        if (n <= 8) return grid_blocks_of<8, true>(device, lane_blocks, tail_blocks, replay_blocks);
+        if (n <= 16) return grid_blocks_of<16, true>(device, lane_blocks, tail_blocks, replay_blocks);
+        return grid_blocks_of<32, true>(device, lane_blocks, tail_blocks, replay_blocks);
+    }
+    if (n <= 8) return grid_blocks_of<8, false>(device, lane_blocks, tail_blocks, replay_blocks);
+    if (n <= 16) return grid_blocks_of<16, false>(device, lane_blocks, tail_blocks, replay_blocks);
+    return grid_blocks_of<32, false>(device, lane_blocks, tail_blocks, replay_blocks);
 }
 size_t pht_mhrs_smem_bytes(int n) {
     return n <= 8 ? sizeof(MhrsSmem<8>) : (n <= 16 ? sizeof(MhrsSmem<16>) : sizeof(MhrsSmem<32>));
 }
 
-cudaError_t pht_launch_mhrs(const SweepParams &p, int lane_blocks, int tail_blocks, int replay_blocks, cudaStream_t st) {
+template <int NC, bool IV>
+static cudaError_t launch_of(const SweepParams &p, int lane_blocks, int tail_blocks, int replay_blocks, cudaStream_t st) {
     SweepParams q = p;
     void *args[] = { &q };
-    const size_t smem = pht_mhrs_smem_bytes(p.n);
-    if (p.n <= 8) k_mhrs_lanes<8><<<lane_blocks, MHRS_THREADS, smem, st>>>(q);
-    else if (p.n <= 16) k_mhrs_lanes<16><<<lane_blocks, MHRS_THREADS, smem, st>>>(q);
-    else k_mhrs_lanes<32><<<lane_blocks, MHRS_THREADS, smem, st>>>(q);
+    const size_t smem = sizeof(MhrsSmem<NC>);
+    k_mhrs_lanes<NC, IV><<<lane_blocks, MHRS_THREADS, smem, st>>>(q);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return e;
-    const void *fn = p.n <= 8 ? (const void *)k_mhrs_tail<8> : (p.n <= 16 ? (const void *)k_mhrs_tail<16> : (const void *)k_mhrs_tail<32>);
-    e = cudaLaunchCooperativeKernel(fn, dim3(tail_blocks), dim3(MHRS_THREADS), args, smem, st);
+    e = cudaLaunchCooperativeKernel((const void *)k_mhrs_tail<NC, IV>, dim3(tail_blocks), dim3(MHRS_THREADS), args, smem, st);
     if (e != cudaSuccess) return e;
-    if (p.n <= 8) k_mhrs_replay<8><<<replay_blocks, MHRS_THREADS, smem, st>>>(q);
-    else if (p.n <= 16) k_mhrs_replay<16><<<replay_blocks, MHRS_THREADS, smem, st>>>(q);
-    else k_mhrs_replay<32><<<replay_blocks, MHRS_THREADS, smem, st>>>(q);
+    k_mhrs_replay<NC><<<replay_blocks, MHRS_THREADS, smem, st>>>(q);
     return cudaGetLastError();
+}
+/* the IV instance runs when the sweep has interval bounds (p.u != nullptr), the plain one otherwise */
+cudaError_t pht_launch_mhrs(const SweepParams &p, int lane_blocks, int tail_blocks, int replay_blocks, cudaStream_t st) {
+    if (p.u != nullptr) {
+        if (p.n <= 8) return launch_of<8, true>(p, lane_blocks, tail_blocks, replay_blocks, st);
+        if (p.n <= 16) return launch_of<16, true>(p, lane_blocks, tail_blocks, replay_blocks, st);
+        return launch_of<32, true>(p, lane_blocks, tail_blocks, replay_blocks, st);
+    }
+    if (p.n <= 8) return launch_of<8, false>(p, lane_blocks, tail_blocks, replay_blocks, st);
+    if (p.n <= 16) return launch_of<16, false>(p, lane_blocks, tail_blocks, replay_blocks, st);
+    return launch_of<32, false>(p, lane_blocks, tail_blocks, replay_blocks, st);
 }

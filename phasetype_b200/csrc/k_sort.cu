@@ -19,6 +19,10 @@ __global__ void k_gather_u8(const uint8_t *src, const uint32_t *perm, uint8_t *d
     const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < l) dst[i] = src[perm[i]];
 }
+__global__ void k_gather_f64(const double *src, const uint32_t *perm, double *dst, long l) {
+    const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < l) dst[i] = src[perm[i]];
+}
 
 /* ys[i] = y[perm[i]] non-increasing, cs[i] = cens[perm[i]]; all pointers device memory of length l */
 cudaError_t pht_sort_by_y_desc(const double *y, const uint8_t *cens, long l, double *ys, uint8_t *cs, uint32_t *perm, cudaStream_t st) {
@@ -36,4 +40,12 @@ cudaError_t pht_sort_by_y_desc(const double *y, const uint8_t *cens, long l, dou
     pht_dev_free(tmp, st);
     pht_dev_free(idx, st);
     return e;
+}
+
+/* interval bounds into the sorted layout (pht_engine_set_upper): the sort itself stays as it is */
+cudaError_t pht_gather_f64(const double *src, const uint32_t *perm, double *dst, long l, cudaStream_t st) {
+    if (l <= 0) return cudaSuccess;
+    const int threads = 256; const unsigned blocks = (unsigned)((l + threads - 1) / threads);
+    k_gather_f64<<<blocks, threads, 0, st>>>(src, perm, dst, l);
+    return cudaGetLastError();
 }

@@ -50,6 +50,19 @@ def simulate_pht(R, s, size, rng, chunk=1 << 20):
     return out
 
 
+def inspection(R, s, l, spacing, k, rng):
+    """Inspection data (interval censoring): absorption times T of the CTMC (R, s) started in state 0, seen only at the
+    inspections spacing, 2 spacing, ..., k spacing.  A unit found failed at inspection i (T in ((i-1) spacing, i spacing])
+    gives the interval y = (i-1) spacing, u = i spacing (y = 1e-12 before the first inspection: the sampler needs y > 0);
+    a unit still working at the last inspection is right-censored there (u = +inf).  Returns (y, u, censored, T)."""
+    t = simulate_pht(R, s, l, rng)
+    i = np.ceil(t / spacing)
+    failed = i <= k
+    y = np.where(failed, np.maximum((i - 1) * spacing, 1e-12), k * spacing)
+    u = np.where(failed, i * spacing, np.inf)
+    return y, u, np.ones(l, dtype=np.int32), t
+
+
 def _general_T(R, s):
     """Every non-zero rate its own parameter, numbered column-major like sorted "Sij"/"si" names would be."""
     n = s.shape[0]
