@@ -65,6 +65,15 @@ void LJMA_Gibbs(int *it, int *mhit, int *method, int *n, int *m, double *nu, dou
                                        the chain sampler (the MH step is skipped for a censored observation) */
 #define PHT_METHOD_MHS_ASLETT 16    /* LJMA_MHsample_Aslett (reverse = 0), src/Simulate_AbsCTMC_eq_Aslett_DCS.c:49-143: the
                                        Aslett-DCS "alive at y" sampler for every observation + independence MH */
+/* The uniformisation path sampler (Hobolth & Stone 2009, section 3.3; the engine's own, no reference counterpart): every
+ * path is drawn from its exact conditional law given the data, for any sub-generator (a Jordan block or a complex
+ * spectrum included), through the uniformised chain R = I + S/lambda, lambda = max_i -S_ii, and a table of its powers
+ * built once per sweep.  Exact, right-censored, interval-censored (pht_engine_set_upper) and left-censored (y = 0 with a
+ * finite bound) observations; the start state is drawn from its conditional law too, so the start-distribution update
+ * (pht_engine_set_pi with beta) works with it.  Lowest priority of the mask; `mhit` is not used.  The table holds
+ * PHT_UNIF_CAP = 4096 powers (33 MB at n = 32): an observation whose lambda y (or lambda (u - y)) needs more raises error
+ * bit 256.  (Bit 32 stays unassigned.) */
+#define PHT_METHOD_UNIF 64
 #define PHT_MAX_PHASES  32
 
 typedef struct pht_engine pht_engine;
@@ -72,7 +81,7 @@ typedef struct pht_engine pht_engine;
 typedef struct pht_config {
     int n;                /* transient phases, 1..PHT_MAX_PHASES */
     int m;                /* number of rate parameters */
-    int method;           /* bit mask as in the reference; priority MHRS > DCS > ECS */
+    int method;           /* bit mask as in the reference; priority MHRS > DCS > ECS (> 8 > 16 > 64, the engine's own) */
     int mhit;             /* Metropolis-Hastings proposals per exact observation (MHRS) */
     const int *T;         /* (n+1)^2 column-major: 0 = structural zero, v>=1 = parameter index */
     const double *C;      /* (n+1)^2 constant multipliers */
@@ -129,22 +138,25 @@ int pht_engine_get_theta(pht_engine *e, double *theta);
 /* Start distribution.  The reference fixes pi = e1 and leaves its update as FIX ME (src/PHT_MCMC_Aslett.c:190-193) although
  * R passes a Dirichlet prior `beta` down to the wrapper (R/phtMCMC2.R:20-21).  pi (n values, may be NULL: keep) sets the
  * distribution the samplers start their paths from; beta (n positive values, may be NULL: no update) switches on the
- * conjugate update pi | paths ~ Dirichlet(beta + B) at the end of every sweep (method MHRS only: a rejection sampler
- * started from pi draws the start state from its conditional law given y; the reference's ECS and DCS samplers draw it
- * from pi itself, which is exact for the degenerate pi the reference uses and nothing else).  pht_engine_pi_rows returns
+ * conjugate update pi | paths ~ Dirichlet(beta + B) at the end of every sweep (methods MHRS and 64 only: a rejection
+ * sampler started from pi, and the uniformisation sampler, draw the start state from its conditional law given y; the
+ * reference's ECS and DCS samplers draw it from pi itself, which is exact for the degenerate pi the reference uses and
+ * nothing else).  pht_engine_pi_rows returns
  * the draws of the last pht_engine_run (rows x n, row-major). */
 int pht_engine_set_pi(pht_engine *e, const double *pi, const double *beta);
 int pht_engine_get_pi(pht_engine *e, double *pi);
 int pht_engine_pi_rows(pht_engine *e, int rows, double *out);
 
-/* Interval-censored observations (method MHRS): the absorption time of local observation k is known to lie in
+/* Interval-censored observations (methods MHRS and 64): the absorption time of local observation k is known to lie in
  * [y_k, u_k].  upper_local holds one u per local observation, in the order of y_local; +INFINITY means no bound
  * (exact or right-censored as before, with the same results bit for bit).  A finite u needs the censoring flag and
  * u > y.  Paths are drawn from their law given y <= T <= u by the same rejection sampler (an attempt survives when it
  * is absorbed in [y, u]); their statistics are those of a right-censored path.  Interval paths end by u, so the
  * configured zbits may be at most pht_choose_zbits(sum over the observations of max(y, u)).  NULL clears the bounds.
  * Every rank of a multi-rank run sets bounds (or none) before the exchange windows are attached.  Refused for ECS,
- * DCS and the two MH variants. */
+ * DCS and the two MH variants.  Method 64 draws the path given y < T <= u directly (no rejection: the cost does not
+ * depend on the width of the interval) and also takes y = 0 with a finite u: a failure before the first inspection
+ * (left-censored); MHRS needs y > 0. */
 int pht_engine_set_upper(pht_engine *e, const double *upper_local);
 
 /* run `nsweeps` Gibbs sweeps; row r of out (nsweeps x m, row-major) is the draw of sweep r.
@@ -166,7 +178,8 @@ int pht_engine_sweep_stats(pht_engine *e, long long *N, long long *B, long long 
 /* per-observation statistics for local observations [first, first+count): B[count],
  * N[count*n*n] (int32), z[count*n]; same kernels, recording to memory instead of reducing */
 int pht_engine_paths(pht_engine *e, long first, long count, int *B, int *N, double *z);
-/* override the spectral data the ECS/DCS kernels use (evals n, Q n*n, Qinv n*n); NULL restores the device solver */
+/* override the spectral data the ECS/DCS kernels use (evals n, Q n*n, Qinv n*n); NULL restores the device solver;
+ * refused for method 64, which uses none */
 int pht_engine_set_spectral(pht_engine *e, const double *evals, const double *Q, const double *Qinv);
 /* current model matrices as the kernels see them (each may be NULL) */
 int pht_engine_get_model(pht_engine *e, double *S, double *s, double *P, double *Pfull,

@@ -22,6 +22,9 @@ SYMBOLS = [
     "pht_engine_set_upper",
 ]
 PEER_HANDLE_BYTES = 128
+# method 64 (include/pht_b200.h PHT_METHOD_UNIF): the uniformisation path sampler; exact, right-, interval- and
+# left-censored observations, any sub-generator
+METHOD_UNIF = 64
 CNT_NAMES = ["paths", "attempts", "jumps", "dens_evals", "env_updates", "brent_evals", "arms_calls",
              "metrop_rejects", "nonfinite", "deferred", "tail_rounds", "errors", "launches", "ns_lane", "ns_tail", "ns_replay",
              "ns_global", "ns_xwait", "global_rounds", "global_items"]
@@ -218,8 +221,9 @@ class Engine:
         return out
 
     def set_upper(self, u):
-        """Interval-censored observations (method MHRS): u[k] is the upper bound of local observation k's absorption time
-        (+inf: none; a finite bound needs the censoring flag and u > y); None clears the bounds.  Interval paths end by u,
+        """Interval-censored observations (methods MHRS and METHOD_UNIF): u[k] is the upper bound of local observation k's absorption time
+        (+inf: none; a finite bound needs the censoring flag and u > y; METHOD_UNIF also takes y = 0, a failure before
+        the first inspection); None clears the bounds.  Interval paths end by u,
         so construct the engine with sum_y_global = the sum of max(y, u) over all observations (or a zbits at most
         pht_choose_zbits of it)."""
         if u is None:

@@ -14,7 +14,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libpht_b200.so")
-CU = ["engine.cu", "k_model.cu", "k_mhrs.cu", "k_sort.cu", "k_dcs.cu", "k_ecs.cu", "k_peak.cu"]
+CU = ["engine.cu", "k_model.cu", "k_mhrs.cu", "k_sort.cu", "k_dcs.cu", "k_ecs.cu", "k_unif.cu", "k_peak.cu"]
 CC = ["gibbs_host.c", "rapi_standin.c"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-fmad=false", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=default"]

@@ -19,6 +19,7 @@
 #include <unistd.h>
 #include <time.h>
 #include "engine_internal.h"
+#include "pht_unif.h"
 
 /* ---------------------------------------------------------------- errors */
 static thread_local char g_err[512] = "";
@@ -88,6 +89,8 @@ struct pht_engine {
      * grids of the kernel instances that read them */
     double *d_u = nullptr, *d_us = nullptr, *d_item_u = nullptr;
     int iv_blocks[3] = { 0, 0, 0 };
+    /* method 64: the uniformisation table (pht_unif.h) and the longest time span it must cover (max of y and of u - y) */
+    double *d_unif = nullptr; double unif_tmax = 0.0;
     /* graph */
     cudaGraphExec_t graph_exec = nullptr; int graph_res_rows = -1; double *graph_res = nullptr;
     unsigned long long graph_launches = 0;      /* kernels one replay of the captured sweep launches */
@@ -182,6 +185,7 @@ static int method_of(const pht_config &c) {       /* dispatch priority of src/PH
     if (c.method & PHT_METHOD_ECS) return PHT_METHOD_ECS;
     if (c.method & PHT_METHOD_MHS_HOBOLTH) return PHT_METHOD_MHS_HOBOLTH;      /* the engine's extension (pht_b200.h) */
     if (c.method & PHT_METHOD_MHS_ASLETT) return PHT_METHOD_MHS_ASLETT;
+    if (c.method & PHT_METHOD_UNIF) return PHT_METHOD_UNIF;
     return 0;
 }
 
@@ -200,6 +204,7 @@ static int enqueue_paths(pht_engine *e, const SweepParams &p, const uint32_t *id
         e->launches += 2; break;
     case PHT_METHOD_DCS: CU(pht_launch_dcs(p, e->grid_blocks, e->stream)); e->launches++; break;           /* unit machine + complex-spectrum kernel */
     case PHT_METHOD_MHS_HOBOLTH: CU(pht_launch_dcs(p, e->grid_blocks, e->stream, true)); e->launches++; break;
+    case PHT_METHOD_UNIF: CU(pht_launch_unif(p, e->d_unif, e->grid_blocks, e->stream)); break;
     case PHT_METHOD_MHS_ASLETT:
         /* every observation through one kernel: the window list in parity mode, else the whole shard (identity) */
         if (lists_given) CU(pht_launch_mhs_aslett(p, e->grid_blocks, idx_exact, n_exact, e->stream));
@@ -211,10 +216,13 @@ static int enqueue_paths(pht_engine *e, const SweepParams &p, const uint32_t *id
     return 0;
 }
 
-/* k_assemble (+ spectral data for ECS / DCS): everything the path kernels read from the model block */
+/* k_assemble (+ spectral data for ECS / DCS, the uniformisation table for method 64): everything the path kernels read
+ * from the model block */
 static int enqueue_model(pht_engine *e, const UpdateParams &u) {
     CU(pht_launch_assemble(u, e->stream)); e->launches++;
-    if (method_of(e->cfg) != PHT_METHOD_MHRS) {
+    if (method_of(e->cfg) == PHT_METHOD_UNIF) {
+        CU(pht_launch_unif_table(u, e->d_unif, e->unif_tmax, e->stream)); e->launches++;
+    } else if (method_of(e->cfg) != PHT_METHOD_MHRS) {
         CU(pht_launch_spectral(u, e->d_inject, e->stream)); e->launches++;
     }
     return 0;
@@ -263,7 +271,7 @@ extern "C" void pht_engine_destroy(pht_engine *e) {
     if (e->ev1) cudaEventDestroy(e->ev1);
     for (void *q : e->ipc_opened) cudaIpcCloseMemHandle(q);
     stage("events, ipc");
-    void *big[] = { e->d_u, e->d_us, e->d_item_u, e->d_recs, e->d_ys, e->d_cs, e->d_perm, e->d_y, e->d_cens, e->d_items /* arena: found, pend0, pend1, done live inside */, e->d_idx_exact, e->d_idx_cens,
+    void *big[] = { e->d_unif, e->d_u, e->d_us, e->d_item_u, e->d_recs, e->d_ys, e->d_cs, e->d_perm, e->d_y, e->d_cens, e->d_items /* arena: found, pend0, pend1, done live inside */, e->d_idx_exact, e->d_idx_cens,
                     e->d_glist, e->d_model, e->d_stats, e->d_state, e->d_T, e->d_C, e->d_nu, e->d_zeta, e->d_var_ptr, e->d_cell_i, e->d_cell_j, e->d_pires, e->d_res };
     for (void *b : big) pht_dev_free(b, e->stream);
     if (e->stream) cudaStreamSynchronize(e->stream);
@@ -381,6 +389,21 @@ extern "C" int pht_engine_create(pht_engine **out, const pht_config *cfg, const 
         CUE(cudaMemsetAsync(e->d_xw, 0, sizeof(XchgWindow), e->stream));
         CUE(cudaMemsetAsync(e->d_xw->gfound, 0xFF, sizeof(e->d_xw->gfound), e->stream));
         CUE(cudaStreamSynchronize(e->stream));
+    }
+    if (method_of(e->cfg) == PHT_METHOD_UNIF) {
+        /* the table (capacity PHT_UNIF_CAP powers; log k! filled once here), the y-descending layout so that the lanes of
+         * a warp run similar Poisson truncations (parity hooks keep the upload order), and the longest span y */
+        CUE(pht_dev_alloc((void **)&e->d_unif, sizeof(double) * pht_unif_table_doubles(n, PHT_UNIF_CAP), e->stream));
+        CUE(pht_unif_init(e->d_unif, n, PHT_UNIF_CAP, e->stream));
+        for (long i = 0; i < l_local; i++) if (y_local[i] > e->unif_tmax) e->unif_tmax = y_local[i];
+        if (l_local > 1 && !getenv("PHT_B200_NO_SORT")) {
+            CUE(pht_dev_alloc((void **)&e->d_ys, ln * sizeof(double), e->stream)); CUE(pht_dev_alloc((void **)&e->d_cs, ln, e->stream));
+            CUE(pht_dev_alloc((void **)&e->d_perm, ln * sizeof(uint32_t), e->stream));
+            CUE(pht_sort_by_y_desc(e->d_y, e->d_cens, l_local, e->d_ys, e->d_cs, e->d_perm, e->stream));
+        }
+        CUE(cudaStreamSynchronize(e->stream));
+        e->grid_blocks = pht_unif_grid_blocks(cfg->device, n);
+        if (e->grid_blocks <= 0) { fail("the uniformisation kernel does not fit on the device: %s", cudaGetErrorString(cudaGetLastError())); pht_engine_destroy(e); return -1; }
     }
     if (method_of(e->cfg) == PHT_METHOD_MHRS) {
         /* Tail work lists: one arena with room for a quarter of the shard (at least 2^20 observations, at most all of
@@ -578,7 +601,8 @@ extern "C" int pht_engine_set_pi(pht_engine *e, const double *pi, const double *
          * rejection sampler from pi).  The reference's ECS and DCS samplers draw the start state from pi itself
          * (src/Simulate_AbsCTMC_eq_Aslett_ECS.c:231-238, src/Simulate_AbsCTMC_gt_Hobolth_DCS.c:88-95) -- exact only for
          * the degenerate pi the reference always uses -- so B carries no information about pi there. */
-        if (method_of(e->cfg) != PHT_METHOD_MHRS) return fail("the start-distribution update needs method MHRS (ECS and DCS draw the start state from pi, not from its conditional law given y)");
+        if (method_of(e->cfg) != PHT_METHOD_MHRS && method_of(e->cfg) != PHT_METHOD_UNIF)
+            return fail("the start-distribution update needs method MHRS or 64 (ECS and DCS draw the start state from pi, not from its conditional law given y)");
         for (int i = 0; i < n; i++) if (!(beta[i] > 0.0)) return fail("beta[%d] = %g: Dirichlet parameters must be positive", i, beta[i]);
         if (!e->d_beta) CU(cudaMalloc(&e->d_beta, sizeof(double) * n));
         CU(cudaMemcpy(e->d_beta, beta, sizeof(double) * n, cudaMemcpyHostToDevice));
@@ -613,10 +637,17 @@ extern "C" int pht_engine_set_upper(pht_engine *e, const double *upper_local) {
         for (double *b : bufs) CU(pht_dev_free(b, e->stream));
         e->d_u = e->d_us = e->d_item_u = nullptr;
         CU(cudaStreamSynchronize(e->stream));
+        if (method_of(e->cfg) == PHT_METHOD_UNIF) {
+            std::vector<double> y((size_t)(e->l_local > 0 ? e->l_local : 1));
+            if (e->l_local > 0) CU(cudaMemcpy(y.data(), e->d_y, sizeof(double) * (size_t)e->l_local, cudaMemcpyDeviceToHost));
+            e->unif_tmax = 0.0;
+            for (long i = 0; i < e->l_local; i++) if (y[(size_t)i] > e->unif_tmax) e->unif_tmax = y[(size_t)i];
+        }
         return 0;
     }
-    if (method_of(e->cfg) != PHT_METHOD_MHRS)
-        return fail("interval-censored observations need method MHRS (ECS, DCS and the MH variants have no conditional law for a bounded absorption time)");
+    const bool unif = method_of(e->cfg) == PHT_METHOD_UNIF;
+    if (method_of(e->cfg) != PHT_METHOD_MHRS && !unif)
+        return fail("interval-censored observations need method MHRS or 64 (ECS, DCS and the MH variants have no conditional law for a bounded absorption time)");
     const long l = e->l_local;
     std::vector<double> y((size_t)(l > 0 ? l : 1)); std::vector<uint8_t> c((size_t)(l > 0 ? l : 1));
     if (l > 0) {
@@ -624,28 +655,33 @@ extern "C" int pht_engine_set_upper(pht_engine *e, const double *upper_local) {
         CU(cudaMemcpy(c.data(), e->d_cens, (size_t)l, cudaMemcpyDeviceToHost));
     }
     /* an interval path ends by u, not by y: the fixed-point scale must leave room for sum max(y, u) */
-    double sum = 0.0;
+    double sum = 0.0, tmax = 0.0;
     for (long i = 0; i < l; i++) {
         const double u = upper_local[i];
+        if (y[(size_t)i] > tmax) tmax = y[(size_t)i];
         if (std::isnan(u)) return fail("upper[%ld] is NaN", i);
         if (u == INFINITY) { sum += y[(size_t)i]; continue; }
         if (!(u > y[(size_t)i])) return fail("upper[%ld] = %g is not above y = %g", i, u, y[(size_t)i]);
         if (!c[(size_t)i]) return fail("upper[%ld] = %g on an exact observation: a finite bound needs the censoring flag", i, u);
-        /* (the rejection loop `while (t < y || t > u)` runs no attempt at all when y = 0) */
-        if (!(y[(size_t)i] > 0.0)) return fail("upper[%ld] = %g with y = %g: an interval needs y > 0 (a tiny y for a failure before the first inspection)", i, u, y[(size_t)i]);
+        /* (the rejection loop `while (t < y || t > u)` runs no attempt at all when y = 0; method 64 takes y = 0 as a
+         * failure before the first inspection: left-censored) */
+        if (!unif && !(y[(size_t)i] > 0.0)) return fail("upper[%ld] = %g with y = %g: an interval needs y > 0 (a tiny y for a failure before the first inspection)", i, u, y[(size_t)i]);
+        if (unif && !(y[(size_t)i] >= 0.0)) return fail("upper[%ld] = %g with y = %g: an interval needs y >= 0", i, u, y[(size_t)i]);
+        if (u - y[(size_t)i] > tmax) tmax = u - y[(size_t)i];
         sum += u;
     }
     if (sum > 0.0 && e->cfg.zbits > pht_choose_zbits(sum))
         return fail("zbits = %d is too fine for these bounds: interval paths end by u, and sum of max(y, u) = %g allows at most %d",
                     e->cfg.zbits, sum, pht_choose_zbits(sum));
     const size_t ln = (size_t)(l > 0 ? l : 1);
-    if (!e->iv_blocks[0] && pht_mhrs_grid_blocks(e->cfg.device, e->cfg.n, true, &e->iv_blocks[0], &e->iv_blocks[1], &e->iv_blocks[2]) != 0) {
+    if (unif) e->unif_tmax = tmax;
+    if (!unif && !e->iv_blocks[0] && pht_mhrs_grid_blocks(e->cfg.device, e->cfg.n, true, &e->iv_blocks[0], &e->iv_blocks[1], &e->iv_blocks[2]) != 0) {
         e->iv_blocks[0] = 0;
         return fail("MHRS interval kernels do not fit on the device: %s", cudaGetErrorString(cudaGetLastError()));
     }
     if (!e->d_u) CU(pht_dev_alloc((void **)&e->d_u, ln * sizeof(double), e->stream));
     if (e->d_ys && !e->d_us) CU(pht_dev_alloc((void **)&e->d_us, ln * sizeof(double), e->stream));
-    if (!e->d_item_u) CU(pht_dev_alloc((void **)&e->d_item_u, (size_t)e->item_cap * sizeof(double), e->stream));
+    if (!unif && !e->d_item_u) CU(pht_dev_alloc((void **)&e->d_item_u, (size_t)e->item_cap * sizeof(double), e->stream));
     if (l > 0) {
         CU(cudaMemcpyAsync(e->d_u, upper_local, sizeof(double) * (size_t)l, cudaMemcpyHostToDevice, e->stream));
         if (e->d_ys) CU(pht_gather_f64(e->d_u, e->d_perm, e->d_us, l, e->stream));
@@ -708,13 +744,15 @@ static int check_state(pht_engine *e) {
         int err = st.error;
         cudaMemsetAsync(&e->d_state->error, 0, sizeof(int), e->stream);
         cudaStreamSynchronize(e->stream);
-        return fail("device error word 0x%x (%s%s%s%s%s%s%s)", err, (err & 2) ? "sojourn total overflows the fixed-point range (lower PHT_B200_ZBITS); " : "",
+        return fail("device error word 0x%x (%s%s%s%s%s%s%s%s%s)", err, (err & 2) ? "sojourn total overflows the fixed-point range (lower PHT_B200_ZBITS); " : "",
                     (err & 4) ? "MHRS tail list overflow; " : "",
                     (err & 8) ? "an observation's survival probability is too small for rejection sampling (more than 4e9 attempts); " : "",
                     (err & 16) ? "(unused) " : "",
                     (err & 32) ? "spectral decomposition failed; " : "",
                     (err & 64) ? "a peer GPU did not arrive at a barrier of the global MHRS tail; " : "",
-                    (err & 128) ? "another rank of the run raised its error word; " : "");
+                    (err & 128) ? "another rank of the run raised its error word; " : "",
+                    (err & PHT_UNIF_ERR_TABLE) ? "the uniformisation sampler needs more powers of R than its table holds (a stiff generator or a very long y); " : "",
+                    (err & PHT_UNIF_ERR_ZERO) ? "every weight of a uniformisation draw underflowed to zero; " : "");
     }
     return 0;
 }
@@ -828,6 +866,8 @@ extern "C" int pht_engine_set_spectral(pht_engine *e, const double *evals, const
     CU(cudaSetDevice(e->cfg.device));
     CU(cudaStreamSynchronize(e->stream));
     const int n = e->cfg.n;
+    if (method_of(e->cfg) == PHT_METHOD_UNIF && evals && Q && Qinv)
+        return fail("method 64 uses no spectral data (it samples through the uniformised chain)");
     if (e->graph_exec) { cudaGraphExecDestroy(e->graph_exec); e->graph_exec = nullptr; }     /* the sweep changes shape */
     if (!evals || !Q || !Qinv) {
         if (e->d_inject) { CU(cudaFree(e->d_inject)); e->d_inject = nullptr; }

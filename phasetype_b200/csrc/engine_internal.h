@@ -4,7 +4,8 @@
  * HBM layout (all per engine = per GPU):
  *   y[l_local]      fp64   observations of this rank's shard (global index rank + k*world)
  *   cens[l_local]   uint8  right-censoring flags (the ABI's int32 is repacked at upload)
- *   u[l_local]      fp64   MHRS only, when interval bounds are set (pht_engine_set_upper): upper bound of each
+ *   unif[]          fp64   method 64 only: the uniformisation table (pht_unif.h; 33 MB at n = 32)
+ *   u[l_local]      fp64   MHRS and method 64 only, when interval bounds are set (pht_engine_set_upper): upper bound of each
  *                          censored observation's absorption time, +inf = none; a copy in the decreasing-y layout
  *   model[]         fp64   the per-sweep model block, offsets from ModelLayout (< 70 KB at n = 32);
  *                          rebuilt on the device every sweep, copied to shared memory by the path kernels
@@ -185,6 +186,14 @@ cudaError_t pht_launch_spectral(const UpdateParams &p, const double *inject, cud
 /* iv: the instance that reads interval bounds (SweepParams::u != nullptr) */
 int pht_mhrs_grid_blocks(int device, int n, bool iv, int *lane_blocks, int *tail_blocks, int *replay_blocks);
 size_t pht_mhrs_smem_bytes(int n);
+/* method 64 (k_unif.cu): log k! into a new table; the per-sweep table kernel (tmax: the longest time span of the shard,
+ * max of y and of u - y); the path kernel and its grid.  The table (pht_unif.h, capacity PHT_UNIF_CAP powers) is a
+ * kernel argument of its own, so that SweepParams / UpdateParams -- and the other kernels' code -- stay as they are. */
+cudaError_t pht_unif_init(double *tab, int n, int cap, cudaStream_t st);
+size_t pht_unif_table_doubles(int n, int cap);
+cudaError_t pht_launch_unif_table(const UpdateParams &p, double *tab, double tmax, cudaStream_t st);
+cudaError_t pht_launch_unif(const SweepParams &p, const double *tab, int grid_blocks, cudaStream_t st);
+int pht_unif_grid_blocks(int device, int n);
 /* large per-call buffers: stream-ordered pool allocations, cached across calls (engine.cu) */
 cudaError_t pht_dev_alloc(void **p, size_t bytes, cudaStream_t st);
 cudaError_t pht_dev_free(void *p, cudaStream_t st);
