@@ -72,7 +72,8 @@ void LJMA_Gibbs(int *it, int *mhit, int *method, int *n, int *m, double *nu, dou
  * finite bound) observations; the start state is drawn from its conditional law too, so the start-distribution update
  * (pht_engine_set_pi with beta) works with it.  Lowest priority of the mask; `mhit` is not used.  The table holds
  * PHT_UNIF_CAP = 4096 powers (33 MB at n = 32): an observation whose lambda y (or lambda (u - y)) needs more raises error
- * bit 256.  (Bit 32 stays unassigned.) */
+ * bit 256.  Delayed entry (left-truncated observations, pht_engine_set_entry) is this method's alone.  (Bit 32 stays
+ * unassigned.) */
 #define PHT_METHOD_UNIF 64
 #define PHT_MAX_PHASES  32
 
@@ -159,6 +160,25 @@ int pht_engine_pi_rows(pht_engine *e, int rows, double *out);
  * (left-censored); MHRS needs y > 0. */
 int pht_engine_set_upper(pht_engine *e, const double *upper_local);
 
+/* Delayed entry, also called left truncation (method 64 only): local observation k entered the study at age a_k because it
+ * was still working then (a component bought used, a patient enrolled at some age), so the sample holds only units with
+ * T > a_k and each contributes L_k / S(a_k).  entry_local holds one a per local observation, in the order of y_local; 0
+ * means no truncation (the results are those without entry ages, bit for bit); NULL clears the ages.  Every sweep draws,
+ * per observation with a > 0, the number M of units of its kind lost before a (M | theta ~ Geometric, P(M = k) =
+ * F(a)^k S(a)) and each lost unit's path given absorption in (0, a]; their start states, transitions and sojourns join
+ * the sweep statistics, which keeps the update conjugate (Dempster, Laird & Rubin 1977).  The observations' own paths
+ * are drawn as before.  Refused: NaN, +-inf, a < 0, a > y (a left-censored record, y = 0, takes no entry age), a call
+ * after the exchange windows are attached (every rank sets ages, or none, before), and a zbits above
+ * pht_choose_zbits(sum over the observations of max(y, u) + a).  That sum counts one ghost path per truncated observation;
+ * the fixed point holds at least 32 times it per sweep, so ghost time up to ~30 times one ghost per observation still
+ * fits, and beyond that error word 2 reports the overflow.  Error bit 1024:
+ * S(a) underflowed, or a ghost count above 2^20 (the model leaves almost no survival at that age).  It ends the run, and
+ * it is a draw: an observation whose S(a) at the chain's current theta is ~1e-6 raises it with probability
+ * exp(-2^20 S(a)) ~ 0.35 per sweep, so entry ages far in the model's tail (a unit entering long after nearly all of its
+ * kind have failed) can stop a chain mid-run even when early sweeps pass.  Refused for MHRS,
+ * ECS, DCS and the two MH variants. */
+int pht_engine_set_entry(pht_engine *e, const double *entry_local);
+
 /* run `nsweeps` Gibbs sweeps; row r of out (nsweeps x m, row-major) is the draw of sweep r.
  * out may be NULL (results stay on the device; fetch later with pht_engine_get_theta). */
 int pht_engine_run(pht_engine *e, int nsweeps, double *out);
@@ -168,7 +188,8 @@ int pht_engine_sync(pht_engine *e);
 /* measurement aid: write `bytes` of scratch (larger than L2) on the sweep stream before every sweep, so that no sweep
  * finds its observations in L2 from the previous one; 0 switches it off (default) */
 int pht_engine_set_l2_flush(pht_engine *e, unsigned long long bytes);
-/* device time in ms of the sweeps enqueued by the last pht_engine_enqueue (after sync) */
+/* device time in ms of the sweeps enqueued by the last pht_engine_enqueue (after sync): all of them, and the path kernels
+ * per sweep (with the ghost pass of delayed entry, pht_engine_set_entry; measured only without the CUDA graph) */
 int pht_engine_last_ms(pht_engine *e, float *total_ms, float *path_kernel_ms);
 
 /* parity hooks ------------------------------------------------------------- */
@@ -178,6 +199,10 @@ int pht_engine_sweep_stats(pht_engine *e, long long *N, long long *B, long long 
 /* per-observation statistics for local observations [first, first+count): B[count],
  * N[count*n*n] (int32), z[count*n]; same kernels, recording to memory instead of reducing */
 int pht_engine_paths(pht_engine *e, long first, long count, int *B, int *N, double *z);
+/* delayed entry (pht_engine_set_entry): the ghost counts M[count] of local observations [first, first+count) in upload
+ * order, and when B is not NULL all total = sum M ghost paths in (observation, ghost index) order: B[total],
+ * N[total*n*n] (int32), z[total*n]; same kernels as a sweep, recording to memory.  Without entry ages M is all zero. */
+int pht_engine_entry_paths(pht_engine *e, long first, long count, int *M, long total, int *B, int *N, double *z);
 /* override the spectral data the ECS/DCS kernels use (evals n, Q n*n, Qinv n*n); NULL restores the device solver;
  * refused for method 64, which uses none */
 int pht_engine_set_spectral(pht_engine *e, const double *evals, const double *Q, const double *Qinv);

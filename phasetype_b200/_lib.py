@@ -19,11 +19,11 @@ SYMBOLS = [
     "pht_engine_get_theta", "pht_engine_run", "pht_engine_enqueue", "pht_engine_sync", "pht_engine_last_ms",
     "pht_engine_sweep_stats", "pht_engine_paths", "pht_engine_set_spectral", "pht_engine_get_model",
     "pht_engine_counters", "pht_fp64_fma_rate", "pht_engine_set_l2_flush", "pht_engine_peer_handle", "pht_engine_peer_attach", "pht_engine_round_trace", "pht_engine_set_pi", "pht_engine_get_pi", "pht_engine_pi_rows",
-    "pht_engine_set_upper",
+    "pht_engine_set_upper", "pht_engine_set_entry", "pht_engine_entry_paths",
 ]
 PEER_HANDLE_BYTES = 128
 # method 64 (include/pht_b200.h PHT_METHOD_UNIF): the uniformisation path sampler; exact, right-, interval- and
-# left-censored observations, any sub-generator
+# left-censored observations, any sub-generator; delayed entry (Engine.set_entry) is this method's alone
 METHOD_UNIF = 64
 CNT_NAMES = ["paths", "attempts", "jumps", "dens_evals", "env_updates", "brent_evals", "arms_calls",
              "metrop_rejects", "nonfinite", "deferred", "tail_rounds", "errors", "launches", "ns_lane", "ns_tail", "ns_replay",
@@ -81,6 +81,8 @@ def lib():
     L.pht_engine_get_pi.argtypes = [C.c_void_p, _dp]
     L.pht_engine_pi_rows.argtypes = [C.c_void_p, C.c_int, _dp]
     L.pht_engine_set_upper.argtypes = [C.c_void_p, C.c_void_p]
+    L.pht_engine_set_entry.argtypes = [C.c_void_p, C.c_void_p]
+    L.pht_engine_entry_paths.argtypes = [C.c_void_p, C.c_long, C.c_long, _ip, C.c_long, C.c_void_p, C.c_void_p, C.c_void_p]
     L.pht_engine_peer_handle.argtypes = [C.c_void_p, C.c_void_p]
     L.pht_engine_peer_attach.argtypes = [C.c_void_p, C.c_void_p]
     _lib = L
@@ -235,6 +237,39 @@ class Engine:
         if not self.l_local:
             a = np.full(1, np.inf)           # an empty shard still takes part (never NULL, which clears)
         _check(lib().pht_engine_set_upper(self._h, a.ctypes.data))
+
+    def set_entry(self, a):
+        """Delayed entry, or left truncation (METHOD_UNIF only): a[k] is the age at which local observation k entered the
+        study (0: none; 0 <= a <= y); None clears the ages.  Each sweep then also draws, per truncated observation, the
+        units of its kind lost before entry and their paths.  Those paths end by a, so construct the engine with
+        sum_y_global = the sum of max(y, u) + a over all observations (or a zbits at most pht_choose_zbits of it)."""
+        if a is None:
+            _check(lib().pht_engine_set_entry(self._h, None))
+            return
+        v = np.ascontiguousarray(a, dtype=np.float64)
+        if v.shape != (self.l_local,):
+            raise EngineError("set_entry: %d entry ages for %d local observations" % (v.size, self.l_local))
+        if not self.l_local:
+            v = np.zeros(1)                  # an empty shard still takes part (never NULL, which clears)
+        _check(lib().pht_engine_set_entry(self._h, v.ctypes.data))
+
+    def entry_paths(self, first=0, count=None, paths=True):
+        """Ghost counts M (count,) of local observations [first, first + count) at the current parameters, and with paths
+        the ghost paths in (observation, ghost index) order: (M, B, N, z) with B (G,), N (G, n*n), z (G, n), G = M.sum()."""
+        n = self.n
+        count = self.l_local - first if count is None else count
+        M = np.zeros(max(int(count), 1), dtype=np.int32)
+        _check(lib().pht_engine_entry_paths(self._h, int(first), int(count), M, 0, None, None, None))
+        M = M[:int(count)]
+        if not paths:
+            return M
+        G = int(M.astype(np.int64).sum())
+        B = np.zeros(max(G, 1), dtype=np.int32); N = np.zeros(max(G, 1) * n * n, dtype=np.int32); z = np.zeros(max(G, 1) * n)
+        M2 = np.zeros(max(int(count), 1), dtype=np.int32)
+        _check(lib().pht_engine_entry_paths(self._h, int(first), int(count), M2, G, B.ctypes.data, N.ctypes.data, z.ctypes.data))
+        if not np.array_equal(M2[:int(count)], M):
+            raise EngineError("entry_paths: ghost counts changed between two calls at the same parameters")
+        return M, B[:G], N[:G * n * n].reshape(G, n * n), z[:G * n].reshape(G, n)
 
     def round_trace(self):
         """(48, 8) array: per tail round number, ns search / ns barrier / ns advance / sum of pending / sum of K / attempts run /

@@ -14,6 +14,7 @@
 #include <cstdarg>
 #include <cmath>
 #include <vector>
+#include <algorithm>
 #include <thread>
 #include <dlfcn.h>
 #include <unistd.h>
@@ -91,6 +92,13 @@ struct pht_engine {
     int iv_blocks[3] = { 0, 0, 0 };
     /* method 64: the uniformisation table (pht_unif.h) and the longest time span it must cover (max of y and of u - y) */
     double *d_unif = nullptr; double unif_tmax = 0.0;
+    /* method 64, delayed entry (pht_engine_set_entry): the ages in upload order (device and host), the truncated
+     * observations (a > 0) by decreasing a with their local indices, their ghost counts and offsets, the entry tables,
+     * the ghost counter, the scan's scratch and the ghost kernel's grid */
+    bool entry_set = false; std::vector<double> h_entry;
+    double *d_entry = nullptr, *d_ea = nullptr; uint32_t *d_eobs = nullptr; long n_trunc = 0;
+    unsigned *d_eM = nullptr; unsigned long long *d_eoff = nullptr, *d_enext = nullptr; double *d_etab = nullptr;
+    void *d_escan = nullptr; size_t escan_bytes = 0; int ghost_blocks = 0, count_blocks = 0;
     /* graph */
     cudaGraphExec_t graph_exec = nullptr; int graph_res_rows = -1; double *graph_res = nullptr;
     unsigned long long graph_launches = 0;      /* kernels one replay of the captured sweep launches */
@@ -228,12 +236,26 @@ static int enqueue_model(pht_engine *e, const UpdateParams &u) {
     return 0;
 }
 
+/* method 64 with entry ages: entry tables, ghost counts, their scan and the ghost paths of the truncated observations,
+ * reduced into the same statistics block (nothing is launched without truncated observations) */
+static int enqueue_entry(pht_engine *e, const UpdateParams &u, const SweepParams &p) {
+    if (!e->entry_set || e->n_trunc == 0) return 0;
+    UnifEntry E; memset(&E, 0, sizeof(E));
+    E.a = e->d_ea; E.obs = e->d_eobs; E.first = 0; E.count = e->n_trunc; E.M = e->d_eM; E.off = e->d_eoff;
+    E.etab = e->d_etab; E.next = e->d_enext; E.scan_tmp = e->d_escan; E.scan_bytes = e->escan_bytes;
+    E.count_blocks = e->count_blocks;
+    CU(pht_launch_unif_entry(u, p, e->d_unif, E, e->ghost_blocks, PHT_ENTRY_COUNTS | PHT_ENTRY_GHOSTS, e->stream));
+    e->launches += 5;
+    return 0;
+}
+
 static int enqueue_sweep(pht_engine *e, double *res, int res_rows, bool time_kernel) {
     UpdateParams u = update_params(e, res, res_rows);
     if (enqueue_model(e, u)) return -1;
     SweepParams p = sweep_params(e);
     if (time_kernel && e->kev_used + 2 <= (int)e->kev.size()) CU(cudaEventRecord(e->kev[e->kev_used++], e->stream));
     if (enqueue_paths(e, p)) return -1;
+    if (enqueue_entry(e, u, p)) return -1;          /* the ghost pass is path work: inside the path-kernel timing */
     if (time_kernel && (e->kev_used & 1)) CU(cudaEventRecord(e->kev[e->kev_used++], e->stream));
     if (e->peer_reduce) {
         ReduceParams r; memset(&r, 0, sizeof(r));
@@ -271,7 +293,7 @@ extern "C" void pht_engine_destroy(pht_engine *e) {
     if (e->ev1) cudaEventDestroy(e->ev1);
     for (void *q : e->ipc_opened) cudaIpcCloseMemHandle(q);
     stage("events, ipc");
-    void *big[] = { e->d_unif, e->d_u, e->d_us, e->d_item_u, e->d_recs, e->d_ys, e->d_cs, e->d_perm, e->d_y, e->d_cens, e->d_items /* arena: found, pend0, pend1, done live inside */, e->d_idx_exact, e->d_idx_cens,
+    void *big[] = { e->d_entry, e->d_ea, e->d_eobs, e->d_eM, e->d_eoff, e->d_enext, e->d_etab, e->d_escan, e->d_unif, e->d_u, e->d_us, e->d_item_u, e->d_recs, e->d_ys, e->d_cs, e->d_perm, e->d_y, e->d_cens, e->d_items /* arena: found, pend0, pend1, done live inside */, e->d_idx_exact, e->d_idx_cens,
                     e->d_glist, e->d_model, e->d_stats, e->d_state, e->d_T, e->d_C, e->d_nu, e->d_zeta, e->d_var_ptr, e->d_cell_i, e->d_cell_j, e->d_pires, e->d_res };
     for (void *b : big) pht_dev_free(b, e->stream);
     if (e->stream) cudaStreamSynchronize(e->stream);
@@ -507,13 +529,15 @@ extern "C" int pht_engine_comm_init(pht_engine *e, const void *id128) {
 
 /* ---------------------------------------------------------------- peer exchange windows (MHRS global tail) */
 struct PeerHandle { unsigned long long pid; unsigned long long ptr; int device; int valid; cudaIpcMemHandle_t ipc; unsigned long long cfg_hash; };
-/* what every rank of a run must agree on (the chain is one chain): key, shape, sampler, fixed-point scale, world size, and
- * whether interval bounds are set (a global tail round searches every rank's items with one kernel instance) */
+/* what every rank of a run must agree on (the chain is one chain): key, shape, sampler, fixed-point scale, world size,
+ * whether interval bounds are set (a global tail round searches every rank's items with one kernel instance) and whether
+ * entry ages are set */
 static unsigned long long cfg_hash(const pht_engine *e) {
     const pht_config &c = e->cfg;
     unsigned long long h = 0xcbf29ce484222325ULL;
     const unsigned long long v[] = { c.seed, (unsigned long long)c.n, (unsigned long long)c.m, (unsigned long long)c.method, (unsigned long long)c.mhit,
-                                     (unsigned long long)c.zbits, (unsigned long long)c.world, e->d_u ? 1ull : 0ull };
+                                     (unsigned long long)c.zbits, (unsigned long long)c.world, e->d_u ? 1ull : 0ull,
+                                     e->entry_set ? 1ull : 0ull };
     for (unsigned long long x : v) for (int b = 0; b < 8; b++) { h ^= (x >> (8 * b)) & 0xffull; h *= 0x100000001b3ULL; }
     return h;
 }
@@ -540,7 +564,7 @@ extern "C" int pht_engine_peer_attach(pht_engine *e, const void *handles) {
     for (int r = 0; r < e->cfg.world; r++) {
         PeerHandle h; memcpy(&h, (const char *)handles + (size_t)r * PHT_PEER_HANDLE_BYTES, sizeof(h));
         if (!h.valid) return fail("rank %d offers no exchange window", r);
-        if (h.cfg_hash != cfg_hash(e)) return fail("rank %d runs a different configuration (seed, n, m, method, mhit, zbits, world or the presence of interval bounds differ from rank %d's): the ranks of a run share one chain", r, e->cfg.rank);
+        if (h.cfg_hash != cfg_hash(e)) return fail("rank %d runs a different configuration (seed, n, m, method, mhit, zbits, world or the presence of interval bounds or of entry ages differ from rank %d's): the ranks of a run share one chain", r, e->cfg.rank);
         if (r == e->cfg.rank) { e->xpeer[r] = e->d_xw; continue; }
         if (h.pid == (unsigned long long)getpid()) {
             /* same process (one host thread per GPU): the peer's pointer is valid here once peer access is on */
@@ -670,8 +694,9 @@ extern "C" int pht_engine_set_upper(pht_engine *e, const double *upper_local) {
         if (u - y[(size_t)i] > tmax) tmax = u - y[(size_t)i];
         sum += u;
     }
+    for (double a : e->h_entry) sum += a;           /* ghost paths of delayed-entry observations (pht_engine_set_entry) */
     if (sum > 0.0 && e->cfg.zbits > pht_choose_zbits(sum))
-        return fail("zbits = %d is too fine for these bounds: interval paths end by u, and sum of max(y, u) = %g allows at most %d",
+        return fail("zbits = %d is too fine for these bounds: interval paths end by u, and sum of max(y, u) (plus the entry ages, when set) = %g allows at most %d",
                     e->cfg.zbits, sum, pht_choose_zbits(sum));
     const size_t ln = (size_t)(l > 0 ? l : 1);
     if (unif) e->unif_tmax = tmax;
@@ -688,6 +713,137 @@ extern "C" int pht_engine_set_upper(pht_engine *e, const double *upper_local) {
     }
     CU(cudaStreamSynchronize(e->stream));
     return 0;
+}
+
+static int entry_free(pht_engine *e) {
+    void *bufs[] = { e->d_entry, e->d_ea, e->d_eobs, e->d_eM, e->d_eoff, e->d_enext, e->d_etab, e->d_escan };
+    for (void *b : bufs) CU(pht_dev_free(b, e->stream));
+    e->d_entry = e->d_ea = e->d_etab = nullptr; e->d_eobs = nullptr; e->d_eM = nullptr; e->d_eoff = e->d_enext = nullptr;
+    e->d_escan = nullptr; e->escan_bytes = 0; e->n_trunc = 0;
+    e->entry_set = false; e->h_entry.clear();
+    CU(cudaStreamSynchronize(e->stream));
+    return 0;
+}
+
+extern "C" int pht_engine_set_entry(pht_engine *e, const double *entry_local) {
+    if (!e) return fail("null engine");
+    if (method_of(e->cfg) != PHT_METHOD_UNIF)
+        return fail("delayed entry (entry ages, left truncation) needs method 64: the units lost before entry are drawn as left-censored paths of the uniformisation sampler");
+    CU(cudaSetDevice(e->cfg.device));
+    CU(cudaStreamSynchronize(e->stream));
+    if (e->peers_attached) return fail("the entry ages of a multi-rank run are set on every rank before the exchange windows are attached");
+    if (e->graph_exec) { cudaGraphExecDestroy(e->graph_exec); e->graph_exec = nullptr; }     /* the sweep changes shape */
+    if (!entry_local) return entry_free(e);
+    const long l = e->l_local;
+    const size_t ln = (size_t)(l > 0 ? l : 1);
+    std::vector<double> y(ln), u(ln, INFINITY);
+    if (l > 0) {
+        CU(cudaMemcpy(y.data(), e->d_y, sizeof(double) * (size_t)l, cudaMemcpyDeviceToHost));
+        if (e->d_u) CU(cudaMemcpy(u.data(), e->d_u, sizeof(double) * (size_t)l, cudaMemcpyDeviceToHost));
+    }
+    /* ghost paths end by their entry age: the fixed-point scale must leave room for sum of max(y, u) + a */
+    double sum = 0.0;
+    std::vector<uint32_t> trunc;
+    for (long i = 0; i < l; i++) {
+        const double a = entry_local[i], yi = y[(size_t)i], ui = u[(size_t)i];
+        if (!std::isfinite(a)) return fail("entry[%ld] = %g: an entry age must be finite", i, a);
+        if (a < 0.0) return fail("entry[%ld] = %g is negative", i, a);
+        if (a > yi) return fail("entry[%ld] = %g is above y = %g: a unit enters before its failure or censoring time (a left-censored record, y = 0, takes no entry age)", i, a, yi);
+        sum += (ui < INFINITY && ui > yi ? ui : yi) + a;
+        if (a > 0.0) trunc.push_back((uint32_t)i);
+    }
+    if (sum > 0.0 && e->cfg.zbits > pht_choose_zbits(sum))
+        return fail("zbits = %d is too fine for these entry ages: ghost paths end by a, and sum of max(y, u) + a = %g allows at most %d",
+                    e->cfg.zbits, sum, pht_choose_zbits(sum));
+    if (!e->ghost_blocks) {
+        e->ghost_blocks = pht_unif_ghost_grid_blocks(e->cfg.device, e->cfg.n);
+        if (e->ghost_blocks <= 0) { e->ghost_blocks = 0; return fail("the ghost-path kernel does not fit on the device: %s", cudaGetErrorString(cudaGetLastError())); }
+        int sms = 0;
+        CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, e->cfg.device));
+        e->count_blocks = 8 * sms;                   /* the count kernel is grid-stride: 8 blocks of 256 per SM */
+    }
+    if (entry_free(e)) return -1;
+    /* the truncated observations by decreasing a (ties by index), so that the lanes of a warp run similar truncations */
+    std::stable_sort(trunc.begin(), trunc.end(), [&](uint32_t i, uint32_t j) { return entry_local[i] > entry_local[j]; });
+    const long nt = (long)trunc.size();
+    std::vector<double> ea((size_t)(nt > 0 ? nt : 1));
+    for (long k = 0; k < nt; k++) ea[(size_t)k] = entry_local[trunc[(size_t)k]];
+    CU(pht_dev_alloc((void **)&e->d_entry, ln * sizeof(double), e->stream));
+    CU(pht_dev_alloc((void **)&e->d_ea, ea.size() * sizeof(double), e->stream));
+    CU(pht_dev_alloc((void **)&e->d_eobs, ea.size() * sizeof(uint32_t), e->stream));
+    CU(pht_dev_alloc((void **)&e->d_eM, (size_t)(nt + 1) * sizeof(unsigned), e->stream));
+    CU(pht_dev_alloc((void **)&e->d_eoff, (size_t)(nt + 1) * sizeof(unsigned long long), e->stream));
+    CU(pht_dev_alloc((void **)&e->d_enext, sizeof(unsigned long long), e->stream));
+    CU(pht_dev_alloc((void **)&e->d_etab, 2 * PHT_UNIF_CAP * sizeof(double), e->stream));
+    e->escan_bytes = pht_unif_entry_scan_bytes(nt);
+    CU(pht_dev_alloc(&e->d_escan, e->escan_bytes ? e->escan_bytes : 1, e->stream));
+    if (l > 0) CU(cudaMemcpyAsync(e->d_entry, entry_local, sizeof(double) * (size_t)l, cudaMemcpyHostToDevice, e->stream));
+    if (nt > 0) {
+        CU(cudaMemcpyAsync(e->d_ea, ea.data(), sizeof(double) * (size_t)nt, cudaMemcpyHostToDevice, e->stream));
+        CU(cudaMemcpyAsync(e->d_eobs, trunc.data(), sizeof(uint32_t) * (size_t)nt, cudaMemcpyHostToDevice, e->stream));
+    }
+    CU(cudaStreamSynchronize(e->stream));
+    e->h_entry.assign(entry_local, entry_local + l);
+    e->n_trunc = nt; e->entry_set = true;
+    return 0;
+}
+
+extern "C" int pht_engine_entry_paths(pht_engine *e, long first, long count, int *M, long total, int *B, int *N, double *z) {
+    if (!e || !M) return fail("null argument");
+    if (method_of(e->cfg) != PHT_METHOD_UNIF) return fail("delayed entry (entry ages, left truncation) needs method 64");
+    if (first < 0 || count < 0 || first + count > e->l_local) return fail("range [%ld, %ld) outside the shard", first, first + count);
+    if (B && (!N || !z)) return fail("null argument");
+    if (count == 0 || !e->entry_set) {
+        for (long i = 0; i < count; i++) M[i] = 0;
+        if (B && total != 0) return fail("%ld ghost paths asked, the window has none (no entry ages set)", total);
+        return 0;
+    }
+    CU(cudaSetDevice(e->cfg.device));
+    const int n = e->cfg.n;
+    unsigned *dM = nullptr; unsigned long long *doff = nullptr; void *tmp = nullptr;
+    int *dB = nullptr, *dN = nullptr; double *dz = nullptr;
+    int rc = -1;
+#define CUP(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { fail("%s failed: %s (%s:%d)", #call, cudaGetErrorString(e_), __FILE__, __LINE__); goto out; } } while (0)
+    {
+        UnifEntry E; memset(&E, 0, sizeof(E));
+        E.scan_bytes = pht_unif_entry_scan_bytes(count);
+        CUP(cudaMalloc(&dM, sizeof(unsigned) * (count + 1))); CUP(cudaMalloc(&doff, sizeof(unsigned long long) * (count + 1)));
+        CUP(cudaMalloc(&tmp, E.scan_bytes ? E.scan_bytes : 1));
+        /* the window in upload order: entry ages d_entry[first + i], local observation first + i */
+        E.a = e->d_entry + first; E.obs = nullptr; E.first = first; E.count = count; E.M = dM; E.off = doff;
+        E.etab = e->d_etab; E.next = e->d_enext; E.scan_tmp = tmp; E.count_blocks = e->count_blocks;
+        UpdateParams u = update_params(e, nullptr, 0);
+        if (enqueue_model(e, u)) goto out;
+        SweepParams p = sweep_params(e);
+        CUP(pht_launch_unif_entry(u, p, e->d_unif, E, e->ghost_blocks, PHT_ENTRY_COUNTS, e->stream));
+        if (pht_engine_sync(e)) goto out;
+        std::vector<unsigned> hM((size_t)count);
+        unsigned long long G = 0;
+        CUP(cudaMemcpy(hM.data(), dM, sizeof(unsigned) * count, cudaMemcpyDeviceToHost));
+        CUP(cudaMemcpy(&G, doff + count, sizeof(G), cudaMemcpyDeviceToHost));
+        for (long i = 0; i < count; i++) M[i] = (int)hM[(size_t)i];
+        if (B) {
+            if ((unsigned long long)total != G) { fail("total = %ld, but the window's ghost counts sum to %llu", total, G); goto out; }
+            if (G > 0) {
+                CUP(cudaMalloc(&dB, sizeof(int) * G)); CUP(cudaMalloc(&dN, sizeof(int) * G * n * n)); CUP(cudaMalloc(&dz, sizeof(double) * G * n));
+                CUP(cudaMemsetAsync(dN, 0, sizeof(int) * G * n * n, e->stream));
+                p.outB = dB; p.outN = dN; p.outz = dz; p.first = 0; p.count = (long)G;
+                CUP(pht_launch_unif_entry(u, p, e->d_unif, E, e->ghost_blocks, PHT_ENTRY_GHOSTS, e->stream));
+                if (pht_engine_sync(e)) goto out;
+                CUP(cudaMemcpy(B, dB, sizeof(int) * G, cudaMemcpyDeviceToHost));
+                CUP(cudaMemcpy(N, dN, sizeof(int) * G * n * n, cudaMemcpyDeviceToHost));
+                CUP(cudaMemcpy(z, dz, sizeof(double) * G * n, cudaMemcpyDeviceToHost));
+            }
+        }
+        rc = 0;
+    }
+#undef CUP
+out:
+    cudaFree(dM); cudaFree(doff); cudaFree(tmp);
+    if (dB) cudaFree(dB);
+    if (dN) cudaFree(dN);
+    if (dz) cudaFree(dz);
+    return rc;
 }
 
 static int ensure_res(pht_engine *e, int rows) {
@@ -744,7 +900,7 @@ static int check_state(pht_engine *e) {
         int err = st.error;
         cudaMemsetAsync(&e->d_state->error, 0, sizeof(int), e->stream);
         cudaStreamSynchronize(e->stream);
-        return fail("device error word 0x%x (%s%s%s%s%s%s%s%s%s)", err, (err & 2) ? "sojourn total overflows the fixed-point range (lower PHT_B200_ZBITS); " : "",
+        return fail("device error word 0x%x (%s%s%s%s%s%s%s%s%s%s)", err, (err & 2) ? "sojourn total overflows the fixed-point range (lower PHT_B200_ZBITS); " : "",
                     (err & 4) ? "MHRS tail list overflow; " : "",
                     (err & 8) ? "an observation's survival probability is too small for rejection sampling (more than 4e9 attempts); " : "",
                     (err & 16) ? "(unused) " : "",
@@ -752,7 +908,8 @@ static int check_state(pht_engine *e) {
                     (err & 64) ? "a peer GPU did not arrive at a barrier of the global MHRS tail; " : "",
                     (err & 128) ? "another rank of the run raised its error word; " : "",
                     (err & PHT_UNIF_ERR_TABLE) ? "the uniformisation sampler needs more powers of R than its table holds (a stiff generator or a very long y); " : "",
-                    (err & PHT_UNIF_ERR_ZERO) ? "every weight of a uniformisation draw underflowed to zero; " : "");
+                    (err & PHT_UNIF_ERR_ZERO) ? "every weight of a uniformisation draw underflowed to zero; " : "",
+                    (err & PHT_UNIF_ERR_ENTRY) ? "the model leaves (almost) no survival at an observation's entry age: S(a) underflowed or more than 2^20 units would have been lost before entry; " : "");
     }
     return 0;
 }
@@ -799,6 +956,7 @@ extern "C" int pht_engine_sweep_stats(pht_engine *e, long long *N, long long *B,
     if (enqueue_model(e, u)) return -1;
     SweepParams p = sweep_params(e);
     if (enqueue_paths(e, p)) return -1;
+    if (enqueue_entry(e, u, p)) return -1;
     if (pht_engine_sync(e)) return -1;
     std::vector<long long> h(stats_len(n));
     CU(cudaMemcpy(h.data(), e->d_stats, sizeof(long long) * h.size(), cudaMemcpyDeviceToHost));

@@ -7,6 +7,9 @@
  *   unif[]          fp64   method 64 only: the uniformisation table (pht_unif.h; 33 MB at n = 32)
  *   u[l_local]      fp64   MHRS and method 64 only, when interval bounds are set (pht_engine_set_upper): upper bound of each
  *                          censored observation's absorption time, +inf = none; a copy in the decreasing-y layout
+ *   entry[]         fp64   method 64 only, when entry ages are set (pht_engine_set_entry): a per observation in upload
+ *                          order; the truncated ones (a > 0) as a list by decreasing a with their local indices, ghost
+ *                          counts and offsets; the entry tables (2 x PHT_UNIF_CAP)
  *   model[]         fp64   the per-sweep model block, offsets from ModelLayout (< 70 KB at n = 32);
  *                          rebuilt on the device every sweep, copied to shared memory by the path kernels
  *   stats[]         int64  N (n*n) | B (n) | z fixed point in two limbs (2n) | error count: the only data that crosses NVLink
@@ -194,6 +197,22 @@ size_t pht_unif_table_doubles(int n, int cap);
 cudaError_t pht_launch_unif_table(const UpdateParams &p, double *tab, double tmax, cudaStream_t st);
 cudaError_t pht_launch_unif(const SweepParams &p, const double *tab, int grid_blocks, cudaStream_t st);
 int pht_unif_grid_blocks(int device, int n);
+/* method 64, delayed entry (k_unif.cu; pht_engine_set_entry): a list of observations with entry ages and its buffers.
+ * Like the table, every pointer is a kernel argument of its own. */
+struct UnifEntry {
+    const double *a; const uint32_t *obs; long first, count;   /* entry age per list entry; local observation index
+                                                                  (obs == nullptr: first + i) */
+    unsigned *M; unsigned long long *off;                      /* ghost counts and their exclusive scan, count + 1 each */
+    double *etab; unsigned long long *next;                    /* sigma_k | phi_k (2 x PHT_UNIF_CAP); ghost hand-out counter */
+    void *scan_tmp; size_t scan_bytes;                         /* CUB scratch of the scan */
+    int count_blocks;                                          /* grid of the (grid-stride) count kernel at most */
+};
+#define PHT_ENTRY_COUNTS 1     /* entry tables, ghost counts, scan */
+#define PHT_ENTRY_GHOSTS 2     /* the ghost paths */
+cudaError_t pht_launch_unif_entry(const UpdateParams &u, const SweepParams &p, const double *tab, const UnifEntry &E, int ghost_blocks,
+                                  int stages, cudaStream_t st);
+size_t pht_unif_entry_scan_bytes(long count);
+int pht_unif_ghost_grid_blocks(int device, int n);
 /* large per-call buffers: stream-ordered pool allocations, cached across calls (engine.cu) */
 cudaError_t pht_dev_alloc(void **p, size_t bytes, cudaStream_t st);
 cudaError_t pht_dev_free(void *p, cudaStream_t st);

@@ -12,10 +12,19 @@
  *                  per-lane n-vectors of scratch live in shared-memory slabs (stride THREADS), the powers in global
  *                  memory (33 MB at n = 32 and full capacity; what a sweep touches stays in L2).
  *
+ * Delayed entry (only when entry ages are set, pht_engine_set_entry; law and draw order in pht_unif.h):
+ *   k_unif_entry_table  sigma_k, phi_k for k <= K_sweep, after k_unif_table (one block)
+ *   k_unif_entry_count  the ghost count M of every truncated observation, walked by decreasing a; then an exclusive
+ *                       CUB scan of the counts (64-bit offsets) leaves the total G in device memory
+ *   k_unif_ghosts       persistent warps over the flat ghost indices [0, G), one left-censored path per lane,
+ *                       reduced into the same statistics block
+ *
  * Bound: FP64 issue.  Per observation the sampler evaluates ~3 K(lambda y) Poisson weights (one pht_exp each) and
  * ~K(lambda y) n multiply-adds for the end-state weights, plus n per uniformised event; the observations are handed out
  * by decreasing y (k_sort.cu), so the lanes of a warp run similar K.
  */
+#include <cub/device/device_scan.cuh>
+#include <cuda/std/functional>
 #include "path_common.cuh"
 
 /* one out-of-line uniform: the sampler draws at a dozen places of a divergent body */
@@ -131,6 +140,137 @@ __global__ void __launch_bounds__(THREADS) k_unif_paths(SweepParams p, const dou
     unsigned long long w_paths = c_paths;
     for (int o = 16; o > 0; o >>= 1) w_paths += __shfl_down_sync(FULL, w_paths, o);
     if ((tid & 31) == 0) atomicAdd(&p.state->counters[PHT_CNT_PATHS], w_paths);
+}
+
+/* ---- delayed entry (pht_unif.h, "Delayed entry"): launched only when entry ages are set */
+
+/* sigma_k and phi_k for k <= K_sweep, after k_unif_table; one block */
+__global__ void __launch_bounds__(UNIF_TABLE_THREADS) k_unif_entry_table(UpdateParams p, const double *tab, double *etab) {
+    const int n = p.n, cap = PHT_UNIF_CAP;
+    const ModelLayout ML = ModelLayout::make(n, p.m);
+    const pht_unif_layout L = pht_unif_layout_make(n, cap);
+    const double *pi = p.model + ML.pi;
+    const int K = (int)tab[1];
+    for (int k = threadIdx.x; k <= K; k += blockDim.x) {
+        etab[k] = pht_unif_sigma_entry(n, tab + L.q + k * n);
+        etab[cap + k] = pht_unif_phi_entry(n, pi, tab + L.g + k * n);
+    }
+}
+
+/* the ghost count of every entry of a list (a[i], local observation obs[i], or first + i when obs is null); M[count] = 0
+ * closes the list for the scan */
+__global__ void __launch_bounds__(256) k_unif_entry_count(SweepParams p, const double *tab, const double *etab, const double *a,
+                                                        const uint32_t *obs, long first, long count, unsigned *M) {
+    const uint32_t iter = p.state->iter;
+    int err = 0;
+    for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i <= count; i += (long)gridDim.x * blockDim.x) {
+        unsigned m = 0u;
+        if (i < count && a[i] > 0.0) {
+            const uint32_t ol = obs ? obs[i] : (uint32_t)(first + i);
+            const double U = pht_unif_at(p.k0, p.k1, iter, p.obs_rank + ol * p.obs_world, 1u, 0u);
+            err |= pht_unif_ghost_count(tab, etab, p.n, PHT_UNIF_CAP, a[i], U, &m);
+        }
+        M[i] = m;
+    }
+    if (err) atomicOr(&p.state->error, err);
+}
+
+/* Ghost paths.  Persistent warps take 32 flat ghost indices g in [0, G) at a time (G = off[count], on the device) and
+ * map each to (list entry i, ghost j): a binary search for the chunk's first index, then per lane a galloping search
+ * from there over the entries with no ghosts.  Each lane runs the shared sampler (y = 0, censored, u = a on sub-stream
+ * 2 + j) and reduces the path into the sweep statistics like k_unif_paths; in parity mode (p.outB) ghost g is record g. */
+template <int THREADS>
+__global__ void __launch_bounds__(THREADS) k_unif_ghosts(SweepParams p, const double *tab, const double *a, const uint32_t *obs,
+                                                         long first, long count, const unsigned long long *off,
+                                                         unsigned long long *next) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const int n = p.n, tid = threadIdx.x, lane = tid & 31;
+    const unsigned FULL = 0xffffffffu;
+    const ModelLayout ML = ModelLayout::make(n, p.m);
+    UnifSmem<THREADS> sm; sm.carve(smem_raw, n);
+    for (int i = tid; i < n * n; i += THREADS) sm.Nacc[i] = 0u;
+    for (int i = tid; i < (n + 1) * (n + 1); i += THREADS) sm.cum[i] = p.model[ML.cum + i];
+    for (int i = tid; i < n; i += THREADS) {
+        sm.s[i] = p.model[ML.s + i]; sm.scale[i] = p.model[ML.scale + i]; sm.pi[i] = p.model[ML.pi + i];
+        sm.zlo[i] = 0ull; sm.zhi[i] = 0; sm.Bacc[i] = 0u;
+    }
+    __syncthreads();
+    const uint32_t iter = p.state->iter;
+    const unsigned long long G = off[count];
+    int err = 0;
+    UnifCount ctx; ctx.p = &p; ctx.Nacc = sm.Nacc; ctx.n = n; ctx.out_idx = 0;
+    for (;;) {
+        unsigned long long base = 0;
+        if (lane == 0) base = atomicAdd(next, (unsigned long long)PATH_CHUNK);
+        base = __shfl_sync(FULL, base, 0);
+        if (base >= G) break;
+        long lo = 0, hi = count;                       /* the entry holding ghost `base`: off[lo] <= base < off[lo + 1] */
+        while (hi - lo > 1) { const long mid = (lo + hi) >> 1; if (off[mid] <= base) lo = mid; else hi = mid; }
+        const unsigned long long g = base + (unsigned long long)lane;
+        if (g < G) {
+            long i = lo;
+            if (off[i + 1] <= g) {                     /* off[count] = G > g bounds the search */
+                long l0 = i, h0 = i, step = 1;
+                for (;;) {
+                    h0 = i + step;
+                    if (h0 >= count - 1) { h0 = count - 1; break; }
+                    if (off[h0 + 1] > g) break;
+                    l0 = h0; step <<= 1;
+                }
+                while (h0 - l0 > 1) { const long mid = (l0 + h0) >> 1; if (off[mid + 1] > g) h0 = mid; else l0 = mid; }
+                i = h0;
+            }
+            const uint32_t ol = obs ? obs[i] : (uint32_t)(first + i);
+            pht_stream st; st.k0 = p.k0; st.k1 = p.k1;
+            pht_stream_seek(&st, iter, p.obs_rank + ol * p.obs_world, 2u + (uint32_t)(g - off[i]), 0u);
+            ctx.out_idx = (long)g;
+            int B = 0;
+            err |= pht_unif_path(tab, n, PHT_UNIF_CAP, sm.s, sm.scale, sm.cum, sm.pi, 0.0, 1, a[i], &st,
+                                 sm.Za + tid, sm.Zb + tid, THREADS, &ctx, &B);
+            path_flush<THREADS>(p, n, sm.Za, sm.zlo, sm.zhi, sm.Bacc, B, ctx.out_idx);
+        }
+        __syncwarp();
+    }
+    if (err) atomicOr(&p.state->error, err);
+    __syncthreads();
+    block_flush<THREADS>(p, n, sm.Nacc, sm.Bacc, sm.zlo, sm.zhi);
+}
+
+size_t pht_unif_entry_scan_bytes(long count) {
+    size_t bytes = 0;
+    cub::DeviceScan::ExclusiveScan(nullptr, bytes, (const unsigned *)nullptr, (unsigned long long *)nullptr, cuda::std::plus<>(),
+                                   0ull, count + 1);
+    return bytes;
+}
+
+int pht_unif_ghost_grid_blocks(int device, int n) {
+    const size_t smem = UnifSmem<UNIF_THREADS>::bytes(n);
+    int per_sm = 0, sms = 0;
+    if (cudaFuncSetAttribute(k_unif_ghosts<UNIF_THREADS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return -1;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_unif_ghosts<UNIF_THREADS>, UNIF_THREADS, smem) != cudaSuccess) return -1;
+    if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device) != cudaSuccess) return -1;
+    return per_sm * sms;
+}
+
+cudaError_t pht_launch_unif_entry(const UpdateParams &u, const SweepParams &p, const double *tab, const UnifEntry &E, int ghost_blocks,
+                                  int stages, cudaStream_t st) {
+    if (stages & PHT_ENTRY_COUNTS) {
+        k_unif_entry_table<<<1, UNIF_TABLE_THREADS, 0, st>>>(u, tab, E.etab);
+        long blocks = (E.count + 1 + 255) / 256;
+        if (blocks > E.count_blocks) blocks = E.count_blocks;
+        k_unif_entry_count<<<(unsigned)blocks, 256, 0, st>>>(p, tab, E.etab, E.a, E.obs, E.first, E.count, E.M);
+        size_t bytes = E.scan_bytes;
+        const cudaError_t e = cub::DeviceScan::ExclusiveScan(E.scan_tmp, bytes, (const unsigned *)E.M, E.off, cuda::std::plus<>(),
+                                                             0ull, E.count + 1, st);
+        if (e != cudaSuccess) return e;
+    }
+    if (stages & PHT_ENTRY_GHOSTS) {
+        const cudaError_t e = cudaMemsetAsync(E.next, 0, sizeof(unsigned long long), st);
+        if (e != cudaSuccess) return e;
+        k_unif_ghosts<UNIF_THREADS><<<ghost_blocks, UNIF_THREADS, UnifSmem<UNIF_THREADS>::bytes(p.n), st>>>(
+            p, tab, E.a, E.obs, E.first, E.count, E.off, E.next);
+    }
+    return cudaGetLastError();
 }
 
 cudaError_t pht_unif_init(double *tab, int n, int cap, cudaStream_t st) {

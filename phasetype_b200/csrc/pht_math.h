@@ -199,4 +199,52 @@ PHT_HD double pht_log(double x) {
     return pht_log_core(ux, 0);
 }
 
+/* log(1 + x), fdlibm's s_log1p.c on the polynomial of pht_log (its Lp1..Lp7 are the Lg1..Lg7 above).
+ * Fast path: 1 + x in [sqrt(1/2), sqrt(2)), i.e. x in [-0.2929, 0.4142): f = x exactly and no reduction.  The general
+ * path takes every x: on the fast range it computes what the fast path computes; elsewhere it reduces u = 1 + x to
+ * 2^k m like pht_log and carries the rounding of u as the correction c = (x - (u - 1)) / u (also where the reduction
+ * gives k = 0, at the edges of the fast range, which fdlibm drops). */
+#define PHT_LOG1P_LO (-0.2928932188134524)        /* sqrt(1/2) - 1 */
+#define PHT_LOG1P_HI 0.41421356237309503          /* sqrt(2) - 1 */
+PHT_HD double pht_log1p_poly(double f, double *hfsq, double *s) {
+    *hfsq = 0.5 * f * f;
+    *s = f / (2.0 + f);
+    const double z = *s * *s;
+    const double w = z * z;
+    const double t1 = w * PHT_FMA(w, PHT_FMA(w, PHT_LC(5), PHT_LC(3)), PHT_LC(1));
+    const double t2 = z * PHT_FMA(w, PHT_FMA(w, PHT_FMA(w, PHT_LC(6), PHT_LC(4)), PHT_LC(2)), PHT_LC(0));
+    return t2 + t1;
+}
+PHT_SLOW double pht_log1p_general(double x) {
+    if (!(x == x)) return x + x;                                  /* NaN */
+    if (x < -1.0) return pht_u2d(0x7ff8000000000000ULL);
+    if (x == -1.0) return -pht_u2d(0x7ff0000000000000ULL);
+    if (x == pht_u2d(0x7ff0000000000000ULL)) return x;
+    const double LN2_HI = 6.93147180369123816490e-01;
+    const double LN2_LO = 1.90821492927058770002e-10;
+    double hfsq, s;
+    if (x >= PHT_LOG1P_LO && x < PHT_LOG1P_HI) {
+        const double R = pht_log1p_poly(x, &hfsq, &s);
+        return x - (hfsq - s * (hfsq + R));
+    }
+    const double u = x < 9007199254740992.0 ? 1.0 + x : x;         /* beyond 2^53, 1 + x rounds to x: no correction */
+    const uint64_t uu = pht_d2u(u);
+    uint32_t hu = (uint32_t)(uu >> 32);
+    int k = (int)(hu >> 20) - 1023;
+    const double c = x < 9007199254740992.0 ? (k > 0 ? 1.0 - (u - x) : x - (u - 1.0)) / u : 0.0;
+    hu &= 0x000fffffu;
+    if (hu < 0x6a09eu) hu |= 0x3ff00000u;                          /* mantissa in [1, sqrt(2)) */
+    else { k += 1; hu |= 0x3fe00000u; }                              /* in [sqrt(1/2), 1) */
+    const double f = pht_u2d(((uint64_t)hu << 32) | (uu & 0xffffffffULL)) - 1.0;
+    const double R = pht_log1p_poly(f, &hfsq, &s);
+    const double dk = (double)k;
+    return dk * LN2_HI - ((hfsq - (s * (hfsq + R) + (dk * LN2_LO + c))) - f);
+}
+PHT_HD double pht_log1p(double x) {
+    if (!(x >= PHT_LOG1P_LO && x < PHT_LOG1P_HI)) return pht_log1p_general(x);
+    double hfsq, s;
+    const double R = pht_log1p_poly(x, &hfsq, &s);
+    return x - (hfsq - s * (hfsq + R));
+}
+
 #endif /* PHT_MATH_H */

@@ -116,6 +116,59 @@ PHT_HD int pht_unif_pick(const double *w, int n, int ws, double U) {
     return last;
 }
 
+/* Delayed entry (left truncation; pht_engine_set_entry).  A unit seen only because it survived to its entry age a > 0
+ * contributes L / S(a).  The augmentation of Dempster, Laird & Rubin (1977) keeps the sweep conjugate: per truncated
+ * observation, M units of the same kind lost before a ("ghosts"), M | theta ~ Geometric with P(M = k) = F(a)^k S(a),
+ * F = 1 - S, and each ghost's whole path given absorption in (0, a] -- the left-censored path (y = 0, u = a) of
+ * pht_unif_path.  Summing F(a)^M over M gives 1 / S(a), so the theta-marginal is prior x prod L_i / S(a_i).
+ * Entry tables (a buffer of their own, 2 x capacity doubles, filled per sweep for k <= K_sweep; a <= y, so K_sweep
+ * covers lambda a):
+ *     sigma_k = sum_c (q_k)_c           S(a) = sum_k Pois(k; lambda a) sigma_k
+ *     phi_k   = sum_c pi_c (g_k)_c      F(a) = sum_k Pois(k; lambda a) phi_k
+ * both sums of non-negative terms, c ascending, so neither probability is formed by cancellation.
+ * Draw order, per observation with a > 0: the ghost count is draw 0 of Philox sub-stream 1 of (sweep, global
+ * observation), M = floor(log U / log F(a)) with log F = log F (F <= 1/2) or log1p(-S) (otherwise); ghost j (0-based)
+ * is pht_unif_path(y = 0, censored, u = a) on sub-stream 2 + j.  The observation's own path stays on sub-stream 0. */
+#define PHT_UNIF_ERR_ENTRY 1024      /* error word: S(a) underflowed, or a ghost count above PHT_UNIF_GHOST_MAX */
+#define PHT_UNIF_GHOST_MAX (1 << 20)
+
+PHT_HD double pht_unif_sigma_entry(int n, const double *qk) {
+    double acc = 0.0;
+    for (int c = 0; c < n; c++) acc += qk[c];
+    return acc;
+}
+PHT_HD double pht_unif_phi_entry(int n, const double *pi, const double *gk) {
+    double acc = 0.0;
+    for (int c = 0; c < n; c++) acc += pi[c] * gk[c];
+    return acc;
+}
+
+/* The ghost count of an observation with entry age a > 0.  tab: the sweep's table; etab: sigma_k at k, phi_k at
+ * cap + k; U: draw 0 of sub-stream 1.  Returns 0 or an error bit; *M = 0 on error. */
+PHT_HD int pht_unif_ghost_count(const double *tab, const double *etab, int n, int cap, double a, double U, unsigned *M) {
+    const pht_unif_layout L = pht_unif_layout_make(n, cap);
+    const double *lgk = tab + L.lgk;
+    const double x = tab[0] * a, lx = x > 0.0 ? pht_log(x) : 0.0;
+    const int K = pht_unif_K(x);
+    *M = 0u;
+    if (K >= cap) return PHT_UNIF_ERR_TABLE;
+    double S = 0.0, F = 0.0;
+    for (int k = 0; k <= K; k++) {
+        const double w = pht_unif_w(x, lx, k, lgk);
+        if (w == 0.0) continue;
+        S += w * etab[k];
+        F += w * etab[cap + k];
+    }
+    if (!(S > 0.0)) return PHT_UNIF_ERR_ENTRY;
+    const double lF = F <= 0.5 ? pht_log(F) : pht_log1p(-S);      /* < 0; -inf when F = 0 (then M = 0) */
+    const double q = pht_log(U) / lF;
+    if (!(q < 2.0 * PHT_UNIF_GHOST_MAX)) return PHT_UNIF_ERR_ENTRY;
+    const unsigned m = (unsigned)q;
+    if (m > (unsigned)PHT_UNIF_GHOST_MAX) return PHT_UNIF_ERR_ENTRY;
+    *M = m;
+    return 0;
+}
+
 /* the sampler itself is compiled where the includer says how transitions are counted: PHT_UNIF_CTX (a type) and
  * PHT_UNIF_COUNT(ctx, from, to); PHT_UNIF_U01(st) may replace the uniform draw by an equivalent call, PHT_UNIF_FN the function's qualifiers */
 #if defined(PHT_UNIF_CTX) && defined(PHT_UNIF_COUNT)

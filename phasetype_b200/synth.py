@@ -63,6 +63,39 @@ def inspection(R, s, l, spacing, k, rng):
     return y, u, np.ones(l, dtype=np.int32), t
 
 
+def delayed_entry(R, s, l, entry, rng, censor=None, spacing=None):
+    """Delayed-entry (left-truncated) data: l units of the CTMC (R, s) started in state 0 that were still working at their
+    entry ages.  entry(k, rng) draws k candidate ages; a unit absorbed at or before its age never enters the sample and is
+    redrawn.  censor(k, rng), when given, draws k study-end ages: a unit still working then is right-censored there
+    (units whose study ends at or before entry are redrawn too).  With spacing the units are inspected every spacing time
+    units from entry on, and a unit found failed gives the interval y = a + (i-1) spacing, u = a + i spacing.
+    Returns (y, a): exact failure times and entry ages; with censor or spacing (y, a, censored, u), u = +inf where there
+    is no upper bound."""
+    ys, As, cs, us = [], [], [], []
+    need = l
+    while need > 0:
+        k = max(2 * need, 1024)
+        t = simulate_pht(R, s, k, rng)
+        a = np.asarray(entry(k, rng), dtype=np.float64)
+        end = np.full(k, np.inf) if censor is None else np.asarray(censor(k, rng), dtype=np.float64)
+        keep = (t > a) & (end > a)
+        t, a, end = t[keep][:need], a[keep][:need], end[keep][:need]
+        cens = t > end
+        y = np.where(cens, end, t)
+        u = np.full(y.shape[0], np.inf)
+        if spacing is not None:
+            i = np.ceil((y - a) / spacing)
+            fail = ~cens
+            y = np.where(fail, a + (i - 1) * spacing, y)
+            u = np.where(fail, a + i * spacing, u)
+            cens = np.ones(y.shape[0], dtype=bool)
+        ys.append(y); As.append(a); cs.append(cens.astype(np.int32)); us.append(u)
+        need -= y.shape[0]
+    if censor is None and spacing is None:
+        return np.concatenate(ys), np.concatenate(As)
+    return np.concatenate(ys), np.concatenate(As), np.concatenate(cs), np.concatenate(us)
+
+
 def _general_T(R, s):
     """Every non-zero rate its own parameter, numbered column-major like sorted "Sij"/"si" names would be."""
     n = s.shape[0]
