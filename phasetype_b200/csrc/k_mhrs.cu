@@ -368,19 +368,19 @@ __device__ __forceinline__ void replay_phase(const SweepParams &p, MhrsSmem<NC> 
 
 /* ------------------------------------------------------------------------------------------ filter walk
  * What a search needs to know of its observation: y in FP32 in units of the largest mean sojourn (smax = max_j
- * scale[j]; the filter clock runs in those units so that its error constants are pure numbers), the part of the
- * per-step error bound that depends on y, the Philox word, and the censoring flag. */
-struct ObsF { float yn; uint32_t og; bool cens; };
-__device__ __forceinline__ void obs_set(ObsF &o, float yn, uint32_t og, bool cens) { o.yn = yn; o.og = og; o.cens = cens; }
-/* IV instance: also the upper bound u in the same units (+inf: none), and bn = the largest clock value a decision is
- * made at (u when finite, else y), at which the part of the error bound that grows with the clock is taken */
-struct ObsFU : ObsF { float un, bn; };
+ * scale[j]; the filter clock runs in those units so that its error constants are pure numbers), the part c0y of the
+ * per-step error bound that depends on y (so that a step need not take it from y again), the Philox word, and the
+ * censoring flag. */
+struct ObsF { float yn, c0y; uint32_t og; bool cens; };
+__device__ __forceinline__ float bound_c0(float bn) { return __fmaf_rn(1.2e-7f, bn, 4.5e-7f); }
+__device__ __forceinline__ void obs_set(ObsF &o, float yn, uint32_t og, bool cens) { o.yn = yn; o.c0y = bound_c0(yn); o.og = og; o.cens = cens; }
+/* IV instance: also the upper bound u in the same units (+inf: none).  c0y is then taken at the largest clock value a
+ * decision is made at (u when finite, else y). */
+struct ObsFU : ObsF { float un; };
 template <bool IV> struct ObsOf { typedef ObsF T; };
 template <> struct ObsOf<true> { typedef ObsFU T; };
 __device__ __forceinline__ void obs_set_u(ObsF &, float) {}
-__device__ __forceinline__ void obs_set_u(ObsFU &o, float un) { o.un = un; o.bn = (un < __int_as_float(0x7f800000)) ? un : o.yn; }
-__device__ __forceinline__ float obs_bound(const ObsF &o) { return o.yn; }
-__device__ __forceinline__ float obs_bound(const ObsFU &o) { return o.bn; }
+__device__ __forceinline__ void obs_set_u(ObsFU &o, float un) { o.un = un; o.c0y = bound_c0((un < __int_as_float(0x7f800000)) ? un : o.yn); }
 /* the bound of the observation at layout position pos (IV), or nothing */
 template <bool IV> __device__ __forceinline__ double upper_at(const double *u, uint32_t pos) {
     if constexpr (IV) return u[pos]; else return 0.0;
@@ -405,22 +405,35 @@ __device__ __forceinline__ void fast_begin(Fast &f, uint32_t a, int n) { f.t = 0
  * (a clock beyond 2y is in no danger: its relative error stays below 1e-3 for the 4096 steps a walk may take here.)
  * The bound accumulated per step is TWICE that sum: 2 * 2^-e + (4.5e-7 + 1.2e-7 y) + 2.5e-7 |L|.  Uniforms with
  * w < 4096 and walks of 4096 steps make the bound infinite, i.e. leave the decision to the exact walker.
- * Outcome of the step: fail (the attempt is dead for certain), surv (alive at y for certain, in state kout), amb (the
+ * Outcome of the step: fail (the attempt is dead for certain), surv (alive at y for certain, in state f.row), amb (the
  * clock is inside the error band at the moment of the test: ask the exact walker), none of them (the walk goes on).
  * IV (interval-censored observations, absorbed in [y, u]): the same bound, with its clock-proportional part taken at u
  * instead of y, gives a second band around u.  The attempt fails as soon as the clock is past u for certain (the clock
- * only grows), survives when absorbed above y and below u for certain, and goes to the exact walker inside either band. */
+ * only grows), survives when absorbed above y and below u for certain, and goes to the exact walker inside either band.
+ *
+ * Almost every step has none of these outcomes, so the step only works out whether the attempt ENDS here and whether
+ * it failed; fast_survives tells surv from amb afterwards, for the attempts that ended without failing.  The step at
+ * which `alive at y` is decided is absorption for a censored observation and any other step for an exact one, so an
+ * attempt ends at absorption, at a step of an exact observation not dead at y for certain, or (IV) past u for certain.
+ * It fails when absorbed before y (exact) or dead at y for certain (censored), or (IV) past u.  Because `over` and
+ * `under` (and `past` and `below`) exclude each other, the outcomes are those of the test above.
+ * c0y = the part of the bound that depends on y (ObsF).  On absorption f.row keeps the state the chain was absorbed
+ * from: the state occupied at the end. */
 template <int NC, bool IV = false>
-__device__ __forceinline__ void fast_step(Fast &f, const typename ObsOf<IV>::T &o, const SweepParams &p, const MhrsSmem<NC> &sm, uint32_t iter, int n,
-                                          bool &fail, bool &surv, bool &amb, int &kout) {
+__device__ __forceinline__ bool fast_step(Fast &f, const typename ObsOf<IV>::T &o, float c0y, const SweepParams &p, const MhrsSmem<NC> &sm,
+                                          uint32_t iter, int n, bool &fail) {
     constexpr int R = NC + 1;
     const pht_u32x4 r = philox_block(f.b, f.a, o.og, iter, p);
     f.b++;
-    const unsigned long long x = (((unsigned long long)r.v[1] << 32) | r.v[0]) >> 12;
     const unsigned g = sm.guide[f.row * GUIDE + (r.v[1] >> (32 - GUIDE_BITS))];
     int k = (int)(g & 0x7fu);
-    /* bit 7: no threshold of the row falls inside the bucket, the guide entry IS the answer (24 of 25 look-ups at 8 phases) */
-    if (!(g & 0x80u)) { const unsigned long long *th = sm.thr + f.row * R; while (x >= th[k]) k++; }
+    /* bit 7: no threshold of the row falls inside the bucket, the guide entry IS the answer (24 of 25 look-ups at 8
+     * phases); only the other buckets need the 52 bits x */
+    if (!(g & 0x80u)) {
+        const unsigned long long x = (((unsigned long long)r.v[1] << 32) | r.v[0]) >> 12;
+        const unsigned long long *th = sm.thr + f.row * R;
+        while (x >= th[k]) k++;
+    }
     const uint32_t w = r.v[3];
     const uint32_t wb = __float_as_uint(__uint2float_rn(w));
     const uint32_t eb = wb >> 23;                                                     /* 127 + exponent of w */
@@ -428,26 +441,29 @@ __device__ __forceinline__ void fast_step(Fast &f, const typename ObsOf<IV>::T &
     const float L = (__uint_as_float(0x4b400000u + eb) - 12583071.0f) + lg2m;        /* (eb - 159) + lg2m: log2 of u */
     f.t = __fmaf_rn(L, sm.A[k], f.t);
     const float trunc = __uint_as_float((254u - eb) << 23);                           /* 2^-(exponent of w) >= 1 / w */
-    const float c0y = __fmaf_rn(1.2e-7f, obs_bound(o), 4.5e-7f);                      /* the part of the bound that depends on y */
     const float step_err = __fmaf_rn(trunc, 2.0f, __fmaf_rn(fabsf(L), 2.5e-7f, c0y));
     const bool flagged = (w < 4096u) || (f.b >> 12) != 0u;
     f.dacc = flagged ? __int_as_float(0x7f800000) : f.dacc + step_err;
     const bool absd = (k == n);
-    const float diff = f.t - o.yn;
-    const bool over = diff > f.dacc, under = -diff > f.dacc;      /* alive at y for certain / dead at y for certain */
-    const bool test = o.cens == absd;                            /* the step at which `alive at y` is decided */
-    surv = test && over;
-    amb = test && !over && !under;
+    const bool under = -(f.t - o.yn) > f.dacc;                    /* dead at y for certain */
+    bool end = absd || (!o.cens && !under);
     fail = absd && (!o.cens || under);
     if constexpr (IV) {
-        const float du = f.t - o.un;
-        const bool past = du > f.dacc, below = -du > f.dacc;        /* above u for certain / below u for certain */
+        const bool past = f.t - o.un > f.dacc;                  /* above u for certain */
+        end = end || past;
         fail = fail || past;
-        amb = test && !under && !past && !(over && below);
-        surv = surv && below;
     }
-    kout = absd ? f.row : k;             /* the state occupied at the end: absorption happens FROM the previous state */
-    f.row = k;
+    f.row = absd ? f.row : k;
+    return end;
+}
+
+/* after a step that ended the attempt without failing: alive at y for certain (and, IV, absorbed below u for certain);
+ * otherwise the step was ambiguous */
+template <bool IV>
+__device__ __forceinline__ bool fast_survives(const Fast &f, const typename ObsOf<IV>::T &o) {
+    bool s = f.t - o.yn > f.dacc;
+    if constexpr (IV) s = s && -(f.t - o.un) > f.dacc;
+    return s;
 }
 
 /* Scan tables of the sweep's model.  thr[row][k] = the smallest x in [0, 2^52] whose uniform (x + 0.5) 2^-52
@@ -639,13 +655,17 @@ __device__ __forceinline__ void tail_search(const TailView &tv, const SweepParam
             }
             __syncwarp();           /* lanes that have just taken an attempt step together with the rest */
             if (active) {
-                bool fail, surv, amb; int k;
-                fast_step<NC, IV>(f, mo, p, sm, iter, n, fail, surv, amb, k);
-                if (surv && !((smask >> k) & 1u)) { surv = false; fail = true; }     /* alive at y in a state that cannot exit: failed */
-                /* (jump-steps are counted when an attempt ends: f.b of them) */
-                if (fail) { c_attempts++; c_jumps += f.b; TAIL_GRAB(); }
-                else if (surv) { c_attempts++; c_jumps += f.b; survived = true; kend = k; active = false; }
-                else if (amb) { c_jumps += f.b; want_exact = true; active = false; }
+                bool fail;
+                /* (at its 80 registers the tail would spill c0y of an exact or right-censored observation: it is taken from y
+                 * in each step instead; the IV instance holds it in place of the bound it is taken at) */
+                if (fast_step<NC, IV>(f, mo, IV ? mo.c0y : bound_c0(mo.yn), p, sm, iter, n, fail)) {
+                    const bool surv = !fail && fast_survives<IV>(f, mo);
+                    if (surv && !((smask >> f.row) & 1u)) fail = true;     /* alive at y in a state that cannot exit: failed */
+                    /* (jump-steps are counted when an attempt ends: f.b of them) */
+                    if (fail) { c_attempts++; c_jumps += f.b; TAIL_GRAB(); }
+                    else if (surv) { c_attempts++; c_jumps += f.b; survived = true; kend = f.row; active = false; }
+                    else { c_jumps += f.b; want_exact = true; active = false; }
+                }
             }
             if (__any_sync(FULL, survived || want_exact)) break;
         }
@@ -763,24 +783,34 @@ __device__ __forceinline__ void lane_phase(const SweepParams &p, MhrsSmem<NC> &s
         __syncwarp();
         /* ---- the search loop proper: steps until some lane has something to report.  No calls, nothing but the
          * filter walk, in here; a failed attempt restarts on the next sub-stream on the spot. */
-        bool surv = false, amb = false, hand = false; int k = 0;
         bool go = (fl & LF_RUN) != 0u;
         /* A lane that has something to report stops walking, but the warp only leaves the loop for the (divergent, ~100
          * instructions at 2 lanes) event code once EV_MIN lanes are waiting or the first of them has waited EV_WAIT steps:
-         * events come every ~150 steps per lane, so the wait costs a lane a few per cent and the event code runs a third as often. */
+         * events come every ~150 steps per lane, so the wait costs a lane a few per cent and the event code runs a third as often.
+         * Two jump-steps per vote: a lane that stops in the first sits out the second, and the vote, its count and the
+         * wait counter (kept in steps) cost half as much per step.  A lane stops when its attempt ended without failing,
+         * or when it failed and the next attempt is the tail's (f.b = 0 then: the walk has restarted). */
         unsigned waited = 0u, ev;
         do {
-            if (go) {
-                bool fail;
-                fast_step<NC, IV>(f, o, p, sm, iter, n, fail, surv, amb, k);
-                if (fail) { c_jumps += f.b; fast_begin(f, f.a + 1u, n); c_attempts++; hand = f.a >= a_lim; }
-                go = !(surv || amb || hand);
+#pragma unroll
+            for (int h = 0; h < 2; h++) {
+                if (go) {
+                    bool fail;
+                    const bool end = fast_step<NC, IV>(f, o, o.c0y, p, sm, iter, n, fail);
+                    if (fail) { c_jumps += f.b; fast_begin(f, f.a + 1u, n); c_attempts++; }
+                    go = fail ? f.a < a_lim : !end;
+                }
             }
             ev = __ballot_sync(FULL, !go);
-            waited += ((ev & running) != 0u) ? 1u : 0u;
+            waited += ((ev & running) != 0u) ? 2u : 0u;
         } while (ev != 0xffffffffu && (unsigned)__popc(ev & running) < EV_MIN && waited < EV_WAIT);
         /* ---- events, a few lanes at a time */
-        if (surv || amb) c_jumps += f.b;            /* the filter steps of the attempt that just ended (failed ones: above) */
+        const bool stopped = (fl & LF_RUN) && !go;
+        bool hand = stopped && f.b == 0u, surv = false, amb = false; int k = f.row;
+        if (stopped && f.b != 0u) {
+            c_jumps += f.b;                         /* the filter steps of the attempt that just ended (failed ones: above) */
+            surv = fast_survives<IV>(f, o); amb = !surv;
+        }
         if (amb) {
             const uint32_t res = exact_attempt<NC, IV>(f.a, false, p.y[pos], o.cens, o.og, p, sm, iter, n, ~0u, upper_at<IV>(p.u, pos));
             surv = res & 1u; k = (int)((res >> 8) & 0xffu); c_jumps += res >> 16;
