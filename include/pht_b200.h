@@ -179,6 +179,29 @@ int pht_engine_set_upper(pht_engine *e, const double *upper_local);
  * ECS, DCS and the two MH variants. */
 int pht_engine_set_entry(pht_engine *e, const double *entry_local);
 
+/* Several chains in one engine (method 64 only).  Chain c is, bit for bit, the chain a single-chain engine created with
+ * Philox key keys[c] draws from the same theta, pi, prior, data, bounds and next_iter: every sweep statistic is an integer
+ * sum, and every chain runs the same table, path and update code on its own model block with its own key.  The chains
+ * share the observations, the bounds and the sorted layout; each has its own model block, statistics block, 33 MB table
+ * (at n = 32) and result rows.  One sweep builds the chains' tables side by side (one block each) and the path kernel
+ * spreads every chain's observations over the GPU, so at small shards C chains cost about what one does.
+ * pht_engine_set_chains: keys holds `chains` Philox keys, NULL = the configured seed + c.  Every chain starts from the
+ * engine's current theta and pi; chains = 1 returns to the single-chain engine, whose results are those of an engine that
+ * never called it.  With several chains the existing calls keep their meaning for chain 0 (pht_engine_get_theta, run's
+ * out, pht_engine_pi_rows, pht_engine_get_model; the parity hooks pht_engine_sweep_stats and pht_engine_paths run chain
+ * 0 alone), while pht_engine_set_theta and pht_engine_set_pi set every chain.  Refused: any method but 64, world > 1 (the
+ * all-reduce carries one chain's statistics), entry ages (pht_engine_set_entry, in either order), chains outside
+ * 1..PHT_MAX_CHAINS, duplicate keys, and a failed allocation (the engine then stays as it was).
+ * pht_engine_set_chain_theta / pht_engine_get_chain_theta: one theta per chain (chains x m, row-major); set also gives
+ * the next sweep index next_iter, as pht_engine_set_theta does.
+ * pht_engine_chain_rows: the draws of the last pht_engine_run, theta as chains x rows x m and pi as chains x rows x n
+ * (either may be NULL; pi needs the prior set, pht_engine_set_pi with beta). */
+#define PHT_MAX_CHAINS 1024
+int pht_engine_set_chains(pht_engine *e, int chains, const uint64_t *keys);
+int pht_engine_set_chain_theta(pht_engine *e, const double *theta, uint32_t next_iter);
+int pht_engine_get_chain_theta(pht_engine *e, double *theta);
+int pht_engine_chain_rows(pht_engine *e, int rows, double *theta_out, double *pi_out);
+
 /* run `nsweeps` Gibbs sweeps; row r of out (nsweeps x m, row-major) is the draw of sweep r.
  * out may be NULL (results stay on the device; fetch later with pht_engine_get_theta). */
 int pht_engine_run(pht_engine *e, int nsweeps, double *out);

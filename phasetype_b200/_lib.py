@@ -20,11 +20,13 @@ SYMBOLS = [
     "pht_engine_sweep_stats", "pht_engine_paths", "pht_engine_set_spectral", "pht_engine_get_model",
     "pht_engine_counters", "pht_fp64_fma_rate", "pht_engine_set_l2_flush", "pht_engine_peer_handle", "pht_engine_peer_attach", "pht_engine_round_trace", "pht_engine_set_pi", "pht_engine_get_pi", "pht_engine_pi_rows",
     "pht_engine_set_upper", "pht_engine_set_entry", "pht_engine_entry_paths",
+    "pht_engine_set_chains", "pht_engine_set_chain_theta", "pht_engine_get_chain_theta", "pht_engine_chain_rows",
 ]
 PEER_HANDLE_BYTES = 128
 # method 64 (include/pht_b200.h PHT_METHOD_UNIF): the uniformisation path sampler; exact, right-, interval- and
 # left-censored observations, any sub-generator; delayed entry (Engine.set_entry) is this method's alone
 METHOD_UNIF = 64
+MAX_CHAINS = 1024            # include/pht_b200.h PHT_MAX_CHAINS: chains one METHOD_UNIF engine can run (Engine.set_chains)
 CNT_NAMES = ["paths", "attempts", "jumps", "dens_evals", "env_updates", "brent_evals", "arms_calls",
              "metrop_rejects", "nonfinite", "deferred", "tail_rounds", "errors", "launches", "ns_lane", "ns_tail", "ns_replay",
              "ns_global", "ns_xwait", "global_rounds", "global_items"]
@@ -83,6 +85,10 @@ def lib():
     L.pht_engine_set_upper.argtypes = [C.c_void_p, C.c_void_p]
     L.pht_engine_set_entry.argtypes = [C.c_void_p, C.c_void_p]
     L.pht_engine_entry_paths.argtypes = [C.c_void_p, C.c_long, C.c_long, _ip, C.c_long, C.c_void_p, C.c_void_p, C.c_void_p]
+    L.pht_engine_set_chains.argtypes = [C.c_void_p, C.c_int, C.c_void_p]
+    L.pht_engine_set_chain_theta.argtypes = [C.c_void_p, _dp, C.c_uint32]
+    L.pht_engine_get_chain_theta.argtypes = [C.c_void_p, _dp]
+    L.pht_engine_chain_rows.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]
     L.pht_engine_peer_handle.argtypes = [C.c_void_p, C.c_void_p]
     L.pht_engine_peer_attach.argtypes = [C.c_void_p, C.c_void_p]
     _lib = L
@@ -123,6 +129,7 @@ class Engine:
                      self._nu.ctypes.data, self._zeta.ctypes.data, int(seed), int(device), int(rank), int(world),
                      self.zbits, int(mhrs_cap), 1 if use_graph else 0)
         self._h = C.c_void_p()
+        self.chains = 1
         _check(L.pht_engine_create(C.byref(self._h), C.byref(cfg), y_local if self.l_local else np.zeros(1),
                                    cens_local if self.l_local else np.zeros(1, dtype=np.int32), self.l_local))
 
@@ -270,6 +277,46 @@ class Engine:
         if not np.array_equal(M2[:int(count)], M):
             raise EngineError("entry_paths: ghost counts changed between two calls at the same parameters")
         return M, B[:G], N[:G * n * n].reshape(G, n * n), z[:G * n].reshape(G, n)
+
+    def set_chains(self, chains, keys=None):
+        """Several chains in this engine (METHOD_UNIF only, one rank, no entry ages): chain c draws with Philox key keys[c]
+        (default: seed + c) and is bit for bit the chain of a single-chain engine with that key.  Every chain starts from
+        the current theta and pi; set_theta and set_pi then set every chain, and the single-chain calls (get_theta, run,
+        pi_rows, model, paths, sweep_stats) refer to chain 0.  chains = 1 returns to the single-chain engine."""
+        chains = int(chains)
+        k = None
+        if keys is not None:
+            k = np.ascontiguousarray(keys, dtype=np.uint64)
+            if k.shape != (chains,):
+                raise EngineError("set_chains: %d keys for %d chains" % (k.size, chains))
+        _check(lib().pht_engine_set_chains(self._h, chains, None if k is None else k.ctypes.data))
+        self.chains = chains
+
+    def set_chain_theta(self, theta, next_iter=1):
+        """One parameter vector per chain: theta of shape (chains, m)."""
+        t = np.ascontiguousarray(theta, dtype=np.float64)
+        if t.shape != (self.chains, self.m):
+            raise EngineError("set_chain_theta: shape %s, expected (%d, %d)" % (t.shape, self.chains, self.m))
+        _check(lib().pht_engine_set_chain_theta(self._h, t.ravel(), int(next_iter)))
+
+    def get_chain_theta(self):
+        out = np.zeros(self.chains * self.m)
+        _check(lib().pht_engine_get_chain_theta(self._h, out))
+        return out.reshape(self.chains, self.m)
+
+    def run_chains(self, nsweeps):
+        """nsweeps sweeps of every chain; returns the draws of theta, shape (chains, nsweeps, m)."""
+        nsweeps = int(nsweeps)
+        _check(lib().pht_engine_run(self._h, nsweeps, None))
+        out = np.zeros((self.chains, nsweeps, self.m))
+        _check(lib().pht_engine_chain_rows(self._h, nsweeps, out.ctypes.data, None))
+        return out
+
+    def chain_pi_rows(self, rows):
+        """The pi draws of the last run, shape (chains, rows, n) (needs set_pi with a prior)."""
+        out = np.zeros((self.chains, int(rows), self.n))
+        _check(lib().pht_engine_chain_rows(self._h, int(rows), None, out.ctypes.data))
+        return out
 
     def round_trace(self):
         """(48, 8) array: per tail round number, ns search / ns barrier / ns advance / sum of pending / sum of K / attempts run /

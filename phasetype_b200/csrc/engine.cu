@@ -92,6 +92,10 @@ struct pht_engine {
     int iv_blocks[3] = { 0, 0, 0 };
     /* method 64: the uniformisation table (pht_unif.h) and the longest time span it must cover (max of y and of u - y) */
     double *d_unif = nullptr; double unif_tmax = 0.0;
+    /* method 64, several chains (pht_engine_set_chains): model, stats, table, res and pires hold `chains` blocks, chain 0
+     * first; the chains' Philox keys (2 x u32 each) and observation counters; the seed that NULL keys count from */
+    int chains = 1; uint32_t *d_keys = nullptr; unsigned long long *d_cnext = nullptr; uint64_t base_seed = 0;
+    int chain_blocks = 0;              /* grid of the several-chain path kernel */
     /* method 64, delayed entry (pht_engine_set_entry): the ages in upload order (device and host), the truncated
      * observations (a > 0) by decreasing a with their local indices, their ghost counts and offsets, the entry tables,
      * the ghost counter, the scan's scratch and the ghost kernel's grid */
@@ -138,6 +142,7 @@ static SweepParams sweep_params(pht_engine *e) {
     p.glist = e->d_glist; p.k_switch = e->k_switch; p.recs = e->d_recs;
     if (e->peers_attached) { p.xw = e->d_xw; for (int r = 0; r < e->cfg.world && r < PHT_MAX_WORLD; r++) p.xpeer[r] = e->xpeer[r]; }
     if (e->d_u) { p.u = e->d_ys ? e->d_us : e->d_u; p.item_u = e->d_item_u; }
+    p.chains = e->chains; p.ckeys = e->d_keys; p.cnext = e->d_cnext;
     return p;
 }
 static UpdateParams update_params(pht_engine *e, double *res, int res_rows) {
@@ -148,6 +153,7 @@ static UpdateParams update_params(pht_engine *e, double *res, int res_rows) {
     u.n = e->cfg.n; u.m = e->cfg.m; u.zbits = e->cfg.zbits;
     u.k0 = (uint32_t)e->cfg.seed; u.k1 = (uint32_t)(e->cfg.seed >> 32);
     u.beta = e->d_beta; u.pires = (e->d_beta && res) ? e->d_pires : nullptr;
+    u.chains = e->chains; u.ckeys = e->d_keys; u.cnext = e->d_cnext;
     return u;
 }
 
@@ -212,7 +218,7 @@ static int enqueue_paths(pht_engine *e, const SweepParams &p, const uint32_t *id
         e->launches += 2; break;
     case PHT_METHOD_DCS: CU(pht_launch_dcs(p, e->grid_blocks, e->stream)); e->launches++; break;           /* unit machine + complex-spectrum kernel */
     case PHT_METHOD_MHS_HOBOLTH: CU(pht_launch_dcs(p, e->grid_blocks, e->stream, true)); e->launches++; break;
-    case PHT_METHOD_UNIF: CU(pht_launch_unif(p, e->d_unif, e->grid_blocks, e->stream)); break;
+    case PHT_METHOD_UNIF: CU(pht_launch_unif(p, e->d_unif, p.chains > 1 ? e->chain_blocks : e->grid_blocks, e->stream)); break;
     case PHT_METHOD_MHS_ASLETT:
         /* every observation through one kernel: the window list in parity mode, else the whole shard (identity) */
         if (lists_given) CU(pht_launch_mhs_aslett(p, e->grid_blocks, idx_exact, n_exact, e->stream));
@@ -293,7 +299,7 @@ extern "C" void pht_engine_destroy(pht_engine *e) {
     if (e->ev1) cudaEventDestroy(e->ev1);
     for (void *q : e->ipc_opened) cudaIpcCloseMemHandle(q);
     stage("events, ipc");
-    void *big[] = { e->d_entry, e->d_ea, e->d_eobs, e->d_eM, e->d_eoff, e->d_enext, e->d_etab, e->d_escan, e->d_unif, e->d_u, e->d_us, e->d_item_u, e->d_recs, e->d_ys, e->d_cs, e->d_perm, e->d_y, e->d_cens, e->d_items /* arena: found, pend0, pend1, done live inside */, e->d_idx_exact, e->d_idx_cens,
+    void *big[] = { e->d_keys, e->d_cnext, e->d_entry, e->d_ea, e->d_eobs, e->d_eM, e->d_eoff, e->d_enext, e->d_etab, e->d_escan, e->d_unif, e->d_u, e->d_us, e->d_item_u, e->d_recs, e->d_ys, e->d_cs, e->d_perm, e->d_y, e->d_cens, e->d_items /* arena: found, pend0, pend1, done live inside */, e->d_idx_exact, e->d_idx_cens,
                     e->d_glist, e->d_model, e->d_stats, e->d_state, e->d_T, e->d_C, e->d_nu, e->d_zeta, e->d_var_ptr, e->d_cell_i, e->d_cell_j, e->d_pires, e->d_res };
     for (void *b : big) pht_dev_free(b, e->stream);
     if (e->stream) cudaStreamSynchronize(e->stream);
@@ -351,6 +357,7 @@ extern "C" int pht_engine_create(pht_engine **out, const pht_config *cfg, const 
     const bool auto_cap = e->cfg.mhrs_cap <= 0;
     if (auto_cap) e->cfg.mhrs_cap = 256;
     e->l_local = l_local;
+    e->base_seed = cfg->seed;
     e->L = ModelLayout::make(n, m);
 #define CUE(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { fail("%s failed: %s", #call, cudaGetErrorString(e_)); pht_engine_destroy(e); return -1; } } while (0)
     CUE(cudaStreamCreateWithFlags(&e->stream, cudaStreamNonBlocking));
@@ -416,7 +423,13 @@ extern "C" int pht_engine_create(pht_engine **out, const pht_config *cfg, const 
         /* the table (capacity PHT_UNIF_CAP powers; log k! filled once here), the y-descending layout so that the lanes of
          * a warp run similar Poisson truncations (parity hooks keep the upload order), and the longest span y */
         CUE(pht_dev_alloc((void **)&e->d_unif, sizeof(double) * pht_unif_table_doubles(n, PHT_UNIF_CAP), e->stream));
-        CUE(pht_unif_init(e->d_unif, n, PHT_UNIF_CAP, e->stream));
+        CUE(pht_unif_init(e->d_unif, n, PHT_UNIF_CAP, 1, e->stream));
+        /* chain 0's key and observation counter (pht_engine_set_chains adds more) */
+        const uint32_t key[2] = { (uint32_t)cfg->seed, (uint32_t)(cfg->seed >> 32) };
+        CUE(pht_dev_alloc((void **)&e->d_keys, sizeof(key), e->stream));
+        CUE(cudaMemcpyAsync(e->d_keys, key, sizeof(key), cudaMemcpyHostToDevice, e->stream));
+        CUE(pht_dev_alloc((void **)&e->d_cnext, sizeof(unsigned long long), e->stream));
+        CUE(cudaMemsetAsync(e->d_cnext, 0, sizeof(unsigned long long), e->stream));
         for (long i = 0; i < l_local; i++) if (y_local[i] > e->unif_tmax) e->unif_tmax = y_local[i];
         if (l_local > 1 && !getenv("PHT_B200_NO_SORT")) {
             CUE(pht_dev_alloc((void **)&e->d_ys, ln * sizeof(double), e->stream)); CUE(pht_dev_alloc((void **)&e->d_cs, ln, e->stream));
@@ -424,7 +437,7 @@ extern "C" int pht_engine_create(pht_engine **out, const pht_config *cfg, const 
             CUE(pht_sort_by_y_desc(e->d_y, e->d_cens, l_local, e->d_ys, e->d_cs, e->d_perm, e->stream));
         }
         CUE(cudaStreamSynchronize(e->stream));
-        e->grid_blocks = pht_unif_grid_blocks(cfg->device, n);
+        e->grid_blocks = pht_unif_grid_blocks(cfg->device, n, false);
         if (e->grid_blocks <= 0) { fail("the uniformisation kernel does not fit on the device: %s", cudaGetErrorString(cudaGetLastError())); pht_engine_destroy(e); return -1; }
     }
     if (method_of(e->cfg) == PHT_METHOD_MHRS) {
@@ -590,15 +603,21 @@ extern "C" int pht_engine_peer_attach(pht_engine *e, const void *handles) {
     return 0;
 }
 
-extern "C" int pht_engine_set_theta(pht_engine *e, const double *theta, uint32_t next_iter) {
-    if (!e || !theta) return fail("null argument");
-    CU(cudaSetDevice(e->cfg.device));
-    CU(cudaStreamSynchronize(e->stream));
-    CU(cudaMemcpy(e->d_model + e->L.theta, theta, sizeof(double) * e->cfg.m, cudaMemcpyHostToDevice));
+/* the next sweep gets index next_iter and assembles its model from start values (src/PHT_MCMC_Aslett.c:268) */
+static int set_next_iter(pht_engine *e, uint32_t next_iter) {
     DevState st; CU(cudaMemcpy(&st, e->d_state, sizeof(st), cudaMemcpyDeviceToHost));
     st.iter = next_iter; st.first_assembly = 1;
     CU(cudaMemcpy(e->d_state, &st, sizeof(st), cudaMemcpyHostToDevice));
     return 0;
+}
+
+extern "C" int pht_engine_set_theta(pht_engine *e, const double *theta, uint32_t next_iter) {
+    if (!e || !theta) return fail("null argument");
+    CU(cudaSetDevice(e->cfg.device));
+    CU(cudaStreamSynchronize(e->stream));
+    for (int c = 0; c < e->chains; c++)           /* every chain */
+        CU(cudaMemcpy(e->d_model + (size_t)c * e->L.total + e->L.theta, theta, sizeof(double) * e->cfg.m, cudaMemcpyHostToDevice));
+    return set_next_iter(e, next_iter);
 }
 extern "C" int pht_engine_get_theta(pht_engine *e, double *theta) {
     if (!e || !theta) return fail("null argument");
@@ -617,7 +636,8 @@ extern "C" int pht_engine_set_pi(pht_engine *e, const double *pi, const double *
         double sum = 0.0;
         for (int i = 0; i < n; i++) { if (!(pi[i] >= 0.0)) return fail("pi[%d] = %g is not a probability", i, pi[i]); sum += pi[i]; }
         if (!(sum > 0.999999 && sum < 1.000001)) return fail("pi sums to %g, not 1", sum);
-        CU(cudaMemcpy(e->d_model + e->L.pi, pi, sizeof(double) * n, cudaMemcpyHostToDevice));
+        for (int c = 0; c < e->chains; c++)       /* every chain */
+            CU(cudaMemcpy(e->d_model + (size_t)c * e->L.total + e->L.pi, pi, sizeof(double) * n, cudaMemcpyHostToDevice));
     }
     if (e->graph_exec) { cudaGraphExecDestroy(e->graph_exec); e->graph_exec = nullptr; }     /* kernel parameters change */
     if (beta) {
@@ -647,6 +667,95 @@ extern "C" int pht_engine_pi_rows(pht_engine *e, int rows, double *out) {
     CU(cudaSetDevice(e->cfg.device));
     CU(cudaStreamSynchronize(e->stream));
     if (rows) CU(cudaMemcpy(out, e->d_pires, sizeof(double) * (size_t)rows * e->cfg.n, cudaMemcpyDeviceToHost));
+    return 0;
+}
+
+/* ---------------------------------------------------------------- several chains (method 64) */
+extern "C" int pht_engine_set_chains(pht_engine *e, int chains, const uint64_t *keys) {
+    if (!e) return fail("null engine");
+    if (method_of(e->cfg) != PHT_METHOD_UNIF)
+        return fail("several chains per engine need method 64 (the uniformisation sampler); MHRS, ECS, DCS and the MH variants run one chain per engine");
+    if (e->cfg.world > 1)
+        return fail("several chains per engine need world = 1: the statistics all-reduce of a multi-rank run carries one chain's block");
+    if (chains < 1 || chains > PHT_MAX_CHAINS) return fail("chains = %d outside 1..%d", chains, PHT_MAX_CHAINS);
+    if (chains > 1 && e->entry_set)
+        return fail("%d chains asked while entry ages (delayed entry) are set: the ghost paths are drawn for one chain; clear them with pht_engine_set_entry(e, NULL) first", chains);
+    std::vector<uint64_t> k((size_t)chains);
+    for (int c = 0; c < chains; c++) k[(size_t)c] = keys ? keys[c] : e->base_seed + (uint64_t)c;
+    { std::vector<uint64_t> sorted(k); std::sort(sorted.begin(), sorted.end());
+      for (size_t i = 1; i < sorted.size(); i++) if (sorted[i] == sorted[i - 1])
+          return fail("duplicate key 0x%llx: two chains with one key would be one chain drawn twice", (unsigned long long)sorted[i]); }
+    CU(cudaSetDevice(e->cfg.device));
+    CU(cudaStreamSynchronize(e->stream));
+    const int n = e->cfg.n;
+    if (chains > 1 && !e->chain_blocks) {
+        e->chain_blocks = pht_unif_grid_blocks(e->cfg.device, n, true);
+        if (e->chain_blocks <= 0) { e->chain_blocks = 0; return fail("the several-chain path kernel does not fit on the device: %s", cudaGetErrorString(cudaGetLastError())); }
+    }
+    const size_t total = (size_t)e->L.total, slen = (size_t)stats_len(n), tab = pht_unif_table_doubles(n, PHT_UNIF_CAP);
+    /* the new buffers first: a failed allocation leaves the engine as it was */
+    double *model = nullptr, *unif = nullptr; long long *stats = nullptr; uint32_t *dkeys = nullptr; unsigned long long *cnext = nullptr;
+    const size_t bytes[] = { sizeof(double) * chains * total, sizeof(long long) * chains * slen, sizeof(double) * chains * tab,
+                             sizeof(uint32_t) * 2 * chains, sizeof(unsigned long long) * chains };
+    void **ptrs[] = { (void **)&model, (void **)&stats, (void **)&unif, (void **)&dkeys, (void **)&cnext };
+    for (int b = 0; b < 5; b++) {
+        const cudaError_t ce = pht_dev_alloc(ptrs[b], bytes[b], e->stream);
+        if (ce != cudaSuccess) {
+            cudaGetLastError();
+            for (int f = 0; f < b; f++) pht_dev_free(*ptrs[f], e->stream);
+            cudaStreamSynchronize(e->stream); cudaGetLastError();
+            return fail("cannot allocate device memory for %d chains (%.1f MB, of which the uniformisation tables take %.1f MB per chain): %s",
+                        chains, (bytes[0] + bytes[1] + bytes[2] + bytes[3] + bytes[4]) / 1e6, sizeof(double) * tab / 1e6, cudaGetErrorString(ce));
+        }
+    }
+    /* every chain starts from chain 0's current theta and pi (the rest of a model block is rebuilt every sweep) */
+    for (int c = 0; c < chains; c++)
+        CU(cudaMemcpyAsync(model + (size_t)c * total, e->d_model, sizeof(double) * total, cudaMemcpyDeviceToDevice, e->stream));
+    CU(cudaMemsetAsync(stats, 0, bytes[1], e->stream));
+    CU(pht_unif_init(unif, n, PHT_UNIF_CAP, chains, e->stream));       /* log k! in every chain's table */
+    std::vector<uint32_t> hk(2 * (size_t)chains);
+    for (int c = 0; c < chains; c++) { hk[2 * (size_t)c] = (uint32_t)k[(size_t)c]; hk[2 * (size_t)c + 1] = (uint32_t)(k[(size_t)c] >> 32); }
+    CU(cudaMemcpyAsync(dkeys, hk.data(), bytes[3], cudaMemcpyHostToDevice, e->stream));
+    CU(cudaMemsetAsync(cnext, 0, bytes[4], e->stream));
+    void *old[] = { e->d_model, e->d_stats, e->d_unif, e->d_keys, e->d_cnext, e->d_res, e->d_pires };
+    for (void *b : old) CU(pht_dev_free(b, e->stream));
+    CU(cudaStreamSynchronize(e->stream));
+    e->d_model = model; e->d_stats = stats; e->d_unif = unif; e->d_keys = dkeys; e->d_cnext = cnext;
+    e->d_res = nullptr; e->d_pires = nullptr; e->res_rows = 0;
+    e->chains = chains;
+    e->cfg.seed = k[0];                            /* chain 0's key is the engine's key (the ghost kernels read it) */
+    if (e->graph_exec) { cudaGraphExecDestroy(e->graph_exec); e->graph_exec = nullptr; }     /* kernel parameters change */
+    return 0;
+}
+
+extern "C" int pht_engine_set_chain_theta(pht_engine *e, const double *theta, uint32_t next_iter) {
+    if (!e || !theta) return fail("null argument");
+    CU(cudaSetDevice(e->cfg.device));
+    CU(cudaStreamSynchronize(e->stream));
+    for (int c = 0; c < e->chains; c++)
+        CU(cudaMemcpy(e->d_model + (size_t)c * e->L.total + e->L.theta, theta + (size_t)c * e->cfg.m, sizeof(double) * e->cfg.m, cudaMemcpyHostToDevice));
+    return set_next_iter(e, next_iter);
+}
+
+extern "C" int pht_engine_get_chain_theta(pht_engine *e, double *theta) {
+    if (!e || !theta) return fail("null argument");
+    CU(cudaSetDevice(e->cfg.device));
+    CU(cudaStreamSynchronize(e->stream));
+    for (int c = 0; c < e->chains; c++)
+        CU(cudaMemcpy(theta + (size_t)c * e->cfg.m, e->d_model + (size_t)c * e->L.total + e->L.theta, sizeof(double) * e->cfg.m, cudaMemcpyDeviceToHost));
+    return 0;
+}
+
+extern "C" int pht_engine_chain_rows(pht_engine *e, int rows, double *theta_out, double *pi_out) {
+    if (!e || rows < 0) return fail("bad argument");
+    if (rows > e->res_rows) return fail("%d rows asked, the last run produced at most %d", rows, e->res_rows);
+    if (pi_out && (!e->d_beta || !e->d_pires)) return fail("pi is not being inferred (pht_engine_set_pi with a prior first)");
+    if (rows == 0) return 0;
+    CU(cudaSetDevice(e->cfg.device));
+    CU(cudaStreamSynchronize(e->stream));
+    const size_t m = (size_t)e->cfg.m, n = (size_t)e->cfg.n, R = (size_t)e->res_rows;
+    if (theta_out) CU(cudaMemcpy2D(theta_out, sizeof(double) * rows * m, e->d_res, sizeof(double) * R * m, sizeof(double) * rows * m, e->chains, cudaMemcpyDeviceToHost));
+    if (pi_out) CU(cudaMemcpy2D(pi_out, sizeof(double) * rows * n, e->d_pires, sizeof(double) * R * n, sizeof(double) * rows * n, e->chains, cudaMemcpyDeviceToHost));
     return 0;
 }
 
@@ -732,6 +841,8 @@ extern "C" int pht_engine_set_entry(pht_engine *e, const double *entry_local) {
     CU(cudaSetDevice(e->cfg.device));
     CU(cudaStreamSynchronize(e->stream));
     if (e->peers_attached) return fail("the entry ages of a multi-rank run are set on every rank before the exchange windows are attached");
+    if (entry_local && e->chains > 1)
+        return fail("entry ages (delayed entry) are not supported with %d chains: the ghost paths are drawn for one chain; pht_engine_set_chains(e, 1, ...) first", e->chains);
     if (e->graph_exec) { cudaGraphExecDestroy(e->graph_exec); e->graph_exec = nullptr; }     /* the sweep changes shape */
     if (!entry_local) return entry_free(e);
     const long l = e->l_local;
@@ -813,8 +924,10 @@ extern "C" int pht_engine_entry_paths(pht_engine *e, long first, long count, int
         E.a = e->d_entry + first; E.obs = nullptr; E.first = first; E.count = count; E.M = dM; E.off = doff;
         E.etab = e->d_etab; E.next = e->d_enext; E.scan_tmp = tmp; E.count_blocks = e->count_blocks;
         UpdateParams u = update_params(e, nullptr, 0);
+        u.chains = 1;
         if (enqueue_model(e, u)) goto out;
         SweepParams p = sweep_params(e);
+        p.chains = 1;
         CUP(pht_launch_unif_entry(u, p, e->d_unif, E, e->ghost_blocks, PHT_ENTRY_COUNTS, e->stream));
         if (pht_engine_sync(e)) goto out;
         std::vector<unsigned> hM((size_t)count);
@@ -846,13 +959,14 @@ out:
     return rc;
 }
 
+/* rows x m draws of theta and rows x n of pi per chain, chain 0 first (chain c's rows start at c x res_rows) */
 static int ensure_res(pht_engine *e, int rows) {
     if (rows <= e->res_rows) return 0;
     CU(cudaStreamSynchronize(e->stream));
     if (e->d_res) { CU(pht_dev_free(e->d_res, e->stream)); e->d_res = nullptr; }
-    CU(pht_dev_alloc((void **)&e->d_res, sizeof(double) * (size_t)rows * e->cfg.m, e->stream));
+    CU(pht_dev_alloc((void **)&e->d_res, sizeof(double) * (size_t)e->chains * rows * e->cfg.m, e->stream));
     if (e->d_pires) { CU(pht_dev_free(e->d_pires, e->stream)); e->d_pires = nullptr; }
-    CU(pht_dev_alloc((void **)&e->d_pires, sizeof(double) * (size_t)rows * e->cfg.n, e->stream));
+    CU(pht_dev_alloc((void **)&e->d_pires, sizeof(double) * (size_t)e->chains * rows * e->cfg.n, e->stream));
     CU(cudaStreamSynchronize(e->stream));
     e->res_rows = rows;
     return 0;
@@ -953,8 +1067,10 @@ extern "C" int pht_engine_sweep_stats(pht_engine *e, long long *N, long long *B,
     CU(cudaSetDevice(e->cfg.device));
     const int n = e->cfg.n;
     UpdateParams u = update_params(e, nullptr, 0);
+    u.chains = 1;                                  /* chain 0 only */
     if (enqueue_model(e, u)) return -1;
     SweepParams p = sweep_params(e);
+    p.chains = 1;
     if (enqueue_paths(e, p)) return -1;
     if (enqueue_entry(e, u, p)) return -1;
     if (pht_engine_sync(e)) return -1;
@@ -986,8 +1102,10 @@ extern "C" int pht_engine_paths(pht_engine *e, long first, long count, int *B, i
         CUP(cudaMemsetAsync(dB, 0, sizeof(int) * count, e->stream)); CUP(cudaMemsetAsync(dN, 0, sizeof(int) * count * n * n, e->stream));
         CUP(cudaMemsetAsync(dz, 0, sizeof(double) * count * n, e->stream));
         UpdateParams u = update_params(e, nullptr, 0);
+        u.chains = 1;                              /* chain 0 only */
         if (enqueue_model(e, u)) goto out;
         SweepParams p = sweep_params(e);
+        p.chains = 1;
         p.y = e->d_y; p.cens = e->d_cens; p.perm = nullptr;         /* the window [first, first + count) is in upload order */
         if (p.u) p.u = e->d_u;
         p.outB = dB; p.outN = dN; p.outz = dz; p.first = first; p.count = count;

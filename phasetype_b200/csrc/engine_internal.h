@@ -14,6 +14,9 @@
  *                          rebuilt on the device every sweep, copied to shared memory by the path kernels
  *   stats[]         int64  N (n*n) | B (n) | z fixed point in two limbs (2n) | error count: the only data that crosses NVLink
  *   state           DevState: sweep index, work counters, event counters, error word
+ * Method 64 with several chains (pht_engine_set_chains) repeats model[], stats[] and unif[] once per chain, chain-major with
+ * chain 0 first, and adds the chains' Philox keys and observation counters; observations, bounds and the sorted layout
+ * stay shared.
  *   items/pend/...  MHRS tail work lists (see k_mhrs.cu)
  */
 #ifndef PHT_ENGINE_INTERNAL_H
@@ -125,6 +128,7 @@ struct DevState {
     /* measurement aid: per tail round (index = round number, accumulated over sweeps) the device-timer ns block 0 spent
      * searching / waiting at the barrier after the search / advancing, and the sum of pending items and of K */
     unsigned long long round_trace[PHT_ROUND_TRACE][8];
+    uint32_t update_ticket;    /* k_update blocks (one per chain) that have finished; the last one advances the sweep */
 };
 
 struct SweepParams {
@@ -150,6 +154,9 @@ struct SweepParams {
     /* interval-censored observations (read by the IV instance of the MHRS kernels only; nullptr = no bounds set):
      * u per position, same layout as y, +inf where there is no bound; and the bound of each tail item, indexed like items */
     const double *u; double *item_u;
+    /* method 64, several chains (pht_engine_set_chains): chains 0 .. chains-1, each with its own model block, stats block,
+     * table and Philox key (ckeys[2c], ckeys[2c+1]) and observation counter cnext[c]; chain 0's blocks come first */
+    int chains; const uint32_t *ckeys; unsigned long long *cnext;
 };
 
 struct UpdateParams {
@@ -159,6 +166,9 @@ struct UpdateParams {
     int n, m, zbits; uint32_t k0, k1;
     const double *beta;        /* Dirichlet prior of the start distribution (n), nullptr: pi stays as it is */
     double *pires;             /* res_rows x n draws of pi, nullptr when pi is not inferred */
+    /* several chains (method 64): one block of k_assemble / k_update / k_unif_table per chain; chain c's rows of res and
+     * pires start at c x res_rows; ckeys as in SweepParams (nullptr: k0, k1); k_assemble zeroes cnext[c] when set */
+    int chains; const uint32_t *ckeys; unsigned long long *cnext;
 };
 
 /* all-reduce of the statistics block through the exchange windows */
@@ -192,11 +202,11 @@ size_t pht_mhrs_smem_bytes(int n);
 /* method 64 (k_unif.cu): log k! into a new table; the per-sweep table kernel (tmax: the longest time span of the shard,
  * max of y and of u - y); the path kernel and its grid.  The table (pht_unif.h, capacity PHT_UNIF_CAP powers) is a
  * kernel argument of its own, so that SweepParams / UpdateParams -- and the other kernels' code -- stay as they are. */
-cudaError_t pht_unif_init(double *tab, int n, int cap, cudaStream_t st);
+cudaError_t pht_unif_init(double *tab, int n, int cap, int chains, cudaStream_t st);   /* log k! of `chains` tables */
 size_t pht_unif_table_doubles(int n, int cap);
 cudaError_t pht_launch_unif_table(const UpdateParams &p, double *tab, double tmax, cudaStream_t st);
 cudaError_t pht_launch_unif(const SweepParams &p, const double *tab, int grid_blocks, cudaStream_t st);
-int pht_unif_grid_blocks(int device, int n);
+int pht_unif_grid_blocks(int device, int n, bool chains);   /* chains: the kernel of several chains (k_unif_chain_paths) */
 /* method 64, delayed entry (k_unif.cu; pht_engine_set_entry): a list of observations with entry ages and its buffers.
  * Like the table, every pointer is a kernel argument of its own. */
 struct UnifEntry {

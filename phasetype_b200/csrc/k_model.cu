@@ -9,6 +9,9 @@
  *   k_update    gather Nsum / zsum per parameter (:340-355) and the conjugate
  *               Gamma draw (:365-366) from the Philox parameter stream.
  *
+ * With several chains (method 64, pht_engine_set_chains) both run one block per
+ * chain, block c on chain c's model, statistics block, key and result rows.
+ *
  * Row i of every matrix is handled by thread i with the reference's own loop
  * order, so each value is bit-identical to the host computation.
  */
@@ -20,16 +23,19 @@
 __global__ void __launch_bounds__(64) k_assemble(UpdateParams p) {
     const int n = p.n, n1 = n + 1, tid = threadIdx.x;
     const ModelLayout L = ModelLayout::make(n, p.m);
-    double *M = p.model;
+    const int c = blockIdx.x;                /* chain (grid = chains) */
+    double *M = p.model + (size_t)c * L.total;
+    long long *stats = p.stats + (size_t)c * stats_len(n);
     const double *theta = M + L.theta;
     double *TT = M + L.TT, *S = M + L.S, *s = M + L.s;
     const bool first = p.state->first_assembly != 0;
 
-    for (int i = tid; i < stats_len(n); i += blockDim.x) p.stats[i] = 0;
-    if (tid == 0) {
+    for (int i = tid; i < stats_len(n); i += blockDim.x) stats[i] = 0;
+    if (tid == 0 && c == 0) {
         p.state->next_obs = 0ull; p.state->unit_counter = 0ull; p.state->replay_next = 0ull;
         p.state->n_items = 0u; p.state->n_pend[0] = 0u; p.state->n_pend[1] = 0u; p.state->n_done = 0u;
     }
+    if (tid == 0 && p.cnext != nullptr) p.cnext[c] = 0ull;
     if (tid <= n) {
         const int i = tid;
         for (int j = 0; j <= n; j++) {
@@ -88,10 +94,17 @@ __global__ void __launch_bounds__(128) k_update(UpdateParams p) {
     const ModelLayout L = ModelLayout::make(n, m);
     const uint32_t iter = p.state->iter;
     const uint32_t row = p.state->res_row;
-    const long long *Nacc = p.stats, *zlo = p.stats + n * n + n, *zhi = p.stats + n * n + 2 * n;
+    /* chain c (grid = chains): its model, statistics, key and rows */
+    const int c = blockIdx.x;
+    double *model = p.model + (size_t)c * L.total;
+    const long long *stats = p.stats + (size_t)c * stats_len(n);
+    const uint32_t k0 = p.ckeys ? p.ckeys[2 * c] : p.k0, k1 = p.ckeys ? p.ckeys[2 * c + 1] : p.k1;
+    double *res = p.res ? p.res + (size_t)c * p.res_rows * m : nullptr;
+    double *pires = p.pires ? p.pires + (size_t)c * p.res_rows * n : nullptr;
+    const long long *Nacc = stats, *zlo = stats + n * n + n, *zhi = stats + n * n + 2 * n;
     const double zscale = pht_u2d((uint64_t)(1023 - p.zbits) << 52);      /* 2^-zbits */
     /* some rank raised its error word this sweep: every rank learns it here and stops at the next synchronisation */
-    if (threadIdx.x == 0 && p.stats[stats_len(n) - 1] != 0 && p.state->error == 0) atomicOr(&p.state->error, 128);
+    if (threadIdx.x == 0 && stats[stats_len(n) - 1] != 0 && p.state->error == 0) atomicOr(&p.state->error, 128);
     for (int v = threadIdx.x; v < m; v += blockDim.x) {
         long long Nsum = 0; double zsum = 0.0;
         /* the reference walks prepend lists, i.e. cells in reverse insertion order (:340-355) */
@@ -104,20 +117,20 @@ __global__ void __launch_bounds__(128) k_update(UpdateParams p) {
             const double zi = (double)(long long)tot * zscale;
             zsum += zi / p.C[i + j * n1];
         }
-        pht_stream st; st.k0 = p.k0; st.k1 = p.k1;
+        pht_stream st; st.k0 = k0; st.k1 = k1;
         pht_stream_seek(&st, iter, PHT_OBS_PARAM, (uint32_t)v, 0);
         const double th = pht_rgamma(&st, p.nu[v] + (double)Nsum, 1.0 / (p.zeta[v] + zsum));   /* :366 */
-        p.model[L.theta + v] = th;
-        if (p.res != nullptr && row < (uint32_t)p.res_rows) p.res[(size_t)row * m + v] = th;
+        model[L.theta + v] = th;
+        if (res != nullptr && row < (uint32_t)p.res_rows) res[(size_t)row * m + v] = th;
     }
     /* start distribution: pi | paths ~ Dirichlet(beta + B), B = start-state counts of the sweep (the conjugate update the
      * reference leaves as FIX ME, src/PHT_MCMC_Aslett.c:190-193; beta is R/phtMCMC2.R:20-21's prior).  Drawn as n
      * Gamma(beta_i + B_i, 1) variates from parameter sub-streams m .. m+n-1, normalised in index order. */
     __shared__ double gpi[PHT_NMAX];
     if (p.beta != nullptr) {
-        const long long *Bacc = p.stats + n * n;
+        const long long *Bacc = stats + n * n;
         for (int i = threadIdx.x; i < n; i += blockDim.x) {
-            pht_stream st; st.k0 = p.k0; st.k1 = p.k1;
+            pht_stream st; st.k0 = k0; st.k1 = k1;
             pht_stream_seek(&st, iter, PHT_OBS_PARAM, (uint32_t)(m + i), 0);
             gpi[i] = pht_rgamma(&st, p.beta[i] + (double)Bacc[i], 1.0);
         }
@@ -129,11 +142,15 @@ __global__ void __launch_bounds__(128) k_update(UpdateParams p) {
             for (int i = 0; i < n; i++) sum += gpi[i];
             for (int i = 0; i < n; i++) {
                 const double v = gpi[i] / sum;
-                p.model[L.pi + i] = v;
-                if (p.pires != nullptr && row < (uint32_t)p.res_rows) p.pires[(size_t)row * n + i] = v;
+                model[L.pi + i] = v;
+                if (pires != nullptr && row < (uint32_t)p.res_rows) pires[(size_t)row * n + i] = v;
             }
         }
-        p.state->iter = iter + 1; p.state->first_assembly = 0; p.state->res_row = row + 1;
+        /* Every block read iter and res_row on entry, so the sweep may advance only once all blocks have: the last block
+         * to finish (a ticket taken after its reads) advances it and resets the ticket for the next launch. */
+        bool last = gridDim.x == 1;
+        if (!last) { __threadfence(); last = atomicAdd(&p.state->update_ticket, 1u) == gridDim.x - 1; }
+        if (last) { p.state->update_ticket = 0u; p.state->iter = iter + 1; p.state->first_assembly = 0; p.state->res_row = row + 1; }
     }
 }
 
@@ -202,11 +219,11 @@ cudaError_t pht_launch_spectral(const UpdateParams &p, const double *inject, cud
 }
 
 cudaError_t pht_launch_assemble(const UpdateParams &p, cudaStream_t st) {
-    k_assemble<<<1, 64, 0, st>>>(p);
+    k_assemble<<<p.chains, 64, 0, st>>>(p);
     return cudaGetLastError();
 }
 cudaError_t pht_launch_update(const UpdateParams &p, cudaStream_t st) {
-    k_update<<<1, 128, 0, st>>>(p);
+    k_update<<<p.chains, 128, 0, st>>>(p);
     return cudaGetLastError();
 }
 

@@ -3,14 +3,15 @@
  * sub-generator (Hobolth & Stone 2009, section 3.3), for exact, right-, interval- and left-censored observations.
  * Law, table, truncation and draw order: pht_unif.h, which this file and the host restatement share.
  *
- *   k_unif_lgk     once per engine: log k! for k < capacity
+ *   k_unif_lgk     once per engine (and per pht_engine_set_chains): log k! for k < capacity, in every chain's table
  *   k_unif_table   once per sweep (in place of k_spectral_solve): lambda, R = I + S/lambda, r = s/lambda and the
- *                  powers R^k, pi R^k, g_k for k <= K_sweep = K(lambda t_max), by sequential products.  One block: the
- *                  products are a chain of K_sweep dependent steps, each n^2 + 2n dot products of length n, so one
- *                  step is one pass of the block over the entries with the previous power in shared memory.
+ *                  powers R^k, pi R^k, g_k for k <= K_sweep = K(lambda t_max), by sequential products.  One block per
+ *                  chain: the products are a chain of K_sweep dependent steps, each n^2 + 2n dot products of length n, so
+ *                  one step is one pass of the block over the entries with the previous power in shared memory.
  *   k_unif_paths   one observation per lane, persistent warps refilled from the global counter (Dispenser); the two
  *                  per-lane n-vectors of scratch live in shared-memory slabs (stride THREADS), the powers in global
- *                  memory (33 MB at n = 32 and full capacity; what a sweep touches stays in L2).
+ *                  memory (33 MB per chain at n = 32 and full capacity; what a sweep touches stays in L2).
+ *   k_unif_chain_paths  the same per observation for several chains: the blocks walk the chains (below)
  *
  * Delayed entry (only when entry ages are set, pht_engine_set_entry; law and draw order in pht_unif.h):
  *   k_unif_entry_table  sigma_k, phi_k for k <= K_sweep, after k_unif_table (one block)
@@ -39,16 +40,21 @@ struct UnifCount { const SweepParams *p; unsigned int *Nacc; long out_idx; int n
 #define UNIF_THREADS 128
 #define UNIF_TABLE_THREADS 256
 
+/* block c fills table c */
 __global__ void k_unif_lgk(double *tab, int n, int cap) {
-    if (threadIdx.x == 0 && blockIdx.x == 0) pht_unif_lgk_fill(tab + pht_unif_layout_make(n, cap).lgk, cap);
+    const pht_unif_layout L = pht_unif_layout_make(n, cap);
+    if (threadIdx.x == 0) pht_unif_lgk_fill(tab + (size_t)blockIdx.x * L.total + L.lgk, cap);
 }
 
+/* block c builds chain c's table from chain c's model block (grid = chains) */
 __global__ void __launch_bounds__(UNIF_TABLE_THREADS) k_unif_table(UpdateParams p, double *tab, double tmax) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int n = p.n, nn = n * n, tid = threadIdx.x, cap = PHT_UNIF_CAP;
     const ModelLayout ML = ModelLayout::make(n, p.m);
     const pht_unif_layout L = pht_unif_layout_make(n, cap);
-    const double *S = p.model + ML.S, *s = p.model + ML.s, *pi = p.model + ML.pi;
+    const double *model = p.model + (size_t)blockIdx.x * ML.total;
+    tab += (size_t)blockIdx.x * L.total;
+    const double *S = model + ML.S, *s = model + ML.s, *pi = model + ML.pi;
     double *sR = reinterpret_cast<double *>(smem_raw), *sr = sR + nn;
     double *P0 = sr + n, *P1 = P0 + nn, *q0 = P1 + nn, *q1 = q0 + n, *g0 = q1 + n, *g1 = g0 + n;
     const double lam = pht_unif_lambda(n, S);
@@ -137,6 +143,90 @@ __global__ void __launch_bounds__(THREADS) k_unif_paths(SweepParams p, const dou
     if (err) atomicOr(&p.state->error, err);
     __syncthreads();
     block_flush<THREADS>(p, n, sm.Nacc, sm.Bacc, sm.zlo, sm.zhi);
+    unsigned long long w_paths = c_paths;
+    for (int o = 16; o > 0; o >>= 1) w_paths += __shfl_down_sync(FULL, w_paths, o);
+    if ((tid & 31) == 0) atomicAdd(&p.state->counters[PHT_CNT_PATHS], w_paths);
+}
+
+/* Several chains (pht_engine_set_chains; one chain and parity mode run k_unif_paths above, 2 % faster at one chain on the
+ * C3 shape).  Persistent blocks walk the chains: block b starts at chain
+ * b mod chains, loads that chain's model into shared memory and its warps take observations 32 at a time from the chain's
+ * counter, with the chain's key.  When the counter runs dry the block flushes its accumulators into the chain's statistics
+ * block and moves on to the next chain that still has work, until it has passed every chain once.  Whether a chain has
+ * work left is read from its counter with plain loads, 32 chains per warp-wide look; every statistic is an integer sum,
+ * so which block draws which observation does not change the result. */
+template <int THREADS>
+__global__ void __launch_bounds__(THREADS, 7) /* 7 blocks of 128 per SM: at most 72 registers */ k_unif_chain_paths(SweepParams p, const double *tab) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    /* the walk's state lives in shared memory, re-read after each barrier, so that it holds no register in the path loop */
+    __shared__ int s_chain, s_left; __shared__ uint32_t s_key[2];
+    __shared__ const double *s_tab; __shared__ unsigned long long *s_counter;
+    const int n = p.n, tid = threadIdx.x;
+    const unsigned FULL = 0xffffffffu;
+    const ModelLayout ML = ModelLayout::make(n, p.m);
+    const int chains = p.chains;
+    UnifSmem<THREADS> sm; sm.carve(smem_raw, n);
+    const uint32_t iter = p.state->iter;
+    unsigned c_paths = 0; int err = 0;
+    Dispenser disp; disp.init(p);
+    UnifCount ctx; ctx.p = &p; ctx.Nacc = sm.Nacc; ctx.n = n; ctx.out_idx = 0;
+    if (tid == 0) { s_chain = (int)(blockIdx.x % (unsigned)chains); s_left = chains; }   /* current chain; chains not passed yet */
+    __syncthreads();
+    for (;;) {
+        if (tid < 32) {                        /* the first chain from the current one on (cyclically) with work left */
+            const int c = s_chain, left = s_left;
+            const unsigned long long span = (unsigned long long)p.l_local;
+            int found = -1;
+            for (int k = 0; k < left && found < 0; k += 32) {
+                int cc = c + k + tid; if (cc >= chains) cc -= chains;
+                const bool work = k + tid < left && *(volatile unsigned long long *)&p.cnext[cc] < span;
+                const unsigned b = __ballot_sync(FULL, work);
+                if (b) found = k + __ffs(b) - 1;
+            }
+            if (tid == 0) {
+                int cn = c + (found < 0 ? 0 : found); if (cn >= chains) cn -= chains;
+                s_chain = cn; s_left = found < 0 ? 0 : left - found;
+                s_key[0] = p.ckeys[2 * cn]; s_key[1] = p.ckeys[2 * cn + 1];
+                s_tab = tab + (size_t)cn * pht_unif_layout_make(n, PHT_UNIF_CAP).total; s_counter = p.cnext + cn;
+            }
+        }
+        __syncthreads();
+        if (s_left == 0) break;
+        {
+            const double *model = p.model + (size_t)s_chain * ML.total;
+            for (int i = tid; i < n * n; i += THREADS) sm.Nacc[i] = 0u;
+            for (int i = tid; i < (n + 1) * (n + 1); i += THREADS) sm.cum[i] = model[ML.cum + i];
+            for (int i = tid; i < n; i += THREADS) {
+                sm.s[i] = model[ML.s + i]; sm.scale[i] = model[ML.scale + i]; sm.pi[i] = model[ML.pi + i];
+                sm.zlo[i] = 0ull; sm.zhi[i] = 0; sm.Bacc[i] = 0u;
+            }
+        }
+        __syncthreads();
+        disp.next = disp.end = 0ull; disp.exhausted = false;
+        for (;;) {
+            const unsigned long long o = disp.take_from(s_counter, FULL, true);
+            const bool have = o != ~0ull;
+            if (__ballot_sync(FULL, have) == 0u) { if (disp.exhausted) break; continue; }
+            if (have) {
+                const uint32_t obs_local = p.perm ? p.perm[o] : (uint32_t)o;
+                pht_stream st; st.k0 = s_key[0]; st.k1 = s_key[1];
+                pht_stream_seek(&st, iter, p.obs_rank + obs_local * p.obs_world, 0u, 0u);
+                ctx.out_idx = (long)o - p.first;
+                int B = 0;
+                err |= pht_unif_path(s_tab, n, PHT_UNIF_CAP, sm.s, sm.scale, sm.cum, sm.pi, p.y[o], p.cens[o],
+                                     p.u ? p.u[o] : INFINITY, &st, sm.Za + tid, sm.Zb + tid, THREADS, &ctx, &B);
+                path_flush<THREADS>(p, n, sm.Za, sm.zlo, sm.zhi, sm.Bacc, B, ctx.out_idx);
+                c_paths++;
+            }
+            __syncwarp();
+        }
+        __syncthreads();
+        block_flush_to<THREADS>(p.stats + (size_t)s_chain * stats_len(n), n, sm.Nacc, sm.Bacc, sm.zlo, sm.zhi);
+        __syncthreads();
+        if (tid == 0) { int cn = s_chain + 1; if (cn == chains) cn = 0; s_chain = cn; s_left = s_left - 1; }
+        __syncthreads();
+    }
+    if (err) atomicOr(&p.state->error, err);
     unsigned long long w_paths = c_paths;
     for (int o = 16; o > 0; o >>= 1) w_paths += __shfl_down_sync(FULL, w_paths, o);
     if ((tid & 31) == 0) atomicAdd(&p.state->counters[PHT_CNT_PATHS], w_paths);
@@ -273,8 +363,8 @@ cudaError_t pht_launch_unif_entry(const UpdateParams &u, const SweepParams &p, c
     return cudaGetLastError();
 }
 
-cudaError_t pht_unif_init(double *tab, int n, int cap, cudaStream_t st) {
-    k_unif_lgk<<<1, 32, 0, st>>>(tab, n, cap);
+cudaError_t pht_unif_init(double *tab, int n, int cap, int chains, cudaStream_t st) {
+    k_unif_lgk<<<chains, 32, 0, st>>>(tab, n, cap);
     return cudaGetLastError();
 }
 
@@ -282,20 +372,23 @@ size_t pht_unif_table_doubles(int n, int cap) { return (size_t)pht_unif_layout_m
 
 cudaError_t pht_launch_unif_table(const UpdateParams &p, double *tab, double tmax, cudaStream_t st) {
     const size_t smem = sizeof(double) * (size_t)(3 * p.n * p.n + 7 * p.n);
-    k_unif_table<<<1, UNIF_TABLE_THREADS, smem, st>>>(p, tab, tmax);
+    k_unif_table<<<p.chains, UNIF_TABLE_THREADS, smem, st>>>(p, tab, tmax);
     return cudaGetLastError();
 }
 
-int pht_unif_grid_blocks(int device, int n) {
+int pht_unif_grid_blocks(int device, int n, bool chains) {
     const size_t smem = UnifSmem<UNIF_THREADS>::bytes(n);
     int per_sm = 0, sms = 0;
-    if (cudaFuncSetAttribute(k_unif_paths<UNIF_THREADS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return -1;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_unif_paths<UNIF_THREADS>, UNIF_THREADS, smem) != cudaSuccess) return -1;
+    const void *k = chains ? (const void *)k_unif_chain_paths<UNIF_THREADS> : (const void *)k_unif_paths<UNIF_THREADS>;
+    if (cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return -1;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, UNIF_THREADS, smem) != cudaSuccess) return -1;
     if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device) != cudaSuccess) return -1;
     return per_sm * sms;
 }
 
 cudaError_t pht_launch_unif(const SweepParams &p, const double *tab, int grid_blocks, cudaStream_t st) {
-    k_unif_paths<UNIF_THREADS><<<grid_blocks, UNIF_THREADS, UnifSmem<UNIF_THREADS>::bytes(p.n), st>>>(p, tab);
+    if (p.chains > 1 && p.outB == nullptr)
+        k_unif_chain_paths<UNIF_THREADS><<<grid_blocks, UNIF_THREADS, UnifSmem<UNIF_THREADS>::bytes(p.n), st>>>(p, tab);
+    else k_unif_paths<UNIF_THREADS><<<grid_blocks, UNIF_THREADS, UnifSmem<UNIF_THREADS>::bytes(p.n), st>>>(p, tab);
     return cudaGetLastError();
 }

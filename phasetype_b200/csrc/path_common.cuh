@@ -24,10 +24,14 @@ struct Dispenser {
     /* every lane of the warp calls this with the same `idle` ballot; returns the observation index for this
      * lane or ~0ull when it got none */
     __device__ __forceinline__ unsigned long long take(const SweepParams &p, unsigned idle, bool me_idle) {
+        return take_from(&p.state->next_obs, idle, me_idle);
+    }
+    /* the same from another counter (method 64 with several chains: one counter per chain) */
+    __device__ __forceinline__ unsigned long long take_from(unsigned long long *counter, unsigned idle, bool me_idle) {
         const unsigned FULL = 0xffffffffu; const int lane = threadIdx.x & 31;
         if (next == end && !exhausted) {
             unsigned long long base = 0;
-            if (lane == 0) base = obs_begin + atomicAdd(&p.state->next_obs, (unsigned long long)PATH_CHUNK);
+            if (lane == 0) base = obs_begin + atomicAdd(counter, (unsigned long long)PATH_CHUNK);
             base = __shfl_sync(FULL, base, 0);
             next = base < obs_end ? base : obs_end;
             end = base + PATH_CHUNK < obs_end ? base + PATH_CHUNK : obs_end;
@@ -148,18 +152,25 @@ __device__ __forceinline__ void count_transition(const SweepParams &p, int n, un
     else atomicAdd(&Nacc[from + to * n], 1u);
 }
 
-/* block accumulators -> global statistics block */
+/* block accumulators -> a statistics block */
 template <int THREADS>
-__device__ __forceinline__ void block_flush(const SweepParams &p, int n, const unsigned int *Nacc, const unsigned int *Bacc,
-                                            const unsigned long long *zlo, const long long *zhi) {
-    if (p.outB != nullptr) return;
-    unsigned long long *g = reinterpret_cast<unsigned long long *>(p.stats);
+__device__ __forceinline__ void block_flush_to(long long *stats, int n, const unsigned int *Nacc, const unsigned int *Bacc,
+                                               const unsigned long long *zlo, const long long *zhi) {
+    unsigned long long *g = reinterpret_cast<unsigned long long *>(stats);
     for (int i = threadIdx.x; i < n * n; i += THREADS) if (Nacc[i]) atomicAdd(&g[i], (unsigned long long)Nacc[i]);
     for (int i = threadIdx.x; i < n; i += THREADS) {
         if (Bacc[i]) atomicAdd(&g[n * n + i], (unsigned long long)Bacc[i]);
         if (zlo[i]) atomicAdd(&g[n * n + n + i], zlo[i]);
         if (zhi[i]) atomicAdd(&g[n * n + 2 * n + i], (unsigned long long)zhi[i]);
     }
+}
+
+/* block accumulators -> global statistics block */
+template <int THREADS>
+__device__ __forceinline__ void block_flush(const SweepParams &p, int n, const unsigned int *Nacc, const unsigned int *Bacc,
+                                            const unsigned long long *zlo, const long long *zhi) {
+    if (p.outB != nullptr) return;
+    block_flush_to<THREADS>(p.stats, n, Nacc, Bacc, zlo, zhi);
 }
 
 #endif
