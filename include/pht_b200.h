@@ -202,6 +202,31 @@ int pht_engine_set_chain_theta(pht_engine *e, const double *theta, uint32_t next
 int pht_engine_get_chain_theta(pht_engine *e, double *theta);
 int pht_engine_chain_rows(pht_engine *e, int rows, double *theta_out, double *pi_out);
 
+/* Groups of observations with their own generator structure, sharing one parameter vector (method 64 only): treatment and
+ * control arms, two hospitals, two production lots.  Group g's structure (T_g, C_g) maps the engine's m parameters theta
+ * (with the engine's nu and zeta; m <= n(n+1) as pht_engine_create takes it) onto its own n-phase generator, e.g. a
+ * Coxian whose progression rates are shared and whose exit rates are per group.  The model stays conjugate: parameter k's full conditional is a Gamma whose statistics
+ * sum, over the groups in ascending order, every cell of the group's structure that carries k (within a group in the order
+ * a single structure uses, the reference's z / C gather included).  pi is one vector per chain, shared by all groups; its
+ * Dirichlet update sums the start-state counts of every group.  Each observation's path is drawn on its own group's model
+ * and is, bit for bit, the path an engine configured with (T_g, C_g) draws for it from the same key, sweep, theta and pi.
+ * pht_engine_set_groups: T and C hold G structures of (n+1)^2 entries each, column-major like pht_config::T / C; group_local
+ * holds the group 0..G-1 of every local observation, in the order of y_local.  T = NULL returns to the configured structure
+ * (G, C and group_local are then ignored).  G = 1 with the configured T and C and every observation in group 0 is the
+ * engine as it was, bit for bit.  Every chain keeps its theta and pi.  The sweep builds one table per group, spanning that
+ * group's own observations, and one per chain; chains x G tables in all (33 MB each at n = 32).
+ * pht_engine_group_stats: as pht_engine_sweep_stats (chain 0, one sweep, no update), per group: N (G x n*n), B (G x n),
+ * zfix (G x n); pht_engine_sweep_stats returns their sum over the groups.  pht_engine_paths records each observation's
+ * path drawn on its own group's model, in upload order.
+ * Refused, each with its own message and leaving the engine as it was: any method but 64; world > 1 (the all-reduce carries
+ * one statistics block); G > 1 with entry ages set (pht_engine_set_entry, in either order: the ghost paths are drawn on
+ * one model); G outside 1..PHT_MAX_GROUPS or chains x G above PHT_MAX_CHAINS (pht_engine_set_chains checks the same
+ * product); a T_g that pht_engine_create would refuse; a parameter used by no group's structure; a group id out of range;
+ * a failed allocation. */
+#define PHT_MAX_GROUPS 64
+int pht_engine_set_groups(pht_engine *e, int G, const int *T, const double *C, const int *group_local);
+int pht_engine_group_stats(pht_engine *e, long long *N, long long *B, long long *zfix);
+
 /* run `nsweeps` Gibbs sweeps; row r of out (nsweeps x m, row-major) is the draw of sweep r.
  * out may be NULL (results stay on the device; fetch later with pht_engine_get_theta). */
 int pht_engine_run(pht_engine *e, int nsweeps, double *out);

@@ -21,12 +21,14 @@ SYMBOLS = [
     "pht_engine_counters", "pht_fp64_fma_rate", "pht_engine_set_l2_flush", "pht_engine_peer_handle", "pht_engine_peer_attach", "pht_engine_round_trace", "pht_engine_set_pi", "pht_engine_get_pi", "pht_engine_pi_rows",
     "pht_engine_set_upper", "pht_engine_set_entry", "pht_engine_entry_paths",
     "pht_engine_set_chains", "pht_engine_set_chain_theta", "pht_engine_get_chain_theta", "pht_engine_chain_rows",
+    "pht_engine_set_groups", "pht_engine_group_stats",
 ]
 PEER_HANDLE_BYTES = 128
 # method 64 (include/pht_b200.h PHT_METHOD_UNIF): the uniformisation path sampler; exact, right-, interval- and
 # left-censored observations, any sub-generator; delayed entry (Engine.set_entry) is this method's alone
 METHOD_UNIF = 64
 MAX_CHAINS = 1024            # include/pht_b200.h PHT_MAX_CHAINS: chains one METHOD_UNIF engine can run (Engine.set_chains)
+MAX_GROUPS = 64              # include/pht_b200.h PHT_MAX_GROUPS: groups with their own structure (Engine.set_groups)
 CNT_NAMES = ["paths", "attempts", "jumps", "dens_evals", "env_updates", "brent_evals", "arms_calls",
              "metrop_rejects", "nonfinite", "deferred", "tail_rounds", "errors", "launches", "ns_lane", "ns_tail", "ns_replay",
              "ns_global", "ns_xwait", "global_rounds", "global_items"]
@@ -89,6 +91,8 @@ def lib():
     L.pht_engine_set_chain_theta.argtypes = [C.c_void_p, _dp, C.c_uint32]
     L.pht_engine_get_chain_theta.argtypes = [C.c_void_p, _dp]
     L.pht_engine_chain_rows.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]
+    L.pht_engine_set_groups.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
+    L.pht_engine_group_stats.argtypes = [C.c_void_p, _lp, _lp, _lp]
     L.pht_engine_peer_handle.argtypes = [C.c_void_p, C.c_void_p]
     L.pht_engine_peer_attach.argtypes = [C.c_void_p, C.c_void_p]
     _lib = L
@@ -130,6 +134,7 @@ class Engine:
                      self.zbits, int(mhrs_cap), 1 if use_graph else 0)
         self._h = C.c_void_p()
         self.chains = 1
+        self.groups = 1
         _check(L.pht_engine_create(C.byref(self._h), C.byref(cfg), y_local if self.l_local else np.zeros(1),
                                    cens_local if self.l_local else np.zeros(1, dtype=np.int32), self.l_local))
 
@@ -317,6 +322,39 @@ class Engine:
         out = np.zeros((self.chains, int(rows), self.n))
         _check(lib().pht_engine_chain_rows(self._h, int(rows), None, out.ctypes.data))
         return out
+
+    def set_groups(self, T, Cmat=None, group=None):
+        """Groups of observations with their own structure over the one parameter vector (METHOD_UNIF only, one rank, no
+        entry ages with more than one group): T and Cmat shaped (G, ...), group g's T and C flattened as the constructor
+        takes them; group[k] in 0..G-1 is the group of local observation k.  Every chain keeps its theta and pi; group
+        g's observations are drawn on (T[g], Cmat[g]), and theta's update sums every group's cells.  T = None returns to
+        the configured structure."""
+        if T is None:
+            _check(lib().pht_engine_set_groups(self._h, 0, None, None, None))
+            self.groups = 1
+            return
+        t = np.asarray(T, dtype=np.int32); c = np.asarray(Cmat, dtype=np.float64)
+        G, n1 = int(t.shape[0]), (self.n + 1) ** 2
+        if t.size != G * n1 or c.size != G * n1:
+            raise EngineError("set_groups: T %s and C %s, expected %d structures of %d entries each" % (t.shape, c.shape, G, n1))
+        t = np.ascontiguousarray(t.reshape(G, n1)); c = np.ascontiguousarray(c.reshape(G, n1))
+        if not G:
+            t = np.zeros((1, n1), dtype=np.int32); c = np.zeros((1, n1))
+        g = np.ascontiguousarray(group, dtype=np.int32)
+        if g.shape != (self.l_local,):
+            raise EngineError("set_groups: %d group ids for %d local observations" % (g.size, self.l_local))
+        if not self.l_local:
+            g = np.zeros(1, dtype=np.int32)
+        _check(lib().pht_engine_set_groups(self._h, G, t.ctypes.data, c.ctypes.data, g.ctypes.data))
+        self.groups = G
+
+    def group_stats(self):
+        """One sweep's statistics of chain 0 per group, without an update: N (G, n*n), B (G, n), zfix (G, n); their sum
+        over the groups is sweep_stats()."""
+        n, G = self.n, self.groups
+        N = np.zeros(G * n * n, dtype=np.int64); B = np.zeros(G * n, dtype=np.int64); z = np.zeros(G * n, dtype=np.int64)
+        _check(lib().pht_engine_group_stats(self._h, N, B, z))
+        return N.reshape(G, n * n), B.reshape(G, n), z.reshape(G, n)
 
     def round_trace(self):
         """(48, 8) array: per tail round number, ns search / ns barrier / ns advance / sum of pending / sum of K / attempts run /

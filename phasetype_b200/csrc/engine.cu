@@ -96,6 +96,14 @@ struct pht_engine {
      * first; the chains' Philox keys (2 x u32 each) and observation counters; the seed that NULL keys count from */
     int chains = 1; uint32_t *d_keys = nullptr; unsigned long long *d_cnext = nullptr; uint64_t base_seed = 0;
     int chain_blocks = 0;              /* grid of the several-chain path kernel */
+    /* method 64, groups (pht_engine_set_groups): G structures in d_T / d_C and the (group, cell) CSR; model, stats, table and
+     * counters per (chain, group) unit, block c G + g.  With G > 1: each group's table span (gtmax), its range of the
+     * grouped layout (gofs, G + 1 offsets), the layout itself (by group, then by decreasing y: y, flags, permutation and u
+     * when bounds are set) and the host copy of the group ids in upload order */
+    int groups = 1;
+    double *d_gtmax = nullptr; unsigned long long *d_gofs = nullptr;
+    double *d_gys = nullptr, *d_gus = nullptr; uint8_t *d_gcs = nullptr; uint32_t *d_gperm = nullptr;
+    std::vector<uint8_t> h_group;
     /* method 64, delayed entry (pht_engine_set_entry): the ages in upload order (device and host), the truncated
      * observations (a > 0) by decreasing a with their local indices, their ghost counts and offsets, the entry tables,
      * the ghost counter, the scan's scratch and the ghost kernel's grid */
@@ -143,6 +151,11 @@ static SweepParams sweep_params(pht_engine *e) {
     if (e->peers_attached) { p.xw = e->d_xw; for (int r = 0; r < e->cfg.world && r < PHT_MAX_WORLD; r++) p.xpeer[r] = e->xpeer[r]; }
     if (e->d_u) { p.u = e->d_ys ? e->d_us : e->d_u; p.item_u = e->d_item_u; }
     p.chains = e->chains; p.ckeys = e->d_keys; p.cnext = e->d_cnext;
+    p.groups = e->groups;
+    if (e->groups > 1) {                           /* the grouped layout: each group a contiguous range (e->d_gofs) */
+        p.y = e->d_gys; p.cens = e->d_gcs; p.perm = e->d_gperm;
+        if (e->d_u) p.u = e->d_gus;
+    }
     return p;
 }
 static UpdateParams update_params(pht_engine *e, double *res, int res_rows) {
@@ -154,6 +167,7 @@ static UpdateParams update_params(pht_engine *e, double *res, int res_rows) {
     u.k0 = (uint32_t)e->cfg.seed; u.k1 = (uint32_t)(e->cfg.seed >> 32);
     u.beta = e->d_beta; u.pires = (e->d_beta && res) ? e->d_pires : nullptr;
     u.chains = e->chains; u.ckeys = e->d_keys; u.cnext = e->d_cnext;
+    u.groups = e->groups; u.gtmax = e->groups > 1 ? e->d_gtmax : nullptr;
     return u;
 }
 
@@ -218,7 +232,9 @@ static int enqueue_paths(pht_engine *e, const SweepParams &p, const uint32_t *id
         e->launches += 2; break;
     case PHT_METHOD_DCS: CU(pht_launch_dcs(p, e->grid_blocks, e->stream)); e->launches++; break;           /* unit machine + complex-spectrum kernel */
     case PHT_METHOD_MHS_HOBOLTH: CU(pht_launch_dcs(p, e->grid_blocks, e->stream, true)); e->launches++; break;
-    case PHT_METHOD_UNIF: CU(pht_launch_unif(p, e->d_unif, p.chains > 1 ? e->chain_blocks : e->grid_blocks, e->stream)); break;
+    case PHT_METHOD_UNIF:
+        CU(pht_launch_unif(p, e->d_unif, p.groups > 1 ? e->d_gofs : nullptr, p.chains > 1 || p.groups > 1 ? e->chain_blocks : e->grid_blocks, e->stream));
+        break;
     case PHT_METHOD_MHS_ASLETT:
         /* every observation through one kernel: the window list in parity mode, else the whole shard (identity) */
         if (lists_given) CU(pht_launch_mhs_aslett(p, e->grid_blocks, idx_exact, n_exact, e->stream));
@@ -299,7 +315,7 @@ extern "C" void pht_engine_destroy(pht_engine *e) {
     if (e->ev1) cudaEventDestroy(e->ev1);
     for (void *q : e->ipc_opened) cudaIpcCloseMemHandle(q);
     stage("events, ipc");
-    void *big[] = { e->d_keys, e->d_cnext, e->d_entry, e->d_ea, e->d_eobs, e->d_eM, e->d_eoff, e->d_enext, e->d_etab, e->d_escan, e->d_unif, e->d_u, e->d_us, e->d_item_u, e->d_recs, e->d_ys, e->d_cs, e->d_perm, e->d_y, e->d_cens, e->d_items /* arena: found, pend0, pend1, done live inside */, e->d_idx_exact, e->d_idx_cens,
+    void *big[] = { e->d_gtmax, e->d_gofs, e->d_gys, e->d_gus, e->d_gcs, e->d_gperm, e->d_keys, e->d_cnext, e->d_entry, e->d_ea, e->d_eobs, e->d_eM, e->d_eoff, e->d_enext, e->d_etab, e->d_escan, e->d_unif, e->d_u, e->d_us, e->d_item_u, e->d_recs, e->d_ys, e->d_cs, e->d_perm, e->d_y, e->d_cens, e->d_items /* arena: found, pend0, pend1, done live inside */, e->d_idx_exact, e->d_idx_cens,
                     e->d_glist, e->d_model, e->d_stats, e->d_state, e->d_T, e->d_C, e->d_nu, e->d_zeta, e->d_var_ptr, e->d_cell_i, e->d_cell_j, e->d_pires, e->d_res };
     for (void *b : big) pht_dev_free(b, e->stream);
     if (e->stream) cudaStreamSynchronize(e->stream);
@@ -615,7 +631,7 @@ extern "C" int pht_engine_set_theta(pht_engine *e, const double *theta, uint32_t
     if (!e || !theta) return fail("null argument");
     CU(cudaSetDevice(e->cfg.device));
     CU(cudaStreamSynchronize(e->stream));
-    for (int c = 0; c < e->chains; c++)           /* every chain */
+    for (int c = 0; c < e->chains * e->groups; c++)           /* every chain, in every group's block */
         CU(cudaMemcpy(e->d_model + (size_t)c * e->L.total + e->L.theta, theta, sizeof(double) * e->cfg.m, cudaMemcpyHostToDevice));
     return set_next_iter(e, next_iter);
 }
@@ -636,7 +652,7 @@ extern "C" int pht_engine_set_pi(pht_engine *e, const double *pi, const double *
         double sum = 0.0;
         for (int i = 0; i < n; i++) { if (!(pi[i] >= 0.0)) return fail("pi[%d] = %g is not a probability", i, pi[i]); sum += pi[i]; }
         if (!(sum > 0.999999 && sum < 1.000001)) return fail("pi sums to %g, not 1", sum);
-        for (int c = 0; c < e->chains; c++)       /* every chain */
+        for (int c = 0; c < e->chains * e->groups; c++)       /* every chain, in every group's block */
             CU(cudaMemcpy(e->d_model + (size_t)c * e->L.total + e->L.pi, pi, sizeof(double) * n, cudaMemcpyHostToDevice));
     }
     if (e->graph_exec) { cudaGraphExecDestroy(e->graph_exec); e->graph_exec = nullptr; }     /* kernel parameters change */
@@ -678,6 +694,8 @@ extern "C" int pht_engine_set_chains(pht_engine *e, int chains, const uint64_t *
     if (e->cfg.world > 1)
         return fail("several chains per engine need world = 1: the statistics all-reduce of a multi-rank run carries one chain's block");
     if (chains < 1 || chains > PHT_MAX_CHAINS) return fail("chains = %d outside 1..%d", chains, PHT_MAX_CHAINS);
+    if ((long)chains * e->groups > PHT_MAX_CHAINS)
+        return fail("chains x groups = %d x %d exceeds %d (pht_engine_set_groups)", chains, e->groups, PHT_MAX_CHAINS);
     if (chains > 1 && e->entry_set)
         return fail("%d chains asked while entry ages (delayed entry) are set: the ghost paths are drawn for one chain; clear them with pht_engine_set_entry(e, NULL) first", chains);
     std::vector<uint64_t> k((size_t)chains);
@@ -688,15 +706,16 @@ extern "C" int pht_engine_set_chains(pht_engine *e, int chains, const uint64_t *
     CU(cudaSetDevice(e->cfg.device));
     CU(cudaStreamSynchronize(e->stream));
     const int n = e->cfg.n;
-    if (chains > 1 && !e->chain_blocks) {
+    const int G = e->groups, units = chains * G;
+    if (units > 1 && !e->chain_blocks) {
         e->chain_blocks = pht_unif_grid_blocks(e->cfg.device, n, true);
         if (e->chain_blocks <= 0) { e->chain_blocks = 0; return fail("the several-chain path kernel does not fit on the device: %s", cudaGetErrorString(cudaGetLastError())); }
     }
     const size_t total = (size_t)e->L.total, slen = (size_t)stats_len(n), tab = pht_unif_table_doubles(n, PHT_UNIF_CAP);
     /* the new buffers first: a failed allocation leaves the engine as it was */
     double *model = nullptr, *unif = nullptr; long long *stats = nullptr; uint32_t *dkeys = nullptr; unsigned long long *cnext = nullptr;
-    const size_t bytes[] = { sizeof(double) * chains * total, sizeof(long long) * chains * slen, sizeof(double) * chains * tab,
-                             sizeof(uint32_t) * 2 * chains, sizeof(unsigned long long) * chains };
+    const size_t bytes[] = { sizeof(double) * units * total, sizeof(long long) * units * slen, sizeof(double) * units * tab,
+                             sizeof(uint32_t) * 2 * chains, sizeof(unsigned long long) * units };
     void **ptrs[] = { (void **)&model, (void **)&stats, (void **)&unif, (void **)&dkeys, (void **)&cnext };
     for (int b = 0; b < 5; b++) {
         const cudaError_t ce = pht_dev_alloc(ptrs[b], bytes[b], e->stream);
@@ -704,15 +723,15 @@ extern "C" int pht_engine_set_chains(pht_engine *e, int chains, const uint64_t *
             cudaGetLastError();
             for (int f = 0; f < b; f++) pht_dev_free(*ptrs[f], e->stream);
             cudaStreamSynchronize(e->stream); cudaGetLastError();
-            return fail("cannot allocate device memory for %d chains (%.1f MB, of which the uniformisation tables take %.1f MB per chain): %s",
+            return fail("cannot allocate device memory for %d chains (%.1f MB, of which the uniformisation tables take %.1f MB per chain and group): %s",
                         chains, (bytes[0] + bytes[1] + bytes[2] + bytes[3] + bytes[4]) / 1e6, sizeof(double) * tab / 1e6, cudaGetErrorString(ce));
         }
     }
     /* every chain starts from chain 0's current theta and pi (the rest of a model block is rebuilt every sweep) */
-    for (int c = 0; c < chains; c++)
+    for (int c = 0; c < units; c++)
         CU(cudaMemcpyAsync(model + (size_t)c * total, e->d_model, sizeof(double) * total, cudaMemcpyDeviceToDevice, e->stream));
     CU(cudaMemsetAsync(stats, 0, bytes[1], e->stream));
-    CU(pht_unif_init(unif, n, PHT_UNIF_CAP, chains, e->stream));       /* log k! in every chain's table */
+    CU(pht_unif_init(unif, n, PHT_UNIF_CAP, units, e->stream));       /* log k! in every unit's table */
     std::vector<uint32_t> hk(2 * (size_t)chains);
     for (int c = 0; c < chains; c++) { hk[2 * (size_t)c] = (uint32_t)k[(size_t)c]; hk[2 * (size_t)c + 1] = (uint32_t)(k[(size_t)c] >> 32); }
     CU(cudaMemcpyAsync(dkeys, hk.data(), bytes[3], cudaMemcpyHostToDevice, e->stream));
@@ -732,8 +751,8 @@ extern "C" int pht_engine_set_chain_theta(pht_engine *e, const double *theta, ui
     if (!e || !theta) return fail("null argument");
     CU(cudaSetDevice(e->cfg.device));
     CU(cudaStreamSynchronize(e->stream));
-    for (int c = 0; c < e->chains; c++)
-        CU(cudaMemcpy(e->d_model + (size_t)c * e->L.total + e->L.theta, theta + (size_t)c * e->cfg.m, sizeof(double) * e->cfg.m, cudaMemcpyHostToDevice));
+    for (int c = 0; c < e->chains * e->groups; c++)            /* chain c / groups, in every group's block */
+        CU(cudaMemcpy(e->d_model + (size_t)c * e->L.total + e->L.theta, theta + (size_t)(c / e->groups) * e->cfg.m, sizeof(double) * e->cfg.m, cudaMemcpyHostToDevice));
     return set_next_iter(e, next_iter);
 }
 
@@ -742,7 +761,7 @@ extern "C" int pht_engine_get_chain_theta(pht_engine *e, double *theta) {
     CU(cudaSetDevice(e->cfg.device));
     CU(cudaStreamSynchronize(e->stream));
     for (int c = 0; c < e->chains; c++)
-        CU(cudaMemcpy(theta + (size_t)c * e->cfg.m, e->d_model + (size_t)c * e->L.total + e->L.theta, sizeof(double) * e->cfg.m, cudaMemcpyDeviceToHost));
+        CU(cudaMemcpy(theta + (size_t)c * e->cfg.m, e->d_model + (size_t)c * e->groups * e->L.total + e->L.theta, sizeof(double) * e->cfg.m, cudaMemcpyDeviceToHost));
     return 0;
 }
 
@@ -756,6 +775,168 @@ extern "C" int pht_engine_chain_rows(pht_engine *e, int rows, double *theta_out,
     const size_t m = (size_t)e->cfg.m, n = (size_t)e->cfg.n, R = (size_t)e->res_rows;
     if (theta_out) CU(cudaMemcpy2D(theta_out, sizeof(double) * rows * m, e->d_res, sizeof(double) * R * m, sizeof(double) * rows * m, e->chains, cudaMemcpyDeviceToHost));
     if (pi_out) CU(cudaMemcpy2D(pi_out, sizeof(double) * rows * n, e->d_pires, sizeof(double) * R * n, sizeof(double) * rows * n, e->chains, cudaMemcpyDeviceToHost));
+    return 0;
+}
+
+/* ---------------------------------------------------------------- groups (method 64) */
+/* each group's table span: the largest y and u - y (finite u) over its observations, as pht_engine_set_upper takes it */
+static int group_tmax(pht_engine *e, const std::vector<uint8_t> &gid, int G, std::vector<double> &tmax) {
+    const long l = e->l_local;
+    std::vector<double> y((size_t)(l > 0 ? l : 1)), u;
+    if (l > 0) CU(cudaMemcpy(y.data(), e->d_y, sizeof(double) * (size_t)l, cudaMemcpyDeviceToHost));
+    if (l > 0 && e->d_u) { u.resize((size_t)l); CU(cudaMemcpy(u.data(), e->d_u, sizeof(double) * (size_t)l, cudaMemcpyDeviceToHost)); }
+    tmax.assign((size_t)G, 0.0);
+    for (long i = 0; i < l; i++) {
+        double &t = tmax[gid[(size_t)i]];
+        if (y[(size_t)i] > t) t = y[(size_t)i];
+        if (!u.empty() && u[(size_t)i] < INFINITY && u[(size_t)i] - y[(size_t)i] > t) t = u[(size_t)i] - y[(size_t)i];
+    }
+    return 0;
+}
+
+/* after the interval bounds change: the groups' table spans and u in the grouped layout */
+static int group_refresh(pht_engine *e) {
+    if (e->groups <= 1) return 0;
+    std::vector<double> t;
+    if (group_tmax(e, e->h_group, e->groups, t)) return -1;
+    CU(cudaMemcpy(e->d_gtmax, t.data(), sizeof(double) * t.size(), cudaMemcpyHostToDevice));
+    const long l = e->l_local;
+    if (e->d_u) {
+        if (!e->d_gus) CU(pht_dev_alloc((void **)&e->d_gus, sizeof(double) * (size_t)(l > 0 ? l : 1), e->stream));
+        CU(pht_gather_f64(e->d_u, e->d_gperm, e->d_gus, l, e->stream));
+    } else if (e->d_gus) { CU(pht_dev_free(e->d_gus, e->stream)); e->d_gus = nullptr; }
+    CU(cudaStreamSynchronize(e->stream));
+    return 0;
+}
+
+extern "C" int pht_engine_set_groups(pht_engine *e, int G, const int *T, const double *C, const int *group_local) {
+    if (!e) return fail("null engine");
+    if (method_of(e->cfg) != PHT_METHOD_UNIF)
+        return fail("groups with their own structure need method 64 (the uniformisation sampler): MHRS, ECS, DCS and the MH variants run one structure per engine");
+    if (e->cfg.world > 1)
+        return fail("groups need world = 1: the statistics all-reduce of a multi-rank run carries one statistics block");
+    const int n = e->cfg.n, m = e->cfg.m, n1 = n + 1, nn1 = n1 * n1;
+    const long l = e->l_local;
+    const bool clear = T == nullptr;
+    std::vector<uint8_t> gid((size_t)(l > 0 ? l : 1), 0);
+    if (clear) { G = 1; T = e->T.data(); C = e->C.data(); }
+    else {
+        if (!C || (!group_local && l > 0)) return fail("null argument");
+        if (G < 1 || G > PHT_MAX_GROUPS) return fail("groups = %d outside 1..%d", G, PHT_MAX_GROUPS);
+    }
+    if ((long)e->chains * G > PHT_MAX_CHAINS)
+        return fail("chains x groups = %d x %d exceeds %d", e->chains, G, PHT_MAX_CHAINS);
+    if (G > 1 && e->entry_set)
+        return fail("%d groups asked while entry ages (delayed entry) are set: the ghost paths are drawn on one model; clear them with pht_engine_set_entry(e, NULL) first", G);
+    if (!clear) {
+        std::vector<char> used((size_t)m, 0);
+        for (int g = 0; g < G; g++) {
+            const int *Tg = T + (size_t)g * nn1;
+            for (int i = 0; i < nn1; i++) {
+                if (Tg[i] < 0 || Tg[i] > m) return fail("group %d: T[%d] = %d outside 0..m", g, i, Tg[i]);
+                if (Tg[i]) used[(size_t)Tg[i] - 1] = 1;
+            }
+            for (int j = 0; j < n1; j++) if (Tg[n + j * n1] != 0)
+                return fail("group %d: T[%d, %d] = %d: row n+1 (the absorbing state) must be all zero", g, n, j, Tg[n + j * n1]);
+        }
+        for (int v = 0; v < m; v++) if (!used[(size_t)v])
+            return fail("parameter %d is used by no group's structure: nothing in the data would inform it", v + 1);
+        for (long k = 0; k < l; k++) {
+            if (group_local[k] < 0 || group_local[k] >= G) return fail("group[%ld] = %d outside 0..%d", k, group_local[k], G - 1);
+            gid[(size_t)k] = (uint8_t)group_local[k];
+        }
+    }
+    CU(cudaSetDevice(e->cfg.device));
+    CU(cudaStreamSynchronize(e->stream));
+    if (G > 1 && !e->chain_blocks) {
+        e->chain_blocks = pht_unif_grid_blocks(e->cfg.device, n, true);
+        if (e->chain_blocks <= 0) { e->chain_blocks = 0; return fail("the several-unit path kernel does not fit on the device: %s", cudaGetErrorString(cudaGetLastError())); }
+    }
+    /* parameter -> cells CSR over (group, parameter): row g m + v lists group g's cells of parameter v in the reference's
+     * insertion order (row-major walk of T_g, as pht_engine_create builds it for one structure) */
+    std::vector<int> var_ptr((size_t)G * m + 1, 0), cell_i, cell_j;
+    for (int g = 0; g < G; g++) for (int i = 0; i < n1; i++) for (int j = 0; j < n1; j++) {
+        const int v = T[(size_t)g * nn1 + i + j * n1]; if (v) var_ptr[(size_t)g * m + v]++;
+    }
+    for (size_t r = 0; r + 1 < var_ptr.size(); r++) var_ptr[r + 1] += var_ptr[r];
+    cell_i.resize(var_ptr.back() > 0 ? var_ptr.back() : 1); cell_j.resize(cell_i.size());
+    { std::vector<int> fill(var_ptr.begin(), var_ptr.end() - 1);
+      for (int g = 0; g < G; g++) for (int i = 0; i < n1; i++) for (int j = 0; j < n1; j++) {
+          const int v = T[(size_t)g * nn1 + i + j * n1];
+          if (v) { const int c = fill[(size_t)g * m + v - 1]++; cell_i[c] = i; cell_j[c] = j; }
+      } }
+    std::vector<double> tmax; std::vector<unsigned long long> gofs((size_t)G + 1, 0ull);
+    if (G > 1) {
+        if (group_tmax(e, gid, G, tmax)) return -1;
+        for (long k = 0; k < l; k++) gofs[(size_t)gid[(size_t)k] + 1]++;
+        for (int g = 0; g < G; g++) gofs[(size_t)g + 1] += gofs[(size_t)g];
+    }
+    /* the new buffers first: a failed allocation (or sort) leaves the engine as it was */
+    const int units = e->chains * G, old_G = e->groups;
+    const size_t total = (size_t)e->L.total, slen = (size_t)stats_len(n), tab = pht_unif_table_doubles(n, PHT_UNIF_CAP);
+    const size_t ln = (size_t)(l > 0 ? l : 1);
+    int *dT = nullptr, *dvp = nullptr, *dci = nullptr, *dcj = nullptr; double *dC = nullptr, *dtmax = nullptr;
+    unsigned long long *dgofs = nullptr, *cnext = nullptr; double *model = nullptr, *unif = nullptr; long long *stats = nullptr;
+    double *gys = nullptr, *gus = nullptr; uint8_t *gcs = nullptr, *dgid = nullptr; uint32_t *gperm = nullptr;
+    struct Buf { void **p; size_t bytes; };
+    std::vector<Buf> bufs = { { (void **)&dT, sizeof(int) * G * nn1 }, { (void **)&dC, sizeof(double) * G * nn1 },
+                              { (void **)&dvp, sizeof(int) * var_ptr.size() }, { (void **)&dci, sizeof(int) * cell_i.size() },
+                              { (void **)&dcj, sizeof(int) * cell_j.size() }, { (void **)&model, sizeof(double) * units * total },
+                              { (void **)&stats, sizeof(long long) * units * slen }, { (void **)&unif, sizeof(double) * units * tab },
+                              { (void **)&cnext, sizeof(unsigned long long) * units } };
+    if (G > 1) {
+        bufs.push_back({ (void **)&dtmax, sizeof(double) * G }); bufs.push_back({ (void **)&dgofs, sizeof(unsigned long long) * (G + 1) });
+        bufs.push_back({ (void **)&gys, sizeof(double) * ln }); bufs.push_back({ (void **)&gcs, ln });
+        bufs.push_back({ (void **)&gperm, sizeof(uint32_t) * ln }); bufs.push_back({ (void **)&dgid, ln });
+        if (e->d_u) bufs.push_back({ (void **)&gus, sizeof(double) * ln });
+    }
+    auto undo = [&](size_t upto) { for (size_t f = 0; f < upto; f++) pht_dev_free(*bufs[f].p, e->stream); cudaStreamSynchronize(e->stream); cudaGetLastError(); };
+    size_t bytes_all = 0;
+    for (const Buf &b : bufs) bytes_all += b.bytes;
+    for (size_t b = 0; b < bufs.size(); b++) {
+        const cudaError_t ce = pht_dev_alloc(bufs[b].p, bufs[b].bytes, e->stream);
+        if (ce != cudaSuccess) {
+            cudaGetLastError(); undo(b);
+            return fail("cannot allocate device memory for %d groups x %d chains (%.1f MB, of which the uniformisation tables take %.1f MB per chain and group): %s",
+                        G, e->chains, bytes_all / 1e6, sizeof(double) * tab / 1e6, cudaGetErrorString(ce));
+        }
+    }
+    cudaError_t ce = cudaSuccess;
+#define STEP(call) do { if (ce == cudaSuccess) ce = (call); } while (0)
+    STEP(cudaMemcpyAsync(dT, T, bufs[0].bytes, cudaMemcpyHostToDevice, e->stream));
+    STEP(cudaMemcpyAsync(dC, C, bufs[1].bytes, cudaMemcpyHostToDevice, e->stream));
+    STEP(cudaMemcpyAsync(dvp, var_ptr.data(), bufs[2].bytes, cudaMemcpyHostToDevice, e->stream));
+    STEP(cudaMemcpyAsync(dci, cell_i.data(), bufs[3].bytes, cudaMemcpyHostToDevice, e->stream));
+    STEP(cudaMemcpyAsync(dcj, cell_j.data(), bufs[4].bytes, cudaMemcpyHostToDevice, e->stream));
+    /* unit (c, g) starts from chain c's current theta and pi (the rest of a model block is rebuilt every sweep) */
+    for (int u = 0; u < units && ce == cudaSuccess; u++)
+        STEP(cudaMemcpyAsync(model + (size_t)u * total, e->d_model + (size_t)(u / G) * old_G * total, sizeof(double) * total, cudaMemcpyDeviceToDevice, e->stream));
+    STEP(cudaMemsetAsync(stats, 0, bufs[6].bytes, e->stream));
+    STEP(pht_unif_init(unif, n, PHT_UNIF_CAP, units, e->stream));      /* log k! in every unit's table */
+    STEP(cudaMemsetAsync(cnext, 0, bufs[8].bytes, e->stream));
+    if (G > 1) {
+        STEP(cudaMemcpyAsync(dtmax, tmax.data(), sizeof(double) * G, cudaMemcpyHostToDevice, e->stream));
+        STEP(cudaMemcpyAsync(dgofs, gofs.data(), sizeof(unsigned long long) * (G + 1), cudaMemcpyHostToDevice, e->stream));
+        if (l > 0) {
+            STEP(cudaMemcpyAsync(dgid, gid.data(), (size_t)l, cudaMemcpyHostToDevice, e->stream));
+            STEP(pht_sort_by_group(e->d_perm, dgid, e->d_y, e->d_cens, l, gys, gcs, gperm, e->stream));
+            if (e->d_u) STEP(pht_gather_f64(e->d_u, gperm, gus, l, e->stream));
+        }
+    }
+    STEP(cudaStreamSynchronize(e->stream));
+#undef STEP
+    if (ce != cudaSuccess) { undo(bufs.size()); return fail("setting up %d groups failed: %s", G, cudaGetErrorString(ce)); }
+    pht_dev_free(dgid, e->stream);
+    void *old[] = { e->d_T, e->d_C, e->d_var_ptr, e->d_cell_i, e->d_cell_j, e->d_model, e->d_stats, e->d_unif, e->d_cnext,
+                    e->d_gtmax, e->d_gofs, e->d_gys, e->d_gcs, e->d_gperm, e->d_gus };
+    for (void *b : old) CU(pht_dev_free(b, e->stream));
+    CU(cudaStreamSynchronize(e->stream));
+    e->d_T = dT; e->d_C = dC; e->d_var_ptr = dvp; e->d_cell_i = dci; e->d_cell_j = dcj;
+    e->d_model = model; e->d_stats = stats; e->d_unif = unif; e->d_cnext = cnext;
+    e->d_gtmax = dtmax; e->d_gofs = dgofs; e->d_gys = gys; e->d_gcs = gcs; e->d_gperm = gperm; e->d_gus = gus;
+    e->groups = G;
+    if (G > 1) e->h_group.assign(gid.begin(), gid.begin() + l); else e->h_group.clear();
+    if (e->graph_exec) { cudaGraphExecDestroy(e->graph_exec); e->graph_exec = nullptr; }     /* kernel parameters change */
     return 0;
 }
 
@@ -776,7 +957,7 @@ extern "C" int pht_engine_set_upper(pht_engine *e, const double *upper_local) {
             e->unif_tmax = 0.0;
             for (long i = 0; i < e->l_local; i++) if (y[(size_t)i] > e->unif_tmax) e->unif_tmax = y[(size_t)i];
         }
-        return 0;
+        return group_refresh(e);
     }
     const bool unif = method_of(e->cfg) == PHT_METHOD_UNIF;
     if (method_of(e->cfg) != PHT_METHOD_MHRS && !unif)
@@ -821,7 +1002,7 @@ extern "C" int pht_engine_set_upper(pht_engine *e, const double *upper_local) {
         if (e->d_ys) CU(pht_gather_f64(e->d_u, e->d_perm, e->d_us, l, e->stream));
     }
     CU(cudaStreamSynchronize(e->stream));
-    return 0;
+    return group_refresh(e);
 }
 
 static int entry_free(pht_engine *e) {
@@ -843,6 +1024,8 @@ extern "C" int pht_engine_set_entry(pht_engine *e, const double *entry_local) {
     if (e->peers_attached) return fail("the entry ages of a multi-rank run are set on every rank before the exchange windows are attached");
     if (entry_local && e->chains > 1)
         return fail("entry ages (delayed entry) are not supported with %d chains: the ghost paths are drawn for one chain; pht_engine_set_chains(e, 1, ...) first", e->chains);
+    if (entry_local && e->groups > 1)
+        return fail("entry ages (delayed entry) are not supported with %d groups: the ghost paths are drawn on one model; pht_engine_set_groups(e, 1, ...) or (e, 0, NULL, ...) first", e->groups);
     if (e->graph_exec) { cudaGraphExecDestroy(e->graph_exec); e->graph_exec = nullptr; }     /* the sweep changes shape */
     if (!entry_local) return entry_free(e);
     const long l = e->l_local;
@@ -1062,10 +1245,9 @@ extern "C" int pht_engine_run(pht_engine *e, int nsweeps, double *out) {
     return 0;
 }
 
-extern "C" int pht_engine_sweep_stats(pht_engine *e, long long *N, long long *B, long long *zfix) {
-    if (!e) return fail("null engine");
+/* one sweep of chain 0 at the current parameters without updating them: its statistics blocks (one per group) into h */
+static int chain0_stats(pht_engine *e, std::vector<long long> &h) {
     CU(cudaSetDevice(e->cfg.device));
-    const int n = e->cfg.n;
     UpdateParams u = update_params(e, nullptr, 0);
     u.chains = 1;                                  /* chain 0 only */
     if (enqueue_model(e, u)) return -1;
@@ -1074,16 +1256,112 @@ extern "C" int pht_engine_sweep_stats(pht_engine *e, long long *N, long long *B,
     if (enqueue_paths(e, p)) return -1;
     if (enqueue_entry(e, u, p)) return -1;
     if (pht_engine_sync(e)) return -1;
-    std::vector<long long> h(stats_len(n));
+    h.resize((size_t)e->groups * stats_len(e->cfg.n));
     CU(cudaMemcpy(h.data(), e->d_stats, sizeof(long long) * h.size(), cudaMemcpyDeviceToHost));
-    if (N) memcpy(N, h.data(), sizeof(long long) * n * n);
-    if (B) memcpy(B, h.data() + n * n, sizeof(long long) * n);
-    if (zfix) for (int i = 0; i < n; i++) {
-        const __int128 tot = ((__int128)h[n * n + 2 * n + i] << 32) + (__int128)(unsigned long long)h[n * n + n + i];
+    return 0;
+}
+
+/* N, B and the fixed-point totals of statistics blocks [g0, g1) of h, summed */
+static int unpack_stats(const pht_engine *e, const long long *h, int blocks, long long *N, long long *B, long long *zfix) {
+    const int n = e->cfg.n, len = stats_len(n);
+    for (int i = 0; i < n * n; i++) { long long a = 0; for (int g = 0; g < blocks; g++) a += h[(size_t)g * len + i]; if (N) N[i] = a; }
+    for (int i = 0; i < n; i++) {
+        long long b = 0; __int128 tot = 0;
+        for (int g = 0; g < blocks; g++) {
+            const long long *q = h + (size_t)g * len;
+            b += q[n * n + i];
+            tot += ((__int128)q[n * n + 2 * n + i] << 32) + (__int128)(unsigned long long)q[n * n + n + i];
+        }
+        if (B) B[i] = b;
         if (tot > (__int128)0x7fffffffffffffffLL || tot < -(__int128)0x7fffffffffffffffLL) return fail("sojourn total of state %d overflows the fixed-point range (zbits = %d)", i, e->cfg.zbits);
-        zfix[i] = (long long)tot;
+        if (zfix) zfix[i] = (long long)tot;
     }
     return 0;
+}
+
+extern "C" int pht_engine_sweep_stats(pht_engine *e, long long *N, long long *B, long long *zfix) {
+    if (!e) return fail("null engine");
+    std::vector<long long> h;
+    if (chain0_stats(e, h)) return -1;
+    return unpack_stats(e, h.data(), e->groups, N, B, zfix);     /* the sum over the groups */
+}
+
+extern "C" int pht_engine_group_stats(pht_engine *e, long long *N, long long *B, long long *zfix) {
+    if (!e) return fail("null engine");
+    if (method_of(e->cfg) != PHT_METHOD_UNIF) return fail("groups with their own structure need method 64");
+    std::vector<long long> h;
+    if (chain0_stats(e, h)) return -1;
+    const int n = e->cfg.n;
+    for (int g = 0; g < e->groups; g++)
+        if (unpack_stats(e, h.data() + (size_t)g * stats_len(n), 1, N ? N + (size_t)g * n * n : nullptr, B ? B + (size_t)g * n : nullptr,
+                         zfix ? zfix + (size_t)g * n : nullptr)) return -1;
+    return 0;
+}
+
+/* pht_engine_paths of a grouped engine: one k_unif_paths launch per group with observations in the window, over that
+ * group's observations of the window (in upload order) on chain 0's model and table of the group; each path is recorded
+ * at its window position */
+static int group_paths(pht_engine *e, long first, long count, int *B, int *N, double *z) {
+    const int n = e->cfg.n, G = e->groups;
+    const size_t tabd = pht_unif_table_doubles(n, PHT_UNIF_CAP);
+    std::vector<double> y((size_t)count), u;
+    std::vector<uint8_t> c((size_t)count);
+    CU(cudaMemcpy(y.data(), e->d_y + first, sizeof(double) * count, cudaMemcpyDeviceToHost));
+    CU(cudaMemcpy(c.data(), e->d_cens + first, (size_t)count, cudaMemcpyDeviceToHost));
+    if (e->d_u) { u.resize((size_t)count); CU(cudaMemcpy(u.data(), e->d_u + first, sizeof(double) * count, cudaMemcpyDeviceToHost)); }
+    UpdateParams up = update_params(e, nullptr, 0);
+    up.chains = 1;                                 /* chain 0 only: its G models and tables */
+    if (enqueue_model(e, up)) return -1;
+    double *dy = nullptr, *du = nullptr, *dz = nullptr; uint8_t *dc = nullptr; uint32_t *dperm = nullptr; int *dB = nullptr, *dN = nullptr;
+    int rc = -1;
+#define CUP(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { fail("%s failed: %s (%s:%d)", #call, cudaGetErrorString(e_), __FILE__, __LINE__); goto out; } } while (0)
+    {
+        CUP(cudaMalloc(&dy, sizeof(double) * count)); CUP(cudaMalloc(&dc, (size_t)count)); CUP(cudaMalloc(&dperm, sizeof(uint32_t) * count));
+        if (e->d_u) CUP(cudaMalloc(&du, sizeof(double) * count));
+        CUP(cudaMalloc(&dB, sizeof(int) * count)); CUP(cudaMalloc(&dN, sizeof(int) * count * n * n)); CUP(cudaMalloc(&dz, sizeof(double) * count * n));
+        for (int g = 0; g < G; g++) {
+            std::vector<long> pos;
+            for (long k = 0; k < count; k++) if (e->h_group[(size_t)(first + k)] == g) pos.push_back(k);
+            if (pos.empty()) continue;
+            const long cnt = (long)pos.size();
+            std::vector<double> yg((size_t)cnt), ug((size_t)cnt); std::vector<uint8_t> cg((size_t)cnt); std::vector<uint32_t> ig((size_t)cnt);
+            for (long k = 0; k < cnt; k++) {
+                const long w = pos[(size_t)k];
+                yg[(size_t)k] = y[(size_t)w]; cg[(size_t)k] = c[(size_t)w]; ig[(size_t)k] = (uint32_t)(first + w);
+                if (du) ug[(size_t)k] = u[(size_t)w];
+            }
+            CUP(cudaMemcpyAsync(dy, yg.data(), sizeof(double) * cnt, cudaMemcpyHostToDevice, e->stream));
+            CUP(cudaMemcpyAsync(dc, cg.data(), (size_t)cnt, cudaMemcpyHostToDevice, e->stream));
+            CUP(cudaMemcpyAsync(dperm, ig.data(), sizeof(uint32_t) * cnt, cudaMemcpyHostToDevice, e->stream));
+            if (du) CUP(cudaMemcpyAsync(du, ug.data(), sizeof(double) * cnt, cudaMemcpyHostToDevice, e->stream));
+            CUP(cudaMemsetAsync(dN, 0, sizeof(int) * cnt * n * n, e->stream));
+            CUP(cudaMemsetAsync(&e->d_state->next_obs, 0, sizeof(unsigned long long), e->stream));   /* each launch hands out from 0 */
+            SweepParams p = sweep_params(e);
+            p.chains = 1; p.groups = 1;
+            p.model = e->d_model + (size_t)g * e->L.total;
+            p.y = dy; p.cens = dc; p.perm = dperm; p.u = du; p.l_local = cnt;
+            p.outB = dB; p.outN = dN; p.outz = dz; p.first = 0; p.count = cnt;
+            CUP(pht_launch_unif(p, e->d_unif + (size_t)g * tabd, nullptr, e->grid_blocks, e->stream));
+            e->launches++;
+            if (pht_engine_sync(e)) goto out;
+            std::vector<int> hB((size_t)cnt), hN((size_t)cnt * n * n); std::vector<double> hz((size_t)cnt * n);
+            CUP(cudaMemcpy(hB.data(), dB, sizeof(int) * cnt, cudaMemcpyDeviceToHost));
+            CUP(cudaMemcpy(hN.data(), dN, sizeof(int) * cnt * n * n, cudaMemcpyDeviceToHost));
+            CUP(cudaMemcpy(hz.data(), dz, sizeof(double) * cnt * n, cudaMemcpyDeviceToHost));
+            for (long k = 0; k < cnt; k++) {
+                const long w = pos[(size_t)k];
+                B[w] = hB[(size_t)k];
+                memcpy(N + (size_t)w * n * n, hN.data() + (size_t)k * n * n, sizeof(int) * n * n);
+                memcpy(z + (size_t)w * n, hz.data() + (size_t)k * n, sizeof(double) * n);
+            }
+        }
+        rc = 0;
+    }
+#undef CUP
+out:
+    cudaFree(dy); cudaFree(dc); cudaFree(dperm); cudaFree(dB); cudaFree(dN); cudaFree(dz);
+    if (du) cudaFree(du);
+    return rc;
 }
 
 extern "C" int pht_engine_paths(pht_engine *e, long first, long count, int *B, int *N, double *z) {
@@ -1091,6 +1369,7 @@ extern "C" int pht_engine_paths(pht_engine *e, long first, long count, int *B, i
     if (first < 0 || count < 0 || first + count > e->l_local) return fail("range [%ld, %ld) outside the shard", first, first + count);
     if (count == 0) return 0;
     CU(cudaSetDevice(e->cfg.device));
+    if (e->groups > 1) return group_paths(e, first, count, B, N, z);
     const int n = e->cfg.n;
     int *dB = nullptr, *dN = nullptr; double *dz = nullptr;
     uint32_t *t_exact = nullptr, *t_cens = nullptr;

@@ -17,6 +17,9 @@
  * Method 64 with several chains (pht_engine_set_chains) repeats model[], stats[] and unif[] once per chain, chain-major with
  * chain 0 first, and adds the chains' Philox keys and observation counters; observations, bounds and the sorted layout
  * stay shared.
+ * Method 64 with groups (pht_engine_set_groups) repeats them once per (chain, group) unit, block c G + g (chain-major, so
+ * block c is chain c when G = 1), each unit with its own observation counter; T, C and the parameter -> cell CSR hold one
+ * structure per group, and the production layout sorts the observations by group, then by decreasing y.
  *   items/pend/...  MHRS tail work lists (see k_mhrs.cu)
  */
 #ifndef PHT_ENGINE_INTERNAL_H
@@ -156,7 +159,10 @@ struct SweepParams {
     const double *u; double *item_u;
     /* method 64, several chains (pht_engine_set_chains): chains 0 .. chains-1, each with its own model block, stats block,
      * table and Philox key (ckeys[2c], ckeys[2c+1]) and observation counter cnext[c]; chain 0's blocks come first */
-    int chains; const uint32_t *ckeys; unsigned long long *cnext;
+    /* method 64, groups (pht_engine_set_groups): unit u = c groups + g has model, stats and table block u and counter
+     * cnext[u]; its layout positions are a kernel argument of the walker (pht_launch_unif).  `groups` sits in the padding
+     * after `chains`, so the structure -- and the other kernels' code -- stays as it was. */
+    int chains, groups; const uint32_t *ckeys; unsigned long long *cnext;
 };
 
 struct UpdateParams {
@@ -169,6 +175,11 @@ struct UpdateParams {
     /* several chains (method 64): one block of k_assemble / k_update / k_unif_table per chain; chain c's rows of res and
      * pires start at c x res_rows; ckeys as in SweepParams (nullptr: k0, k1); k_assemble zeroes cnext[c] when set */
     int chains; const uint32_t *ckeys; unsigned long long *cnext;
+    /* groups (method 64): k_assemble and k_unif_table run one block per (chain, group) unit c groups + g, on T, C + g (n+1)^2
+     * and the table span gtmax[g] (nullptr: the tmax argument); k_update (one block per chain) walks var_ptr[g m + v] ..
+     * var_ptr[g m + v + 1] for g = 0 .. groups - 1 and writes theta and pi into every unit of its chain.  groups = 1 with
+     * var_ptr of m + 1 entries is the single-structure engine. */
+    int groups; const double *gtmax;
 };
 
 /* all-reduce of the statistics block through the exchange windows */
@@ -205,7 +216,8 @@ size_t pht_mhrs_smem_bytes(int n);
 cudaError_t pht_unif_init(double *tab, int n, int cap, int chains, cudaStream_t st);   /* log k! of `chains` tables */
 size_t pht_unif_table_doubles(int n, int cap);
 cudaError_t pht_launch_unif_table(const UpdateParams &p, double *tab, double tmax, cudaStream_t st);
-cudaError_t pht_launch_unif(const SweepParams &p, const double *tab, int grid_blocks, cudaStream_t st);
+/* gofs: G + 1 offsets, group g's observations at layout positions [gofs[g], gofs[g + 1]) (nullptr: one group, [0, l_local)) */
+cudaError_t pht_launch_unif(const SweepParams &p, const double *tab, const unsigned long long *gofs, int grid_blocks, cudaStream_t st);
 int pht_unif_grid_blocks(int device, int n, bool chains);   /* chains: the kernel of several chains (k_unif_chain_paths) */
 /* method 64, delayed entry (k_unif.cu; pht_engine_set_entry): a list of observations with entry ages and its buffers.
  * Like the table, every pointer is a kernel argument of its own. */
@@ -227,6 +239,11 @@ int pht_unif_ghost_grid_blocks(int device, int n);
 cudaError_t pht_dev_alloc(void **p, size_t bytes, cudaStream_t st);
 cudaError_t pht_dev_free(void *p, cudaStream_t st);
 cudaError_t pht_sort_by_y_desc(const double *y, const uint8_t *cens, long l, double *ys, uint8_t *cs, uint32_t *perm, cudaStream_t st);
+/* the grouped layout (pht_engine_set_groups): a stable radix sort by group id (ascending) of the y-descending permutation
+ * perm_y (nullptr: the upload order), so each group is a contiguous range still ordered by decreasing y; group holds the
+ * id of every local observation in upload order.  Writes perm, ys = y[perm], cs = cens[perm]. */
+cudaError_t pht_sort_by_group(const uint32_t *perm_y, const uint8_t *group, const double *y, const uint8_t *cens, long l,
+                              double *ys, uint8_t *cs, uint32_t *perm, cudaStream_t st);
 /* dst[i] = src[perm[i]] (device arrays of length l) */
 cudaError_t pht_gather_f64(const double *src, const uint32_t *perm, double *dst, long l, cudaStream_t st);
 

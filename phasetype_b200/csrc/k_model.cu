@@ -10,7 +10,9 @@
  *               Gamma draw (:365-366) from the Philox parameter stream.
  *
  * With several chains (method 64, pht_engine_set_chains) both run one block per
- * chain, block c on chain c's model, statistics block, key and result rows.
+ * chain, block c on chain c's model, statistics block, key and result rows.  With
+ * groups (pht_engine_set_groups) k_assemble runs one block per (chain, group) unit
+ * on the group's T and C, and k_update's block c gathers over the groups of chain c.
  *
  * Row i of every matrix is handled by thread i with the reference's own loop
  * order, so each value is bit-identical to the host computation.
@@ -23,12 +25,14 @@
 __global__ void __launch_bounds__(64) k_assemble(UpdateParams p) {
     const int n = p.n, n1 = n + 1, tid = threadIdx.x;
     const ModelLayout L = ModelLayout::make(n, p.m);
-    const int c = blockIdx.x;                /* chain (grid = chains) */
+    const int c = blockIdx.x;                /* unit: chain c / groups, group c % groups (grid = chains x groups) */
     double *M = p.model + (size_t)c * L.total;
     long long *stats = p.stats + (size_t)c * stats_len(n);
     const double *theta = M + L.theta;
     double *TT = M + L.TT, *S = M + L.S, *s = M + L.s;
     const bool first = p.state->first_assembly != 0;
+    const size_t gofs = (size_t)(c % p.groups) * n1 * n1;
+    const int *T = p.T + gofs; const double *Cm = p.C + gofs;
 
     for (int i = tid; i < stats_len(n); i += blockDim.x) stats[i] = 0;
     if (tid == 0 && c == 0) {
@@ -39,14 +43,14 @@ __global__ void __launch_bounds__(64) k_assemble(UpdateParams p) {
     if (tid <= n) {
         const int i = tid;
         for (int j = 0; j <= n; j++) {
-            const int v = p.T[i + j * n1];
-            if (j != i || v != 0) TT[i + j * n1] = v ? theta[v - 1] * p.C[i + j * n1] : 0.0;
+            const int v = T[i + j * n1];
+            if (j != i || v != 0) TT[i + j * n1] = v ? theta[v - 1] * Cm[i + j * n1] : 0.0;
         }
         /* diagonal = -(row sum): ascending columns when assembled from the start
          * values (:215,229), descending afterwards (TTDiag is a prepend list, :226,389-393) */
         double acc = 0.0;
-        if (first) { for (int j = 0; j <= n; j++) if (p.T[i + j * n1] != 0) acc -= TT[i + j * n1]; }
-        else       { for (int j = n; j >= 0; j--) if (p.T[i + j * n1] != 0) acc -= TT[i + j * n1]; }
+        if (first) { for (int j = 0; j <= n; j++) if (T[i + j * n1] != 0) acc -= TT[i + j * n1]; }
+        else       { for (int j = n; j >= 0; j--) if (T[i + j * n1] != 0) acc -= TT[i + j * n1]; }
         if (i < n || first) TT[i + i * n1] = acc;
     }
     __syncthreads();
@@ -94,33 +98,38 @@ __global__ void __launch_bounds__(128) k_update(UpdateParams p) {
     const ModelLayout L = ModelLayout::make(n, m);
     const uint32_t iter = p.state->iter;
     const uint32_t row = p.state->res_row;
-    /* chain c (grid = chains): its model, statistics, key and rows */
-    const int c = blockIdx.x;
-    double *model = p.model + (size_t)c * L.total;
-    const long long *stats = p.stats + (size_t)c * stats_len(n);
+    /* chain c (grid = chains): its model and statistics blocks (one per group, c G .. c G + G - 1), key and rows */
+    const int c = blockIdx.x, G = p.groups;
+    double *model = p.model + (size_t)c * G * L.total;
+    const long long *stats = p.stats + (size_t)c * G * stats_len(n);
     const uint32_t k0 = p.ckeys ? p.ckeys[2 * c] : p.k0, k1 = p.ckeys ? p.ckeys[2 * c + 1] : p.k1;
     double *res = p.res ? p.res + (size_t)c * p.res_rows * m : nullptr;
     double *pires = p.pires ? p.pires + (size_t)c * p.res_rows * n : nullptr;
-    const long long *Nacc = stats, *zlo = stats + n * n + n, *zhi = stats + n * n + 2 * n;
     const double zscale = pht_u2d((uint64_t)(1023 - p.zbits) << 52);      /* 2^-zbits */
     /* some rank raised its error word this sweep: every rank learns it here and stops at the next synchronisation */
     if (threadIdx.x == 0 && stats[stats_len(n) - 1] != 0 && p.state->error == 0) atomicOr(&p.state->error, 128);
     for (int v = threadIdx.x; v < m; v += blockDim.x) {
         long long Nsum = 0; double zsum = 0.0;
-        /* the reference walks prepend lists, i.e. cells in reverse insertion order (:340-355) */
-        for (int c = p.var_ptr[v + 1] - 1; c >= p.var_ptr[v]; c--) {
-            const int i = p.cell_i[c], j = p.cell_j[c];
-            Nsum += (j == n) ? Nacc[i + i * n] : Nacc[i + j * n];
-            /* the two limbs of the fixed-point total; it must fit the int64 it is converted from (else: error word 2) */
-            const __int128 tot = ((__int128)zhi[i] << 32) + (__int128)(unsigned long long)zlo[i];
-            if (tot > (__int128)0x7fffffffffffffffLL || tot < -(__int128)0x7fffffffffffffffLL) atomicOr(&p.state->error, 2);
-            const double zi = (double)(long long)tot * zscale;
-            zsum += zi / p.C[i + j * n1];
+        /* groups in ascending order; within a group the reference walks prepend lists, i.e. cells in reverse insertion
+         * order (:340-355) */
+        for (int g = 0; g < G; g++) {
+            const long long *gs = stats + (size_t)g * stats_len(n);
+            const long long *Nacc = gs, *zlo = gs + n * n + n, *zhi = gs + n * n + 2 * n;
+            const double *Cg = p.C + (size_t)g * n1 * n1;
+            for (int c = p.var_ptr[g * m + v + 1] - 1; c >= p.var_ptr[g * m + v]; c--) {
+                const int i = p.cell_i[c], j = p.cell_j[c];
+                Nsum += (j == n) ? Nacc[i + i * n] : Nacc[i + j * n];
+                /* the two limbs of the fixed-point total; it must fit the int64 it is converted from (else: error word 2) */
+                const __int128 tot = ((__int128)zhi[i] << 32) + (__int128)(unsigned long long)zlo[i];
+                if (tot > (__int128)0x7fffffffffffffffLL || tot < -(__int128)0x7fffffffffffffffLL) atomicOr(&p.state->error, 2);
+                const double zi = (double)(long long)tot * zscale;
+                zsum += zi / Cg[i + j * n1];
+            }
         }
         pht_stream st; st.k0 = k0; st.k1 = k1;
         pht_stream_seek(&st, iter, PHT_OBS_PARAM, (uint32_t)v, 0);
         const double th = pht_rgamma(&st, p.nu[v] + (double)Nsum, 1.0 / (p.zeta[v] + zsum));   /* :366 */
-        model[L.theta + v] = th;
+        for (int g = 0; g < G; g++) model[(size_t)g * L.total + L.theta + v] = th;     /* theta lives in every group's block */
         if (res != nullptr && row < (uint32_t)p.res_rows) res[(size_t)row * m + v] = th;
     }
     /* start distribution: pi | paths ~ Dirichlet(beta + B), B = start-state counts of the sweep (the conjugate update the
@@ -128,11 +137,12 @@ __global__ void __launch_bounds__(128) k_update(UpdateParams p) {
      * Gamma(beta_i + B_i, 1) variates from parameter sub-streams m .. m+n-1, normalised in index order. */
     __shared__ double gpi[PHT_NMAX];
     if (p.beta != nullptr) {
-        const long long *Bacc = stats + n * n;
         for (int i = threadIdx.x; i < n; i += blockDim.x) {
+            long long Bsum = 0;                 /* start-state counts summed over the groups: one pi per chain */
+            for (int g = 0; g < G; g++) Bsum += stats[(size_t)g * stats_len(n) + n * n + i];
             pht_stream st; st.k0 = k0; st.k1 = k1;
             pht_stream_seek(&st, iter, PHT_OBS_PARAM, (uint32_t)(m + i), 0);
-            gpi[i] = pht_rgamma(&st, p.beta[i] + (double)Bacc[i], 1.0);
+            gpi[i] = pht_rgamma(&st, p.beta[i] + (double)Bsum, 1.0);
         }
     }
     __syncthreads();
@@ -142,7 +152,7 @@ __global__ void __launch_bounds__(128) k_update(UpdateParams p) {
             for (int i = 0; i < n; i++) sum += gpi[i];
             for (int i = 0; i < n; i++) {
                 const double v = gpi[i] / sum;
-                model[L.pi + i] = v;
+                for (int g = 0; g < G; g++) model[(size_t)g * L.total + L.pi + i] = v;
                 if (pires != nullptr && row < (uint32_t)p.res_rows) pires[(size_t)row * n + i] = v;
             }
         }
@@ -219,7 +229,7 @@ cudaError_t pht_launch_spectral(const UpdateParams &p, const double *inject, cud
 }
 
 cudaError_t pht_launch_assemble(const UpdateParams &p, cudaStream_t st) {
-    k_assemble<<<p.chains, 64, 0, st>>>(p);
+    k_assemble<<<p.chains * p.groups, 64, 0, st>>>(p);
     return cudaGetLastError();
 }
 cudaError_t pht_launch_update(const UpdateParams &p, cudaStream_t st) {

@@ -11,7 +11,8 @@
  *   k_unif_paths   one observation per lane, persistent warps refilled from the global counter (Dispenser); the two
  *                  per-lane n-vectors of scratch live in shared-memory slabs (stride THREADS), the powers in global
  *                  memory (33 MB per chain at n = 32 and full capacity; what a sweep touches stays in L2).
- *   k_unif_chain_paths  the same per observation for several chains: the blocks walk the chains (below)
+ *   k_unif_chain_paths  the same per observation for several chains or groups: the blocks walk the (chain, group)
+ *                  units (below)
  *
  * Delayed entry (only when entry ages are set, pht_engine_set_entry; law and draw order in pht_unif.h):
  *   k_unif_entry_table  sigma_k, phi_k for k <= K_sweep, after k_unif_table (one block)
@@ -46,7 +47,8 @@ __global__ void k_unif_lgk(double *tab, int n, int cap) {
     if (threadIdx.x == 0) pht_unif_lgk_fill(tab + (size_t)blockIdx.x * L.total + L.lgk, cap);
 }
 
-/* block c builds chain c's table from chain c's model block (grid = chains) */
+/* block c builds unit c's table from unit c's model block (grid = chains x groups); a group's table spans its own
+ * observations (gtmax[c % groups]): a path never reads a power beyond its own K(lambda y), so the span changes no bit */
 __global__ void __launch_bounds__(UNIF_TABLE_THREADS) k_unif_table(UpdateParams p, double *tab, double tmax) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int n = p.n, nn = n * n, tid = threadIdx.x, cap = PHT_UNIF_CAP;
@@ -58,6 +60,7 @@ __global__ void __launch_bounds__(UNIF_TABLE_THREADS) k_unif_table(UpdateParams 
     double *sR = reinterpret_cast<double *>(smem_raw), *sr = sR + nn;
     double *P0 = sr + n, *P1 = P0 + nn, *q0 = P1 + nn, *q1 = q0 + n, *g0 = q1 + n, *g1 = g0 + n;
     const double lam = pht_unif_lambda(n, S);
+    if (p.gtmax) tmax = p.gtmax[blockIdx.x % p.groups];
     int K = pht_unif_K(lam * tmax);
     if (K >= cap) { if (tid == 0) atomicOr(&p.state->error, PHT_UNIF_ERR_TABLE); K = cap - 1; }
     for (int e = tid; e < nn; e += blockDim.x) {
@@ -148,23 +151,26 @@ __global__ void __launch_bounds__(THREADS) k_unif_paths(SweepParams p, const dou
     if ((tid & 31) == 0) atomicAdd(&p.state->counters[PHT_CNT_PATHS], w_paths);
 }
 
-/* Several chains (pht_engine_set_chains; one chain and parity mode run k_unif_paths above, 2 % faster at one chain on the
- * C3 shape).  Persistent blocks walk the chains: block b starts at chain
- * b mod chains, loads that chain's model into shared memory and its warps take observations 32 at a time from the chain's
- * counter, with the chain's key.  When the counter runs dry the block flushes its accumulators into the chain's statistics
- * block and moves on to the next chain that still has work, until it has passed every chain once.  Whether a chain has
- * work left is read from its counter with plain loads, 32 chains per warp-wide look; every statistic is an integer sum,
- * so which block draws which observation does not change the result. */
+/* Several chains or groups (pht_engine_set_chains, pht_engine_set_groups; one chain of one group and parity mode run
+ * k_unif_paths above, 2 % faster at one chain on the C3 shape).  The work comes in units u = c groups + g: chain c's paths
+ * of group g's observations, layout positions [gofs[g], gofs[g + 1]), drawn with chain c's key on unit u's model and
+ * table into unit u's statistics block, handed out by unit u's counter.  Persistent blocks walk the units: block b starts
+ * at unit b mod units, loads that unit's model into shared memory and its warps take observations 32 at a time from the
+ * unit's counter.  When the counter runs dry the block flushes its accumulators into the unit's statistics block and
+ * moves on to the next unit that still has work, until it has passed every unit once.  Whether a unit has work left is
+ * read from its counter with plain loads, 32 units per warp-wide look; every statistic is an integer sum, so which block
+ * draws which observation does not change the result. */
 template <int THREADS>
-__global__ void __launch_bounds__(THREADS, 7) /* 7 blocks of 128 per SM: at most 72 registers */ k_unif_chain_paths(SweepParams p, const double *tab) {
+__global__ void __launch_bounds__(THREADS, 7) /* 7 blocks of 128 per SM: at most 72 registers */ k_unif_chain_paths(SweepParams p, const double *tab,
+                                                                                                             const unsigned long long *gofs) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     /* the walk's state lives in shared memory, re-read after each barrier, so that it holds no register in the path loop */
     __shared__ int s_chain, s_left; __shared__ uint32_t s_key[2];
-    __shared__ const double *s_tab; __shared__ unsigned long long *s_counter;
+    __shared__ const double *s_tab; __shared__ unsigned long long *s_counter, s_begin, s_end;
     const int n = p.n, tid = threadIdx.x;
     const unsigned FULL = 0xffffffffu;
     const ModelLayout ML = ModelLayout::make(n, p.m);
-    const int chains = p.chains;
+    const int chains = p.chains * p.groups;       /* units (s_chain: the current one) */
     UnifSmem<THREADS> sm; sm.carve(smem_raw, n);
     const uint32_t iter = p.state->iter;
     unsigned c_paths = 0; int err = 0;
@@ -175,10 +181,11 @@ __global__ void __launch_bounds__(THREADS, 7) /* 7 blocks of 128 per SM: at most
     for (;;) {
         if (tid < 32) {                        /* the first chain from the current one on (cyclically) with work left */
             const int c = s_chain, left = s_left;
-            const unsigned long long span = (unsigned long long)p.l_local;
             int found = -1;
             for (int k = 0; k < left && found < 0; k += 32) {
                 int cc = c + k + tid; if (cc >= chains) cc -= chains;
+                const int g = cc % p.groups;
+                const unsigned long long span = gofs ? gofs[g + 1] - gofs[g] : (unsigned long long)p.l_local;
                 const bool work = k + tid < left && *(volatile unsigned long long *)&p.cnext[cc] < span;
                 const unsigned b = __ballot_sync(FULL, work);
                 if (b) found = k + __ffs(b) - 1;
@@ -186,8 +193,10 @@ __global__ void __launch_bounds__(THREADS, 7) /* 7 blocks of 128 per SM: at most
             if (tid == 0) {
                 int cn = c + (found < 0 ? 0 : found); if (cn >= chains) cn -= chains;
                 s_chain = cn; s_left = found < 0 ? 0 : left - found;
-                s_key[0] = p.ckeys[2 * cn]; s_key[1] = p.ckeys[2 * cn + 1];
+                const int ch = cn / p.groups, g = cn - ch * p.groups;
+                s_key[0] = p.ckeys[2 * ch]; s_key[1] = p.ckeys[2 * ch + 1];
                 s_tab = tab + (size_t)cn * pht_unif_layout_make(n, PHT_UNIF_CAP).total; s_counter = p.cnext + cn;
+                s_begin = gofs ? gofs[g] : 0ull; s_end = gofs ? gofs[g + 1] : (unsigned long long)p.l_local;
             }
         }
         __syncthreads();
@@ -202,7 +211,7 @@ __global__ void __launch_bounds__(THREADS, 7) /* 7 blocks of 128 per SM: at most
             }
         }
         __syncthreads();
-        disp.next = disp.end = 0ull; disp.exhausted = false;
+        disp.next = disp.end = 0ull; disp.exhausted = false; disp.obs_begin = s_begin; disp.obs_end = s_end;
         for (;;) {
             const unsigned long long o = disp.take_from(s_counter, FULL, true);
             const bool have = o != ~0ull;
@@ -372,11 +381,11 @@ size_t pht_unif_table_doubles(int n, int cap) { return (size_t)pht_unif_layout_m
 
 cudaError_t pht_launch_unif_table(const UpdateParams &p, double *tab, double tmax, cudaStream_t st) {
     const size_t smem = sizeof(double) * (size_t)(3 * p.n * p.n + 7 * p.n);
-    k_unif_table<<<p.chains, UNIF_TABLE_THREADS, smem, st>>>(p, tab, tmax);
+    k_unif_table<<<p.chains * p.groups, UNIF_TABLE_THREADS, smem, st>>>(p, tab, tmax);
     return cudaGetLastError();
 }
 
-int pht_unif_grid_blocks(int device, int n, bool chains) {
+int pht_unif_grid_blocks(int device, int n, bool chains) {     /* chains: the walker (several chains or groups) */
     const size_t smem = UnifSmem<UNIF_THREADS>::bytes(n);
     int per_sm = 0, sms = 0;
     const void *k = chains ? (const void *)k_unif_chain_paths<UNIF_THREADS> : (const void *)k_unif_paths<UNIF_THREADS>;
@@ -386,9 +395,9 @@ int pht_unif_grid_blocks(int device, int n, bool chains) {
     return per_sm * sms;
 }
 
-cudaError_t pht_launch_unif(const SweepParams &p, const double *tab, int grid_blocks, cudaStream_t st) {
-    if (p.chains > 1 && p.outB == nullptr)
-        k_unif_chain_paths<UNIF_THREADS><<<grid_blocks, UNIF_THREADS, UnifSmem<UNIF_THREADS>::bytes(p.n), st>>>(p, tab);
+cudaError_t pht_launch_unif(const SweepParams &p, const double *tab, const unsigned long long *gofs, int grid_blocks, cudaStream_t st) {
+    if ((p.chains > 1 || p.groups > 1) && p.outB == nullptr)
+        k_unif_chain_paths<UNIF_THREADS><<<grid_blocks, UNIF_THREADS, UnifSmem<UNIF_THREADS>::bytes(p.n), st>>>(p, tab, gofs);
     else k_unif_paths<UNIF_THREADS><<<grid_blocks, UNIF_THREADS, UnifSmem<UNIF_THREADS>::bytes(p.n), st>>>(p, tab);
     return cudaGetLastError();
 }

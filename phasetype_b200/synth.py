@@ -96,6 +96,29 @@ def delayed_entry(R, s, l, entry, rng, censor=None, spacing=None):
     return np.concatenate(ys), np.concatenate(As), np.concatenate(cs), np.concatenate(us)
 
 
+def structure_rates(T, C, theta, n):
+    """(R, s) of the generator that theta maps to through the structure (T, C): column-major flat (n+1)^2, as pht_config
+    takes them."""
+    T = np.asarray(T).reshape(n + 1, n + 1, order="F"); C = np.asarray(C, dtype=np.float64).reshape(n + 1, n + 1, order="F")
+    rate = np.where(T > 0, np.asarray(theta, dtype=np.float64)[np.maximum(T, 1) - 1] * C, 0.0)
+    R = rate[:n, :n].copy(); np.fill_diagonal(R, 0.0)
+    return R, rate[:n, n].copy()
+
+
+def groups(T, C, theta, n, sizes, rng, censor=None):
+    """Grouped data (Engine.set_groups): G structures T[g], C[g] (column-major flat (n+1)^2 each) over one parameter vector
+    theta.  Group g gets sizes[g] absorption times of its own generator (structure_rates), started in state 0
+    (simulate_pht).  censor(k, rng), when given, draws k censoring times: a unit still working then is right-censored
+    there.  Returns (y, censored, group), the groups one after another."""
+    ys, cs, gs = [], [], []
+    for g, k in enumerate(sizes):
+        R, s = structure_rates(T[g], C[g], theta, n)
+        t = simulate_pht(R, s, int(k), rng)
+        end = np.full(int(k), np.inf) if censor is None else np.asarray(censor(int(k), rng), dtype=np.float64)
+        ys.append(np.minimum(t, end)); cs.append((t > end).astype(np.int32)); gs.append(np.full(int(k), g, dtype=np.int32))
+    return np.concatenate(ys), np.concatenate(cs), np.concatenate(gs)
+
+
 def _general_T(R, s):
     """Every non-zero rate its own parameter, numbered column-major like sorted "Sij"/"si" names would be."""
     n = s.shape[0]
