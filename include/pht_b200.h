@@ -72,7 +72,8 @@ void LJMA_Gibbs(int *it, int *mhit, int *method, int *n, int *m, double *nu, dou
  * finite bound) observations; the start state is drawn from its conditional law too, so the start-distribution update
  * (pht_engine_set_pi with beta) works with it.  Lowest priority of the mask; `mhit` is not used.  The table holds
  * PHT_UNIF_CAP = 4096 powers (33 MB at n = 32): an observation whose lambda y (or lambda (u - y)) needs more raises error
- * bit 256.  Delayed entry (left-truncated observations, pht_engine_set_entry) is this method's alone.  (Bit 32 stays
+ * bit 256.  Delayed entry (left-truncated observations, pht_engine_set_entry) is this method's alone, and so are counts
+ * (tied observations as records drawn once per record, pht_engine_set_counts).  (Bit 32 stays
  * unassigned.) */
 #define PHT_METHOD_UNIF 64
 #define PHT_MAX_PHASES  32
@@ -226,6 +227,25 @@ int pht_engine_chain_rows(pht_engine *e, int rows, double *theta_out, double *pi
 #define PHT_MAX_GROUPS 64
 int pht_engine_set_groups(pht_engine *e, int G, const int *T, const double *C, const int *group_local);
 int pht_engine_group_stats(pht_engine *e, long long *N, long long *B, long long *zfix);
+
+/* Observations with counts (method 64 only): tied and tabulated data -- inspection data, administrative censoring, life
+ * tables -- as records (y_k, flag_k, u_k) with a count w_k >= 0 each.  counts_local holds one count per local record, in
+ * the order of y_local.  The engine is then, bit for bit, the engine created on the expanded data (each record repeated
+ * w_k times in upload order, as np.repeat does) with the same configuration, zbits, key, theta, pi, prior, bounds, chains
+ * and groups: unit j of record k is expanded observation base_k + j, base the exclusive prefix sum of the counts in upload
+ * order, and its path is drawn on Philox sub-stream 0 of (sweep, base_k + j), as that observation's is.  Every sweep
+ * statistic is an integer sum, so the statistics and the theta and pi rows are the expanded engine's.  Each record's
+ * weights are computed once per sweep for all its units (k_unif_records); records with few units run through the
+ * per-observation kernels.  A count of 0 removes the record from the likelihood; all counts 1 give the results without
+ * counts; NULL returns to plain records, bit for bit the engine that never called this.  Chains (pht_engine_set_chains)
+ * and groups (pht_engine_set_groups) work with counts, set in either order; bounds (pht_engine_set_upper) may change
+ * while counts are set.  Construct the engine with zbits at most pht_choose_zbits(sum_k w_k max(y_k, u_k)).
+ * Refused, each with its own message and leaving the engine as it was: any method but 64; world > 1 (the expanded index
+ * is a single-rank numbering) and a call after the exchange windows are attached; entry ages (pht_engine_set_entry, in
+ * either order: a record's ghost count would be a sum of w Geometric draws); counts summing to 2^32 or more (the Philox
+ * observation word is 32 bits); a configured zbits above pht_choose_zbits(sum_k w_k max(y_k, u_k)), which
+ * pht_engine_set_upper also applies while counts are set; and pht_engine_paths while counts are set. */
+int pht_engine_set_counts(pht_engine *e, const uint32_t *counts_local);
 
 /* run `nsweeps` Gibbs sweeps; row r of out (nsweeps x m, row-major) is the draw of sweep r.
  * out may be NULL (results stay on the device; fetch later with pht_engine_get_theta). */

@@ -21,7 +21,7 @@ SYMBOLS = [
     "pht_engine_counters", "pht_fp64_fma_rate", "pht_engine_set_l2_flush", "pht_engine_peer_handle", "pht_engine_peer_attach", "pht_engine_round_trace", "pht_engine_set_pi", "pht_engine_get_pi", "pht_engine_pi_rows",
     "pht_engine_set_upper", "pht_engine_set_entry", "pht_engine_entry_paths",
     "pht_engine_set_chains", "pht_engine_set_chain_theta", "pht_engine_get_chain_theta", "pht_engine_chain_rows",
-    "pht_engine_set_groups", "pht_engine_group_stats",
+    "pht_engine_set_groups", "pht_engine_group_stats", "pht_engine_set_counts",
 ]
 PEER_HANDLE_BYTES = 128
 # method 64 (include/pht_b200.h PHT_METHOD_UNIF): the uniformisation path sampler; exact, right-, interval- and
@@ -93,6 +93,7 @@ def lib():
     L.pht_engine_chain_rows.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]
     L.pht_engine_set_groups.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
     L.pht_engine_group_stats.argtypes = [C.c_void_p, _lp, _lp, _lp]
+    L.pht_engine_set_counts.argtypes = [C.c_void_p, C.c_void_p]
     L.pht_engine_peer_handle.argtypes = [C.c_void_p, C.c_void_p]
     L.pht_engine_peer_attach.argtypes = [C.c_void_p, C.c_void_p]
     _lib = L
@@ -347,6 +348,24 @@ class Engine:
             g = np.zeros(1, dtype=np.int32)
         _check(lib().pht_engine_set_groups(self._h, G, t.ctypes.data, c.ctypes.data, g.ctypes.data))
         self.groups = G
+
+    def set_counts(self, counts):
+        """Observations with counts (METHOD_UNIF only, one rank, no entry ages): local record k stands for counts[k] >= 0
+        tied units, and the engine is bit for bit the engine on np.repeat(records, counts) (synth.tabulate builds such
+        records).  Every unit's path ends by max(y, u), so construct the engine with sum_y_global = the sum of
+        counts x max(y, u) over the records (or a zbits at most pht_choose_zbits of it).  None returns to plain records."""
+        if counts is None:
+            _check(lib().pht_engine_set_counts(self._h, None))
+            return
+        w = np.asarray(counts)
+        if w.shape != (self.l_local,):
+            raise EngineError("set_counts: %d counts for %d local records" % (w.size, self.l_local))
+        if w.size and (w.min() < 0 or w.max() > 0xffffffff):
+            raise EngineError("set_counts: counts must lie in 0 .. 2^32 - 1")
+        w = np.ascontiguousarray(w, dtype=np.uint32)
+        if not self.l_local:
+            w = np.zeros(1, dtype=np.uint32)     # an empty shard still takes part (never NULL, which clears)
+        _check(lib().pht_engine_set_counts(self._h, w.ctypes.data))
 
     def group_stats(self):
         """One sweep's statistics of chain 0 per group, without an update: N (G, n*n), B (G, n), zfix (G, n); their sum

@@ -13,6 +13,7 @@
 #include <cstring>
 #include <cstdarg>
 #include <cmath>
+#include <string>
 #include <vector>
 #include <algorithm>
 #include <thread>
@@ -111,6 +112,16 @@ struct pht_engine {
     double *d_entry = nullptr, *d_ea = nullptr; uint32_t *d_eobs = nullptr; long n_trunc = 0;
     unsigned *d_eM = nullptr; unsigned long long *d_eoff = nullptr, *d_enext = nullptr; double *d_etab = nullptr;
     void *d_escan = nullptr; size_t escan_bytes = 0; int ghost_blocks = 0, count_blocks = 0;
+    /* method 64, counts (pht_engine_set_counts): the counts in upload order; the records below the threshold expanded into
+     * the ordinary layout (y, flags, u, the expanded index of every unit) with its group offsets, run by the per-observation
+     * kernels; the records at or above it (y, flags, u, expanded index of unit 0) and their work items, run by
+     * k_unif_records; its hand-out counter and grid; the threshold and the chunk size */
+    bool counts_set = false; std::vector<uint32_t> h_counts;
+    double *d_cy = nullptr, *d_cu = nullptr; uint8_t *d_cc = nullptr; uint32_t *d_cperm = nullptr; unsigned long long *d_cgofs = nullptr;
+    long n_low = 0;
+    double *d_ry = nullptr, *d_ru = nullptr; uint8_t *d_rc = nullptr; uint32_t *d_rbase = nullptr; uint4 *d_ritems = nullptr;
+    long n_items = 0; unsigned long long *d_rnext = nullptr; int rec_blocks = 0;
+    uint32_t counts_threshold = 0, counts_chunk = 0;
     /* graph */
     cudaGraphExec_t graph_exec = nullptr; int graph_res_rows = -1; double *graph_res = nullptr;
     unsigned long long graph_launches = 0;      /* kernels one replay of the captured sweep launches */
@@ -217,6 +228,27 @@ static int method_of(const pht_config &c) {       /* dispatch priority of src/PH
     return 0;
 }
 
+static int counts_build(pht_engine *e);      /* pht_engine_set_counts: the counted records' layouts */
+
+/* method 64 with counts: the expanded records below the threshold through the per-observation kernels (their own layout
+ * and group offsets), then k_unif_records over the items of the others; both add to the same statistics blocks */
+static int enqueue_counts(pht_engine *e, const SweepParams &p) {
+    if (e->n_low > 0) {
+        SweepParams q = p;
+        q.y = e->d_cy; q.cens = e->d_cc; q.perm = e->d_cperm; q.u = e->d_cu; q.l_local = e->n_low;
+        CU(pht_launch_unif(q, e->d_unif, q.groups > 1 ? e->d_cgofs : nullptr, q.chains > 1 || q.groups > 1 ? e->chain_blocks : e->grid_blocks, e->stream));
+        e->launches++;
+    }
+    if (e->n_items > 0) {
+        UnifRecords R; memset(&R, 0, sizeof(R));
+        R.y = e->d_ry; R.u = e->d_ru; R.cens = e->d_rc; R.base = e->d_rbase; R.items = e->d_ritems; R.n_items = e->n_items; R.next = e->d_rnext;
+        CU(pht_launch_unif_records(p, e->d_unif, R, e->rec_blocks, e->stream));
+        e->launches++;
+    }
+    e->launches--;                                 /* enqueue_paths counts one */
+    return 0;
+}
+
 /* enqueue the path kernel of the configured method */
 static int enqueue_paths(pht_engine *e, const SweepParams &p, const uint32_t *idx_exact = nullptr, unsigned long long n_exact = 0,
                          const uint32_t *idx_cens = nullptr, unsigned long long n_cens = 0, bool lists_given = false) {
@@ -233,6 +265,7 @@ static int enqueue_paths(pht_engine *e, const SweepParams &p, const uint32_t *id
     case PHT_METHOD_DCS: CU(pht_launch_dcs(p, e->grid_blocks, e->stream)); e->launches++; break;           /* unit machine + complex-spectrum kernel */
     case PHT_METHOD_MHS_HOBOLTH: CU(pht_launch_dcs(p, e->grid_blocks, e->stream, true)); e->launches++; break;
     case PHT_METHOD_UNIF:
+        if (e->counts_set) { if (enqueue_counts(e, p)) return -1; break; }
         CU(pht_launch_unif(p, e->d_unif, p.groups > 1 ? e->d_gofs : nullptr, p.chains > 1 || p.groups > 1 ? e->chain_blocks : e->grid_blocks, e->stream));
         break;
     case PHT_METHOD_MHS_ASLETT:
@@ -315,7 +348,7 @@ extern "C" void pht_engine_destroy(pht_engine *e) {
     if (e->ev1) cudaEventDestroy(e->ev1);
     for (void *q : e->ipc_opened) cudaIpcCloseMemHandle(q);
     stage("events, ipc");
-    void *big[] = { e->d_gtmax, e->d_gofs, e->d_gys, e->d_gus, e->d_gcs, e->d_gperm, e->d_keys, e->d_cnext, e->d_entry, e->d_ea, e->d_eobs, e->d_eM, e->d_eoff, e->d_enext, e->d_etab, e->d_escan, e->d_unif, e->d_u, e->d_us, e->d_item_u, e->d_recs, e->d_ys, e->d_cs, e->d_perm, e->d_y, e->d_cens, e->d_items /* arena: found, pend0, pend1, done live inside */, e->d_idx_exact, e->d_idx_cens,
+    void *big[] = { e->d_cy, e->d_cu, e->d_cc, e->d_cperm, e->d_cgofs, e->d_ry, e->d_ru, e->d_rc, e->d_rbase, e->d_ritems, e->d_rnext, e->d_gtmax, e->d_gofs, e->d_gys, e->d_gus, e->d_gcs, e->d_gperm, e->d_keys, e->d_cnext, e->d_entry, e->d_ea, e->d_eobs, e->d_eM, e->d_eoff, e->d_enext, e->d_etab, e->d_escan, e->d_unif, e->d_u, e->d_us, e->d_item_u, e->d_recs, e->d_ys, e->d_cs, e->d_perm, e->d_y, e->d_cens, e->d_items /* arena: found, pend0, pend1, done live inside */, e->d_idx_exact, e->d_idx_cens,
                     e->d_glist, e->d_model, e->d_stats, e->d_state, e->d_T, e->d_C, e->d_nu, e->d_zeta, e->d_var_ptr, e->d_cell_i, e->d_cell_j, e->d_pires, e->d_res };
     for (void *b : big) pht_dev_free(b, e->stream);
     if (e->stream) cudaStreamSynchronize(e->stream);
@@ -937,6 +970,139 @@ extern "C" int pht_engine_set_groups(pht_engine *e, int G, const int *T, const d
     e->groups = G;
     if (G > 1) e->h_group.assign(gid.begin(), gid.begin() + l); else e->h_group.clear();
     if (e->graph_exec) { cudaGraphExecDestroy(e->graph_exec); e->graph_exec = nullptr; }     /* kernel parameters change */
+    return e->counts_set ? counts_build(e) : 0;      /* the counted records follow the grouped layout */
+}
+
+/* ---------------------------------------------------------------- counts (method 64) */
+/* Records at or above the threshold go to k_unif_records in items of at most the chunk size; the others are expanded once
+ * into the ordinary layout.  Chosen from the "sweep" lines of profiles/counts_bench.jsonl (NVIDIA B200, 1000 W; C3 shape,
+ * 1e7 units, ms per sweep at chunk 32 / 64 / 256 / 1024): exact times rounded to 0.01 (501 records) 8.62 / 11.80 / 15.26 /
+ * 22.64 at any threshold; rounded to 1e-4 (50001 records of ~200 units) at threshold 64: 9.24 / 11.53 / 13.81 / 24.15,
+ * against 9.51 at 16, 9.48 at 256 and 10.47 at 1024 with chunk 32.  One item per warp round keeps every warp busy to the
+ * end of the sweep, which outweighs preparing a record once per 32 units instead of once per 1024.
+ * PHT_B200_COUNTS_THRESHOLD and PHT_B200_COUNTS_CHUNK override them for that sweep; the results do not depend on either. */
+#define PHT_COUNTS_THRESHOLD 64
+#define PHT_COUNTS_CHUNK 32
+
+static int counts_free(pht_engine *e) {
+    void *bufs[] = { e->d_cy, e->d_cu, e->d_cc, e->d_cperm, e->d_cgofs, e->d_ry, e->d_ru, e->d_rc, e->d_rbase, e->d_ritems, e->d_rnext };
+    for (void *b : bufs) CU(pht_dev_free(b, e->stream));
+    e->d_cy = e->d_cu = e->d_ry = e->d_ru = nullptr; e->d_cc = e->d_rc = nullptr; e->d_cperm = e->d_rbase = nullptr;
+    e->d_cgofs = e->d_rnext = nullptr; e->d_ritems = nullptr; e->n_low = 0; e->n_items = 0;
+    CU(cudaStreamSynchronize(e->stream));
+    return 0;
+}
+
+/* both layouts of the counted records from e->h_counts, in the engine's layout order (by group, then by decreasing y);
+ * unit j of record k is expanded observation base_k + j, base the exclusive prefix sum of the counts in upload order */
+static int counts_build(pht_engine *e) {
+    const long l = e->l_local;
+    const int G = e->groups;
+    const size_t ln = (size_t)(l > 0 ? l : 1);
+    std::vector<double> y(ln), u; std::vector<uint8_t> c(ln); std::vector<uint32_t> order(ln);
+    const uint32_t *dperm = G > 1 ? e->d_gperm : e->d_perm;
+    if (l > 0) {
+        CU(cudaMemcpy(y.data(), e->d_y, sizeof(double) * (size_t)l, cudaMemcpyDeviceToHost));
+        CU(cudaMemcpy(c.data(), e->d_cens, (size_t)l, cudaMemcpyDeviceToHost));
+        if (e->d_u) { u.resize(ln); CU(cudaMemcpy(u.data(), e->d_u, sizeof(double) * (size_t)l, cudaMemcpyDeviceToHost)); }
+        if (dperm) CU(cudaMemcpy(order.data(), dperm, sizeof(uint32_t) * (size_t)l, cudaMemcpyDeviceToHost));
+        else for (long i = 0; i < l; i++) order[(size_t)i] = (uint32_t)i;
+    }
+    std::vector<uint32_t> base(ln);
+    { uint64_t acc = 0; for (long i = 0; i < l; i++) { base[(size_t)i] = (uint32_t)acc; acc += e->h_counts[(size_t)i]; } }
+    const uint32_t thr = e->counts_threshold, ch = e->counts_chunk;
+    std::vector<double> ly, lu, ry, ru; std::vector<uint8_t> lc, rc; std::vector<uint32_t> lperm, rbase; std::vector<uint4> items;
+    std::vector<unsigned long long> lgofs((size_t)G + 1, 0ull);
+    for (long pos = 0; pos < l; pos++) {
+        const uint32_t k = order[(size_t)pos], w = e->h_counts[k];
+        if (w == 0u) continue;
+        const uint32_t g = G > 1 ? e->h_group[k] : 0u;
+        if (w >= thr) {
+            const uint32_t r = (uint32_t)ry.size();
+            ry.push_back(y[k]); rc.push_back(c[k]); rbase.push_back(base[k]);
+            if (!u.empty()) ru.push_back(u[k]);
+            for (uint32_t j0 = 0; j0 < w; j0 += ch) { items.push_back(make_uint4(r, j0, w - j0 < ch ? w - j0 : ch, g)); if (w - j0 <= ch) break; }
+        } else {
+            for (uint32_t j = 0; j < w; j++) {
+                ly.push_back(y[k]); lc.push_back(c[k]); lperm.push_back(base[k] + j);
+                if (!u.empty()) lu.push_back(u[k]);
+            }
+            lgofs[(size_t)g + 1] += w;
+        }
+    }
+    for (int g = 0; g < G; g++) lgofs[(size_t)g + 1] += lgofs[(size_t)g];
+    if (counts_free(e)) return -1;
+    auto up = [&](void **dst, const void *src, size_t bytes) -> cudaError_t {
+        cudaError_t ce = pht_dev_alloc(dst, bytes ? bytes : 1, e->stream);
+        if (ce == cudaSuccess && bytes) ce = cudaMemcpyAsync(*dst, src, bytes, cudaMemcpyHostToDevice, e->stream);
+        return ce;
+    };
+    CU(up((void **)&e->d_cy, ly.data(), sizeof(double) * ly.size()));
+    CU(up((void **)&e->d_cc, lc.data(), lc.size()));
+    CU(up((void **)&e->d_cperm, lperm.data(), sizeof(uint32_t) * lperm.size()));
+    if (!u.empty()) CU(up((void **)&e->d_cu, lu.data(), sizeof(double) * lu.size()));
+    CU(up((void **)&e->d_cgofs, lgofs.data(), sizeof(unsigned long long) * lgofs.size()));
+    CU(up((void **)&e->d_ry, ry.data(), sizeof(double) * ry.size()));
+    CU(up((void **)&e->d_rc, rc.data(), rc.size()));
+    CU(up((void **)&e->d_rbase, rbase.data(), sizeof(uint32_t) * rbase.size()));
+    if (!u.empty()) CU(up((void **)&e->d_ru, ru.data(), sizeof(double) * ru.size()));
+    CU(up((void **)&e->d_ritems, items.data(), sizeof(uint4) * items.size()));
+    CU(pht_dev_alloc((void **)&e->d_rnext, sizeof(unsigned long long), e->stream));
+    CU(cudaStreamSynchronize(e->stream));
+    e->n_low = (long)ly.size(); e->n_items = (long)items.size();
+    if (e->graph_exec) { cudaGraphExecDestroy(e->graph_exec); e->graph_exec = nullptr; }     /* kernel parameters change */
+    return 0;
+}
+
+extern "C" int pht_engine_set_counts(pht_engine *e, const uint32_t *counts_local) {
+    if (!e) return fail("null engine");
+    if (method_of(e->cfg) != PHT_METHOD_UNIF)
+        return fail("counts (tied observations as records) need method 64 (the uniformisation sampler): MHRS, ECS, DCS and the MH variants draw one path per observation");
+    if (e->peers_attached) return fail("counts cannot be set after the exchange windows are attached (counts need a single-rank engine)");
+    if (e->cfg.world > 1) return fail("counts need world = 1: the expanded index of a unit is a single-rank numbering");
+    CU(cudaSetDevice(e->cfg.device));
+    CU(cudaStreamSynchronize(e->stream));
+    if (!counts_local) {
+        if (!e->counts_set) return 0;
+        e->counts_set = false; e->h_counts.clear();
+        if (e->graph_exec) { cudaGraphExecDestroy(e->graph_exec); e->graph_exec = nullptr; }
+        return counts_free(e);
+    }
+    if (e->entry_set)
+        return fail("counts are not supported with entry ages (delayed entry): a record's ghost count would be a sum of w Geometric draws; clear the ages with pht_engine_set_entry(e, NULL) first");
+    const long l = e->l_local;
+    unsigned long long total = 0;
+    for (long i = 0; i < l; i++) total += counts_local[i];
+    if (total >= (1ull << 32))
+        return fail("the counts sum to %llu: the expanded observation index (Philox counter word 2) is 32 bits, so the sum must stay below 2^32", total);
+    /* every unit's path ends by max(y, u): the fixed-point scale must leave room for sum_k w_k max(y_k, u_k) */
+    std::vector<double> y((size_t)(l > 0 ? l : 1)), u;
+    if (l > 0) CU(cudaMemcpy(y.data(), e->d_y, sizeof(double) * (size_t)l, cudaMemcpyDeviceToHost));
+    if (l > 0 && e->d_u) { u.resize((size_t)l); CU(cudaMemcpy(u.data(), e->d_u, sizeof(double) * (size_t)l, cudaMemcpyDeviceToHost)); }
+    double sum = 0.0;
+    for (long i = 0; i < l; i++) {
+        const double ui = u.empty() ? INFINITY : u[(size_t)i];
+        sum += (double)counts_local[i] * (ui < INFINITY ? ui : y[(size_t)i]);
+    }
+    if (sum > 0.0 && e->cfg.zbits > pht_choose_zbits(sum))
+        return fail("zbits = %d is too fine for these counts: sum of count x max(y, u) = %g allows at most %d", e->cfg.zbits, sum, pht_choose_zbits(sum));
+    if (!e->rec_blocks) {
+        e->rec_blocks = pht_unif_records_grid_blocks(e->cfg.device, e->cfg.n);
+        if (e->rec_blocks <= 0) { e->rec_blocks = 0; return fail("the record kernel does not fit on the device: %s", cudaGetErrorString(cudaGetLastError())); }
+    }
+    e->counts_threshold = PHT_COUNTS_THRESHOLD; e->counts_chunk = PHT_COUNTS_CHUNK;
+    if (const char *ev = getenv("PHT_B200_COUNTS_THRESHOLD")) { const long v = atol(ev); if (v >= 1) e->counts_threshold = (uint32_t)v; }
+    if (const char *ev = getenv("PHT_B200_COUNTS_CHUNK")) { const long v = atol(ev); if (v >= 1 && v <= (1l << 24)) e->counts_chunk = (uint32_t)v; }
+    std::vector<uint32_t> old; old.swap(e->h_counts);
+    const bool had = e->counts_set;
+    e->h_counts.assign(counts_local, counts_local + l);
+    e->counts_set = true;
+    if (counts_build(e)) {                          /* a failed allocation: back to the previous counts */
+        const std::string msg = g_err;
+        e->h_counts.swap(old); e->counts_set = had;
+        if (had) counts_build(e); else counts_free(e);
+        return fail("%s", msg.c_str());
+    }
     return 0;
 }
 
@@ -957,7 +1123,8 @@ extern "C" int pht_engine_set_upper(pht_engine *e, const double *upper_local) {
             e->unif_tmax = 0.0;
             for (long i = 0; i < e->l_local; i++) if (y[(size_t)i] > e->unif_tmax) e->unif_tmax = y[(size_t)i];
         }
-        return group_refresh(e);
+        if (group_refresh(e)) return -1;
+        return e->counts_set ? counts_build(e) : 0;
     }
     const bool unif = method_of(e->cfg) == PHT_METHOD_UNIF;
     if (method_of(e->cfg) != PHT_METHOD_MHRS && !unif)
@@ -968,13 +1135,14 @@ extern "C" int pht_engine_set_upper(pht_engine *e, const double *upper_local) {
         CU(cudaMemcpy(y.data(), e->d_y, sizeof(double) * (size_t)l, cudaMemcpyDeviceToHost));
         CU(cudaMemcpy(c.data(), e->d_cens, (size_t)l, cudaMemcpyDeviceToHost));
     }
-    /* an interval path ends by u, not by y: the fixed-point scale must leave room for sum max(y, u) */
+    /* an interval path ends by u, not by y: the fixed-point scale must leave room for sum max(y, u) (each record counted
+     * as often as its count, when counts are set) */
     double sum = 0.0, tmax = 0.0;
     for (long i = 0; i < l; i++) {
-        const double u = upper_local[i];
+        const double u = upper_local[i], wgt = e->counts_set ? (double)e->h_counts[(size_t)i] : 1.0;
         if (y[(size_t)i] > tmax) tmax = y[(size_t)i];
         if (std::isnan(u)) return fail("upper[%ld] is NaN", i);
-        if (u == INFINITY) { sum += y[(size_t)i]; continue; }
+        if (u == INFINITY) { sum += wgt * y[(size_t)i]; continue; }
         if (!(u > y[(size_t)i])) return fail("upper[%ld] = %g is not above y = %g", i, u, y[(size_t)i]);
         if (!c[(size_t)i]) return fail("upper[%ld] = %g on an exact observation: a finite bound needs the censoring flag", i, u);
         /* (the rejection loop `while (t < y || t > u)` runs no attempt at all when y = 0; method 64 takes y = 0 as a
@@ -982,11 +1150,11 @@ extern "C" int pht_engine_set_upper(pht_engine *e, const double *upper_local) {
         if (!unif && !(y[(size_t)i] > 0.0)) return fail("upper[%ld] = %g with y = %g: an interval needs y > 0 (a tiny y for a failure before the first inspection)", i, u, y[(size_t)i]);
         if (unif && !(y[(size_t)i] >= 0.0)) return fail("upper[%ld] = %g with y = %g: an interval needs y >= 0", i, u, y[(size_t)i]);
         if (u - y[(size_t)i] > tmax) tmax = u - y[(size_t)i];
-        sum += u;
+        sum += wgt * u;
     }
     for (double a : e->h_entry) sum += a;           /* ghost paths of delayed-entry observations (pht_engine_set_entry) */
     if (sum > 0.0 && e->cfg.zbits > pht_choose_zbits(sum))
-        return fail("zbits = %d is too fine for these bounds: interval paths end by u, and sum of max(y, u) (plus the entry ages, when set) = %g allows at most %d",
+        return fail("zbits = %d is too fine for these bounds: interval paths end by u, and sum of max(y, u) (plus the entry ages, when set; times the counts, when set) = %g allows at most %d",
                     e->cfg.zbits, sum, pht_choose_zbits(sum));
     const size_t ln = (size_t)(l > 0 ? l : 1);
     if (unif) e->unif_tmax = tmax;
@@ -1002,7 +1170,8 @@ extern "C" int pht_engine_set_upper(pht_engine *e, const double *upper_local) {
         if (e->d_ys) CU(pht_gather_f64(e->d_u, e->d_perm, e->d_us, l, e->stream));
     }
     CU(cudaStreamSynchronize(e->stream));
-    return group_refresh(e);
+    if (group_refresh(e)) return -1;
+    return e->counts_set ? counts_build(e) : 0;
 }
 
 static int entry_free(pht_engine *e) {
@@ -1024,6 +1193,8 @@ extern "C" int pht_engine_set_entry(pht_engine *e, const double *entry_local) {
     if (e->peers_attached) return fail("the entry ages of a multi-rank run are set on every rank before the exchange windows are attached");
     if (entry_local && e->chains > 1)
         return fail("entry ages (delayed entry) are not supported with %d chains: the ghost paths are drawn for one chain; pht_engine_set_chains(e, 1, ...) first", e->chains);
+    if (entry_local && e->counts_set)
+        return fail("entry ages (delayed entry) are not supported with counts: a record's ghost count would be a sum of w Geometric draws; clear the counts with pht_engine_set_counts(e, NULL) first");
     if (entry_local && e->groups > 1)
         return fail("entry ages (delayed entry) are not supported with %d groups: the ghost paths are drawn on one model; pht_engine_set_groups(e, 1, ...) or (e, 0, NULL, ...) first", e->groups);
     if (e->graph_exec) { cudaGraphExecDestroy(e->graph_exec); e->graph_exec = nullptr; }     /* the sweep changes shape */
@@ -1367,6 +1538,7 @@ out:
 extern "C" int pht_engine_paths(pht_engine *e, long first, long count, int *B, int *N, double *z) {
     if (!e || !B || !N || !z) return fail("null argument");
     if (first < 0 || count < 0 || first + count > e->l_local) return fail("range [%ld, %ld) outside the shard", first, first + count);
+    if (e->counts_set) return fail("per-observation paths are not recorded while counts are set: compare with an engine on the expanded data instead");
     if (count == 0) return 0;
     CU(cudaSetDevice(e->cfg.device));
     if (e->groups > 1) return group_paths(e, first, count, B, N, z);

@@ -235,6 +235,16 @@ cudaError_t pht_launch_unif_entry(const UpdateParams &u, const SweepParams &p, c
                                   int stages, cudaStream_t st);
 size_t pht_unif_entry_scan_bytes(long count);
 int pht_unif_ghost_grid_blocks(int device, int n);
+/* method 64, records with counts (k_unif.cu; pht_engine_set_counts): the records at or above the count threshold, in the
+ * layout order (by group, then by decreasing y), and their work items.  Kernel arguments of their own, like the table. */
+struct UnifRecords {
+    const double *y, *u; const uint8_t *cens;   /* per record; u nullptr: no bounds */
+    const uint32_t *base;                        /* expanded index of the record's unit 0 */
+    const uint4 *items; long n_items;            /* (record, first unit, units, group) */
+    unsigned long long *next;                    /* hand-out counter, zeroed by the launcher */
+};
+cudaError_t pht_launch_unif_records(const SweepParams &p, const double *tab, const UnifRecords &R, int grid_blocks, cudaStream_t st);
+int pht_unif_records_grid_blocks(int device, int n);
 /* large per-call buffers: stream-ordered pool allocations, cached across calls (engine.cu) */
 cudaError_t pht_dev_alloc(void **p, size_t bytes, cudaStream_t st);
 cudaError_t pht_dev_free(void *p, cudaStream_t st);

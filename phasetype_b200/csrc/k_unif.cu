@@ -21,6 +21,11 @@
  *   k_unif_ghosts       persistent warps over the flat ghost indices [0, G), one left-censored path per lane,
  *                       reduced into the same statistics block
  *
+ * Counts (only when counts are set, pht_engine_set_counts; record form in pht_unif.h):
+ *   k_unif_records      persistent warps over (chain, record chunk) items: a warp prepares the record's weights once
+ *                       into its shared-memory slab, its lanes draw the chunk's units; records with few units run
+ *                       through k_unif_paths / k_unif_chain_paths in an expanded layout of their own
+ *
  * Bound: FP64 issue.  Per observation the sampler evaluates ~3 K(lambda y) Poisson weights (one pht_exp each) and
  * ~K(lambda y) n multiply-adds for the end-state weights, plus n per uniformised event; the observations are handed out
  * by decreasing y (k_sort.cu), so the lanes of a warp run similar K.
@@ -333,6 +338,112 @@ __global__ void __launch_bounds__(THREADS) k_unif_ghosts(SweepParams p, const do
     if (err) atomicOr(&p.state->error, err);
     __syncthreads();
     block_flush<THREADS>(p, n, sm.Nacc, sm.Bacc, sm.zlo, sm.zhi);
+}
+
+/* ---- records with counts (pht_engine_set_counts; pht_unif.h, "Records with counts"): launched only when counts are set.
+ * Work items are (record, chunk of at most PHT_COUNTS_CHUNK units) of the records at or above the count threshold; the
+ * hand-out runs over (chain, item), unit = c groups + item's group as in k_unif_chain_paths.  A persistent warp takes one
+ * work item at a time, prepares the record into its shared-memory slab (lanes over k for the weights, over states and
+ * cells for the vector and the matrix), then its lanes draw the chunk's units, one per lane, 32 at a time, into the
+ * warp's own accumulators, which are flushed into the unit's statistics block after every item (so no 32-bit counter
+ * can wrap, whatever the count).  Unit j of record k is expanded observation base_k + j: Philox sub-stream 0 of (sweep,
+ * base_k + j) with chain c's key. */
+#define UNIF_REC_KB 255              /* weights a slab holds per record (k = 0 .. KB); beyond, pht_unif_w recomputes them */
+
+struct UnifRecSlab {
+    double *w1, *w2, *v, *mx; unsigned long long *zlo; long long *zhi; unsigned int *Nacc, *Bacc;
+    __host__ __device__ static size_t bytes(int n) {
+        return sizeof(double) * (size_t)(2 * (UNIF_REC_KB + 1) + n + n * n + 2 * n) + sizeof(unsigned int) * (size_t)(n * n + n);
+    }
+    __device__ __forceinline__ void carve(unsigned char *raw, int n) {
+        double *d = reinterpret_cast<double *>(raw);
+        w1 = d; d += UNIF_REC_KB + 1; w2 = d; d += UNIF_REC_KB + 1; v = d; d += n; mx = d; d += n * n;
+        zlo = reinterpret_cast<unsigned long long *>(d); d += n; zhi = reinterpret_cast<long long *>(d); d += n;
+        Nacc = reinterpret_cast<unsigned int *>(d); Bacc = Nacc + n * n;
+    }
+};
+template <int THREADS>
+static size_t unif_rec_smem(int n) {       /* per-lane path scratch (stride THREADS) + one slab per warp, 16-byte aligned */
+    return sizeof(double) * (size_t)(2 * n * THREADS) + (size_t)(THREADS / 32) * ((UnifRecSlab::bytes(n) + 15) & ~(size_t)15);
+}
+
+template <int THREADS>
+__global__ void __launch_bounds__(THREADS) k_unif_records(SweepParams p, const double *tab, UnifRecords R) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const int n = p.n, tid = threadIdx.x, lane = tid & 31, cap = PHT_UNIF_CAP;
+    const unsigned FULL = 0xffffffffu;
+    const ModelLayout ML = ModelLayout::make(n, p.m);
+    const pht_unif_layout TL = pht_unif_layout_make(n, cap);
+    double *Za = reinterpret_cast<double *>(smem_raw), *Zb = Za + n * THREADS;
+    UnifRecSlab w;
+    w.carve(smem_raw + sizeof(double) * (size_t)(2 * n * THREADS) + (size_t)(tid >> 5) * ((UnifRecSlab::bytes(n) + 15) & ~(size_t)15), n);
+    for (int i = lane; i < n * n; i += 32) w.Nacc[i] = 0u;
+    for (int i = lane; i < n; i += 32) { w.Bacc[i] = 0u; w.zlo[i] = 0ull; w.zhi[i] = 0; }
+    __syncwarp();
+    const uint32_t iter = p.state->iter;
+    const unsigned long long work = (unsigned long long)p.chains * (unsigned long long)R.n_items;
+    unsigned long long c_paths = 0; int err = 0;
+    UnifCount ctx; ctx.p = &p; ctx.Nacc = w.Nacc; ctx.n = n; ctx.out_idx = 0;
+    for (;;) {
+        unsigned long long f = 0;
+        if (lane == 0) f = atomicAdd(R.next, 1ull);
+        f = __shfl_sync(FULL, f, 0);
+        if (f >= work) break;
+        const unsigned c = (unsigned)(f / (unsigned long long)R.n_items);
+        const uint4 it = R.items[f - (unsigned long long)c * R.n_items];       /* record, first unit, units, group */
+        const int unit = (int)c * p.groups + (int)it.w;
+        const double *utab = tab + (size_t)unit * TL.total, *model = p.model + (size_t)unit * ML.total;
+        pht_unif_rec rc;
+        const int e0 = pht_unif_rec_init(&rc, utab, cap, R.y[it.x], R.cens[it.x], R.u ? R.u[it.x] : INFINITY, UNIF_REC_KB);
+        if (e0) { err |= e0; continue; }
+        rc.w1 = w.w1; rc.w2 = w.w2; rc.v = w.v; rc.mx = w.mx;
+        const double *lgk = utab + TL.lgk;
+        const int k1 = rc.K1 < UNIF_REC_KB ? rc.K1 : UNIF_REC_KB, k2 = !rc.iv ? -1 : rc.K2 < UNIF_REC_KB ? rc.K2 : UNIF_REC_KB;
+        for (int k = lane; k <= k1; k += 32) w.w1[k] = pht_unif_w(rc.x, rc.lx, k, lgk);
+        for (int k = lane; k <= k2; k += 32) w.w2[k] = pht_unif_w(rc.x2, rc.lx2, k, lgk);
+        __syncwarp();
+        if (lane < n) w.v[lane] = pht_unif_rec_v_entry(&rc, utab, n, cap, model + ML.s, lane);
+        if (rc.y > 0.0 && (int)utab[2] > 1)
+            for (int e = lane; e < n * n; e += 32) w.mx[e] = pht_unif_rec_m_entry(&rc, utab, n, cap, model + ML.pi, e % n, e / n);
+        __syncwarp();
+        const uint32_t k0 = p.ckeys[2 * c], k1key = p.ckeys[2 * c + 1], base = R.base[it.x] + it.y;
+        for (unsigned j = lane; j < it.z; j += 32) {
+            pht_stream st; st.k0 = k0; st.k1 = k1key;
+            pht_stream_seek(&st, iter, base + j, 0u, 0u);
+            int B = 0;
+            err |= pht_unif_rec_path(utab, n, cap, model + ML.scale, model + ML.cum, &rc, &st, Za + tid, Zb + tid, THREADS, &ctx, &B);
+            path_flush<THREADS>(p, n, Za, w.zlo, w.zhi, w.Bacc, B, 0);
+            c_paths++;
+        }
+        __syncwarp();
+        unsigned long long *g = reinterpret_cast<unsigned long long *>(p.stats + (size_t)unit * stats_len(n));
+        for (int i = lane; i < n * n; i += 32) if (w.Nacc[i]) { atomicAdd(&g[i], (unsigned long long)w.Nacc[i]); w.Nacc[i] = 0u; }
+        for (int i = lane; i < n; i += 32) {
+            if (w.Bacc[i]) { atomicAdd(&g[n * n + i], (unsigned long long)w.Bacc[i]); w.Bacc[i] = 0u; }
+            if (w.zlo[i]) { atomicAdd(&g[n * n + n + i], w.zlo[i]); w.zlo[i] = 0ull; }
+            if (w.zhi[i]) { atomicAdd(&g[n * n + 2 * n + i], (unsigned long long)w.zhi[i]); w.zhi[i] = 0; }
+        }
+        __syncwarp();
+    }
+    if (err) atomicOr(&p.state->error, err);
+    for (int o = 16; o > 0; o >>= 1) c_paths += __shfl_down_sync(FULL, c_paths, o);
+    if (lane == 0) atomicAdd(&p.state->counters[PHT_CNT_PATHS], c_paths);
+}
+
+int pht_unif_records_grid_blocks(int device, int n) {
+    const size_t smem = unif_rec_smem<UNIF_THREADS>(n);
+    int per_sm = 0, sms = 0;
+    if (cudaFuncSetAttribute(k_unif_records<UNIF_THREADS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return -1;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_unif_records<UNIF_THREADS>, UNIF_THREADS, smem) != cudaSuccess) return -1;
+    if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device) != cudaSuccess) return -1;
+    return per_sm * sms;
+}
+
+cudaError_t pht_launch_unif_records(const SweepParams &p, const double *tab, const UnifRecords &R, int grid_blocks, cudaStream_t st) {
+    const cudaError_t e = cudaMemsetAsync(R.next, 0, sizeof(unsigned long long), st);
+    if (e != cudaSuccess) return e;
+    k_unif_records<UNIF_THREADS><<<grid_blocks, UNIF_THREADS, unif_rec_smem<UNIF_THREADS>(p.n), st>>>(p, tab, R);
+    return cudaGetLastError();
 }
 
 size_t pht_unif_entry_scan_bytes(long count) {

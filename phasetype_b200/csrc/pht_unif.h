@@ -169,6 +169,74 @@ PHT_HD int pht_unif_ghost_count(const double *tab, const double *etab, int n, in
     return 0;
 }
 
+/* Records with counts (pht_engine_set_counts).  The w tied units of a record (y, flag, u) are w observations whose
+ * paths differ only in their Philox streams, so everything pht_unif_path computes before its first draw is computed
+ * once per record: the Poisson weights of k <= K1 (and of 1 <= k <= K2 for an interval), the n weights of the state at y,
+ * and, when pi has more than one positive entry and y > 0, the n x n weights of the start state given the state at y.
+ * pht_unif_rec_path then draws one unit from them.  Every quantity is the same expression, summed in the same order with
+ * the same zero-weight skips, as in pht_unif_path, so a unit's path is bit for bit that observation's path.  The two
+ * forms are separate code: a lane cannot hold K weights of its own, a warp preparing one record can.
+ * Weight buffers hold k <= kb; weights beyond are recomputed by pht_unif_w, which gives the same bits. */
+typedef struct {
+    double y, u, d, x, lx, x2, lx2;
+    int cens, iv, K1, K2, kb;
+    const double *w1, *w2;       /* w1[k] = Pois(k; lambda y), k <= min(K1, kb); w2[k] = Pois(k; lambda (u - y)), 1 <= k <= min(K2, kb) */
+    const double *v;             /* the n weights of the state at y (step 1, before the pick) */
+    const double *mx;            /* column b (n x n, column-major): pi_c sum_k w1[k] (R^k)_cb (only y > 0 and npos > 1) */
+} pht_unif_rec;
+
+/* the record's scalars; 0 or PHT_UNIF_ERR_TABLE (the same test as pht_unif_path) */
+PHT_HD int pht_unif_rec_init(pht_unif_rec *rc, const double *tab, int cap, double y, int cens, double u, int kb) {
+    const double lam = tab[0];
+    rc->y = y; rc->cens = cens; rc->u = u; rc->kb = kb;
+    rc->iv = cens && u <= 1.7976931348623157e308;
+    rc->x = lam * y; rc->lx = rc->x > 0.0 ? pht_log(rc->x) : 0.0;
+    rc->d = rc->iv ? u - y : 0.0; rc->x2 = lam * rc->d; rc->lx2 = rc->x2 > 0.0 ? pht_log(rc->x2) : 0.0;
+    rc->K1 = pht_unif_K(rc->x); rc->K2 = rc->iv ? pht_unif_K(rc->x2) : 0;
+    return (rc->K1 >= cap || rc->K2 >= cap) ? PHT_UNIF_ERR_TABLE : 0;
+}
+PHT_HD double pht_unif_rec_w1(const pht_unif_rec *rc, int k, const double *lgk) {
+    return k <= rc->kb ? rc->w1[k] : pht_unif_w(rc->x, rc->lx, k, lgk);
+}
+PHT_HD double pht_unif_rec_w2(const pht_unif_rec *rc, int k, const double *lgk) {
+    return k <= rc->kb ? rc->w2[k] : pht_unif_w(rc->x2, rc->lx2, k, lgk);
+}
+/* entry c of the weights of the state at y (pht_unif_path step 1); the weight buffers must be filled */
+PHT_HD double pht_unif_rec_v_entry(const pht_unif_rec *rc, const double *tab, int n, int cap, const double *s, int c) {
+    const pht_unif_layout L = pht_unif_layout_make(n, cap);
+    const double *lgk = tab + L.lgk;
+    double v = 0.0;
+    for (int k = 0; k <= rc->K1; k++) {
+        const double w = pht_unif_rec_w1(rc, k, lgk);
+        if (w == 0.0) continue;
+        v += w * tab[L.q + k * n + c];
+    }
+    if (rc->iv) {
+        double z = 0.0;
+        for (int k = 1; k <= rc->K2; k++) {
+            const double w = pht_unif_rec_w2(rc, k, lgk);
+            if (w == 0.0) continue;
+            z += w * tab[L.g + k * n + c];
+        }
+        v = v * z;
+    } else if (!rc->cens) {
+        v = v * s[c];
+    }
+    return v;
+}
+/* entry (c, b) of the start-state weights (pht_unif_path step 2 for state b at y) */
+PHT_HD double pht_unif_rec_m_entry(const pht_unif_rec *rc, const double *tab, int n, int cap, const double *pi, int c, int b) {
+    const pht_unif_layout L = pht_unif_layout_make(n, cap);
+    const double *lgk = tab + L.lgk;
+    double a = 0.0;
+    for (int k = 0; k <= rc->K1; k++) {
+        const double w = pht_unif_rec_w1(rc, k, lgk);
+        if (w == 0.0) continue;
+        a += w * tab[L.P + k * n * n + b * n + c];
+    }
+    return pi[c] * a;
+}
+
 /* the sampler itself is compiled where the includer says how transitions are counted: PHT_UNIF_CTX (a type) and
  * PHT_UNIF_COUNT(ctx, from, to); PHT_UNIF_U01(st) may replace the uniform draw by an equivalent call, PHT_UNIF_FN the function's qualifiers */
 #if defined(PHT_UNIF_CTX) && defined(PHT_UNIF_COUNT)
@@ -297,6 +365,119 @@ PHT_UNIF_FN int pht_unif_path(const double *tab, int n, int cap, const double *s
         double sofar = 0.0; int kk = -1;
         for (int k = 1; k <= K2; k++) {
             const double v = pht_unif_w(x2, lx2, k, lgk) * tab[L.g + k * n + b];
+            if (v > 0.0) { sofar += v; kk = k; if (sofar >= target) break; }
+        }
+        int cur = b, absorbed = 0; double et = 0.0;
+        for (int i = 1; i <= kk; i++) {
+            const double e = -pht_log(PHT_UNIF_U01(st));
+            et += e;
+            if (absorbed) continue;
+            zb[cur * zs] += e;
+            const double *gn = tab + L.g + (kk - i) * n;
+            double t2 = 0.0;
+            for (int q = 0; q < n; q++) t2 += R[cur + q * n] * gn[q];
+            t2 += r[cur];
+            if (!(t2 > 0.0)) return PHT_UNIF_ERR_ZERO;
+            const double tg = PHT_UNIF_U01(st) * t2;
+            double so = 0.0; int c = -1;
+            for (int q = 0; q < n; q++) {
+                const double v = R[cur + q * n] * gn[q];
+                if (v > 0.0) { so += v; c = q; if (so >= tg) break; }
+            }
+            if (!(so >= tg) && r[cur] > 0.0) c = n;      /* absorption: the last category */
+            if (c == n) { PHT_UNIF_COUNT(ctx, cur, cur); absorbed = 1; }
+            else { if (c != cur) PHT_UNIF_COUNT(ctx, cur, c); cur = c; }
+        }
+        const double e = -pht_log(PHT_UNIF_U01(st));
+        et += e;
+        const double sc = d / et;
+        for (int c = 0; c < n; c++) if (zb[c * zs] != 0.0) za[c * zs] = za[c * zs] + zb[c * zs] * sc;
+    }
+    return 0;
+}
+
+/* One unit of a prepared record (pht_unif_rec: scalars, weight buffers, rc->v and, when y > 0 and pi has more than one
+ * positive entry, rc->mx): the draws of pht_unif_path from the same stream, with the same results.  Arguments as there. */
+PHT_UNIF_FN int pht_unif_rec_path(const double *tab, int n, int cap, const double *scale, const double *cum,
+                                  const pht_unif_rec *rc, pht_stream *st, double *za, double *zb, int zs, PHT_UNIF_CTX *ctx, int *B) {
+    const pht_unif_layout L = pht_unif_layout_make(n, cap);
+    const int npos = (int)tab[2], a1 = (int)tab[3];
+    const double *lgk = tab + L.lgk, *R = tab + L.R, *r = tab + L.r;
+    const double y = rc->y, d = rc->d;
+    const int cens = rc->cens, iv = rc->iv, K1 = rc->K1, K2 = rc->K2;
+    *B = 0;
+
+    /* 1.-2. the state at y and the start state from the record's weights */
+    const int b = pht_unif_pick(rc->v, n, 1, PHT_UNIF_U01(st));
+    if (b < 0) return PHT_UNIF_ERR_ZERO;
+    int a;
+    if (y > 0.0 && npos > 1) {
+        a = pht_unif_pick(rc->mx + b * n, n, 1, PHT_UNIF_U01(st));
+        if (a < 0) return PHT_UNIF_ERR_ZERO;
+    } else a = y > 0.0 ? a1 : b;
+    *B = a;
+    for (int c = 0; c < n; c++) { za[c * zs] = 0.0; zb[c * zs] = 0.0; }
+
+    /* 3.-4. the bridge a -> b on [0, y] */
+    if (y > 0.0) {
+        double tot = 0.0;
+        for (int k = 0; k <= K1; k++) tot += pht_unif_rec_w1(rc, k, lgk) * tab[L.P + k * n * n + a + b * n];
+        if (!(tot > 0.0)) return PHT_UNIF_ERR_ZERO;
+        const double target = PHT_UNIF_U01(st) * tot;
+        double sofar = 0.0; int kk = -1;
+        for (int k = 0; k <= K1; k++) {
+            const double v = pht_unif_rec_w1(rc, k, lgk) * tab[L.P + k * n * n + a + b * n];
+            if (v > 0.0) { sofar += v; kk = k; if (sofar >= target) break; }
+        }
+        int cur = a; double et = 0.0;
+        for (int i = 1; i <= kk; i++) {
+            const double e = -pht_log(PHT_UNIF_U01(st));
+            za[cur * zs] += e; et += e;
+            int c = b;
+            if (i < kk) {
+                const double *Pn = tab + L.P + (kk - i) * n * n + b * n;
+                double t2 = 0.0;
+                for (int q = 0; q < n; q++) t2 += R[cur + q * n] * Pn[q];
+                if (!(t2 > 0.0)) return PHT_UNIF_ERR_ZERO;
+                const double tg = PHT_UNIF_U01(st) * t2;
+                double so = 0.0; c = -1;
+                for (int q = 0; q < n; q++) {
+                    const double v = R[cur + q * n] * Pn[q];
+                    if (v > 0.0) { so += v; c = q; if (so >= tg) break; }
+                }
+            }
+            if (c != cur) PHT_UNIF_COUNT(ctx, cur, c);
+            cur = c;
+        }
+        const double e = -pht_log(PHT_UNIF_U01(st));
+        za[cur * zs] += e; et += e;
+        const double sc = y / et;
+        for (int c = 0; c < n; c++) if (za[c * zs] != 0.0) za[c * zs] = za[c * zs] * sc;
+    }
+
+    /* 5. after y */
+    if (!cens) {
+        PHT_UNIF_COUNT(ctx, b, b);
+    } else if (!iv) {
+        int j = b;
+        for (;;) {
+            const double t = scale[j] * -pht_log(PHT_UNIF_U01(st));
+            const double target = PHT_UNIF_U01(st);
+            const double *cr = cum + j * (n + 1);
+            int k = 0;
+            while (k < n && cr[k] < target) k++;
+            za[j * zs] += t;
+            if (k < n) { PHT_UNIF_COUNT(ctx, j, k); j = k; }
+            else { PHT_UNIF_COUNT(ctx, j, j); break; }
+        }
+    } else {
+        double tot = 0.0;
+        for (int k = 1; k <= K2; k++) tot += pht_unif_rec_w2(rc, k, lgk) * tab[L.g + k * n + b];
+        if (!(tot > 0.0)) return PHT_UNIF_ERR_ZERO;
+        const double target = PHT_UNIF_U01(st) * tot;
+        double sofar = 0.0; int kk = -1;
+        for (int k = 1; k <= K2; k++) {
+            const double v = pht_unif_rec_w2(rc, k, lgk) * tab[L.g + k * n + b];
             if (v > 0.0) { sofar += v; kk = k; if (sofar >= target) break; }
         }
         int cur = b, absorbed = 0; double et = 0.0;

@@ -63,6 +63,20 @@ def inspection(R, s, l, spacing, k, rng):
     return y, u, np.ones(l, dtype=np.int32), t
 
 
+def tabulate(y, cens, u=None):
+    """Tied observations as records with counts (Engine.set_counts): the distinct (y, cens, u) in order of first occurrence
+    and how often each occurs.  Returns (y, cens, u, counts) with u None when no u was given; np.repeat of the records by
+    the counts gives back the observations, grouped by record."""
+    y = np.asarray(y, dtype=np.float64); c = np.asarray(cens, dtype=np.int32)
+    cols = [y.view(np.uint64), c.astype(np.uint64)]
+    if u is not None:
+        cols.append(np.asarray(u, dtype=np.float64).view(np.uint64))
+    _, first, counts = np.unique(np.stack(cols, axis=1), axis=0, return_index=True, return_counts=True)
+    order = np.argsort(first, kind="stable")
+    idx = first[order]
+    return (y[idx], c[idx], None if u is None else np.asarray(u, dtype=np.float64)[idx], counts[order].astype(np.uint32))
+
+
 def delayed_entry(R, s, l, entry, rng, censor=None, spacing=None):
     """Delayed-entry (left-truncated) data: l units of the CTMC (R, s) started in state 0 that were still working at their
     entry ages.  entry(k, rng) draws k candidate ages; a unit absorbed at or before its age never enters the sample and is
