@@ -73,7 +73,8 @@ void LJMA_Gibbs(int *it, int *mhit, int *method, int *n, int *m, double *nu, dou
  * (pht_engine_set_pi with beta) works with it.  Lowest priority of the mask; `mhit` is not used.  The table holds
  * PHT_UNIF_CAP = 4096 powers (33 MB at n = 32): an observation whose lambda y (or lambda (u - y)) needs more raises error
  * bit 256.  Delayed entry (left-truncated observations, pht_engine_set_entry) is this method's alone, and so are counts
- * (tied observations as records drawn once per record, pht_engine_set_counts).  (Bit 32 stays
+ * (tied observations as records drawn once per record, pht_engine_set_counts) and panel observations (the phases a unit
+ * was seen in at inspection times, pht_engine_set_visits).  (Bit 32 stays
  * unassigned.) */
 #define PHT_METHOD_UNIF 64
 #define PHT_MAX_PHASES  32
@@ -246,6 +247,31 @@ int pht_engine_group_stats(pht_engine *e, long long *N, long long *B, long long 
  * observation word is 32 bits); a configured zbits above pht_choose_zbits(sum_k w_k max(y_k, u_k)), which
  * pht_engine_set_upper also applies while counts are set; and pht_engine_paths while counts are set. */
 int pht_engine_set_counts(pht_engine *e, const uint32_t *counts_local);
+
+/* Panel observations (method 64 only): what a unit was doing before it failed -- a disease stage recorded at clinic visits,
+ * a degradation level read at inspections, the state of a multi-state model known at panel times.  Local observation k
+ * carries visits (t_kj, A_kj), j = 1..m_k, 0 <= t_k1 < ... < t_km <= y_k: at time t the unit was in one of the phases of
+ * the set A, a uint32 bitmask (bit c: phase c).  A one-phase mask is a phase seen exactly, a mask of several phases an
+ * observed stage made of several latent phases, a mask of every phase only "alive at t"; t = 0 gives the possible start
+ * states.  The terminal information is unchanged (exact, right-censored, or (y, u] through pht_engine_set_upper).  Each
+ * panel path is drawn from its exact conditional law given pi, the visits and the terminal information: a backward pass
+ * over the visits, then the visit states and a bridge per gap (pht_unif.h, "Panel observations"); the sweep statistics and
+ * both updates stay as they are.  offsets_local holds l_local + 1 offsets in the order of y_local (a CSR: observation k's
+ * visits are t and mask [offsets[k], offsets[k + 1])); NULL clears the visits.  Observations without visits draw exactly
+ * the paths they draw without this call, and an engine whose observations have no visits is, bit for bit, the engine
+ * that never called it.  Chains and groups (either order), interval bounds and delayed entry (either order; a first
+ * visit at or after the entry age) work with visits.  Refused, each with its own message and leaving the engine as it was: any method but 64; world > 1 and a call
+ * after the exchange windows are attached; counts (pht_engine_set_counts, in either order); visit times that are
+ * negative, not increasing or above y; a visit on an observation with y = 0 other than a single one at t = 0; an empty
+ * mask or one with bits at or above n; more than PHT_MAX_VISITS visits on one observation; a visit sequence that the
+ * start distribution and the structure (T and C, or T_g and C_g of the observation's group) cannot produce, by
+ * reachability from the support of chain 0's pi (the start state itself for a visit at t = 0) over the structure's nonzero
+ * cells, with an exit after the last visit for exact and interval data (its first draw would find only zero weights);
+ * a failed allocation.  While visits are set, pht_engine_set_pi and pht_engine_set_groups apply the same check to the
+ * new pi or structures and refuse, leaving the engine as it was, what the visits cannot follow.  The device holds, besides the visits,
+ * (most visits of one observation + 1) x n doubles of scratch per resident lane of the panel kernel. */
+#define PHT_MAX_VISITS 1024
+int pht_engine_set_visits(pht_engine *e, const int64_t *offsets_local, const double *t, const uint32_t *mask);
 
 /* run `nsweeps` Gibbs sweeps; row r of out (nsweeps x m, row-major) is the draw of sweep r.
  * out may be NULL (results stay on the device; fetch later with pht_engine_get_theta). */

@@ -21,7 +21,7 @@ SYMBOLS = [
     "pht_engine_counters", "pht_fp64_fma_rate", "pht_engine_set_l2_flush", "pht_engine_peer_handle", "pht_engine_peer_attach", "pht_engine_round_trace", "pht_engine_set_pi", "pht_engine_get_pi", "pht_engine_pi_rows",
     "pht_engine_set_upper", "pht_engine_set_entry", "pht_engine_entry_paths",
     "pht_engine_set_chains", "pht_engine_set_chain_theta", "pht_engine_get_chain_theta", "pht_engine_chain_rows",
-    "pht_engine_set_groups", "pht_engine_group_stats", "pht_engine_set_counts",
+    "pht_engine_set_groups", "pht_engine_group_stats", "pht_engine_set_counts", "pht_engine_set_visits",
 ]
 PEER_HANDLE_BYTES = 128
 # method 64 (include/pht_b200.h PHT_METHOD_UNIF): the uniformisation path sampler; exact, right-, interval- and
@@ -29,6 +29,7 @@ PEER_HANDLE_BYTES = 128
 METHOD_UNIF = 64
 MAX_CHAINS = 1024            # include/pht_b200.h PHT_MAX_CHAINS: chains one METHOD_UNIF engine can run (Engine.set_chains)
 MAX_GROUPS = 64              # include/pht_b200.h PHT_MAX_GROUPS: groups with their own structure (Engine.set_groups)
+MAX_VISITS = 1024            # include/pht_b200.h PHT_MAX_VISITS: visits of one observation (Engine.set_visits)
 CNT_NAMES = ["paths", "attempts", "jumps", "dens_evals", "env_updates", "brent_evals", "arms_calls",
              "metrop_rejects", "nonfinite", "deferred", "tail_rounds", "errors", "launches", "ns_lane", "ns_tail", "ns_replay",
              "ns_global", "ns_xwait", "global_rounds", "global_items"]
@@ -94,6 +95,7 @@ def lib():
     L.pht_engine_set_groups.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
     L.pht_engine_group_stats.argtypes = [C.c_void_p, _lp, _lp, _lp]
     L.pht_engine_set_counts.argtypes = [C.c_void_p, C.c_void_p]
+    L.pht_engine_set_visits.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     L.pht_engine_peer_handle.argtypes = [C.c_void_p, C.c_void_p]
     L.pht_engine_peer_attach.argtypes = [C.c_void_p, C.c_void_p]
     _lib = L
@@ -366,6 +368,28 @@ class Engine:
         if not self.l_local:
             w = np.zeros(1, dtype=np.uint32)     # an empty shard still takes part (never NULL, which clears)
         _check(lib().pht_engine_set_counts(self._h, w.ctypes.data))
+
+    def set_visits(self, offsets, t=None, mask=None):
+        """Panel observations (METHOD_UNIF only, one rank, no counts): local observation k was seen at times
+        t[offsets[k]:offsets[k + 1]] (increasing, within [0, y_k]) in one of the phases of mask[...] (uint32 bitmasks,
+        bit c: phase c; synth.stage_masks builds stage masks).  offsets has l_local + 1 entries starting at 0.  Each path is
+        then drawn given its visits too; observations without visits draw the paths they drew before.  None clears them."""
+        if offsets is None:
+            _check(lib().pht_engine_set_visits(self._h, None, None, None))
+            return
+        off = np.ascontiguousarray(offsets, dtype=np.int64)
+        if off.shape != (self.l_local + 1,):
+            raise EngineError("set_visits: %d offsets for %d local observations (expected l_local + 1)" % (off.size, self.l_local))
+        total = int(off[-1]) if off.size else 0
+        tv = np.ascontiguousarray(t if t is not None else np.zeros(0), dtype=np.float64)
+        mv = np.asarray(mask if mask is not None else np.zeros(0, dtype=np.uint32))
+        if tv.shape != (total,) or mv.shape != (total,):
+            raise EngineError("set_visits: %d times and %d masks for %d visits" % (tv.size, mv.size, total))
+        if mv.size and (mv.min() < 0 or mv.max() > 0xffffffff):
+            raise EngineError("set_visits: masks must lie in 0 .. 2^32 - 1")
+        mv = np.ascontiguousarray(mv, dtype=np.uint32)
+        tv = tv if total else np.zeros(1); mv = mv if total else np.zeros(1, dtype=np.uint32)
+        _check(lib().pht_engine_set_visits(self._h, off.ctypes.data, tv.ctypes.data, mv.ctypes.data))
 
     def group_stats(self):
         """One sweep's statistics of chain 0 per group, without an update: N (G, n*n), B (G, n), zfix (G, n); their sum

@@ -61,6 +61,16 @@ static int nccl_load() {
 static const int NCCL_INT64 = 4, NCCL_SUM = 0;     /* ncclInt64, ncclSum (stable enum values of nccl.h) */
 
 /* ---------------------------------------------------------------- engine */
+/* method 64 with visits: the observations without visits in the ordinary layout of their own (y, flags, u, local index and
+ * group offsets), run by the per-observation kernels; the panel observations in theirs (the same, plus chunk offsets and
+ * the visit CSR) and the beta scratch of k_unif_panel_paths, with its hand-out counter; both by group, then by decreasing y */
+struct PanelBufs {
+    double *py = nullptr, *pu = nullptr; uint8_t *pc = nullptr; uint32_t *pperm = nullptr; unsigned long long *pgofs = nullptr;
+    double *vy = nullptr, *vu = nullptr, *vt = nullptr, *beta = nullptr; uint8_t *vc = nullptr; uint32_t *vperm = nullptr, *vm = nullptr;
+    unsigned long long *vgofs = nullptr, *vcoff = nullptr, *voff = nullptr, *vnext = nullptr;
+    long n_plain = 0, n_panel = 0;
+};
+
 struct pht_engine {
     pht_config cfg;
     std::vector<int> T; std::vector<double> C, nu, zeta;
@@ -122,6 +132,10 @@ struct pht_engine {
     double *d_ry = nullptr, *d_ru = nullptr; uint8_t *d_rc = nullptr; uint32_t *d_rbase = nullptr; uint4 *d_ritems = nullptr;
     long n_items = 0; unsigned long long *d_rnext = nullptr; int rec_blocks = 0;
     uint32_t counts_threshold = 0, counts_chunk = 0;
+    /* method 64, panel observations (pht_engine_set_visits): the visits in upload order (host CSR) and the two layouts
+     * (PanelBufs below); the panel kernel's grid */
+    bool visits_set = false; std::vector<int64_t> h_voff; std::vector<double> h_vt; std::vector<uint32_t> h_vm;
+    PanelBufs pan; int panel_blocks = 0;
     /* graph */
     cudaGraphExec_t graph_exec = nullptr; int graph_res_rows = -1; double *graph_res = nullptr;
     unsigned long long graph_launches = 0;      /* kernels one replay of the captured sweep launches */
@@ -229,6 +243,30 @@ static int method_of(const pht_config &c) {       /* dispatch priority of src/PH
 }
 
 static int counts_build(pht_engine *e);      /* pht_engine_set_counts: the counted records' layouts */
+static int visits_build(pht_engine *e);      /* pht_engine_set_visits: the panel and plain layouts */
+static int engine_visits_reachable(pht_engine *e, const int64_t *off, const double *t, const uint32_t *mask, const double *pi,
+                                   int G, const int *T, const double *C, const uint8_t *gid);
+
+static UnifPanel panel_args(const PanelBufs &b) {
+    UnifPanel V; memset(&V, 0, sizeof(V));
+    V.y = b.vy; V.u = b.vu; V.cens = b.vc; V.perm = b.vperm; V.gofs = b.vgofs; V.coff = b.vcoff;
+    V.voff = b.voff; V.vt = b.vt; V.vm = b.vm; V.beta = b.beta; V.next = b.vnext;
+    return V;
+}
+
+/* method 64 with visits: the observations without visits through the per-observation kernels (their own layout and group
+ * offsets), then k_unif_panel_paths over the panel observations; both add to the same statistics blocks */
+static int enqueue_panel(pht_engine *e, const SweepParams &p) {
+    const PanelBufs &b = e->pan;
+    if (b.n_plain > 0) {
+        SweepParams q = p;
+        q.y = b.py; q.cens = b.pc; q.perm = b.pperm; q.u = b.pu; q.l_local = b.n_plain;
+        CU(pht_launch_unif(q, e->d_unif, q.groups > 1 ? b.pgofs : nullptr, q.chains > 1 || q.groups > 1 ? e->chain_blocks : e->grid_blocks, e->stream));
+        e->launches++;
+    }
+    CU(pht_launch_unif_panel(p, e->d_unif, panel_args(b), e->panel_blocks, e->stream));
+    return 0;                                      /* enqueue_paths counts the panel kernel */
+}
 
 /* method 64 with counts: the expanded records below the threshold through the per-observation kernels (their own layout
  * and group offsets), then k_unif_records over the items of the others; both add to the same statistics blocks */
@@ -266,6 +304,7 @@ static int enqueue_paths(pht_engine *e, const SweepParams &p, const uint32_t *id
     case PHT_METHOD_MHS_HOBOLTH: CU(pht_launch_dcs(p, e->grid_blocks, e->stream, true)); e->launches++; break;
     case PHT_METHOD_UNIF:
         if (e->counts_set) { if (enqueue_counts(e, p)) return -1; break; }
+        if (e->visits_set && p.outB == nullptr) { if (enqueue_panel(e, p)) return -1; break; }   /* (pht_engine_paths: panel_window) */
         CU(pht_launch_unif(p, e->d_unif, p.groups > 1 ? e->d_gofs : nullptr, p.chains > 1 || p.groups > 1 ? e->chain_blocks : e->grid_blocks, e->stream));
         break;
     case PHT_METHOD_MHS_ASLETT:
@@ -348,6 +387,9 @@ extern "C" void pht_engine_destroy(pht_engine *e) {
     if (e->ev1) cudaEventDestroy(e->ev1);
     for (void *q : e->ipc_opened) cudaIpcCloseMemHandle(q);
     stage("events, ipc");
+    { const PanelBufs &b = e->pan;
+      void *pb[] = { b.py, b.pu, b.pc, b.pperm, b.pgofs, b.vy, b.vu, b.vt, b.beta, b.vc, b.vperm, b.vm, b.vgofs, b.vcoff, b.voff, b.vnext };
+      for (void *q : pb) pht_dev_free(q, e->stream); }
     void *big[] = { e->d_cy, e->d_cu, e->d_cc, e->d_cperm, e->d_cgofs, e->d_ry, e->d_ru, e->d_rc, e->d_rbase, e->d_ritems, e->d_rnext, e->d_gtmax, e->d_gofs, e->d_gys, e->d_gus, e->d_gcs, e->d_gperm, e->d_keys, e->d_cnext, e->d_entry, e->d_ea, e->d_eobs, e->d_eM, e->d_eoff, e->d_enext, e->d_etab, e->d_escan, e->d_unif, e->d_u, e->d_us, e->d_item_u, e->d_recs, e->d_ys, e->d_cs, e->d_perm, e->d_y, e->d_cens, e->d_items /* arena: found, pend0, pend1, done live inside */, e->d_idx_exact, e->d_idx_cens,
                     e->d_glist, e->d_model, e->d_stats, e->d_state, e->d_T, e->d_C, e->d_nu, e->d_zeta, e->d_var_ptr, e->d_cell_i, e->d_cell_j, e->d_pires, e->d_res };
     for (void *b : big) pht_dev_free(b, e->stream);
@@ -685,6 +727,8 @@ extern "C" int pht_engine_set_pi(pht_engine *e, const double *pi, const double *
         double sum = 0.0;
         for (int i = 0; i < n; i++) { if (!(pi[i] >= 0.0)) return fail("pi[%d] = %g is not a probability", i, pi[i]); sum += pi[i]; }
         if (!(sum > 0.999999 && sum < 1.000001)) return fail("pi sums to %g, not 1", sum);
+        if (e->visits_set && engine_visits_reachable(e, e->h_voff.data(), e->h_vt.data(), e->h_vm.data(), pi, 0, nullptr, nullptr, nullptr))
+            return -1;                             /* (pht_engine_set_visits: a visit sequence this pi cannot start) */
         for (int c = 0; c < e->chains * e->groups; c++)       /* every chain, in every group's block */
             CU(cudaMemcpy(e->d_model + (size_t)c * e->L.total + e->L.pi, pi, sizeof(double) * n, cudaMemcpyHostToDevice));
     }
@@ -881,6 +925,8 @@ extern "C" int pht_engine_set_groups(pht_engine *e, int G, const int *T, const d
     }
     CU(cudaSetDevice(e->cfg.device));
     CU(cudaStreamSynchronize(e->stream));
+    if (e->visits_set && engine_visits_reachable(e, e->h_voff.data(), e->h_vt.data(), e->h_vm.data(), nullptr, G, T, C,
+                                                 G > 1 ? gid.data() : nullptr)) return -1;
     if (G > 1 && !e->chain_blocks) {
         e->chain_blocks = pht_unif_grid_blocks(e->cfg.device, n, true);
         if (e->chain_blocks <= 0) { e->chain_blocks = 0; return fail("the several-unit path kernel does not fit on the device: %s", cudaGetErrorString(cudaGetLastError())); }
@@ -970,6 +1016,7 @@ extern "C" int pht_engine_set_groups(pht_engine *e, int G, const int *T, const d
     e->groups = G;
     if (G > 1) e->h_group.assign(gid.begin(), gid.begin() + l); else e->h_group.clear();
     if (e->graph_exec) { cudaGraphExecDestroy(e->graph_exec); e->graph_exec = nullptr; }     /* kernel parameters change */
+    if (e->visits_set) return visits_build(e);     /* the panel layouts follow the grouped layout */
     return e->counts_set ? counts_build(e) : 0;      /* the counted records follow the grouped layout */
 }
 
@@ -1068,6 +1115,8 @@ extern "C" int pht_engine_set_counts(pht_engine *e, const uint32_t *counts_local
         if (e->graph_exec) { cudaGraphExecDestroy(e->graph_exec); e->graph_exec = nullptr; }
         return counts_free(e);
     }
+    if (e->visits_set)
+        return fail("counts are not supported with visits (panel observations): the units of a record would share their visits; clear the visits with pht_engine_set_visits(e, NULL, NULL, NULL) first");
     if (e->entry_set)
         return fail("counts are not supported with entry ages (delayed entry): a record's ghost count would be a sum of w Geometric draws; clear the ages with pht_engine_set_entry(e, NULL) first");
     const long l = e->l_local;
@@ -1106,6 +1155,311 @@ extern "C" int pht_engine_set_counts(pht_engine *e, const uint32_t *counts_local
     return 0;
 }
 
+/* ---------------------------------------------------------------- panel observations (method 64) */
+static void panel_free(PanelBufs &b, cudaStream_t st) {
+    void *bufs[] = { b.py, b.pu, b.pc, b.pperm, b.pgofs, b.vy, b.vu, b.vt, b.beta, b.vc, b.vperm, b.vm, b.vgofs, b.vcoff, b.voff, b.vnext };
+    for (void *q : bufs) pht_dev_free(q, st);
+    b = PanelBufs();
+    cudaStreamSynchronize(st);
+}
+
+/* Both layouts from the visits in e->h_voff / h_vt / h_vm, in the engine's layout order (by group, then by decreasing y):
+ * y, flags, u, local index and group offsets of each; the panel observations' chunk offsets and visits; the beta scratch
+ * ((most visits + 1) n doubles per resident lane of the panel kernel).  A failed allocation leaves e->pan as it was. */
+static int visits_build(pht_engine *e) {
+    const long l = e->l_local;
+    const int G = e->groups, n = e->cfg.n;
+    const size_t ln = (size_t)(l > 0 ? l : 1);
+    std::vector<double> y(ln), u; std::vector<uint8_t> c(ln); std::vector<uint32_t> order(ln);
+    const uint32_t *dperm = G > 1 ? e->d_gperm : e->d_perm;
+    if (l > 0) {
+        CU(cudaMemcpy(y.data(), e->d_y, sizeof(double) * (size_t)l, cudaMemcpyDeviceToHost));
+        CU(cudaMemcpy(c.data(), e->d_cens, (size_t)l, cudaMemcpyDeviceToHost));
+        if (e->d_u) { u.resize(ln); CU(cudaMemcpy(u.data(), e->d_u, sizeof(double) * (size_t)l, cudaMemcpyDeviceToHost)); }
+        if (dperm) CU(cudaMemcpy(order.data(), dperm, sizeof(uint32_t) * (size_t)l, cudaMemcpyDeviceToHost));
+        else for (long i = 0; i < l; i++) order[(size_t)i] = (uint32_t)i;
+    }
+    std::vector<double> py, pu, vy, vu, vt; std::vector<uint8_t> pc, vc; std::vector<uint32_t> pperm, vperm, vm;
+    std::vector<unsigned long long> pgofs((size_t)G + 1, 0ull), vgofs((size_t)G + 1, 0ull), vcoff((size_t)G + 1, 0ull), voff(1, 0ull);
+    long mmax = 0;
+    for (long pos = 0; pos < l; pos++) {
+        const uint32_t k = order[(size_t)pos], g = G > 1 ? e->h_group[k] : 0u;
+        const long m = (long)(e->h_voff[k + 1] - e->h_voff[k]);
+        if (m == 0) {
+            py.push_back(y[k]); pc.push_back(c[k]); pperm.push_back(k);
+            if (!u.empty()) pu.push_back(u[k]);
+            pgofs[(size_t)g + 1]++;
+            continue;
+        }
+        vy.push_back(y[k]); vc.push_back(c[k]); vperm.push_back(k);
+        if (!u.empty()) vu.push_back(u[k]);
+        vgofs[(size_t)g + 1]++;
+        for (int64_t q = e->h_voff[k]; q < e->h_voff[k + 1]; q++) { vt.push_back(e->h_vt[(size_t)q]); vm.push_back(e->h_vm[(size_t)q]); }
+        voff.push_back(vt.size());
+        if (m > mmax) mmax = m;
+    }
+    for (int g = 0; g < G; g++) {
+        vcoff[(size_t)g + 1] = vcoff[(size_t)g] + (vgofs[(size_t)g + 1] + 31) / 32;
+        pgofs[(size_t)g + 1] += pgofs[(size_t)g]; vgofs[(size_t)g + 1] += vgofs[(size_t)g];
+    }
+    PanelBufs b;
+    cudaError_t ce = cudaSuccess;
+    auto up = [&](void **dst, const void *src, size_t bytes) {
+        if (ce == cudaSuccess) ce = pht_dev_alloc(dst, bytes ? bytes : 1, e->stream);
+        if (ce == cudaSuccess && bytes && src) ce = cudaMemcpyAsync(*dst, src, bytes, cudaMemcpyHostToDevice, e->stream);
+    };
+    up((void **)&b.py, py.data(), sizeof(double) * py.size()); up((void **)&b.pc, pc.data(), pc.size());
+    up((void **)&b.pperm, pperm.data(), sizeof(uint32_t) * pperm.size()); up((void **)&b.pgofs, pgofs.data(), sizeof(unsigned long long) * pgofs.size());
+    up((void **)&b.vy, vy.data(), sizeof(double) * vy.size()); up((void **)&b.vc, vc.data(), vc.size());
+    up((void **)&b.vperm, vperm.data(), sizeof(uint32_t) * vperm.size()); up((void **)&b.vgofs, vgofs.data(), sizeof(unsigned long long) * vgofs.size());
+    up((void **)&b.vcoff, vcoff.data(), sizeof(unsigned long long) * vcoff.size()); up((void **)&b.voff, voff.data(), sizeof(unsigned long long) * voff.size());
+    up((void **)&b.vt, vt.data(), sizeof(double) * vt.size()); up((void **)&b.vm, vm.data(), sizeof(uint32_t) * vm.size());
+    if (!u.empty()) { up((void **)&b.pu, pu.data(), sizeof(double) * pu.size()); up((void **)&b.vu, vu.data(), sizeof(double) * vu.size()); }
+    up((void **)&b.vnext, nullptr, sizeof(unsigned long long));
+    const size_t beta_bytes = sizeof(double) * (size_t)e->panel_blocks * PHT_UNIF_PANEL_THREADS * (size_t)(mmax + 1) * (size_t)n;
+    up((void **)&b.beta, nullptr, beta_bytes);
+    if (ce == cudaSuccess) ce = cudaStreamSynchronize(e->stream);
+    if (ce != cudaSuccess) {
+        cudaGetLastError(); panel_free(b, e->stream); cudaGetLastError();
+        return fail("cannot allocate device memory for the panel observations (%.1f MB of beta scratch for %ld visits per observation at most): %s",
+                    beta_bytes / 1e6, mmax, cudaGetErrorString(ce));
+    }
+    panel_free(e->pan, e->stream);
+    b.n_plain = (long)py.size(); b.n_panel = (long)vy.size();
+    e->pan = b;
+    if (e->graph_exec) { cudaGraphExecDestroy(e->graph_exec); e->graph_exec = nullptr; }     /* kernel parameters change */
+    return 0;
+}
+
+/* for every phase, the phases reachable from it through the nonzero cells of the structure (itself included); bit n: an exit */
+static void reach_sets(int n, const int *T, const double *C, std::vector<uint64_t> &reach) {
+    const int n1 = n + 1;
+    reach.assign((size_t)n, 0ull);
+    for (int i = 0; i < n; i++) {
+        reach[(size_t)i] = 1ull << i;
+        for (int j = 0; j <= n; j++) if (j != i && T[i + j * n1] != 0 && C[i + j * n1] != 0.0) reach[(size_t)i] |= 1ull << j;
+    }
+    for (bool grew = true; grew;) {
+        grew = false;
+        for (int i = 0; i < n; i++) {
+            uint64_t r = reach[(size_t)i];
+            for (int j = 0; j < n; j++) if ((r >> j) & 1ull) r |= reach[(size_t)j];
+            if (r != reach[(size_t)i]) { reach[(size_t)i] = r; grew = true; }
+        }
+    }
+}
+
+/* Whether every observation's visits can happen: the phases it can be in at each visit, starting from the support of pi
+ * (the start state itself when t_1 = 0) and moving along the nonzero cells of its group's structure (T, C: G structures of
+ * (n+1)^2, gid: the group of every observation, or nullptr for one group), and for exact and interval data an exit after
+ * the last visit (from the phase at y itself when an exact observation's last visit is at y).  0, or fail() naming the
+ * first observation that cannot be drawn (its first draw would find only zero weights: error word 512). */
+static int visits_reachable(int n, int G, const int *T, const double *C, const uint8_t *gid, const double *pi, long l,
+                            const double *y, const uint8_t *c, const double *u, const int64_t *off, const double *t,
+                            const uint32_t *mask) {
+    const int n1 = n + 1;
+    std::vector<std::vector<uint64_t>> reach((size_t)G);
+    for (int g = 0; g < G; g++) reach_sets(n, T + (size_t)g * n1 * n1, C + (size_t)g * n1 * n1, reach[(size_t)g]);
+    uint64_t start = 0;
+    for (int i = 0; i < n; i++) if (pi[i] > 0.0) start |= 1ull << i;
+    for (long k = 0; k < l; k++) {
+        const int64_t v0 = off[k], m = off[k + 1] - v0;
+        if (m == 0) continue;
+        const size_t g = gid ? (size_t)gid[k] : 0;
+        const std::vector<uint64_t> &R = reach[g];
+        auto step = [&](uint64_t from) { uint64_t r = 0; for (int i = 0; i < n; i++) if ((from >> i) & 1ull) r |= R[(size_t)i]; return r; };
+        uint64_t cur = (t[v0] == 0.0 ? start : step(start)) & mask[v0];
+        for (int64_t q = v0 + 1; q < v0 + m && cur; q++) cur = step(cur) & mask[q];
+        if (!cur) return fail("observation %ld: the start distribution and the structure cannot produce its visit sequence (no path from pi's support through the masks' phases)", k);
+        const bool iv = u && u[k] < INFINITY;
+        if (!c[k] || iv) {
+            const size_t g0 = g * n1 * n1;
+            const bool direct = !c[k] && t[v0 + m - 1] == y[k];
+            bool ok = false;
+            for (int i = 0; i < n; i++) {
+                if (!((cur >> i) & 1ull)) continue;
+                if (direct) ok = ok || (T[g0 + i + n * n1] != 0 && C[g0 + i + n * n1] != 0.0);
+                else ok = ok || ((R[(size_t)i] >> n) & 1ull);
+            }
+            if (!ok) return fail("observation %ld: the structure cannot absorb after its last visit (no exit from the phases its visits allow)", k);
+        }
+    }
+    return 0;
+}
+
+/* visits_reachable for the engine's visits (or the given ones) and data, against its structures and the given pi (nullptr:
+ * chain 0's current pi), T / C / gid (nullptr: the engine's own) */
+static int engine_visits_reachable(pht_engine *e, const int64_t *off, const double *t, const uint32_t *mask, const double *pi,
+                                   int G, const int *T, const double *C, const uint8_t *gid) {
+    const long l = e->l_local;
+    const int n = e->cfg.n, n1 = n + 1;
+    const size_t ln = (size_t)(l > 0 ? l : 1);
+    std::vector<double> y(ln), u, p((size_t)n); std::vector<uint8_t> c(ln);
+    std::vector<int> Th; std::vector<double> Ch;
+    if (l > 0) {
+        CU(cudaMemcpy(y.data(), e->d_y, sizeof(double) * (size_t)l, cudaMemcpyDeviceToHost));
+        CU(cudaMemcpy(c.data(), e->d_cens, (size_t)l, cudaMemcpyDeviceToHost));
+        if (e->d_u) { u.resize(ln); CU(cudaMemcpy(u.data(), e->d_u, sizeof(double) * (size_t)l, cudaMemcpyDeviceToHost)); }
+    }
+    if (pi) p.assign(pi, pi + n);
+    else CU(cudaMemcpy(p.data(), e->d_model + e->L.pi, sizeof(double) * (size_t)n, cudaMemcpyDeviceToHost));
+    if (!T) {
+        G = e->groups;
+        Th.resize((size_t)G * n1 * n1); Ch.resize(Th.size());
+        CU(cudaMemcpy(Th.data(), e->d_T, sizeof(int) * Th.size(), cudaMemcpyDeviceToHost));
+        CU(cudaMemcpy(Ch.data(), e->d_C, sizeof(double) * Ch.size(), cudaMemcpyDeviceToHost));
+        T = Th.data(); C = Ch.data();
+        gid = G > 1 ? e->h_group.data() : nullptr;
+    }
+    return visits_reachable(n, G, T, C, gid, p.data(), l, y.data(), c.data(), u.empty() ? nullptr : u.data(), off, t, mask);
+}
+
+extern "C" int pht_engine_set_visits(pht_engine *e, const int64_t *offsets_local, const double *t, const uint32_t *mask) {
+    if (!e) return fail("null engine");
+    if (method_of(e->cfg) != PHT_METHOD_UNIF)
+        return fail("visits (panel observations) need method 64 (the uniformisation sampler): MHRS, ECS, DCS and the MH variants draw paths given the absorption time alone");
+    if (e->peers_attached) return fail("visits cannot be set after the exchange windows are attached (visits need a single-rank engine)");
+    if (e->cfg.world > 1) return fail("visits need world = 1: the panel observations are laid out and handed out on one rank");
+    CU(cudaSetDevice(e->cfg.device));
+    CU(cudaStreamSynchronize(e->stream));
+    if (!offsets_local) {
+        if (!e->visits_set) return 0;
+        e->visits_set = false; e->h_voff.clear(); e->h_vt.clear(); e->h_vm.clear();
+        panel_free(e->pan, e->stream);
+        if (e->graph_exec) { cudaGraphExecDestroy(e->graph_exec); e->graph_exec = nullptr; }
+        return 0;
+    }
+    if (e->counts_set)
+        return fail("visits are not supported with counts: the units of a record would share their visits; clear the counts with pht_engine_set_counts(e, NULL) first");
+    const long l = e->l_local;
+    const int n = e->cfg.n;
+    if (offsets_local[0] != 0) return fail("offsets[0] = %lld: the visit offsets start at 0", (long long)offsets_local[0]);
+    for (long k = 0; k < l; k++) {
+        const int64_t m = offsets_local[k + 1] - offsets_local[k];
+        if (m < 0) return fail("offsets[%ld] = %lld is below offsets[%ld] = %lld: the visit offsets must not decrease", k + 1, (long long)offsets_local[k + 1], k, (long long)offsets_local[k]);
+        if (m > PHT_MAX_VISITS) return fail("observation %ld has %lld visits, more than PHT_MAX_VISITS = %d", k, (long long)m, PHT_MAX_VISITS);
+    }
+    const size_t ln = (size_t)(l > 0 ? l : 1);
+    std::vector<double> y(ln);
+    if (l > 0) CU(cudaMemcpy(y.data(), e->d_y, sizeof(double) * (size_t)l, cudaMemcpyDeviceToHost));
+    const uint32_t all = n == 32 ? 0xffffffffu : (1u << n) - 1u;
+    bool any = false;
+    for (long k = 0; k < l; k++) {
+        const int64_t v0 = offsets_local[k], m = offsets_local[k + 1] - v0;
+        if (m == 0) continue;
+        any = true;
+        const double yk = y[(size_t)k];
+        if (yk == 0.0 && (m > 1 || t[v0] != 0.0))
+            return fail("observation %ld has y = 0: it takes a single visit at t = 0 (the stage at the start), no other", k);
+        for (int64_t q = v0; q < v0 + m; q++) {
+            if (!(t[q] >= 0.0)) return fail("visit %lld of observation %ld: t = %g is negative or NaN", (long long)(q - v0), k, t[q]);
+            if (t[q] > yk) return fail("visit %lld of observation %ld: t = %g is above y = %g", (long long)(q - v0), k, t[q], yk);
+            if (q > v0 && !(t[q] > t[q - 1])) return fail("visit %lld of observation %ld: t = %g does not follow t = %g (the times must increase)", (long long)(q - v0), k, t[q], t[q - 1]);
+            if (mask[q] == 0u) return fail("visit %lld of observation %ld has an empty mask", (long long)(q - v0), k);
+            if (mask[q] & ~all) return fail("visit %lld of observation %ld: mask 0x%x has bits at or above n = %d", (long long)(q - v0), k, mask[q], n);
+        }
+        if (e->entry_set && t[v0] < e->h_entry[(size_t)k])
+            return fail("observation %ld: its first visit t = %g is before its entry age a = %g", k, t[v0], e->h_entry[(size_t)k]);
+    }
+    if (any && engine_visits_reachable(e, offsets_local, t, mask, nullptr, 0, nullptr, nullptr, nullptr)) return -1;
+    if (!e->panel_blocks) {
+        e->panel_blocks = pht_unif_panel_grid_blocks(e->cfg.device, n);
+        if (e->panel_blocks <= 0) { e->panel_blocks = 0; return fail("the panel path kernel does not fit on the device: %s", cudaGetErrorString(cudaGetLastError())); }
+    }
+    if (!any) {                                    /* no visits at all: the plain engine */
+        if (e->visits_set) { e->visits_set = false; e->h_voff.clear(); e->h_vt.clear(); e->h_vm.clear(); panel_free(e->pan, e->stream); }
+        if (e->graph_exec) { cudaGraphExecDestroy(e->graph_exec); e->graph_exec = nullptr; }
+        return 0;
+    }
+    const int64_t total = offsets_local[l];
+    std::vector<int64_t> ovoff; std::vector<double> ovt; std::vector<uint32_t> ovm;
+    ovoff.swap(e->h_voff); ovt.swap(e->h_vt); ovm.swap(e->h_vm);
+    e->h_voff.assign(offsets_local, offsets_local + l + 1);
+    e->h_vt.assign(t, t + total); e->h_vm.assign(mask, mask + total);
+    if (visits_build(e)) {                          /* a failed allocation: back to the previous visits */
+        e->h_voff.swap(ovoff); e->h_vt.swap(ovt); e->h_vm.swap(ovm);
+        return -1;
+    }
+    e->visits_set = true;
+    return 0;
+}
+
+/* pht_engine_paths with visits: the window's panel observations through k_unif_panel_paths (chain 0, every group on its own
+ * model and table), recorded at their window positions over what the plain kernels recorded there */
+static int panel_window(pht_engine *e, long first, long count, int *B, int *N, double *z) {
+    const int n = e->cfg.n, G = e->groups;
+    std::vector<std::vector<uint32_t>> byg((size_t)G);
+    for (long k = first; k < first + count; k++)
+        if (e->h_voff[(size_t)k + 1] > e->h_voff[(size_t)k]) byg[G > 1 ? e->h_group[(size_t)k] : 0].push_back((uint32_t)k);
+    std::vector<uint32_t> perm; std::vector<unsigned long long> gofs((size_t)G + 1, 0ull), coff((size_t)G + 1, 0ull), voff(1, 0ull);
+    std::vector<double> vt; std::vector<uint32_t> vm;
+    for (int g = 0; g < G; g++) {
+        for (uint32_t k : byg[(size_t)g]) {
+            perm.push_back(k);
+            for (int64_t q = e->h_voff[k]; q < e->h_voff[(size_t)k + 1]; q++) { vt.push_back(e->h_vt[(size_t)q]); vm.push_back(e->h_vm[(size_t)q]); }
+            voff.push_back(vt.size());
+        }
+        gofs[(size_t)g + 1] = perm.size();
+        coff[(size_t)g + 1] = coff[(size_t)g] + (byg[(size_t)g].size() + 31) / 32;
+    }
+    const long cnt = (long)perm.size();
+    if (cnt == 0) return 0;
+    std::vector<double> yw((size_t)count), uw, y((size_t)cnt), u; std::vector<uint8_t> cw((size_t)count), c((size_t)cnt);
+    CU(cudaMemcpy(yw.data(), e->d_y + first, sizeof(double) * count, cudaMemcpyDeviceToHost));
+    CU(cudaMemcpy(cw.data(), e->d_cens + first, (size_t)count, cudaMemcpyDeviceToHost));
+    if (e->d_u) { uw.resize((size_t)count); u.resize((size_t)cnt); CU(cudaMemcpy(uw.data(), e->d_u + first, sizeof(double) * count, cudaMemcpyDeviceToHost)); }
+    for (long j = 0; j < cnt; j++) {
+        const size_t wpos = (size_t)(perm[(size_t)j] - first);
+        y[(size_t)j] = yw[wpos]; c[(size_t)j] = cw[wpos];
+        if (!u.empty()) u[(size_t)j] = uw[wpos];
+    }
+    PanelBufs w;
+    int *dB = nullptr, *dN = nullptr; double *dz = nullptr;
+    int rc = -1;
+#define CUP(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { fail("%s failed: %s (%s:%d)", #call, cudaGetErrorString(e_), __FILE__, __LINE__); goto out; } } while (0)
+    {
+        auto up = [&](void **dst, const void *src, size_t bytes) -> cudaError_t {
+            cudaError_t ce = cudaMalloc(dst, bytes ? bytes : 1);
+            if (ce == cudaSuccess && bytes && src) ce = cudaMemcpy(*dst, src, bytes, cudaMemcpyHostToDevice);
+            return ce;
+        };
+        CUP(up((void **)&w.vy, y.data(), sizeof(double) * cnt)); CUP(up((void **)&w.vc, c.data(), (size_t)cnt));
+        if (!u.empty()) CUP(up((void **)&w.vu, u.data(), sizeof(double) * cnt));
+        CUP(up((void **)&w.vperm, perm.data(), sizeof(uint32_t) * cnt)); CUP(up((void **)&w.vgofs, gofs.data(), sizeof(unsigned long long) * gofs.size()));
+        CUP(up((void **)&w.vcoff, coff.data(), sizeof(unsigned long long) * coff.size())); CUP(up((void **)&w.voff, voff.data(), sizeof(unsigned long long) * voff.size()));
+        CUP(up((void **)&w.vt, vt.data(), sizeof(double) * vt.size())); CUP(up((void **)&w.vm, vm.data(), sizeof(uint32_t) * vm.size()));
+        CUP(up((void **)&w.vnext, nullptr, sizeof(unsigned long long)));
+        w.beta = e->pan.beta;                       /* sized for the longest panel of the engine */
+        CUP(cudaMalloc(&dB, sizeof(int) * count)); CUP(cudaMalloc(&dN, sizeof(int) * count * n * n)); CUP(cudaMalloc(&dz, sizeof(double) * count * n));
+        CUP(cudaMemset(dN, 0, sizeof(int) * count * n * n));
+        UpdateParams up_ = update_params(e, nullptr, 0);
+        up_.chains = 1;
+        if (enqueue_model(e, up_)) goto out;
+        SweepParams p = sweep_params(e);
+        p.chains = 1;
+        p.outB = dB; p.outN = dN; p.outz = dz; p.first = first; p.count = count;
+        CUP(pht_launch_unif_panel(p, e->d_unif, panel_args(w), e->panel_blocks, e->stream));
+        e->launches++;
+        if (pht_engine_sync(e)) goto out;
+        std::vector<int> hB((size_t)count), hN((size_t)count * n * n); std::vector<double> hz((size_t)count * n);
+        CUP(cudaMemcpy(hB.data(), dB, sizeof(int) * count, cudaMemcpyDeviceToHost));
+        CUP(cudaMemcpy(hN.data(), dN, sizeof(int) * count * n * n, cudaMemcpyDeviceToHost));
+        CUP(cudaMemcpy(hz.data(), dz, sizeof(double) * count * n, cudaMemcpyDeviceToHost));
+        for (uint32_t k : perm) {
+            const size_t wpos = (size_t)(k - first);
+            B[wpos] = hB[wpos];
+            memcpy(N + wpos * n * n, hN.data() + wpos * n * n, sizeof(int) * n * n);
+            memcpy(z + wpos * n, hz.data() + wpos * n, sizeof(double) * n);
+        }
+        rc = 0;
+    }
+#undef CUP
+out:
+    void *bufs[] = { w.vy, w.vc, w.vu, w.vperm, w.vgofs, w.vcoff, w.voff, w.vt, w.vm, w.vnext, dB, dN, dz };
+    for (void *q : bufs) if (q) cudaFree(q);
+    return rc;
+}
+
 extern "C" int pht_engine_set_upper(pht_engine *e, const double *upper_local) {
     if (!e) return fail("null engine");
     CU(cudaSetDevice(e->cfg.device));
@@ -1124,6 +1478,7 @@ extern "C" int pht_engine_set_upper(pht_engine *e, const double *upper_local) {
             for (long i = 0; i < e->l_local; i++) if (y[(size_t)i] > e->unif_tmax) e->unif_tmax = y[(size_t)i];
         }
         if (group_refresh(e)) return -1;
+        if (e->visits_set) return visits_build(e);
         return e->counts_set ? counts_build(e) : 0;
     }
     const bool unif = method_of(e->cfg) == PHT_METHOD_UNIF;
@@ -1171,6 +1526,7 @@ extern "C" int pht_engine_set_upper(pht_engine *e, const double *upper_local) {
     }
     CU(cudaStreamSynchronize(e->stream));
     if (group_refresh(e)) return -1;
+    if (e->visits_set) return visits_build(e);     /* u in the panel layouts */
     return e->counts_set ? counts_build(e) : 0;
 }
 
@@ -1214,6 +1570,8 @@ extern "C" int pht_engine_set_entry(pht_engine *e, const double *entry_local) {
         if (!std::isfinite(a)) return fail("entry[%ld] = %g: an entry age must be finite", i, a);
         if (a < 0.0) return fail("entry[%ld] = %g is negative", i, a);
         if (a > yi) return fail("entry[%ld] = %g is above y = %g: a unit enters before its failure or censoring time (a left-censored record, y = 0, takes no entry age)", i, a, yi);
+        if (e->visits_set && e->h_voff[(size_t)i + 1] > e->h_voff[(size_t)i] && e->h_vt[(size_t)e->h_voff[(size_t)i]] < a)
+            return fail("entry[%ld] = %g is after the observation's first visit t = %g", i, a, e->h_vt[(size_t)e->h_voff[(size_t)i]]);
         sum += (ui < INFINITY && ui > yi ? ui : yi) + a;
         if (a > 0.0) trunc.push_back((uint32_t)i);
     }
@@ -1541,7 +1899,10 @@ extern "C" int pht_engine_paths(pht_engine *e, long first, long count, int *B, i
     if (e->counts_set) return fail("per-observation paths are not recorded while counts are set: compare with an engine on the expanded data instead");
     if (count == 0) return 0;
     CU(cudaSetDevice(e->cfg.device));
-    if (e->groups > 1) return group_paths(e, first, count, B, N, z);
+    if (e->groups > 1) {
+        if (group_paths(e, first, count, B, N, z)) return -1;
+        return e->visits_set ? panel_window(e, first, count, B, N, z) : 0;
+    }
     const int n = e->cfg.n;
     int *dB = nullptr, *dN = nullptr; double *dz = nullptr;
     uint32_t *t_exact = nullptr, *t_cens = nullptr;
@@ -1585,6 +1946,7 @@ out:
     cudaFree(dB); cudaFree(dN); cudaFree(dz);
     if (t_exact) cudaFree(t_exact);
     if (t_cens) cudaFree(t_cens);
+    if (rc == 0 && e->visits_set) rc = panel_window(e, first, count, B, N, z);
     return rc;
 }
 

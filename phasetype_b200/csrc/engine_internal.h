@@ -245,6 +245,21 @@ struct UnifRecords {
 };
 cudaError_t pht_launch_unif_records(const SweepParams &p, const double *tab, const UnifRecords &R, int grid_blocks, cudaStream_t st);
 int pht_unif_records_grid_blocks(int device, int n);
+/* method 64, panel observations (k_unif.cu; pht_engine_set_visits): the observations with visits in their own layout (by
+ * group, then by decreasing y) and their visits.  Kernel arguments of their own, like the table. */
+struct UnifPanel {
+    const double *y, *u; const uint8_t *cens;    /* per panel observation; u nullptr: no bounds */
+    const uint32_t *perm;                        /* local observation index */
+    const unsigned long long *gofs, *coff;       /* G + 1 each: group g's panel observations [gofs[g], gofs[g + 1]), its chunks
+                                                    of 32 [coff[g], coff[g + 1]) */
+    const unsigned long long *voff;              /* visits of panel observation j: [voff[j], voff[j + 1]) of vt, vm */
+    const double *vt; const uint32_t *vm;
+    double *beta;                                /* backward-pass scratch: (most visits + 1) n doubles per resident lane */
+    unsigned long long *next;                    /* hand-out counter, zeroed by the launcher */
+};
+#define PHT_UNIF_PANEL_THREADS 128           /* threads per block of the panel kernel (its beta scratch is per lane) */
+cudaError_t pht_launch_unif_panel(const SweepParams &p, const double *tab, const UnifPanel &V, int grid_blocks, cudaStream_t st);
+int pht_unif_panel_grid_blocks(int device, int n);
 /* large per-call buffers: stream-ordered pool allocations, cached across calls (engine.cu) */
 cudaError_t pht_dev_alloc(void **p, size_t bytes, cudaStream_t st);
 cudaError_t pht_dev_free(void *p, cudaStream_t st);

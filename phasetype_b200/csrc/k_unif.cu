@@ -446,6 +446,104 @@ cudaError_t pht_launch_unif_records(const SweepParams &p, const double *tab, con
     return cudaGetLastError();
 }
 
+/* ---- panel observations (pht_engine_set_visits; pht_unif.h, "Panel observations"): launched only when some observation
+ * has visits, over those observations alone (the others run through k_unif_paths / k_unif_chain_paths in a layout of their
+ * own).  Work items are (chain, chunk of at most 32 panel observations of one group), chunk r of chain c at flat index
+ * c chunks + r, so every item belongs to one unit c groups + g.  A persistent warp takes one item at a time; its lanes draw
+ * one observation each (model and table of the unit from global memory) into the warp's own accumulators, which are
+ * flushed into the unit's statistics block after every item.  The lanes' n-vectors of path scratch live in shared-memory
+ * slabs as in k_unif_paths; the beta history, (visits + 1) n doubles per observation, in global scratch, one slot per
+ * resident lane (stride: the grid's lanes, so a warp's lanes touch adjacent words). */
+struct UnifPanelAcc {
+    unsigned long long *zlo; long long *zhi; unsigned int *Nacc, *Bacc;
+    __host__ __device__ static size_t bytes(int n) { return sizeof(double) * (size_t)(2 * n) + sizeof(unsigned int) * (size_t)(n * n + n); }
+    __device__ __forceinline__ void carve(unsigned char *raw, int n) {
+        zlo = reinterpret_cast<unsigned long long *>(raw); zhi = reinterpret_cast<long long *>(zlo + n);
+        Nacc = reinterpret_cast<unsigned int *>(zhi + n); Bacc = Nacc + n * n;
+    }
+};
+template <int THREADS>
+static size_t unif_panel_smem(int n) {     /* per-lane path scratch (stride THREADS) + one accumulator set per warp, 16-byte aligned */
+    return sizeof(double) * (size_t)(2 * n * THREADS) + (size_t)(THREADS / 32) * ((UnifPanelAcc::bytes(n) + 15) & ~(size_t)15);
+}
+
+template <int THREADS>
+__global__ void __launch_bounds__(THREADS) k_unif_panel_paths(SweepParams p, const double *tab, UnifPanel V) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const int n = p.n, tid = threadIdx.x, lane = tid & 31, cap = PHT_UNIF_CAP, G = p.groups;
+    const unsigned FULL = 0xffffffffu;
+    const ModelLayout ML = ModelLayout::make(n, p.m);
+    const size_t tabd = (size_t)pht_unif_layout_make(n, cap).total;
+    double *Za = reinterpret_cast<double *>(smem_raw), *Zb = Za + n * THREADS;
+    UnifPanelAcc w;
+    w.carve(smem_raw + sizeof(double) * (size_t)(2 * n * THREADS) + (size_t)(tid >> 5) * ((UnifPanelAcc::bytes(n) + 15) & ~(size_t)15), n);
+    for (int i = lane; i < n * n; i += 32) w.Nacc[i] = 0u;
+    for (int i = lane; i < n; i += 32) { w.Bacc[i] = 0u; w.zlo[i] = 0ull; w.zhi[i] = 0; }
+    __syncwarp();
+    const uint32_t iter = p.state->iter;
+    const long bs = (long)gridDim.x * THREADS;
+    double *beta = V.beta + (size_t)blockIdx.x * THREADS + tid;
+    const unsigned long long chunks = V.coff[G], work = (unsigned long long)p.chains * chunks;
+    unsigned long long c_paths = 0; int err = 0;
+    UnifCount ctx; ctx.p = &p; ctx.Nacc = w.Nacc; ctx.n = n; ctx.out_idx = 0;
+    for (;;) {
+        unsigned long long f = 0;
+        if (lane == 0) f = atomicAdd(V.next, 1ull);
+        f = __shfl_sync(FULL, f, 0);
+        if (f >= work) break;
+        const unsigned c = (unsigned)(f / chunks);
+        const unsigned long long r = f - (unsigned long long)c * chunks;
+        int g = 0;
+        while (V.coff[g + 1] <= r) g++;
+        const unsigned long long j0 = V.gofs[g] + (r - V.coff[g]) * 32ull, j = j0 + (unsigned long long)lane;
+        const int unit = (int)c * G + g;
+        const double *utab = tab + (size_t)unit * tabd, *model = p.model + (size_t)unit * ML.total;
+        if (j < V.gofs[g + 1]) {
+            const uint32_t ol = V.perm[j];
+            pht_stream st; st.k0 = p.ckeys[2 * c]; st.k1 = p.ckeys[2 * c + 1];
+            pht_stream_seek(&st, iter, p.obs_rank + ol * p.obs_world, 0u, 0u);
+            ctx.out_idx = (long)ol - p.first;
+            const unsigned long long v0 = V.voff[j];
+            int B = 0;
+            err |= pht_unif_panel_path(utab, n, cap, model + ML.s, model + ML.scale, model + ML.cum, model + ML.pi, V.y[j], V.cens[j],
+                                       V.u ? V.u[j] : INFINITY, (int)(V.voff[j + 1] - v0), V.vt + v0, V.vm + v0, beta, bs, &st,
+                                       Za + tid, Zb + tid, THREADS, &ctx, &B);
+            path_flush<THREADS>(p, n, Za, w.zlo, w.zhi, w.Bacc, B, ctx.out_idx);
+            c_paths++;
+        }
+        __syncwarp();
+        if (p.outB == nullptr) {
+            unsigned long long *gs = reinterpret_cast<unsigned long long *>(p.stats + (size_t)unit * stats_len(n));
+            for (int i = lane; i < n * n; i += 32) if (w.Nacc[i]) { atomicAdd(&gs[i], (unsigned long long)w.Nacc[i]); w.Nacc[i] = 0u; }
+            for (int i = lane; i < n; i += 32) {
+                if (w.Bacc[i]) { atomicAdd(&gs[n * n + i], (unsigned long long)w.Bacc[i]); w.Bacc[i] = 0u; }
+                if (w.zlo[i]) { atomicAdd(&gs[n * n + n + i], w.zlo[i]); w.zlo[i] = 0ull; }
+                if (w.zhi[i]) { atomicAdd(&gs[n * n + 2 * n + i], (unsigned long long)w.zhi[i]); w.zhi[i] = 0; }
+            }
+        }
+        __syncwarp();
+    }
+    if (err) atomicOr(&p.state->error, err);
+    for (int o = 16; o > 0; o >>= 1) c_paths += __shfl_down_sync(FULL, c_paths, o);
+    if (lane == 0) atomicAdd(&p.state->counters[PHT_CNT_PATHS], c_paths);
+}
+
+int pht_unif_panel_grid_blocks(int device, int n) {
+    const size_t smem = unif_panel_smem<PHT_UNIF_PANEL_THREADS>(n);
+    int per_sm = 0, sms = 0;
+    if (cudaFuncSetAttribute(k_unif_panel_paths<PHT_UNIF_PANEL_THREADS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return -1;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_unif_panel_paths<PHT_UNIF_PANEL_THREADS>, PHT_UNIF_PANEL_THREADS, smem) != cudaSuccess) return -1;
+    if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device) != cudaSuccess) return -1;
+    return per_sm * sms;
+}
+
+cudaError_t pht_launch_unif_panel(const SweepParams &p, const double *tab, const UnifPanel &V, int grid_blocks, cudaStream_t st) {
+    const cudaError_t e = cudaMemsetAsync(V.next, 0, sizeof(unsigned long long), st);
+    if (e != cudaSuccess) return e;
+    k_unif_panel_paths<PHT_UNIF_PANEL_THREADS><<<grid_blocks, PHT_UNIF_PANEL_THREADS, unif_panel_smem<PHT_UNIF_PANEL_THREADS>(p.n), st>>>(p, tab, V);
+    return cudaGetLastError();
+}
+
 size_t pht_unif_entry_scan_bytes(long count) {
     size_t bytes = 0;
     cub::DeviceScan::ExclusiveScan(nullptr, bytes, (const unsigned *)nullptr, (unsigned long long *)nullptr, cuda::std::plus<>(),

@@ -237,6 +237,74 @@ PHT_HD double pht_unif_rec_m_entry(const pht_unif_rec *rc, const double *tab, in
     return pi[c] * a;
 }
 
+/* Panel observations (pht_engine_set_visits).  Observation i carries visits (t_j, A_j), j = 1..m, 0 <= t_1 < ... < t_m <= y,
+ * A_j a non-empty set of phases (bit c of a uint32 mask: phase c).  The path law is that of the absorbing chain given pi,
+ * the visits and the terminal information: a hidden Markov chain over the visit states, each gap a bridge with fixed ends.
+ * Backward pass (no draws), with t_0 = 0 and d_{m+1} = y - t_m:
+ *     v = s (exact), 1 (right-censored) or sum_{k>=1} Pois(k; lambda (u - y)) g_k (interval, as in pht_unif_path step 1),
+ *     beta_m = 1[A_m] . e^{S d_{m+1}} v,   beta_{j-1} = 1[A_{j-1}] . e^{S (t_j - t_{j-1})} beta_j,   beta_0 = e^{S t_1} beta_1
+ * (no mask on beta_0; t_1 = 0 makes it beta_1 itself), every e^{Sd} w as sum_{k <= K(lambda d)} Pois(k; lambda d) R^k w with
+ * the zero-weight skip of pht_unif_path, k ascending, then the entries of R^k w in column order.  Each beta is scaled by the
+ * power of two that brings its largest entry into [1, 2): exact, and no draw depends on it, so a long panel cannot
+ * underflow.  The draws, all on Philox sub-stream 0 of (sweep, global observation), in this order:
+ *   1. a, the start state, from pi_a beta_0(a) -- only when pi has more than one positive entry (else the first of them);
+ *   2. for j = 1..m the visit state x_j from (e^{S(t_j - t_{j-1})})_{x_{j-1} x} beta_j(x) (x_0 = a); a gap of length 0
+ *      (t_1 = 0) gives x_1 = a and a one-phase mask its phase, neither with a draw;
+ *   3. b, the state at y, from (e^{S d_{m+1}})_{x_m b} v_b (pht_unif_path step 1 with row x_m of R^k in place of q_k);
+ *      none when t_m = y (b = x_m);
+ *   4. the bridges x_0 -> x_1, ..., x_{m-1} -> x_m, x_m -> b in time order, each with the event-count / spacing /
+ *      next-state draws of pht_unif_path steps 3-4 and its spacings scaled to its own length; a gap of length 0 draws
+ *      nothing;
+ *   5. step 5 of pht_unif_path from b.
+ * B is the start state a.  Sub-streams 1 and 2 + j stay the ghosts' (delayed entry).  Every gap is at most y, so the
+ * sweep's table covers it.  Scratch: (m + 1) n doubles of beta per observation (entry c of beta_j at (j n + c) bs). */
+
+/* out = e^{S d} w (x = lambda d, lx = log x, K = K(x)); w and out may not overlap */
+PHT_HD void pht_unif_expv(const double *tab, int n, int cap, double x, double lx, int K, const double *w, long ws, double *out, long os) {
+    const pht_unif_layout L = pht_unif_layout_make(n, cap);
+    const double *lgk = tab + L.lgk;
+    for (int c = 0; c < n; c++) out[c * os] = 0.0;
+    for (int k = 0; k <= K; k++) {
+        const double p = pht_unif_w(x, lx, k, lgk);
+        if (p == 0.0) continue;
+        const double *P = tab + L.P + k * n * n;
+        for (int c = 0; c < n; c++) {
+            double acc = 0.0;
+            for (int e = 0; e < n; e++) acc += P[c + e * n] * w[e * ws];
+            out[c * os] += p * acc;
+        }
+    }
+}
+
+/* row a of e^{S d} (x = lambda d): out_c = sum_k Pois(k; x) (R^k)_ac, k ascending with the zero-weight skip */
+PHT_HD void pht_unif_exprow(const double *tab, int n, int cap, double x, double lx, int K, int a, double *out, int os) {
+    const pht_unif_layout L = pht_unif_layout_make(n, cap);
+    const double *lgk = tab + L.lgk;
+    for (int c = 0; c < n; c++) out[c * os] = 0.0;
+    for (int k = 0; k <= K; k++) {
+        const double p = pht_unif_w(x, lx, k, lgk);
+        if (p == 0.0) continue;
+        const double *P = tab + L.P + k * n * n + a;
+        for (int c = 0; c < n; c++) out[c * os] += p * P[c * n];
+    }
+}
+
+/* scale w (mask bits clear: zero) by the power of two that brings its largest entry into [1, 2); 0 or PHT_UNIF_ERR_ZERO */
+PHT_HD int pht_unif_rescale(double *w, long ws, int n, uint32_t mask) {
+    double mx = 0.0;
+    for (int c = 0; c < n; c++) {
+        if (!((mask >> c) & 1u)) w[c * ws] = 0.0;
+        else if (w[c * ws] > mx) mx = w[c * ws];
+    }
+    if (!(mx > 0.0)) return PHT_UNIF_ERR_ZERO;
+    int ex = (int)((pht_d2u(mx) >> 52) & 0x7ff);
+    if (ex < 1) ex = 1;
+    if (ex > 2045) ex = 2045;
+    const double sc = pht_u2d((uint64_t)(2046 - ex) << 52);      /* 2^(1023 - ex) */
+    for (int c = 0; c < n; c++) w[c * ws] = w[c * ws] * sc;
+    return 0;
+}
+
 /* the sampler itself is compiled where the includer says how transitions are counted: PHT_UNIF_CTX (a type) and
  * PHT_UNIF_COUNT(ctx, from, to); PHT_UNIF_U01(st) may replace the uniform draw by an equivalent call, PHT_UNIF_FN the function's qualifiers */
 #if defined(PHT_UNIF_CTX) && defined(PHT_UNIF_COUNT)
@@ -478,6 +546,204 @@ PHT_UNIF_FN int pht_unif_rec_path(const double *tab, int n, int cap, const doubl
         double sofar = 0.0; int kk = -1;
         for (int k = 1; k <= K2; k++) {
             const double v = pht_unif_rec_w2(rc, k, lgk) * tab[L.g + k * n + b];
+            if (v > 0.0) { sofar += v; kk = k; if (sofar >= target) break; }
+        }
+        int cur = b, absorbed = 0; double et = 0.0;
+        for (int i = 1; i <= kk; i++) {
+            const double e = -pht_log(PHT_UNIF_U01(st));
+            et += e;
+            if (absorbed) continue;
+            zb[cur * zs] += e;
+            const double *gn = tab + L.g + (kk - i) * n;
+            double t2 = 0.0;
+            for (int q = 0; q < n; q++) t2 += R[cur + q * n] * gn[q];
+            t2 += r[cur];
+            if (!(t2 > 0.0)) return PHT_UNIF_ERR_ZERO;
+            const double tg = PHT_UNIF_U01(st) * t2;
+            double so = 0.0; int c = -1;
+            for (int q = 0; q < n; q++) {
+                const double v = R[cur + q * n] * gn[q];
+                if (v > 0.0) { so += v; c = q; if (so >= tg) break; }
+            }
+            if (!(so >= tg) && r[cur] > 0.0) c = n;      /* absorption: the last category */
+            if (c == n) { PHT_UNIF_COUNT(ctx, cur, cur); absorbed = 1; }
+            else { if (c != cur) PHT_UNIF_COUNT(ctx, cur, c); cur = c; }
+        }
+        const double e = -pht_log(PHT_UNIF_U01(st));
+        et += e;
+        const double sc = d / et;
+        for (int c = 0; c < n; c++) if (zb[c * zs] != 0.0) za[c * zs] = za[c * zs] + zb[c * zs] * sc;
+    }
+    return 0;
+}
+
+/* A bridge a -> b over a gap of length d > 0 (x = lambda d, K = K(x)): the draws of pht_unif_path steps 3-4.  Its sojourns
+ * (spacings scaled to d) are added to za; zb is scratch that is left zero. */
+PHT_UNIF_FN int pht_unif_bridge(const double *tab, int n, int cap, double d, double x, double lx, int K, int a, int b,
+                                pht_stream *st, double *za, double *zb, int zs, PHT_UNIF_CTX *ctx) {
+    const pht_unif_layout L = pht_unif_layout_make(n, cap);
+    const double *lgk = tab + L.lgk, *R = tab + L.R;
+    double tot = 0.0;
+    for (int k = 0; k <= K; k++) tot += pht_unif_w(x, lx, k, lgk) * tab[L.P + k * n * n + a + b * n];
+    if (!(tot > 0.0)) return PHT_UNIF_ERR_ZERO;
+    const double target = PHT_UNIF_U01(st) * tot;
+    double sofar = 0.0; int kk = -1;
+    for (int k = 0; k <= K; k++) {
+        const double v = pht_unif_w(x, lx, k, lgk) * tab[L.P + k * n * n + a + b * n];
+        if (v > 0.0) { sofar += v; kk = k; if (sofar >= target) break; }
+    }
+    int cur = a; double et = 0.0;
+    for (int i = 1; i <= kk; i++) {
+        const double e = -pht_log(PHT_UNIF_U01(st));
+        zb[cur * zs] += e; et += e;
+        int c = b;
+        if (i < kk) {
+            const double *Pn = tab + L.P + (kk - i) * n * n + b * n;
+            double t2 = 0.0;
+            for (int q = 0; q < n; q++) t2 += R[cur + q * n] * Pn[q];
+            if (!(t2 > 0.0)) return PHT_UNIF_ERR_ZERO;
+            const double tg = PHT_UNIF_U01(st) * t2;
+            double so = 0.0; c = -1;
+            for (int q = 0; q < n; q++) {
+                const double v = R[cur + q * n] * Pn[q];
+                if (v > 0.0) { so += v; c = q; if (so >= tg) break; }
+            }
+        }
+        if (c != cur) PHT_UNIF_COUNT(ctx, cur, c);
+        cur = c;
+    }
+    const double e = -pht_log(PHT_UNIF_U01(st));
+    zb[cur * zs] += e; et += e;
+    const double sc = d / et;
+    for (int c = 0; c < n; c++) if (zb[c * zs] != 0.0) { za[c * zs] = za[c * zs] + zb[c * zs] * sc; zb[c * zs] = 0.0; }
+    return 0;
+}
+
+/* One panel observation (law and draw order above): m >= 1 visits at times vt[0..m-1] with masks vm[0..m-1]; beta:
+ * (m + 1) n doubles of scratch with stride bs.  Other arguments as pht_unif_path. */
+PHT_UNIF_FN int pht_unif_panel_path(const double *tab, int n, int cap, const double *s, const double *scale, const double *cum,
+                                    const double *pi, double y, int cens, double u, int m, const double *vt, const uint32_t *vm,
+                                    double *beta, long bs, pht_stream *st, double *za, double *zb, int zs, PHT_UNIF_CTX *ctx, int *B) {
+    const pht_unif_layout L = pht_unif_layout_make(n, cap);
+    const double lam = tab[0];
+    const int npos = (int)tab[2], a1 = (int)tab[3];
+    const double *lgk = tab + L.lgk, *R = tab + L.R, *r = tab + L.r;
+    const int iv = cens && u <= 1.7976931348623157e308;
+    const double d = iv ? u - y : 0.0, x2 = lam * d, lx2 = x2 > 0.0 ? pht_log(x2) : 0.0;
+    const int K2 = iv ? pht_unif_K(x2) : 0;
+    const double dy = y - vt[m - 1];
+    *B = 0;
+    if (pht_unif_K(lam * y) >= cap || K2 >= cap) return PHT_UNIF_ERR_TABLE;
+#define PHT_BETA(j, c) beta[((long)(j) * n + (c)) * bs]
+
+    /* terminal weights v (into za) and the backward pass */
+    if (iv) {
+        for (int c = 0; c < n; c++) za[c * zs] = 0.0;
+        for (int k = 1; k <= K2; k++) {
+            const double w = pht_unif_w(x2, lx2, k, lgk);
+            if (w == 0.0) continue;
+            const double *g = tab + L.g + k * n;
+            for (int c = 0; c < n; c++) za[c * zs] += w * g[c];
+        }
+    } else for (int c = 0; c < n; c++) za[c * zs] = cens ? 1.0 : s[c];
+    for (int j = m; j >= 0; j--) {
+        const double gap = j == m ? dy : vt[j] - (j > 0 ? vt[j - 1] : 0.0);
+        const double x = lam * gap, lx = x > 0.0 ? pht_log(x) : 0.0;
+        if (j == m) pht_unif_expv(tab, n, cap, x, lx, pht_unif_K(x), za, zs, &PHT_BETA(j, 0), bs);
+        else pht_unif_expv(tab, n, cap, x, lx, pht_unif_K(x), &PHT_BETA(j + 1, 0), bs, &PHT_BETA(j, 0), bs);
+        if (pht_unif_rescale(&PHT_BETA(j, 0), bs, n, j > 0 ? vm[j - 1] : 0xffffffffu)) return PHT_UNIF_ERR_ZERO;
+    }
+
+    /* 1. the start state */
+    int a;
+    if (npos > 1) {
+        for (int c = 0; c < n; c++) za[c * zs] = pi[c] * PHT_BETA(0, c);
+        a = pht_unif_pick(za, n, zs, PHT_UNIF_U01(st));
+        if (a < 0) return PHT_UNIF_ERR_ZERO;
+    } else {
+        a = a1;
+        if (!(PHT_BETA(0, a) > 0.0)) return PHT_UNIF_ERR_ZERO;
+    }
+    *B = a;
+
+    /* 2. the visit states; x_j replaces beta_j(0), which no later draw reads */
+    int prev = a;
+    for (int j = 1; j <= m; j++) {
+        const double gap = vt[j - 1] - (j > 1 ? vt[j - 2] : 0.0);
+        const uint32_t mk = vm[j - 1];
+        int x;
+        if (gap == 0.0) x = prev;
+        else if ((mk & (mk - 1u)) == 0u) { x = 0; while (!((mk >> x) & 1u)) x++; }
+        else {
+            const double xx = lam * gap;
+            pht_unif_exprow(tab, n, cap, xx, xx > 0.0 ? pht_log(xx) : 0.0, pht_unif_K(xx), prev, za, zs);
+            for (int c = 0; c < n; c++) za[c * zs] = za[c * zs] * PHT_BETA(j, c);
+            x = pht_unif_pick(za, n, zs, PHT_UNIF_U01(st));
+            if (x < 0) return PHT_UNIF_ERR_ZERO;
+        }
+        PHT_BETA(j, 0) = (double)x;
+        prev = x;
+    }
+
+    /* 3. the state at y */
+    int b = prev;
+    if (dy > 0.0) {
+        const double xx = lam * dy;
+        pht_unif_exprow(tab, n, cap, xx, xx > 0.0 ? pht_log(xx) : 0.0, pht_unif_K(xx), prev, za, zs);
+        if (iv) {
+            for (int c = 0; c < n; c++) zb[c * zs] = 0.0;
+            for (int k = 1; k <= K2; k++) {
+                const double w = pht_unif_w(x2, lx2, k, lgk);
+                if (w == 0.0) continue;
+                const double *g = tab + L.g + k * n;
+                for (int c = 0; c < n; c++) zb[c * zs] += w * g[c];
+            }
+            for (int c = 0; c < n; c++) za[c * zs] = za[c * zs] * zb[c * zs];
+        } else if (!cens) {
+            for (int c = 0; c < n; c++) za[c * zs] = za[c * zs] * s[c];
+        }
+        b = pht_unif_pick(za, n, zs, PHT_UNIF_U01(st));
+        if (b < 0) return PHT_UNIF_ERR_ZERO;
+    }
+    for (int c = 0; c < n; c++) { za[c * zs] = 0.0; zb[c * zs] = 0.0; }
+
+    /* 4. the bridges in time order */
+    prev = a;
+    for (int j = 1; j <= m + 1; j++) {
+        const double gap = j > m ? dy : vt[j - 1] - (j > 1 ? vt[j - 2] : 0.0);
+        const int x = j > m ? b : (int)PHT_BETA(j, 0);
+        if (gap > 0.0) {
+            const double xx = lam * gap;
+            const int e = pht_unif_bridge(tab, n, cap, gap, xx, xx > 0.0 ? pht_log(xx) : 0.0, pht_unif_K(xx), prev, x, st, za, zb, zs, ctx);
+            if (e) return e;
+        }
+        prev = x;
+    }
+#undef PHT_BETA
+
+    /* 5. after y */
+    if (!cens) {
+        PHT_UNIF_COUNT(ctx, b, b);
+    } else if (!iv) {
+        int j = b;
+        for (;;) {
+            const double t = scale[j] * -pht_log(PHT_UNIF_U01(st));
+            const double target = PHT_UNIF_U01(st);
+            const double *cr = cum + j * (n + 1);
+            int k = 0;
+            while (k < n && cr[k] < target) k++;
+            za[j * zs] += t;
+            if (k < n) { PHT_UNIF_COUNT(ctx, j, k); j = k; }
+            else { PHT_UNIF_COUNT(ctx, j, j); break; }
+        }
+    } else {
+        double tot = 0.0;
+        for (int k = 1; k <= K2; k++) tot += pht_unif_w(x2, lx2, k, lgk) * tab[L.g + k * n + b];
+        if (!(tot > 0.0)) return PHT_UNIF_ERR_ZERO;
+        const double target = PHT_UNIF_U01(st) * tot;
+        double sofar = 0.0; int kk = -1;
+        for (int k = 1; k <= K2; k++) {
+            const double v = pht_unif_w(x2, lx2, k, lgk) * tab[L.g + k * n + b];
             if (v > 0.0) { sofar += v; kk = k; if (sofar >= target) break; }
         }
         int cur = b, absorbed = 0; double et = 0.0;

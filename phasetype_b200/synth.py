@@ -63,6 +63,47 @@ def inspection(R, s, l, spacing, k, rng):
     return y, u, np.ones(l, dtype=np.int32), t
 
 
+def stage_masks(stage_of_phase):
+    """The uint32 phase mask of every stage: stage_of_phase[c] is the observed stage of phase c (stages 0, 1, ...); entry k
+    of the result has bit c set for every phase c of stage k."""
+    st = np.asarray(stage_of_phase, dtype=np.int64)
+    return np.array([sum(1 << int(c) for c in np.flatnonzero(st == k)) for k in range(int(st.max()) + 1)], dtype=np.uint32)
+
+
+def panel(R, s, l, spacing, k, stage_of_phase, rng, censor=None):
+    """Panel data (Engine.set_visits): l units of the CTMC (R, s) started in state 0, inspected at spacing, 2 spacing, ...,
+    up to k times while still working; each inspection records the mask of the stage (stage_masks) of the phase occupied
+    then.  The absorption time is exact; censor(l, rng), when given, draws censoring times: a unit still working then is
+    right-censored there, and only inspections up to it are kept.  Returns (y, censored, offsets, t, mask)."""
+    n = s.shape[0]
+    masks = stage_masks(stage_of_phase)
+    stage = np.asarray(stage_of_phase, dtype=np.int64)
+    rate = R.sum(1) + s
+    cum = np.cumsum(np.concatenate([R, s[:, None]], axis=1) / rate[:, None], axis=1)
+    cum[:, -1] = 1.0
+    end = np.full(l, np.inf) if censor is None else np.asarray(censor(l, rng), dtype=np.float64)
+    ins = spacing * np.arange(1, k + 1)
+    seen = np.full((l, k), -1, dtype=np.int64)           # phase at each inspection (-1: absorbed or after the end)
+    t = np.zeros(l); state = np.zeros(l, dtype=np.int64); alive = np.arange(l)
+    while alive.size:
+        st = state[alive]
+        t1 = t[alive] + rng.exponential(1.0, alive.size) / rate[st]
+        inside = (ins[None, :] >= t[alive][:, None]) & (ins[None, :] < t1[:, None])
+        rows, cols = np.nonzero(inside)
+        seen[alive[rows], cols] = st[rows]
+        t[alive] = t1
+        nxt = (rng.random(alive.size)[:, None] >= cum[st]).sum(1)
+        state[alive] = nxt
+        alive = alive[nxt < n]
+    cens = t > end
+    y = np.where(cens, end, t)
+    keep = (seen >= 0) & (ins[None, :] <= y[:, None])
+    counts = keep.sum(1)
+    offsets = np.concatenate([[0], np.cumsum(counts)]).astype(np.int64)
+    rows, cols = np.nonzero(keep)
+    return y, cens.astype(np.int32), offsets, ins[cols], masks[stage[seen[rows, cols]]]
+
+
 def tabulate(y, cens, u=None):
     """Tied observations as records with counts (Engine.set_counts): the distinct (y, cens, u) in order of first occurrence
     and how often each occurs.  Returns (y, cens, u, counts) with u None when no u was given; np.repeat of the records by
