@@ -273,6 +273,40 @@ int pht_engine_set_counts(pht_engine *e, const uint32_t *counts_local);
 #define PHT_MAX_VISITS 1024
 int pht_engine_set_visits(pht_engine *e, const int64_t *offsets_local, const double *t, const uint32_t *mask);
 
+/* Misclassified panel observations (method 64 only): panel observations read by an imperfect instrument (a biopsy grade,
+ * an angiogram, a screening test, a wear gauge), a hidden Markov model over the visits.  Visit j of local observation k
+ * records an observed stage stage[j] in 0..stages-1 instead of a mask; the emission matrix E (n x stages, row-major, rows
+ * summing to 1) gives P(stage o read | phase c) = E[c stages + o].  Each panel path is drawn from its exact conditional
+ * law given pi, E, the visits and the terminal information (pht_unif.h, "Misclassified panel observations").  alpha
+ * (n x stages, may be NULL) is a Dirichlet prior on E's rows: after theta and pi, every sweep draws each row c of E from
+ * Dirichlet(alpha[c, .] + K[c, .]), K[c, o] the visits drawn in phase c and read as stage o, as Gamma variates on
+ * parameter sub-streams m + n + c stages + o normalised in index order; alpha[c, o] = 0 is a structural zero (E[c, o] = 0
+ * and stays 0), a positive alpha is at least 0.1 (smaller shapes draw E[c, o] = 0 often enough to make a visit impossible),
+ * and E's support must equal alpha's.  With alpha NULL, E stays fixed.  Every chain has its own E and draws; E is shared
+ * by the groups.  With E the 0/1 indicator of a partition of the phases into stages and alpha NULL, the engine is bit for
+ * bit the engine given the stage masks through pht_engine_set_visits.  offsets_local and t are as in
+ * pht_engine_set_visits; this call replaces any mask visits and pht_engine_set_visits replaces stage visits; offsets_local
+ * NULL clears the visits.  Refused, each with its own message and leaving the engine as it was: what pht_engine_set_visits
+ * refuses for its method, ranks, counts (either order), times and visit counts; stages outside 1..PHT_MAX_STAGES or a
+ * stage index at or above stages; an E entry negative or NaN, or a row not summing to 1 within 1e-12; an alpha entry
+ * negative or NaN, positive but below 0.1, or an alpha whose support differs from E's; a visit sequence no path can
+ * produce (pht_engine_set_visits' check with each visit's mask the support of its E column, applied again by
+ * pht_engine_set_pi, pht_engine_set_groups and pht_engine_set_emission while stage visits are set); a failed allocation. */
+#define PHT_MAX_STAGES 32
+int pht_engine_set_stage_visits(pht_engine *e, int stages, const double *E, const double *alpha, const int64_t *offsets_local,
+                                const double *t, const uint32_t *stage);
+/* E and / or its prior of an engine with stage visits: E (not NULL) is set in every chain, as pht_engine_set_pi does;
+ * NULL E leaves every chain its own E (a given alpha must then match the support of each); NULL alpha: E fixed from now
+ * on.  Refusals as pht_engine_set_stage_visits. */
+int pht_engine_set_emission(pht_engine *e, const double *E, const double *alpha);
+/* chain 0's current E (n x stages) */
+int pht_engine_get_emission(pht_engine *e, double *E);
+/* the E draws of the last run: chains x rows x n x stages, chain 0 first (needs alpha) */
+int pht_engine_emission_rows(pht_engine *e, int rows, double *out);
+/* parity hook: K (n x stages) of one sweep of chain 0 at the current parameters, without an update (as
+ * pht_engine_sweep_stats) */
+int pht_engine_emission_stats(pht_engine *e, long long *K);
+
 /* run `nsweeps` Gibbs sweeps; row r of out (nsweeps x m, row-major) is the draw of sweep r.
  * out may be NULL (results stay on the device; fetch later with pht_engine_get_theta). */
 int pht_engine_run(pht_engine *e, int nsweeps, double *out);

@@ -22,6 +22,8 @@ SYMBOLS = [
     "pht_engine_set_upper", "pht_engine_set_entry", "pht_engine_entry_paths",
     "pht_engine_set_chains", "pht_engine_set_chain_theta", "pht_engine_get_chain_theta", "pht_engine_chain_rows",
     "pht_engine_set_groups", "pht_engine_group_stats", "pht_engine_set_counts", "pht_engine_set_visits",
+    "pht_engine_set_stage_visits", "pht_engine_set_emission", "pht_engine_get_emission", "pht_engine_emission_rows",
+    "pht_engine_emission_stats",
 ]
 PEER_HANDLE_BYTES = 128
 # method 64 (include/pht_b200.h PHT_METHOD_UNIF): the uniformisation path sampler; exact, right-, interval- and
@@ -30,6 +32,7 @@ METHOD_UNIF = 64
 MAX_CHAINS = 1024            # include/pht_b200.h PHT_MAX_CHAINS: chains one METHOD_UNIF engine can run (Engine.set_chains)
 MAX_GROUPS = 64              # include/pht_b200.h PHT_MAX_GROUPS: groups with their own structure (Engine.set_groups)
 MAX_VISITS = 1024            # include/pht_b200.h PHT_MAX_VISITS: visits of one observation (Engine.set_visits)
+MAX_STAGES = 32              # include/pht_b200.h PHT_MAX_STAGES: observed stages of stage visits (Engine.set_stage_visits)
 CNT_NAMES = ["paths", "attempts", "jumps", "dens_evals", "env_updates", "brent_evals", "arms_calls",
              "metrop_rejects", "nonfinite", "deferred", "tail_rounds", "errors", "launches", "ns_lane", "ns_tail", "ns_replay",
              "ns_global", "ns_xwait", "global_rounds", "global_items"]
@@ -96,6 +99,11 @@ def lib():
     L.pht_engine_group_stats.argtypes = [C.c_void_p, _lp, _lp, _lp]
     L.pht_engine_set_counts.argtypes = [C.c_void_p, C.c_void_p]
     L.pht_engine_set_visits.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+    L.pht_engine_set_stage_visits.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+    L.pht_engine_set_emission.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
+    L.pht_engine_get_emission.argtypes = [C.c_void_p, _dp]
+    L.pht_engine_emission_rows.argtypes = [C.c_void_p, C.c_int, _dp]
+    L.pht_engine_emission_stats.argtypes = [C.c_void_p, _lp]
     L.pht_engine_peer_handle.argtypes = [C.c_void_p, C.c_void_p]
     L.pht_engine_peer_attach.argtypes = [C.c_void_p, C.c_void_p]
     _lib = L
@@ -138,6 +146,7 @@ class Engine:
         self._h = C.c_void_p()
         self.chains = 1
         self.groups = 1
+        self.stages = 0
         _check(L.pht_engine_create(C.byref(self._h), C.byref(cfg), y_local if self.l_local else np.zeros(1),
                                    cens_local if self.l_local else np.zeros(1, dtype=np.int32), self.l_local))
 
@@ -376,6 +385,7 @@ class Engine:
         then drawn given its visits too; observations without visits draw the paths they drew before.  None clears them."""
         if offsets is None:
             _check(lib().pht_engine_set_visits(self._h, None, None, None))
+            self.stages = 0                  # mask visits replace stage visits
             return
         off = np.ascontiguousarray(offsets, dtype=np.int64)
         if off.shape != (self.l_local + 1,):
@@ -390,6 +400,70 @@ class Engine:
         mv = np.ascontiguousarray(mv, dtype=np.uint32)
         tv = tv if total else np.zeros(1); mv = mv if total else np.zeros(1, dtype=np.uint32)
         _check(lib().pht_engine_set_visits(self._h, off.ctypes.data, tv.ctypes.data, mv.ctypes.data))
+        self.stages = 0
+
+    def set_stage_visits(self, E, offsets, t=None, stage=None, alpha=None):
+        """Misclassified panel observations (METHOD_UNIF only, one rank, no counts): local observation k was read at times
+        t[offsets[k]:offsets[k + 1]] (as set_visits) as the stages stage[...] in 0..S-1, through the emission matrix E
+        (n, S): P(stage o read | phase c) = E[c, o], rows summing to 1.  alpha (n, S), when given, is a Dirichlet prior on
+        E's rows (0: a structural zero, else >= 0.1, with E's support): every sweep then also draws E.  Replaces mask
+        visits; offsets None clears the visits."""
+        if offsets is None:
+            _check(lib().pht_engine_set_stage_visits(self._h, 0, None, None, None, None, None))
+            self.stages = 0
+            return
+        Em = np.ascontiguousarray(E, dtype=np.float64)
+        if Em.ndim != 2 or Em.shape[0] != self.n:
+            raise EngineError("set_stage_visits: E has shape %s, expected (%d, stages)" % (Em.shape, self.n))
+        S = int(Em.shape[1])
+        a = None if alpha is None else np.ascontiguousarray(alpha, dtype=np.float64)
+        if a is not None and a.shape != Em.shape:
+            raise EngineError("set_stage_visits: alpha has shape %s, E %s" % (a.shape, Em.shape))
+        off = np.ascontiguousarray(offsets, dtype=np.int64)
+        if off.shape != (self.l_local + 1,):
+            raise EngineError("set_stage_visits: %d offsets for %d local observations (expected l_local + 1)" % (off.size, self.l_local))
+        total = int(off[-1]) if off.size else 0
+        tv = np.ascontiguousarray(t if t is not None else np.zeros(0), dtype=np.float64)
+        sv = np.asarray(stage if stage is not None else np.zeros(0, dtype=np.uint32))
+        if tv.shape != (total,) or sv.shape != (total,):
+            raise EngineError("set_stage_visits: %d times and %d stages for %d visits" % (tv.size, sv.size, total))
+        if sv.size and (sv.min() < 0 or sv.max() > 0xffffffff):
+            raise EngineError("set_stage_visits: stages must lie in 0 .. 2^32 - 1")
+        sv = np.ascontiguousarray(sv, dtype=np.uint32)
+        tv = tv if total else np.zeros(1); sv = sv if total else np.zeros(1, dtype=np.uint32)
+        _check(lib().pht_engine_set_stage_visits(self._h, S, Em.ctypes.data, None if a is None else a.ctypes.data,
+                                                 off.ctypes.data, tv.ctypes.data, sv.ctypes.data))
+        self.stages = S
+
+    def set_emission(self, E=None, alpha=None):
+        """E (n, S) of every chain and / or its Dirichlet prior (None E: each chain keeps its own E; None alpha: E fixed from
+        now on)."""
+        S = self.stages
+        Em = None if E is None else np.ascontiguousarray(E, dtype=np.float64)
+        a = None if alpha is None else np.ascontiguousarray(alpha, dtype=np.float64)
+        for x, what in ((Em, "E"), (a, "alpha")):
+            if x is not None and S and x.shape != (self.n, S):
+                raise EngineError("set_emission: %s has shape %s, expected (%d, %d)" % (what, x.shape, self.n, S))
+        _check(lib().pht_engine_set_emission(self._h, None if Em is None else Em.ctypes.data, None if a is None else a.ctypes.data))
+
+    def emission(self):
+        """Chain 0's current E, shape (n, S)."""
+        out = np.zeros(self.n * max(self.stages, 1))
+        _check(lib().pht_engine_get_emission(self._h, out))
+        return out.reshape(self.n, -1)
+
+    def emission_rows(self, rows):
+        """The E draws of the last run, shape (chains, rows, n, S) (needs alpha)."""
+        S = max(self.stages, 1)
+        out = np.zeros(max(self.chains * int(rows) * self.n * S, 1))
+        _check(lib().pht_engine_emission_rows(self._h, int(rows), out))
+        return out[:self.chains * int(rows) * self.n * S].reshape(self.chains, int(rows), self.n, S)
+
+    def emission_stats(self):
+        """K (n, S) of one sweep of chain 0 without an update: visits drawn in phase c and read as stage o."""
+        K = np.zeros(self.n * max(self.stages, 1), dtype=np.int64)
+        _check(lib().pht_engine_emission_stats(self._h, K))
+        return K.reshape(self.n, -1)
 
     def group_stats(self):
         """One sweep's statistics of chain 0 per group, without an update: N (G, n*n), B (G, n), zfix (G, n); their sum

@@ -136,6 +136,12 @@ struct pht_engine {
      * (PanelBufs below); the panel kernel's grid */
     bool visits_set = false; std::vector<int64_t> h_voff; std::vector<double> h_vt; std::vector<uint32_t> h_vm;
     PanelBufs pan; int panel_blocks = 0;
+    /* method 64, misclassified panel observations (pht_engine_set_stage_visits; h_vm then holds stage indices): the stages
+     * (0: mask visits), the support of each column of E as a phase mask, E and K per chain (chains x n x stages), the prior
+     * (nullptr: E fixed), the E draws of the last run (chains x eres_rows x n x stages) and the kernel's grid */
+    int stages = 0; std::vector<uint32_t> h_colmask;
+    double *d_E = nullptr, *d_alpha = nullptr, *d_Eres = nullptr; unsigned long long *d_K = nullptr;
+    int eres_rows = 0, emis_blocks = 0;
     /* graph */
     cudaGraphExec_t graph_exec = nullptr; int graph_res_rows = -1; double *graph_res = nullptr;
     unsigned long long graph_launches = 0;      /* kernels one replay of the captured sweep launches */
@@ -254,6 +260,27 @@ static UnifPanel panel_args(const PanelBufs &b) {
     return V;
 }
 
+/* the observation process of stage visits; the E draws recorded only when the sweep records its rows */
+static UnifEmis emis_args(const pht_engine *e, bool record) {
+    UnifEmis X; memset(&X, 0, sizeof(X));
+    X.E = e->d_E; X.alpha = e->d_alpha; X.K = e->d_K; X.Eres = record ? e->d_Eres : nullptr; X.S = e->stages;
+    return X;
+}
+
+/* the panel kernel of the visits set: k_unif_emis_paths for stage visits, else k_unif_panel_paths */
+static cudaError_t launch_panel_kernel(pht_engine *e, const SweepParams &p, const UnifPanel &V) {
+    if (e->stages) return pht_launch_unif_emis(p, e->d_unif, V, emis_args(e, false), e->emis_blocks, e->stream);
+    return pht_launch_unif_panel(p, e->d_unif, V, e->panel_blocks, e->stream);
+}
+
+/* the phase mask of every visit: the masks themselves (colmask empty), or for stage visits the support of the stage's
+ * column of E (colmask[o]) */
+static std::vector<uint32_t> visit_masks(const uint32_t *v, size_t count, const std::vector<uint32_t> &colmask) {
+    std::vector<uint32_t> mk(v, v + count);
+    if (!colmask.empty()) for (uint32_t &x : mk) x = colmask[x];
+    return mk;
+}
+
 /* method 64 with visits: the observations without visits through the per-observation kernels (their own layout and group
  * offsets), then k_unif_panel_paths over the panel observations; both add to the same statistics blocks */
 static int enqueue_panel(pht_engine *e, const SweepParams &p) {
@@ -264,7 +291,7 @@ static int enqueue_panel(pht_engine *e, const SweepParams &p) {
         CU(pht_launch_unif(q, e->d_unif, q.groups > 1 ? b.pgofs : nullptr, q.chains > 1 || q.groups > 1 ? e->chain_blocks : e->grid_blocks, e->stream));
         e->launches++;
     }
-    CU(pht_launch_unif_panel(p, e->d_unif, panel_args(b), e->panel_blocks, e->stream));
+    CU(launch_panel_kernel(e, p, panel_args(b)));
     return 0;                                      /* enqueue_paths counts the panel kernel */
 }
 
@@ -363,6 +390,7 @@ static int enqueue_sweep(pht_engine *e, double *res, int res_rows, bool time_ker
         if (rc != 0) return fail("ncclAllReduce failed: %s", g_nccl.GetErrorString ? g_nccl.GetErrorString(rc) : "?");
     }
     CU(pht_launch_update(u, e->stream)); e->launches++;
+    if (e->stages && e->d_alpha) { CU(pht_launch_emis_update(u, emis_args(e, res != nullptr), e->stream)); e->launches++; }
     return 0;
 }
 
@@ -390,6 +418,8 @@ extern "C" void pht_engine_destroy(pht_engine *e) {
     { const PanelBufs &b = e->pan;
       void *pb[] = { b.py, b.pu, b.pc, b.pperm, b.pgofs, b.vy, b.vu, b.vt, b.beta, b.vc, b.vperm, b.vm, b.vgofs, b.vcoff, b.voff, b.vnext };
       for (void *q : pb) pht_dev_free(q, e->stream); }
+    { void *eb[] = { e->d_E, e->d_alpha, e->d_Eres, e->d_K };
+      for (void *q : eb) pht_dev_free(q, e->stream); }
     void *big[] = { e->d_cy, e->d_cu, e->d_cc, e->d_cperm, e->d_cgofs, e->d_ry, e->d_ru, e->d_rc, e->d_rbase, e->d_ritems, e->d_rnext, e->d_gtmax, e->d_gofs, e->d_gys, e->d_gus, e->d_gcs, e->d_gperm, e->d_keys, e->d_cnext, e->d_entry, e->d_ea, e->d_eobs, e->d_eM, e->d_eoff, e->d_enext, e->d_etab, e->d_escan, e->d_unif, e->d_u, e->d_us, e->d_item_u, e->d_recs, e->d_ys, e->d_cs, e->d_perm, e->d_y, e->d_cens, e->d_items /* arena: found, pend0, pend1, done live inside */, e->d_idx_exact, e->d_idx_cens,
                     e->d_glist, e->d_model, e->d_stats, e->d_state, e->d_T, e->d_C, e->d_nu, e->d_zeta, e->d_var_ptr, e->d_cell_i, e->d_cell_j, e->d_pires, e->d_res };
     for (void *b : big) pht_dev_free(b, e->stream);
@@ -727,7 +757,8 @@ extern "C" int pht_engine_set_pi(pht_engine *e, const double *pi, const double *
         double sum = 0.0;
         for (int i = 0; i < n; i++) { if (!(pi[i] >= 0.0)) return fail("pi[%d] = %g is not a probability", i, pi[i]); sum += pi[i]; }
         if (!(sum > 0.999999 && sum < 1.000001)) return fail("pi sums to %g, not 1", sum);
-        if (e->visits_set && engine_visits_reachable(e, e->h_voff.data(), e->h_vt.data(), e->h_vm.data(), pi, 0, nullptr, nullptr, nullptr))
+        if (e->visits_set && engine_visits_reachable(e, e->h_voff.data(), e->h_vt.data(), visit_masks(e->h_vm.data(), e->h_vm.size(), e->h_colmask).data(),
+                                                     pi, 0, nullptr, nullptr, nullptr))
             return -1;                             /* (pht_engine_set_visits: a visit sequence this pi cannot start) */
         for (int c = 0; c < e->chains * e->groups; c++)       /* every chain, in every group's block */
             CU(cudaMemcpy(e->d_model + (size_t)c * e->L.total + e->L.pi, pi, sizeof(double) * n, cudaMemcpyHostToDevice));
@@ -804,6 +835,22 @@ extern "C" int pht_engine_set_chains(pht_engine *e, int chains, const uint64_t *
                         chains, (bytes[0] + bytes[1] + bytes[2] + bytes[3] + bytes[4]) / 1e6, sizeof(double) * tab / 1e6, cudaGetErrorString(ce));
         }
     }
+    /* stage visits: E and K per chain, every chain starting from chain 0's E */
+    double *dE = nullptr; unsigned long long *dK = nullptr;
+    const size_t nS = (size_t)n * e->stages;
+    if (e->stages) {
+        cudaError_t ce = pht_dev_alloc((void **)&dE, sizeof(double) * chains * nS, e->stream);
+        if (ce == cudaSuccess) ce = pht_dev_alloc((void **)&dK, sizeof(unsigned long long) * chains * nS, e->stream);
+        if (ce != cudaSuccess) {
+            cudaGetLastError();
+            for (int f = 0; f < 5; f++) pht_dev_free(*ptrs[f], e->stream);
+            pht_dev_free(dE, e->stream);
+            cudaStreamSynchronize(e->stream); cudaGetLastError();
+            return fail("cannot allocate device memory for the emission matrices of %d chains: %s", chains, cudaGetErrorString(ce));
+        }
+        for (int c = 0; c < chains; c++) CU(cudaMemcpyAsync(dE + c * nS, e->d_E, sizeof(double) * nS, cudaMemcpyDeviceToDevice, e->stream));
+        CU(cudaMemsetAsync(dK, 0, sizeof(unsigned long long) * chains * nS, e->stream));
+    }
     /* every chain starts from chain 0's current theta and pi (the rest of a model block is rebuilt every sweep) */
     for (int c = 0; c < units; c++)
         CU(cudaMemcpyAsync(model + (size_t)c * total, e->d_model, sizeof(double) * total, cudaMemcpyDeviceToDevice, e->stream));
@@ -813,11 +860,12 @@ extern "C" int pht_engine_set_chains(pht_engine *e, int chains, const uint64_t *
     for (int c = 0; c < chains; c++) { hk[2 * (size_t)c] = (uint32_t)k[(size_t)c]; hk[2 * (size_t)c + 1] = (uint32_t)(k[(size_t)c] >> 32); }
     CU(cudaMemcpyAsync(dkeys, hk.data(), bytes[3], cudaMemcpyHostToDevice, e->stream));
     CU(cudaMemsetAsync(cnext, 0, bytes[4], e->stream));
-    void *old[] = { e->d_model, e->d_stats, e->d_unif, e->d_keys, e->d_cnext, e->d_res, e->d_pires };
+    void *old[] = { e->d_model, e->d_stats, e->d_unif, e->d_keys, e->d_cnext, e->d_res, e->d_pires, e->d_E, e->d_K, e->d_Eres };
     for (void *b : old) CU(pht_dev_free(b, e->stream));
     CU(cudaStreamSynchronize(e->stream));
     e->d_model = model; e->d_stats = stats; e->d_unif = unif; e->d_keys = dkeys; e->d_cnext = cnext;
     e->d_res = nullptr; e->d_pires = nullptr; e->res_rows = 0;
+    e->d_E = dE; e->d_K = dK; e->d_Eres = nullptr; e->eres_rows = 0;
     e->chains = chains;
     e->cfg.seed = k[0];                            /* chain 0's key is the engine's key (the ghost kernels read it) */
     if (e->graph_exec) { cudaGraphExecDestroy(e->graph_exec); e->graph_exec = nullptr; }     /* kernel parameters change */
@@ -925,7 +973,7 @@ extern "C" int pht_engine_set_groups(pht_engine *e, int G, const int *T, const d
     }
     CU(cudaSetDevice(e->cfg.device));
     CU(cudaStreamSynchronize(e->stream));
-    if (e->visits_set && engine_visits_reachable(e, e->h_voff.data(), e->h_vt.data(), e->h_vm.data(), nullptr, G, T, C,
+    if (e->visits_set && engine_visits_reachable(e, e->h_voff.data(), e->h_vt.data(), visit_masks(e->h_vm.data(), e->h_vm.size(), e->h_colmask).data(), nullptr, G, T, C,
                                                  G > 1 ? gid.data() : nullptr)) return -1;
     if (G > 1 && !e->chain_blocks) {
         e->chain_blocks = pht_unif_grid_blocks(e->cfg.device, n, true);
@@ -1314,12 +1362,19 @@ static int engine_visits_reachable(pht_engine *e, const int64_t *off, const doub
     return visits_reachable(n, G, T, C, gid, p.data(), l, y.data(), c.data(), u.empty() ? nullptr : u.data(), off, t, mask);
 }
 
-extern "C" int pht_engine_set_visits(pht_engine *e, const int64_t *offsets_local, const double *t, const uint32_t *mask) {
-    if (!e) return fail("null engine");
+/* the engine refusals common to mask and stage visits */
+static int visits_refused(const pht_engine *e) {
     if (method_of(e->cfg) != PHT_METHOD_UNIF)
         return fail("visits (panel observations) need method 64 (the uniformisation sampler): MHRS, ECS, DCS and the MH variants draw paths given the absorption time alone");
     if (e->peers_attached) return fail("visits cannot be set after the exchange windows are attached (visits need a single-rank engine)");
     if (e->cfg.world > 1) return fail("visits need world = 1: the panel observations are laid out and handed out on one rank");
+    return 0;
+}
+
+/* pht_engine_set_visits and pht_engine_set_stage_visits: checks and stores the visits; val holds masks (colmask empty) or
+ * stage indices into colmask, the support of every column of E.  The caller keeps the observation process. */
+static int visits_upload(pht_engine *e, const int64_t *offsets_local, const double *t, const uint32_t *val, const std::vector<uint32_t> &colmask) {
+    if (visits_refused(e)) return -1;
     CU(cudaSetDevice(e->cfg.device));
     CU(cudaStreamSynchronize(e->stream));
     if (!offsets_local) {
@@ -1355,13 +1410,18 @@ extern "C" int pht_engine_set_visits(pht_engine *e, const int64_t *offsets_local
             if (!(t[q] >= 0.0)) return fail("visit %lld of observation %ld: t = %g is negative or NaN", (long long)(q - v0), k, t[q]);
             if (t[q] > yk) return fail("visit %lld of observation %ld: t = %g is above y = %g", (long long)(q - v0), k, t[q], yk);
             if (q > v0 && !(t[q] > t[q - 1])) return fail("visit %lld of observation %ld: t = %g does not follow t = %g (the times must increase)", (long long)(q - v0), k, t[q], t[q - 1]);
-            if (mask[q] == 0u) return fail("visit %lld of observation %ld has an empty mask", (long long)(q - v0), k);
-            if (mask[q] & ~all) return fail("visit %lld of observation %ld: mask 0x%x has bits at or above n = %d", (long long)(q - v0), k, mask[q], n);
+            if (!colmask.empty()) {
+                if (val[q] >= colmask.size()) return fail("visit %lld of observation %ld: stage %u is not below stages = %d", (long long)(q - v0), k, val[q], (int)colmask.size());
+                continue;
+            }
+            if (val[q] == 0u) return fail("visit %lld of observation %ld has an empty mask", (long long)(q - v0), k);
+            if (val[q] & ~all) return fail("visit %lld of observation %ld: mask 0x%x has bits at or above n = %d", (long long)(q - v0), k, val[q], n);
         }
         if (e->entry_set && t[v0] < e->h_entry[(size_t)k])
             return fail("observation %ld: its first visit t = %g is before its entry age a = %g", k, t[v0], e->h_entry[(size_t)k]);
     }
-    if (any && engine_visits_reachable(e, offsets_local, t, mask, nullptr, 0, nullptr, nullptr, nullptr)) return -1;
+    if (any && engine_visits_reachable(e, offsets_local, t, visit_masks(val, (size_t)offsets_local[l], colmask).data(), nullptr, 0, nullptr, nullptr, nullptr))
+        return -1;
     if (!e->panel_blocks) {
         e->panel_blocks = pht_unif_panel_grid_blocks(e->cfg.device, n);
         if (e->panel_blocks <= 0) { e->panel_blocks = 0; return fail("the panel path kernel does not fit on the device: %s", cudaGetErrorString(cudaGetLastError())); }
@@ -1375,12 +1435,175 @@ extern "C" int pht_engine_set_visits(pht_engine *e, const int64_t *offsets_local
     std::vector<int64_t> ovoff; std::vector<double> ovt; std::vector<uint32_t> ovm;
     ovoff.swap(e->h_voff); ovt.swap(e->h_vt); ovm.swap(e->h_vm);
     e->h_voff.assign(offsets_local, offsets_local + l + 1);
-    e->h_vt.assign(t, t + total); e->h_vm.assign(mask, mask + total);
+    e->h_vt.assign(t, t + total); e->h_vm.assign(val, val + total);
     if (visits_build(e)) {                          /* a failed allocation: back to the previous visits */
         e->h_voff.swap(ovoff); e->h_vt.swap(ovt); e->h_vm.swap(ovm);
         return -1;
     }
     e->visits_set = true;
+    return 0;
+}
+
+/* back to mask visits (or none): the observation process of stage visits goes */
+static void emission_free(pht_engine *e) {
+    void *bufs[] = { e->d_E, e->d_alpha, e->d_Eres, e->d_K };
+    for (void *q : bufs) pht_dev_free(q, e->stream);
+    cudaStreamSynchronize(e->stream);
+    e->d_E = e->d_alpha = e->d_Eres = nullptr; e->d_K = nullptr;
+    e->stages = 0; e->h_colmask.clear(); e->eres_rows = 0;
+}
+
+extern "C" int pht_engine_set_visits(pht_engine *e, const int64_t *offsets_local, const double *t, const uint32_t *mask) {
+    if (!e) return fail("null engine");
+    if (visits_upload(e, offsets_local, t, mask, std::vector<uint32_t>())) return -1;
+    emission_free(e);
+    return 0;
+}
+
+/* alpha (n x S) checked as pht_engine_set_stage_visits states, against the support of E (n x S) */
+static int alpha_check(int n, int S, const double *E, const double *alpha) {
+    for (int c = 0; c < n; c++)
+        for (int o = 0; o < S; o++) {
+            const double a = alpha[c * S + o], v = E[c * S + o];
+            if (!(a >= 0.0) || !std::isfinite(a)) return fail("alpha[%d, %d] = %g: Dirichlet parameters must be finite and not negative", c, o, a);
+            if (a > 0.0 && a < 0.1) return fail("alpha[%d, %d] = %g is below 0.1: Gamma draws of such shapes underflow to 0 often enough to make a visit impossible mid-run (0 is a structural zero)", c, o, a);
+            if ((a > 0.0) != (v > 0.0)) return fail("alpha[%d, %d] = %g but E[%d, %d] = %g: E's support must equal alpha's (alpha = 0 is a structural zero)", c, o, a, c, o, v);
+        }
+    return 0;
+}
+
+/* E (n x S) and alpha (n x S or nullptr) checked as pht_engine_set_stage_visits states; colmask receives E's column supports */
+static int emission_check(int n, int S, const double *E, const double *alpha, std::vector<uint32_t> &colmask) {
+    colmask.assign((size_t)S, 0u);
+    for (int c = 0; c < n; c++) {
+        double sum = 0.0;
+        for (int o = 0; o < S; o++) {
+            const double v = E[c * S + o];
+            if (!(v >= 0.0) || !std::isfinite(v)) return fail("E[%d, %d] = %g is not a probability", c, o, v);
+            sum += v;
+            if (v > 0.0) colmask[(size_t)o] |= 1u << c;
+        }
+        if (!(std::fabs(sum - 1.0) <= 1e-12)) return fail("row %d of E sums to %.17g, not 1 (within 1e-12)", c, sum);
+    }
+    return alpha ? alpha_check(n, S, E, alpha) : 0;
+}
+
+static int emis_grid(pht_engine *e, int S) {
+    const int b = pht_unif_emis_grid_blocks(e->cfg.device, e->cfg.n, S);
+    if (b <= 0) return fail("the stage-visit path kernel does not fit on the device: %s", cudaGetErrorString(cudaGetLastError()));
+    return b;
+}
+
+extern "C" int pht_engine_set_stage_visits(pht_engine *e, int stages, const double *E, const double *alpha, const int64_t *offsets_local,
+                                           const double *t, const uint32_t *stage) {
+    if (!e) return fail("null engine");
+    if (!offsets_local) {
+        if (visits_upload(e, nullptr, nullptr, nullptr, std::vector<uint32_t>())) return -1;
+        emission_free(e);
+        return 0;
+    }
+    if (visits_refused(e)) return -1;
+    if (stages < 1 || stages > PHT_MAX_STAGES) return fail("stages = %d outside 1..%d", stages, PHT_MAX_STAGES);
+    if (!E) return fail("null emission matrix");
+    const int n = e->cfg.n, S = stages;
+    const size_t nS = (size_t)n * S, chains = (size_t)e->chains;
+    std::vector<uint32_t> colmask;
+    if (emission_check(n, S, E, alpha, colmask)) return -1;
+    CU(cudaSetDevice(e->cfg.device));
+    CU(cudaStreamSynchronize(e->stream));
+    if (!e->panel_blocks) {
+        e->panel_blocks = pht_unif_panel_grid_blocks(e->cfg.device, n);
+        if (e->panel_blocks <= 0) { e->panel_blocks = 0; return fail("the panel path kernel does not fit on the device: %s", cudaGetErrorString(cudaGetLastError())); }
+    }
+    const int blocks = emis_grid(e, S);
+    if (blocks < 0) return -1;
+    /* the new observation process first: a refusal or a failed allocation leaves the engine as it was */
+    double *dE = nullptr, *dalpha = nullptr; unsigned long long *dK = nullptr;
+    cudaError_t ce = pht_dev_alloc((void **)&dE, sizeof(double) * chains * nS, e->stream);
+    if (ce == cudaSuccess) ce = pht_dev_alloc((void **)&dK, sizeof(unsigned long long) * chains * nS, e->stream);
+    if (ce == cudaSuccess && alpha) ce = pht_dev_alloc((void **)&dalpha, sizeof(double) * nS, e->stream);
+    for (size_t c = 0; c < chains && ce == cudaSuccess; c++) ce = cudaMemcpyAsync(dE + c * nS, E, sizeof(double) * nS, cudaMemcpyHostToDevice, e->stream);
+    if (ce == cudaSuccess) ce = cudaMemsetAsync(dK, 0, sizeof(unsigned long long) * chains * nS, e->stream);
+    if (ce == cudaSuccess && alpha) ce = cudaMemcpyAsync(dalpha, alpha, sizeof(double) * nS, cudaMemcpyHostToDevice, e->stream);
+    if (ce == cudaSuccess) ce = cudaStreamSynchronize(e->stream);
+    auto drop = [&]() { void *b[] = { dE, dK, dalpha }; for (void *q : b) pht_dev_free(q, e->stream); cudaStreamSynchronize(e->stream); };
+    if (ce != cudaSuccess) {
+        cudaGetLastError(); drop(); cudaGetLastError();
+        return fail("cannot allocate device memory for the emission matrices: %s", cudaGetErrorString(ce));
+    }
+    if (visits_upload(e, offsets_local, t, stage, colmask)) { drop(); return -1; }
+    emission_free(e);
+    if (!e->visits_set) { drop(); return 0; }      /* no visits at all: the plain engine */
+    e->d_E = dE; e->d_K = dK; e->d_alpha = dalpha;
+    e->stages = S; e->h_colmask = colmask; e->emis_blocks = std::min(blocks, e->panel_blocks);
+    if (e->graph_exec) { cudaGraphExecDestroy(e->graph_exec); e->graph_exec = nullptr; }
+    return 0;
+}
+
+/* E NULL keeps every chain's own E (a prior is then checked against each of them); the new buffers are filled before
+ * the old ones go, so a refusal or a failed copy leaves the engine as it was */
+extern "C" int pht_engine_set_emission(pht_engine *e, const double *E, const double *alpha) {
+    if (!e) return fail("null engine");
+    if (!e->stages) return fail("the emission matrix belongs to stage visits: set them with pht_engine_set_stage_visits first");
+    const int n = e->cfg.n, S = e->stages;
+    const size_t nS = (size_t)n * S, chains = (size_t)e->chains;
+    CU(cudaSetDevice(e->cfg.device));
+    CU(cudaStreamSynchronize(e->stream));
+    std::vector<uint32_t> colmask = e->h_colmask;
+    if (E) {
+        if (emission_check(n, S, E, alpha, colmask)) return -1;
+        if (colmask != e->h_colmask &&
+            engine_visits_reachable(e, e->h_voff.data(), e->h_vt.data(), visit_masks(e->h_vm.data(), e->h_vm.size(), colmask).data(), nullptr, 0, nullptr, nullptr, nullptr))
+            return -1;
+    } else if (alpha) {
+        std::vector<double> cur(chains * nS);
+        CU(cudaMemcpy(cur.data(), e->d_E, sizeof(double) * cur.size(), cudaMemcpyDeviceToHost));
+        for (size_t c = 0; c < chains; c++)
+            if (alpha_check(n, S, cur.data() + c * nS, alpha)) {
+                const std::string msg = pht_last_error();
+                return fail("%s (chain %zu's E)", msg.c_str(), c);
+            }
+    }
+    double *dE = nullptr, *dalpha = nullptr;
+    cudaError_t ce = cudaSuccess;
+    if (E) ce = pht_dev_alloc((void **)&dE, sizeof(double) * chains * nS, e->stream);
+    for (size_t c = 0; c < chains && E && ce == cudaSuccess; c++) ce = cudaMemcpyAsync(dE + c * nS, E, sizeof(double) * nS, cudaMemcpyHostToDevice, e->stream);
+    if (alpha && ce == cudaSuccess) ce = pht_dev_alloc((void **)&dalpha, sizeof(double) * nS, e->stream);
+    if (alpha && ce == cudaSuccess) ce = cudaMemcpyAsync(dalpha, alpha, sizeof(double) * nS, cudaMemcpyHostToDevice, e->stream);
+    if (ce == cudaSuccess) ce = cudaStreamSynchronize(e->stream);
+    if (ce != cudaSuccess) {
+        cudaGetLastError();
+        pht_dev_free(dE, e->stream); pht_dev_free(dalpha, e->stream);
+        cudaStreamSynchronize(e->stream); cudaGetLastError();
+        return fail("cannot set the emission matrix or its prior: %s", cudaGetErrorString(ce));
+    }
+    if (E) { pht_dev_free(e->d_E, e->stream); e->d_E = dE; }
+    pht_dev_free(e->d_alpha, e->stream); e->d_alpha = dalpha;
+    cudaStreamSynchronize(e->stream);
+    e->h_colmask = colmask;
+    if (e->graph_exec) { cudaGraphExecDestroy(e->graph_exec); e->graph_exec = nullptr; }     /* new pointers; the update comes or goes */
+    return 0;
+}
+
+extern "C" int pht_engine_get_emission(pht_engine *e, double *E) {
+    if (!e || !E) return fail("null argument");
+    if (!e->stages) return fail("no stage visits are set (pht_engine_set_stage_visits)");
+    CU(cudaSetDevice(e->cfg.device));
+    CU(cudaStreamSynchronize(e->stream));
+    CU(cudaMemcpy(E, e->d_E, sizeof(double) * (size_t)e->cfg.n * e->stages, cudaMemcpyDeviceToHost));
+    return 0;
+}
+
+extern "C" int pht_engine_emission_rows(pht_engine *e, int rows, double *out) {
+    if (!e || rows < 0) return fail("bad argument");
+    if (!e->stages || !e->d_alpha) return fail("E is not being inferred (pht_engine_set_stage_visits or pht_engine_set_emission with a prior first)");
+    if (rows > e->eres_rows || !e->d_Eres) return fail("%d rows asked, the last run produced at most %d", rows, e->d_Eres ? e->eres_rows : 0);
+    if (rows == 0) return 0;
+    if (!out) return fail("null argument");
+    CU(cudaSetDevice(e->cfg.device));
+    CU(cudaStreamSynchronize(e->stream));
+    const size_t nS = (size_t)e->cfg.n * e->stages, R = (size_t)e->eres_rows;
+    CU(cudaMemcpy2D(out, sizeof(double) * rows * nS, e->d_Eres, sizeof(double) * R * nS, sizeof(double) * rows * nS, e->chains, cudaMemcpyDeviceToHost));
     return 0;
 }
 
@@ -1438,7 +1661,7 @@ static int panel_window(pht_engine *e, long first, long count, int *B, int *N, d
         SweepParams p = sweep_params(e);
         p.chains = 1;
         p.outB = dB; p.outN = dN; p.outz = dz; p.first = first; p.count = count;
-        CUP(pht_launch_unif_panel(p, e->d_unif, panel_args(w), e->panel_blocks, e->stream));
+        CUP(launch_panel_kernel(e, p, panel_args(w)));
         e->launches++;
         if (pht_engine_sync(e)) goto out;
         std::vector<int> hB((size_t)count), hN((size_t)count * n * n); std::vector<double> hz((size_t)count * n);
@@ -1688,6 +1911,14 @@ extern "C" int pht_engine_enqueue(pht_engine *e, int nsweeps) {
     if (!e || nsweeps < 0) return fail("bad argument");
     CU(cudaSetDevice(e->cfg.device));
     if (ensure_res(e, nsweeps > 0 ? nsweeps : 1)) return -1;
+    if (e->stages && e->d_alpha && (!e->d_Eres || e->eres_rows != e->res_rows)) {    /* rows of the E draws, like res */
+        CU(cudaStreamSynchronize(e->stream));
+        if (e->d_Eres) { CU(pht_dev_free(e->d_Eres, e->stream)); e->d_Eres = nullptr; e->eres_rows = 0; }
+        CU(pht_dev_alloc((void **)&e->d_Eres, sizeof(double) * (size_t)e->chains * e->res_rows * e->cfg.n * e->stages, e->stream));
+        CU(cudaStreamSynchronize(e->stream));
+        e->eres_rows = e->res_rows;
+        if (e->graph_exec) { cudaGraphExecDestroy(e->graph_exec); e->graph_exec = nullptr; }
+    }
     CU(cudaMemsetAsync(&e->d_state->res_row, 0, sizeof(uint32_t), e->stream));
     e->kev_used = 0;
     const bool graph = e->cfg.use_graph != 0;
@@ -1813,6 +2044,15 @@ extern "C" int pht_engine_sweep_stats(pht_engine *e, long long *N, long long *B,
     std::vector<long long> h;
     if (chain0_stats(e, h)) return -1;
     return unpack_stats(e, h.data(), e->groups, N, B, zfix);     /* the sum over the groups */
+}
+
+extern "C" int pht_engine_emission_stats(pht_engine *e, long long *K) {
+    if (!e || !K) return fail("null argument");
+    if (!e->stages) return fail("no stage visits are set (pht_engine_set_stage_visits)");
+    std::vector<long long> h;
+    if (chain0_stats(e, h)) return -1;
+    CU(cudaMemcpy(K, e->d_K, sizeof(long long) * (size_t)e->cfg.n * e->stages, cudaMemcpyDeviceToHost));
+    return 0;
 }
 
 extern "C" int pht_engine_group_stats(pht_engine *e, long long *N, long long *B, long long *zfix) {

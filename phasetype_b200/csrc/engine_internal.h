@@ -260,6 +260,21 @@ struct UnifPanel {
 #define PHT_UNIF_PANEL_THREADS 128           /* threads per block of the panel kernel (its beta scratch is per lane) */
 cudaError_t pht_launch_unif_panel(const SweepParams &p, const double *tab, const UnifPanel &V, int grid_blocks, cudaStream_t st);
 int pht_unif_panel_grid_blocks(int device, int n);
+/* method 64, misclassified panel observations (k_unif.cu; pht_engine_set_stage_visits): the stage visits travel in UnifPanel
+ * (vm holds each visit's stage index), the observation process here.  Kernel arguments of their own. */
+struct UnifEmis {
+    double *E;                                   /* chains x n x S emission matrices, chain c's at c n S (row-major) */
+    const double *alpha;                         /* n x S Dirichlet prior, 0 a structural zero; nullptr: E stays fixed */
+    unsigned long long *K;                       /* chains x n x S: the sweep's visits in phase c read as stage o, zeroed by
+                                                    the path launcher */
+    double *Eres;                                /* per chain res_rows x n x S draws of E, chain c's at c res_rows n S;
+                                                    nullptr: not recorded */
+    int S;
+};
+cudaError_t pht_launch_unif_emis(const SweepParams &p, const double *tab, const UnifPanel &V, const UnifEmis &X, int grid_blocks, cudaStream_t st);
+int pht_unif_emis_grid_blocks(int device, int n, int S);
+/* after k_update (one block per chain): E's rows from Dirichlet(alpha + K) on parameter sub-streams m + n + c S + o */
+cudaError_t pht_launch_emis_update(const UpdateParams &u, const UnifEmis &X, cudaStream_t st);
 /* large per-call buffers: stream-ordered pool allocations, cached across calls (engine.cu) */
 cudaError_t pht_dev_alloc(void **p, size_t bytes, cudaStream_t st);
 cudaError_t pht_dev_free(void *p, cudaStream_t st);

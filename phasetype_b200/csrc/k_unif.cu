@@ -467,6 +467,7 @@ static size_t unif_panel_smem(int n) {     /* per-lane path scratch (stride THRE
     return sizeof(double) * (size_t)(2 * n * THREADS) + (size_t)(THREADS / 32) * ((UnifPanelAcc::bytes(n) + 15) & ~(size_t)15);
 }
 
+/* twin: k_unif_emis_paths below repeats this kernel for stage visits; a fix to one belongs in the other */
 template <int THREADS>
 __global__ void __launch_bounds__(THREADS) k_unif_panel_paths(SweepParams p, const double *tab, UnifPanel V) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -541,6 +542,141 @@ cudaError_t pht_launch_unif_panel(const SweepParams &p, const double *tab, const
     const cudaError_t e = cudaMemsetAsync(V.next, 0, sizeof(unsigned long long), st);
     if (e != cudaSuccess) return e;
     k_unif_panel_paths<PHT_UNIF_PANEL_THREADS><<<grid_blocks, PHT_UNIF_PANEL_THREADS, unif_panel_smem<PHT_UNIF_PANEL_THREADS>(p.n), st>>>(p, tab, V);
+    return cudaGetLastError();
+}
+
+/* ---- misclassified panel observations (pht_engine_set_stage_visits; pht_unif.h, "Misclassified panel observations"):
+ * k_unif_panel_paths with stage indices in V.vm and the emission matrix of the item's chain, drawn by pht_unif_emis_path.
+ * Besides the statistics, every warp counts its lanes' visits by (drawn phase, stage read) in n S shared-memory counters
+ * of its own, flushed into the chain's 64-bit K block after every item, as the statistics are.  Counted only when the
+ * statistics are (p.outB nullptr). */
+template <int THREADS>
+static size_t unif_emis_smem(int n, int S) {
+    return unif_panel_smem<THREADS>(n) + (size_t)(THREADS / 32) * sizeof(unsigned int) * (size_t)(n * S);
+}
+
+/* twin of k_unif_panel_paths above (kept apart so that its SASS stays as it is); a fix to one belongs in the other.  The
+ * minimum of 4 blocks lets ptxas use the registers it needs: without it, it settles on 72 registers and spills */
+template <int THREADS>
+__global__ void __launch_bounds__(THREADS, 4) k_unif_emis_paths(SweepParams p, const double *tab, UnifPanel V, UnifEmis X) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const int n = p.n, tid = threadIdx.x, lane = tid & 31, cap = PHT_UNIF_CAP, G = p.groups, S = X.S, nS = n * S;
+    const unsigned FULL = 0xffffffffu;
+    const ModelLayout ML = ModelLayout::make(n, p.m);
+    const size_t tabd = (size_t)pht_unif_layout_make(n, cap).total;
+    double *Za = reinterpret_cast<double *>(smem_raw), *Zb = Za + n * THREADS;
+    UnifPanelAcc w;
+    w.carve(smem_raw + sizeof(double) * (size_t)(2 * n * THREADS) + (size_t)(tid >> 5) * ((UnifPanelAcc::bytes(n) + 15) & ~(size_t)15), n);
+    unsigned int *Kacc = reinterpret_cast<unsigned int *>(smem_raw + sizeof(double) * (size_t)(2 * n * THREADS)
+                                                          + (size_t)(THREADS / 32) * ((UnifPanelAcc::bytes(n) + 15) & ~(size_t)15)) + (size_t)(tid >> 5) * nS;
+    for (int i = lane; i < n * n; i += 32) w.Nacc[i] = 0u;
+    for (int i = lane; i < n; i += 32) { w.Bacc[i] = 0u; w.zlo[i] = 0ull; w.zhi[i] = 0; }
+    for (int i = lane; i < nS; i += 32) Kacc[i] = 0u;
+    __syncwarp();
+    const uint32_t iter = p.state->iter;
+    const long bs = (long)gridDim.x * THREADS;
+    double *beta = V.beta + (size_t)blockIdx.x * THREADS + tid;
+    const unsigned long long chunks = V.coff[G], work = (unsigned long long)p.chains * chunks;
+    unsigned long long c_paths = 0; int err = 0;
+    UnifCount ctx; ctx.p = &p; ctx.Nacc = w.Nacc; ctx.n = n; ctx.out_idx = 0;
+    for (;;) {
+        unsigned long long f = 0;
+        if (lane == 0) f = atomicAdd(V.next, 1ull);
+        f = __shfl_sync(FULL, f, 0);
+        if (f >= work) break;
+        const unsigned c = (unsigned)(f / chunks);
+        const unsigned long long r = f - (unsigned long long)c * chunks;
+        int g = 0;
+        while (V.coff[g + 1] <= r) g++;
+        const unsigned long long j0 = V.gofs[g] + (r - V.coff[g]) * 32ull, j = j0 + (unsigned long long)lane;
+        const int unit = (int)c * G + g;
+        const double *utab = tab + (size_t)unit * tabd, *model = p.model + (size_t)unit * ML.total;
+        if (j < V.gofs[g + 1]) {
+            const uint32_t ol = V.perm[j];
+            pht_stream st; st.k0 = p.ckeys[2 * c]; st.k1 = p.ckeys[2 * c + 1];
+            pht_stream_seek(&st, iter, p.obs_rank + ol * p.obs_world, 0u, 0u);
+            ctx.out_idx = (long)ol - p.first;
+            const unsigned long long v0 = V.voff[j];
+            const int m = (int)(V.voff[j + 1] - v0);
+            int B = 0;
+            const int e = pht_unif_emis_path(utab, n, cap, model + ML.s, model + ML.scale, model + ML.cum, model + ML.pi, V.y[j], V.cens[j],
+                                             V.u ? V.u[j] : INFINITY, m, V.vt + v0, V.vm + v0, X.E + (size_t)c * nS, S, beta, bs, &st,
+                                             Za + tid, Zb + tid, THREADS, &ctx, &B);
+            err |= e;
+            path_flush<THREADS>(p, n, Za, w.zlo, w.zhi, w.Bacc, B, ctx.out_idx);
+            if (e == 0 && p.outB == nullptr)
+                for (int q = 1; q <= m; q++) atomicAdd(&Kacc[(int)beta[(long)q * n * bs] * S + (int)V.vm[v0 + q - 1]], 1u);
+            c_paths++;
+        }
+        __syncwarp();
+        if (p.outB == nullptr) {
+            unsigned long long *gs = reinterpret_cast<unsigned long long *>(p.stats + (size_t)unit * stats_len(n));
+            for (int i = lane; i < n * n; i += 32) if (w.Nacc[i]) { atomicAdd(&gs[i], (unsigned long long)w.Nacc[i]); w.Nacc[i] = 0u; }
+            for (int i = lane; i < n; i += 32) {
+                if (w.Bacc[i]) { atomicAdd(&gs[n * n + i], (unsigned long long)w.Bacc[i]); w.Bacc[i] = 0u; }
+                if (w.zlo[i]) { atomicAdd(&gs[n * n + n + i], w.zlo[i]); w.zlo[i] = 0ull; }
+                if (w.zhi[i]) { atomicAdd(&gs[n * n + 2 * n + i], (unsigned long long)w.zhi[i]); w.zhi[i] = 0; }
+            }
+            unsigned long long *Kc = X.K + (size_t)c * nS;
+            for (int i = lane; i < nS; i += 32) if (Kacc[i]) { atomicAdd(&Kc[i], (unsigned long long)Kacc[i]); Kacc[i] = 0u; }
+        }
+        __syncwarp();
+    }
+    if (err) atomicOr(&p.state->error, err);
+    for (int o = 16; o > 0; o >>= 1) c_paths += __shfl_down_sync(FULL, c_paths, o);
+    if (lane == 0) atomicAdd(&p.state->counters[PHT_CNT_PATHS], c_paths);
+}
+
+int pht_unif_emis_grid_blocks(int device, int n, int S) {
+    const size_t smem = unif_emis_smem<PHT_UNIF_PANEL_THREADS>(n, S);
+    int per_sm = 0, sms = 0;
+    if (cudaFuncSetAttribute(k_unif_emis_paths<PHT_UNIF_PANEL_THREADS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return -1;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_unif_emis_paths<PHT_UNIF_PANEL_THREADS>, PHT_UNIF_PANEL_THREADS, smem) != cudaSuccess) return -1;
+    if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device) != cudaSuccess) return -1;
+    return per_sm * sms;
+}
+
+cudaError_t pht_launch_unif_emis(const SweepParams &p, const double *tab, const UnifPanel &V, const UnifEmis &X, int grid_blocks, cudaStream_t st) {
+    cudaError_t e = cudaMemsetAsync(V.next, 0, sizeof(unsigned long long), st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(X.K, 0, sizeof(unsigned long long) * (size_t)p.chains * p.n * X.S, st);
+    if (e != cudaSuccess) return e;
+    k_unif_emis_paths<PHT_UNIF_PANEL_THREADS><<<grid_blocks, PHT_UNIF_PANEL_THREADS, unif_emis_smem<PHT_UNIF_PANEL_THREADS>(p.n, X.S), st>>>(p, tab, V, X);
+    return cudaGetLastError();
+}
+
+/* block c: chain c's E rows.  k_update has advanced the sweep, so this sweep is iter - 1 and its row res_row - 1.  Cell
+ * (c, o) with alpha > 0 draws Gamma(alpha + K, 1) on parameter sub-stream m + n + c S + o; each row is normalised in index
+ * order, as pi is; cells with alpha = 0 stay 0. */
+__global__ void __launch_bounds__(128) k_emis_update(UpdateParams p, UnifEmis X) {
+    __shared__ double gam[PHT_NMAX * PHT_MAX_STAGES];
+    const int n = p.n, S = X.S, nS = n * S, c = blockIdx.x;
+    const uint32_t iter = p.state->iter - 1u, row = p.state->res_row - 1u;
+    const uint32_t k0 = p.ckeys ? p.ckeys[2 * c] : p.k0, k1 = p.ckeys ? p.ckeys[2 * c + 1] : p.k1;
+    double *E = X.E + (size_t)c * nS;
+    const unsigned long long *K = X.K + (size_t)c * nS;
+    for (int i = threadIdx.x; i < nS; i += blockDim.x) {
+        double v = 0.0;
+        if (X.alpha[i] > 0.0) {
+            pht_stream st; st.k0 = k0; st.k1 = k1;
+            pht_stream_seek(&st, iter, PHT_OBS_PARAM, (uint32_t)(p.m + n + i), 0);
+            v = pht_rgamma(&st, X.alpha[i] + (double)K[i], 1.0);
+        }
+        gam[i] = v;
+    }
+    __syncthreads();
+    for (int r = threadIdx.x; r < n; r += blockDim.x) {
+        double sum = 0.0;
+        for (int o = 0; o < S; o++) sum += gam[r * S + o];
+        for (int o = 0; o < S; o++) {
+            const double v = X.alpha[r * S + o] > 0.0 ? gam[r * S + o] / sum : 0.0;
+            E[r * S + o] = v;
+            if (X.Eres != nullptr && row < (uint32_t)p.res_rows) X.Eres[((size_t)c * p.res_rows + row) * nS + r * S + o] = v;
+        }
+    }
+}
+
+cudaError_t pht_launch_emis_update(const UpdateParams &u, const UnifEmis &X, cudaStream_t st) {
+    k_emis_update<<<u.chains, 128, 0, st>>>(u, X);
     return cudaGetLastError();
 }
 

@@ -305,6 +305,23 @@ PHT_HD int pht_unif_rescale(double *w, long ws, int n, uint32_t mask) {
     return 0;
 }
 
+/* Misclassified panel observations (pht_engine_set_stage_visits).  Visit j records an observed stage o_j in 0..S-1 instead
+ * of a mask, read through the emission matrix E (n x S, row-major): P(stage o read | phase c) = E[c S + o].  The law is
+ * that of panel observations with the indicator 1[A_j] replaced by the emission column E[., o_j]:
+ *     beta_m = E[., o_m] . e^{S d_{m+1}} v,   beta_{j-1} = E[., o_{j-1}] . e^{S (t_j - t_{j-1})} beta_j,
+ * each beta rescaled by pht_unif_rescale with the mask set to the support of its column.  The draws and their order are
+ * those of pht_unif_panel_path (steps 1-5), a visit state drawn only when the column's support has more than one phase
+ * and the gap is not 0.  With E the 0/1 indicator of a partition into stages, every weight is the mask form's weight
+ * (multiplying by 1.0 and zeroing outside the support are exact), so the paths are bit for bit those of the masks.
+ * Each drawn visit state x_j is left in entry 0 of beta_j, where the caller counts K[x_j S + o_j] for E's update. */
+
+/* the support of column o of E (n x S, row-major) as a phase mask */
+PHT_HD uint32_t pht_unif_col_support(const double *E, int n, int S, uint32_t o) {
+    uint32_t mk = 0u;
+    for (int c = 0; c < n; c++) if (E[c * S + (int)o] > 0.0) mk |= 1u << c;
+    return mk;
+}
+
 /* the sampler itself is compiled where the includer says how transitions are counted: PHT_UNIF_CTX (a type) and
  * PHT_UNIF_COUNT(ctx, from, to); PHT_UNIF_U01(st) may replace the uniform draw by an equivalent call, PHT_UNIF_FN the function's qualifiers */
 #if defined(PHT_UNIF_CTX) && defined(PHT_UNIF_COUNT)
@@ -619,7 +636,8 @@ PHT_UNIF_FN int pht_unif_bridge(const double *tab, int n, int cap, double d, dou
     return 0;
 }
 
-/* One panel observation (law and draw order above): m >= 1 visits at times vt[0..m-1] with masks vm[0..m-1]; beta:
+/* Twin: pht_unif_emis_path below repeats this function with emission columns; a fix to one belongs in the other.
+ * One panel observation (law and draw order above): m >= 1 visits at times vt[0..m-1] with masks vm[0..m-1]; beta:
  * (m + 1) n doubles of scratch with stride bs.  Other arguments as pht_unif_path. */
 PHT_UNIF_FN int pht_unif_panel_path(const double *tab, int n, int cap, const double *s, const double *scale, const double *cum,
                                     const double *pi, double y, int cens, double u, int m, const double *vt, const uint32_t *vm,
@@ -671,6 +689,170 @@ PHT_UNIF_FN int pht_unif_panel_path(const double *tab, int n, int cap, const dou
     for (int j = 1; j <= m; j++) {
         const double gap = vt[j - 1] - (j > 1 ? vt[j - 2] : 0.0);
         const uint32_t mk = vm[j - 1];
+        int x;
+        if (gap == 0.0) x = prev;
+        else if ((mk & (mk - 1u)) == 0u) { x = 0; while (!((mk >> x) & 1u)) x++; }
+        else {
+            const double xx = lam * gap;
+            pht_unif_exprow(tab, n, cap, xx, xx > 0.0 ? pht_log(xx) : 0.0, pht_unif_K(xx), prev, za, zs);
+            for (int c = 0; c < n; c++) za[c * zs] = za[c * zs] * PHT_BETA(j, c);
+            x = pht_unif_pick(za, n, zs, PHT_UNIF_U01(st));
+            if (x < 0) return PHT_UNIF_ERR_ZERO;
+        }
+        PHT_BETA(j, 0) = (double)x;
+        prev = x;
+    }
+
+    /* 3. the state at y */
+    int b = prev;
+    if (dy > 0.0) {
+        const double xx = lam * dy;
+        pht_unif_exprow(tab, n, cap, xx, xx > 0.0 ? pht_log(xx) : 0.0, pht_unif_K(xx), prev, za, zs);
+        if (iv) {
+            for (int c = 0; c < n; c++) zb[c * zs] = 0.0;
+            for (int k = 1; k <= K2; k++) {
+                const double w = pht_unif_w(x2, lx2, k, lgk);
+                if (w == 0.0) continue;
+                const double *g = tab + L.g + k * n;
+                for (int c = 0; c < n; c++) zb[c * zs] += w * g[c];
+            }
+            for (int c = 0; c < n; c++) za[c * zs] = za[c * zs] * zb[c * zs];
+        } else if (!cens) {
+            for (int c = 0; c < n; c++) za[c * zs] = za[c * zs] * s[c];
+        }
+        b = pht_unif_pick(za, n, zs, PHT_UNIF_U01(st));
+        if (b < 0) return PHT_UNIF_ERR_ZERO;
+    }
+    for (int c = 0; c < n; c++) { za[c * zs] = 0.0; zb[c * zs] = 0.0; }
+
+    /* 4. the bridges in time order */
+    prev = a;
+    for (int j = 1; j <= m + 1; j++) {
+        const double gap = j > m ? dy : vt[j - 1] - (j > 1 ? vt[j - 2] : 0.0);
+        const int x = j > m ? b : (int)PHT_BETA(j, 0);
+        if (gap > 0.0) {
+            const double xx = lam * gap;
+            const int e = pht_unif_bridge(tab, n, cap, gap, xx, xx > 0.0 ? pht_log(xx) : 0.0, pht_unif_K(xx), prev, x, st, za, zb, zs, ctx);
+            if (e) return e;
+        }
+        prev = x;
+    }
+#undef PHT_BETA
+
+    /* 5. after y */
+    if (!cens) {
+        PHT_UNIF_COUNT(ctx, b, b);
+    } else if (!iv) {
+        int j = b;
+        for (;;) {
+            const double t = scale[j] * -pht_log(PHT_UNIF_U01(st));
+            const double target = PHT_UNIF_U01(st);
+            const double *cr = cum + j * (n + 1);
+            int k = 0;
+            while (k < n && cr[k] < target) k++;
+            za[j * zs] += t;
+            if (k < n) { PHT_UNIF_COUNT(ctx, j, k); j = k; }
+            else { PHT_UNIF_COUNT(ctx, j, j); break; }
+        }
+    } else {
+        double tot = 0.0;
+        for (int k = 1; k <= K2; k++) tot += pht_unif_w(x2, lx2, k, lgk) * tab[L.g + k * n + b];
+        if (!(tot > 0.0)) return PHT_UNIF_ERR_ZERO;
+        const double target = PHT_UNIF_U01(st) * tot;
+        double sofar = 0.0; int kk = -1;
+        for (int k = 1; k <= K2; k++) {
+            const double v = pht_unif_w(x2, lx2, k, lgk) * tab[L.g + k * n + b];
+            if (v > 0.0) { sofar += v; kk = k; if (sofar >= target) break; }
+        }
+        int cur = b, absorbed = 0; double et = 0.0;
+        for (int i = 1; i <= kk; i++) {
+            const double e = -pht_log(PHT_UNIF_U01(st));
+            et += e;
+            if (absorbed) continue;
+            zb[cur * zs] += e;
+            const double *gn = tab + L.g + (kk - i) * n;
+            double t2 = 0.0;
+            for (int q = 0; q < n; q++) t2 += R[cur + q * n] * gn[q];
+            t2 += r[cur];
+            if (!(t2 > 0.0)) return PHT_UNIF_ERR_ZERO;
+            const double tg = PHT_UNIF_U01(st) * t2;
+            double so = 0.0; int c = -1;
+            for (int q = 0; q < n; q++) {
+                const double v = R[cur + q * n] * gn[q];
+                if (v > 0.0) { so += v; c = q; if (so >= tg) break; }
+            }
+            if (!(so >= tg) && r[cur] > 0.0) c = n;      /* absorption: the last category */
+            if (c == n) { PHT_UNIF_COUNT(ctx, cur, cur); absorbed = 1; }
+            else { if (c != cur) PHT_UNIF_COUNT(ctx, cur, c); cur = c; }
+        }
+        const double e = -pht_log(PHT_UNIF_U01(st));
+        et += e;
+        const double sc = d / et;
+        for (int c = 0; c < n; c++) if (zb[c * zs] != 0.0) za[c * zs] = za[c * zs] + zb[c * zs] * sc;
+    }
+    return 0;
+}
+/* Twin of pht_unif_panel_path above (kept apart so that its code and SASS stay as they are); a fix to one belongs in the
+ * other.  One misclassified panel observation (law above "Misclassified panel observations"): m >= 1 visits at times vt[0..m-1]
+ * with observed stages vo[0..m-1], read through E (n x S, row-major); beta: (m + 1) n doubles of scratch with stride bs,
+ * entry 0 of beta_j holding the drawn x_j on return.  Other arguments as pht_unif_panel_path. */
+PHT_UNIF_FN int pht_unif_emis_path(const double *tab, int n, int cap, const double *s, const double *scale, const double *cum,
+                                   const double *pi, double y, int cens, double u, int m, const double *vt, const uint32_t *vo,
+                                   const double *E, int S, double *beta, long bs, pht_stream *st, double *za, double *zb, int zs,
+                                   PHT_UNIF_CTX *ctx, int *B) {
+    const pht_unif_layout L = pht_unif_layout_make(n, cap);
+    const double lam = tab[0];
+    const int npos = (int)tab[2], a1 = (int)tab[3];
+    const double *lgk = tab + L.lgk, *R = tab + L.R, *r = tab + L.r;
+    const int iv = cens && u <= 1.7976931348623157e308;
+    const double d = iv ? u - y : 0.0, x2 = lam * d, lx2 = x2 > 0.0 ? pht_log(x2) : 0.0;
+    const int K2 = iv ? pht_unif_K(x2) : 0;
+    const double dy = y - vt[m - 1];
+    *B = 0;
+    if (pht_unif_K(lam * y) >= cap || K2 >= cap) return PHT_UNIF_ERR_TABLE;
+#define PHT_BETA(j, c) beta[((long)(j) * n + (c)) * bs]
+
+    /* terminal weights v (into za) and the backward pass */
+    if (iv) {
+        for (int c = 0; c < n; c++) za[c * zs] = 0.0;
+        for (int k = 1; k <= K2; k++) {
+            const double w = pht_unif_w(x2, lx2, k, lgk);
+            if (w == 0.0) continue;
+            const double *g = tab + L.g + k * n;
+            for (int c = 0; c < n; c++) za[c * zs] += w * g[c];
+        }
+    } else for (int c = 0; c < n; c++) za[c * zs] = cens ? 1.0 : s[c];
+    for (int j = m; j >= 0; j--) {
+        const double gap = j == m ? dy : vt[j] - (j > 0 ? vt[j - 1] : 0.0);
+        const double x = lam * gap, lx = x > 0.0 ? pht_log(x) : 0.0;
+        if (j == m) pht_unif_expv(tab, n, cap, x, lx, pht_unif_K(x), za, zs, &PHT_BETA(j, 0), bs);
+        else pht_unif_expv(tab, n, cap, x, lx, pht_unif_K(x), &PHT_BETA(j + 1, 0), bs, &PHT_BETA(j, 0), bs);
+        uint32_t mk = 0xffffffffu;
+        if (j > 0) {
+            const uint32_t o = vo[j - 1];
+            mk = pht_unif_col_support(E, n, S, o);
+            for (int c = 0; c < n; c++) PHT_BETA(j, c) = PHT_BETA(j, c) * E[c * S + (int)o];
+        }
+        if (pht_unif_rescale(&PHT_BETA(j, 0), bs, n, mk)) return PHT_UNIF_ERR_ZERO;
+    }
+
+    /* 1. the start state */
+    int a;
+    if (npos > 1) {
+        for (int c = 0; c < n; c++) za[c * zs] = pi[c] * PHT_BETA(0, c);
+        a = pht_unif_pick(za, n, zs, PHT_UNIF_U01(st));
+        if (a < 0) return PHT_UNIF_ERR_ZERO;
+    } else {
+        a = a1;
+        if (!(PHT_BETA(0, a) > 0.0)) return PHT_UNIF_ERR_ZERO;
+    }
+    *B = a;
+
+    /* 2. the visit states; x_j replaces beta_j(0), which no later draw reads */
+    int prev = a;
+    for (int j = 1; j <= m; j++) {
+        const double gap = vt[j - 1] - (j > 1 ? vt[j - 2] : 0.0);
+        const uint32_t mk = pht_unif_col_support(E, n, S, vo[j - 1]);
         int x;
         if (gap == 0.0) x = prev;
         else if ((mk & (mk - 1u)) == 0u) { x = 0; while (!((mk >> x) & 1u)) x++; }

@@ -104,6 +104,20 @@ def panel(R, s, l, spacing, k, stage_of_phase, rng, censor=None):
     return y, cens.astype(np.int32), offsets, ins[cols], masks[stage[seen[rows, cols]]]
 
 
+def misclassified_panel(R, s, l, spacing, k, E, rng, censor=None):
+    """Misclassified panel data (Engine.set_stage_visits): panel(R, s, l, spacing, k, ...) with every phase seen exactly,
+    then each visit's stage read from row c of the emission matrix E (n, S) for the true phase c.  Returns (y, censored,
+    offsets, t, stage, phase), phase the true phase at each visit."""
+    n = s.shape[0]
+    E = np.asarray(E, dtype=np.float64)
+    y, cens, offsets, t, mask = panel(R, s, l, spacing, k, np.arange(n), rng, censor=censor)
+    phase = np.log2(mask.astype(np.float64)).astype(np.int64)
+    cum = np.cumsum(E, axis=1)
+    cum[:, -1] = 1.0
+    stage = (rng.random(phase.size)[:, None] >= cum[phase]).sum(1)
+    return y, cens, offsets, t, stage.astype(np.uint32), phase
+
+
 def tabulate(y, cens, u=None):
     """Tied observations as records with counts (Engine.set_counts): the distinct (y, cens, u) in order of first occurrence
     and how often each occurs.  Returns (y, cens, u, counts) with u None when no u was given; np.repeat of the records by
